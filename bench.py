@@ -12,6 +12,18 @@ compressed payloads resident in HBM; `e2e` = the same through g4_decode_tiles wi
 the payloads and D2H of the decoded raster inside the timed region.  Encode throughput of the same shard is
 reported in `encode`.
 
+--dump-outputs DIR: after the timed steps, writes what the last timed step returned to a caller of decodeTiles --
+`raster.npy` (the decoded raster, or a fixed seeded sample of it) and `status.npy` (the per-tile status) -- as float64
+(float32 for a float32 raster; both exact), one pair per rank at N>1.  All ranks together write at most DUMP_SAMPLES
+raster samples (32 MiB) plus the tile statuses.  The inputs are the seeded synthetic terrain, so two builds run with the
+same arguments can be compared file for file.  (The GPU arm only: --impl reference decodes a smaller sample.)
+
+--steps K: K timed decode steps; the untimed per-kernel-timing passes and the e2e line run K decode passes as well
+(the tile-record pack / unpack line is a fixed 1 + 3 passes of another operation).
+
+Run __graft_entry__.build() first: bench.py loads the libraries it made instead of rebuilding them, writes only to
+--dump-outputs, and caches no bytecode in the tree.
+
 --impl reference: the reference's algorithm on the host cores.  The reference is Java and no JVM exists in this
 image, so this arm times the C++ oracle (oracle/, a line-by-line restatement) with a tile thread pool over all host
 cores on a bounded sample of the same workload.
@@ -28,6 +40,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as build() left it, __pycache__ included
 
 ORACLE_IDS = {"GvrsHuffman": 0, "GvrsDeflate": 1, "GvrsFloat": 2, "GvrsCanonicalHuffman": 3, "LSOP12": 4}
 GLOBAL_TILE_ROWS = 240  # config 3: 43200 / 180
@@ -46,6 +59,27 @@ CONFIGS = {
 SWEEP_TILES = [(60, 60), (90, 120), (120, 120), (128, 128), (180, 240), (256, 256), (512, 512)]
 SWEEP_GRID = (23040, 15360)  # rows = lcm of the tile heights, cols = 2 x lcm of the tile widths; 1.42 GB raw per GPU (11x the L2)
 METRIC = "GVRS tile decode GB/s of raw samples (config 3 shard, 180x240 tiles)"
+DUMP_SAMPLES = 1 << 22  # raster samples written by --dump-outputs over all ranks: 32 MiB as float64
+DUMP_SEED = 20240601
+
+
+def dump_outputs(path, raster, status, rank, world):
+    """Writes the decoded raster and the per-tile status of one decodeTiles call to path/raster.npy and path/status.npy
+    (per rank when world > 1).  Each rank writes its whole raster if it has at most DUMP_SAMPLES // world samples, else a
+    seeded sample of that many positions drawn over its flat index."""
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    flat = raster.reshape(-1)
+    per_rank = DUMP_SAMPLES // world
+    if flat.numel() > per_rank:
+        idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, flat.numel(), per_rank, dtype=np.int64))
+        values = flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+    else:
+        values = raster.cpu().numpy()
+    suffix = "_rank%d" % rank if world > 1 else ""
+    np.save(os.path.join(path, "raster%s.npy" % suffix), values.astype(np.float32 if values.dtype == np.float32 else np.float64))
+    np.save(os.path.join(path, "status%s.npy" % suffix), status.cpu().numpy().astype(np.float64))
 
 
 def peaks():
@@ -166,7 +200,6 @@ def run_reference(args, rank, cfg):
         return
     from oracle import g4oracle as oracle
 
-    oracle.build()
     threads = oracle.hardware_threads()
     smp = cpu_sample(cfg, threads, 24.0, oracle)
     for _ in range(args.warmup):
@@ -238,6 +271,8 @@ def run_sweep(args, torch, dist, g4, L, ctx, dev, stream, rank, world, barrier):
         sweep.append({"tile": "%dx%d" % (tr, tc), "decode_gbs": gbs, "ms_per_step": 1000.0 * float(t[0]) / args.steps,
                       "bits_per_sample": bps, "hbm_frac_per_gpu": (4.0 + bps / 8.0) / 4.0 * gbs / world / peak,
                       "tile_choice": {c: int(hist[k]) for k, c in enumerate(codecs)} | {"raw": int(hist[255])}})
+    if args.dump_outputs:  # the last timed step is that of the last tile size
+        dump_outputs(args.dump_outputs, out, master.lastStatus, rank, world)
     if rank == 0:
         best = max(sweep, key=lambda s: s["decode_gbs"])
         print(json.dumps({"metric": "GVRS tile decode GB/s of raw samples (config 5 tile-size sweep)", "value": best["decode_gbs"],
@@ -325,7 +360,13 @@ def main():
                                                  "Huffman/Triangle half of the config-3 path on its own)")
     ap.add_argument("--strong", action="store_true",
                     help="config 3, strong scaling: the WHOLE 43200x86400 grid (240 tile rows) split over the ranks (N=1: one GPU holds it all)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the last step's decoded raster (sampled) and tile status to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; --impl reference decodes only a sample of the workload")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -463,9 +504,11 @@ def main():
     torch.cuda.synchronize(dev)
     assert int((master.lastStatus != 0).sum()) == 0, "a tile failed to decode in the timed region"
     assert torch.equal(out.view(torch.int32), grid.view(torch.int32)), "decode does not reproduce the input raster"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, master.lastStatus, rank, world)
     # per-kernel-set device time (CUDA events inside the library, on the launching stream): separate, untimed passes
     kernel_ms = {}
-    for _ in range(min(args.steps, 5)):
+    for _ in range(args.steps):
         master.decodeTiles(batch, out=out)
         torch.cuda.synchronize(dev)
         for c in codecs:
@@ -515,7 +558,7 @@ def main():
         h_len = batch.lens.cpu().numpy().astype(np.uint32)
         h_grid = torch.empty((rows, cols), dtype=grid.dtype).pin_memory()
         hb = g4.TileBatch(h_arena.numpy(), h_off, h_len, None, None, None, batch.total_bytes, batch.band)
-        e2e_steps = max(2, min(args.steps, 4))
+        e2e_steps = args.steps
         master.decodeTiles(hb, out=h_grid.numpy())
         barrier()
         x0, x1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -567,7 +610,6 @@ def main():
     if world == 1:
         from oracle import g4oracle as oracle
 
-        oracle.build()
         threads = oracle.hardware_threads()
         ccfg = dict(cfg, codecs=codecs)
         r1 = cpu_arm(ccfg, 1, args.cpu_seconds / 3, oracle)

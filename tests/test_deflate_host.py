@@ -13,12 +13,14 @@ import subprocess
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+# the nvcc gridfour_b200/csrc/Makefile builds with: PATH first, then the toolkit at CUDA_HOME
+NVCC = shutil.which("nvcc") or shutil.which(os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc"))
 
 
-@pytest.mark.skipif(shutil.which("nvcc") is None, reason="nvcc not on PATH")
+@pytest.mark.skipif(NVCC is None, reason="no nvcc on PATH or under CUDA_HOME")
 def test_deflate_encoder_matches_zlib_bytes(tmp_path):
     exe = str(tmp_path / "deflate_vs_zlib")
-    subprocess.check_call(["nvcc", "-Wno-deprecated-gpu-targets", "-x", "cu", "-O2", "-std=c++17", "-o", exe,
+    subprocess.check_call([NVCC, "-Wno-deprecated-gpu-targets", "-x", "cu", "-O2", "-std=c++17", "-o", exe,
                            os.path.join(HERE, "host", "deflate_vs_zlib.cu"), "-lz"])
     r = subprocess.run([exe, "140000"], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-2000:]
