@@ -113,8 +113,6 @@ struct g4_context {
   DevBuf sGrid, sArena, sOffsets, sLens, sCodec, sPred, sStatus;
   // host-buffer decode pipeline: payload H2D / kernels / raster D2H of consecutive chunks overlap
   cudaStream_t copyIn = nullptr, copyOut = nullptr;
-  cudaStream_t lsopStream = nullptr;  // LSOP12 decode: wavefront of chunk k beside kernels H/T of chunk k+1
-  cudaEvent_t lsopEv[5] = {};
   cudaEvent_t evIn[16] = {}, evDone[16] = {}, evStart = nullptr, evOrder = nullptr;
   // optional per-kernel timing (CUDA events on the launching stream): [0]=decode, [1]=encode, by codec kind
   bool timing = false;
@@ -210,8 +208,7 @@ int run_streams(g4_context* ctx, int nStreams, int capExtra, int level, int* cou
     st.rank = ctx->stRank.as<uint16_t>();
     st.table = ctx->stTable.as<uint32_t>();
     st.tableQ = ctx->stTable.as<uint32_t>() + (span + 16);
-    static const bool lazyOff = getenv("G4_DEFLATE_LAZY") && atoi(getenv("G4_DEFLATE_LAZY")) == 0;
-    st.lazy = (level >= 9 && !lazyOff) ? 1 : 0;
+    st.lazy = level >= 9 ? 1 : 0;
     st.maxLen = 0;
     for (int j = j0; j < j1; j++)
       if (ctx->hostLen[size_t(j)] <= stagedMax && ctx->hostLen[size_t(j)] > st.maxLen) st.maxLen = ctx->hostLen[size_t(j)];
@@ -322,7 +319,7 @@ int launch_decoder(g4_context* ctx, int codecId, DecodeArgs& a, int nCtas) {
       CK(ctx->lsopMeta.ensure(huffman2_tree_bytes(nTiles)));
       HuffFusedScratch fused{ctx->lsopStage.as<uint32_t>(), ctx->lsopMeta.as<uint8_t>(), ctx->defer.as<int>(), ctx->counters.as<int>() + 48, ctx->smCount};
       int nLaunch = 0;
-      CK(launch_huffman_decode(a, nCtas, ctx->stream, &fused, &nLaunch));
+      CK(launch_huffman_decode(a, nCtas, ctx->stream, fused, &nLaunch));
       ctx->launches += uint64_t(nLaunch);
       return G4_OK;
     }
@@ -352,14 +349,9 @@ int launch_decoder(g4_context* ctx, int codecId, DecodeArgs& a, int nCtas) {
       CK(cudaMemsetAsync(ctx->lsopCks.p, 0, size_t(nTiles) * 8, ctx->stream));
       a.lsopCks = ctx->lsopCks.as<uint32_t>();
     {
-      if (!ctx->lsopStream) {
-        CK(cudaStreamCreateWithFlags(&ctx->lsopStream, cudaStreamNonBlocking));
-        for (int k = 0; k < 5; k++) CK(cudaEventCreateWithFlags(&ctx->lsopEv[k], cudaEventDisableTiming));
-      }
       int nLaunch = 0;
       LsopFastArgs fast{};
-      static const bool fastOff = getenv("G4_LSOP_FAST") && atoi(getenv("G4_LSOP_FAST")) == 0;
-      const bool useFast = !fastOff && lsop_fast_geometry(a.band, a.grid, &fast.g);
+      const bool useFast = lsop_fast_geometry(a.band, a.grid, &fast.g);
       if (useFast) {
         CK(ctx->lsopSide.ensure(lsop_fast_side_bytes(fast.g, nTiles)));
         CK(ctx->lsopExc.ensure(lsop_fast_exc_bytes(nTiles)));
@@ -369,11 +361,9 @@ int launch_decoder(g4_context* ctx, int codecId, DecodeArgs& a, int nCtas) {
         fast.resid = ctx->lsopResid.as<uint8_t>();
         if (lsop_fast_stage_bytes(ctx->smCount)) CK(ctx->lsopStage.ensure(lsop_fast_stage_bytes(ctx->smCount)));
         fast.textStage = ctx->lsopStage.as<uint8_t>();
-        static const int lookbackEnv = getenv("G4_TEXT_LOOKBACK") ? atoi(getenv("G4_TEXT_LOOKBACK")) : 0;
-        fast.textLookback = lookbackEnv > 0 ? uint32_t(lookbackEnv) : 96u;
       }
       CK(launch_lsop_decode(a, ctx->coef.as<float>(), ctx->lsopMeta.as<uint8_t>(), ctx->defer.as<int>(), ctx->counters.as<int>() + 56,
-                            nCtas, nTiles, ctx->stream, ctx->lsopStream, ctx->lsopEv, &nLaunch, useFast ? &fast : nullptr, ctx->smCount));
+                            nCtas, nTiles, ctx->stream, &nLaunch, useFast ? &fast : nullptr, ctx->smCount));
       CK(launch_lsop_value_checksum(a, nTiles, ctx->stream));
       ctx->launches += uint64_t(nLaunch) + 1;
       return G4_OK;
@@ -709,11 +699,6 @@ void g4_context_destroy(g4_context* ctx) {
   }
   if (ctx->evStart) cudaEventDestroy(ctx->evStart);
   if (ctx->evOrder) cudaEventDestroy(ctx->evOrder);
-  if (ctx->lsopStream) {
-    cudaStreamSynchronize(ctx->lsopStream);
-    cudaStreamDestroy(ctx->lsopStream);
-    for (int k = 0; k < 5; k++) cudaEventDestroy(ctx->lsopEv[k]);
-  }
   for (auto& b : ctx->slots) b.release();
   DevBuf* bufs[] = {&ctx->candLens, &ctx->candPreds, &ctx->candStatus, &ctx->counters, &ctx->scratch, &ctx->lists, &ctx->src,
                     &ctx->total, &ctx->coef, &ctx->defer, &ctx->lsopMeta, &ctx->lsopSide, &ctx->lsopExc, &ctx->lsopResid, &ctx->lsopStage, &ctx->tileRefs, &ctx->lsopCks, &ctx->wide, &ctx->encScratch, &ctx->region, &ctx->jobLen, &ctx->jobOff, &ctx->jobOut, &ctx->jobTotal,

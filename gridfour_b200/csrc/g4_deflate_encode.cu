@@ -199,27 +199,28 @@ __global__ void __launch_bounds__(kSortThreads) deflate_sort_kernel(StagedArgs a
 // scattered 32-byte sector per entry, and DRAM's rate of such writes -- not the matching -- set the kernel's time
 // (43 GB written + 76 GB read for 1.4 GB of input, profiles/).  The table of a stream (4 bytes per position) therefore
 // fills in shared memory and leaves with coalesced stores; streams too long for that keep the scattered store.
-// W = chain length of the level (slots that must stay behind a round), SB = slots per round, tabCap = entries of the
-// shared-memory table.
+// kMatchChain = chain length of the levels below 9 (slots that must stay behind a round; level 9 takes deflate_lazy_kernel),
+// SB = slots per round, tabCap = entries of the shared-memory table.
 // GROUPS: the CTA works as that many independent thread groups, each with its own window, taking the rounds of a stream
 // in turn and synchronising with a named barrier of its own: while one group waits for the gathers that fill its window,
 // the other walks (with one 205 KB CTA per SM there is no second CTA to do that).
-template <int W, int SB, int GROUPS, int NT_MAX, int MIN_CTAS>
+constexpr int kMatchChain = 128;
+template <int SB, int GROUPS, int NT_MAX, int MIN_CTAS>
 __global__ void __launch_bounds__(NT_MAX, MIN_CTAS) deflate_match_window_kernel(StagedArgs a, uint32_t tabCap) {
   extern __shared__ __align__(16) unsigned char matchSm[];
   const uint32_t nThr = blockDim.x / GROUPS, grp = threadIdx.x / nThr, tid = threadIdx.x - grp * nThr;
-  unsigned char* winSm = matchSm + size_t(grp) * (size_t(W + SB) * 16);
+  unsigned char* winSm = matchSm + size_t(grp) * (size_t(kMatchChain + SB) * 16);
   uint2* keyS = reinterpret_cast<uint2*>(winSm);
-  uint32_t* filtS = reinterpret_cast<uint32_t*>(winSm + size_t(W + SB) * 8);
-  uint32_t* hpS = reinterpret_cast<uint32_t*>(winSm + size_t(W + SB) * 12);  // hash << 16 | position: rises with the slot
-  uint32_t* tabS = reinterpret_cast<uint32_t*>(matchSm + size_t(GROUPS) * size_t(W + SB) * 16);
+  uint32_t* filtS = reinterpret_cast<uint32_t*>(winSm + size_t(kMatchChain + SB) * 8);
+  uint32_t* hpS = reinterpret_cast<uint32_t*>(winSm + size_t(kMatchChain + SB) * 12);  // hash << 16 | position: rises with the slot
+  uint32_t* tabS = reinterpret_cast<uint32_t*>(matchSm + size_t(GROUPS) * size_t(kMatchChain + SB) * 16);
   __shared__ int sj;
   auto group_sync = [&]() {
     if (GROUPS == 1) __syncthreads();
     else asm volatile("bar.sync %0, %1;" ::"r"(1u + grp), "r"(nThr) : "memory");
   };
   const DeflateLevel L = deflate_level(a.level);
-  const uint32_t maxChain = uint32_t(L.maxChain) < uint32_t(W) ? uint32_t(L.maxChain) : uint32_t(W);
+  const uint32_t maxChain = uint32_t(L.maxChain) < uint32_t(kMatchChain) ? uint32_t(L.maxChain) : uint32_t(kMatchChain);
   const uint32_t quarter = uint32_t(L.maxChain) >> 2;
   for (;;) {
     __syncthreads();
@@ -238,7 +239,8 @@ __global__ void __launch_bounds__(NT_MAX, MIN_CTAS) deflate_match_window_kernel(
     const bool inSm = nPos <= tabCap;
     for (uint32_t base = grp * uint32_t(SB); base < nPos; base += uint32_t(GROUPS) * uint32_t(SB)) {
       const uint32_t end = base + SB < nPos ? base + SB : nPos;
-      const uint32_t first = base >= uint32_t(W) ? base - uint32_t(W) : 0u;  // window = slots [first, end), index = slot + W - base
+      // window = slots [first, end), index = slot + kMatchChain - base
+      const uint32_t first = base >= uint32_t(kMatchChain) ? base - uint32_t(kMatchChain) : 0u;
       group_sync();
       for (uint32_t s = first + tid; s < end; s += nThr) {
         const uint32_t p = sorted[s];
@@ -247,16 +249,16 @@ __global__ void __launch_bounds__(NT_MAX, MIN_CTAS) deflate_match_window_kernel(
         const uint32_t sh = uint32_t(ad & 3u) * 8u;
         const uint32_t w0 = q[0], w1 = q[1], w2 = q[2];  // in[] is padded with 16 zero bytes past n
         const uint32_t kl = __funnelshift_r(w0, w1, sh), kh = __funnelshift_r(w1, w2, sh);
-        hpS[s + W - base] = (((((kl & 0xffu) << 10) ^ (((kl >> 8) & 0xffu) << 5) ^ ((kl >> 16) & 0xffu)) & uint32_t(kDefHashMask)) << 16) | p;
-        keyS[s + W - base] = make_uint2(kl, kh);
+        hpS[s + kMatchChain - base] = (((((kl & 0xffu) << 10) ^ (((kl >> 8) & 0xffu) << 5) ^ ((kl >> 16) & 0xffu)) & uint32_t(kDefHashMask)) << 16) | p;
+        keyS[s + kMatchChain - base] = make_uint2(kl, kh);
         // 32-bit filter word.  Inside a hash bucket, byte 1 fixes byte 2 and the low five bits of byte 0 (the hash is
         // b0 << 10 ^ b1 << 5 ^ b2, 15 bits), so {b0 >> 5, b1} is the whole 3-byte prefix; then bytes 3, 4 and five bits
         // of byte 5.  Fields in byte order: a mask over the low bits tests "at least that many bytes in common".
-        filtS[s + W - base] = ((kl >> 5) & 7u) | (((kl >> 8) & 0xffu) << 3) | ((kl >> 24) << 11) | ((kh & 0xffu) << 19) | (((kh >> 8) & 31u) << 27);
+        filtS[s + kMatchChain - base] = ((kl >> 5) & 7u) | (((kl >> 8) & 0xffu) << 3) | ((kl >> 24) << 11) | ((kh & 0xffu) << 19) | (((kh >> 8) & 31u) << 27);
       }
       group_sync();
       for (uint32_t slot = base + tid; slot < end; slot += nThr) {
-        const uint32_t li = slot + W - base;
+        const uint32_t li = slot + kMatchChain - base;
         const uint2 my = keyS[li];
         const uint32_t hp = hpS[li];
         const uint32_t p = hp & 0xffffu;
@@ -523,18 +525,15 @@ __global__ void __launch_bounds__(128, 12) deflate_lazy_kernel(StagedArgs a) {
 // flight), so that a step of the lazy loop costs a shared-memory read instead of a DRAM round trip that the 31 other
 // lanes of the warp wait for as well.
 constexpr int kDecChunk = 16, kDecRing = 4, kDecRow = kDecChunk * kDecRing;  // chunk: 16 entries = 64 bytes + 16 input bytes
-// LANES streams per warp: the loop is a chain of dependent instructions (about 80 per step with the ring upkeep), so
-// what it needs is warps per scheduler, not lanes per warp.
-template <int LANES>
+// One stream per lane of a one-warp CTA (fewer streams per warp measured slower, DESIGN.md 6.1.1).
 __global__ void __launch_bounds__(32) deflate_decide_ring_kernel(StagedArgs a) {
-  __shared__ __align__(16) uint32_t tabS[LANES][kDecRow + 4];  // +4 entries: rows 16 bytes apart in the banks
-  __shared__ __align__(16) uint8_t byteS[LANES][kDecRow + 16];
+  __shared__ __align__(16) uint32_t tabS[32][kDecRow + 4];  // +4 entries: rows 16 bytes apart in the banks
+  __shared__ __align__(16) uint8_t byteS[32][kDecRow + 16];
   // symbols leave 16 bytes at a time (8 distances / 16 length-or-literal bytes): a warp's scalar stores are 32 L2
   // transactions each, and at two per step they, not the loop, set the kernel's time
-  __shared__ __align__(16) uint16_t distS[LANES][8 + 8];
-  __shared__ __align__(16) uint8_t lcS[LANES][16 + 16];
+  __shared__ __align__(16) uint16_t distS[32][8 + 8];
+  __shared__ __align__(16) uint8_t lcS[32][16 + 16];
   const int lane = threadIdx.x;
-  if (lane >= LANES) return;
   const DeflateLevel L = deflate_level(a.level);
   const uint32_t tabBase = uint32_t(__cvta_generic_to_shared(&tabS[lane][0]));
   const uint32_t byteBase = uint32_t(__cvta_generic_to_shared(&byteS[lane][0]));
@@ -1119,20 +1118,16 @@ cudaError_t launch_deflate_staged(const StagedArgs& a, int smCount, cudaStream_t
     const int warps = nChunk < smCount * 48 ? nChunk : smCount * 48;
     deflate_lazy_kernel<<<(warps + 3) / 4, 128, 0, s>>>(a);
   } else {
-  // match: shared memory = the candidate window + the stream's table (4 bytes per position) when that fits
-  {
-    const bool deep = deflate_level(a.level).maxChain > 128;
-    static const bool oneGroup = getenv("G4_MATCH_GROUPS") && atoi(getenv("G4_MATCH_GROUPS")) == 1;
-    size_t win = deep ? size_t(4096 + 2048) * 16 : size_t(128 + 1920) * 16;  // two groups of (128 + 896) slots: the same
-    const size_t winBig = size_t(2) * (128 + 1408) * 16;                     // two groups of 1,536 slots
+    // match: shared memory = the candidate window + the stream's table (4 bytes per position) when that fits
+    size_t win = size_t(128 + 1920) * 16;                // two groups of (128 + 896) slots: the same
+    const size_t winBig = size_t(2) * (128 + 1408) * 16;  // two groups of 1,536 slots
     const size_t smMax = 227 * 1024 - 2048;
     size_t tabBytes = (size_t(a.maxLen) * 4 + 15) & ~size_t(15);
     if (win + tabBytes > smMax) tabBytes = 0;  // too long: scattered stores
     int perSm = int(smMax / (win + tabBytes));
     if (perSm > 8) perSm = 8;
-    if (deep && perSm > 2) perSm = 2;
     // one CTA per SM anyway: the larger windows if they fit beside the table (fewer rounds, less of each window re-filled)
-    const bool big = !deep && !oneGroup && perSm == 1 && winBig + tabBytes <= smMax;
+    const bool big = perSm == 1 && winBig + tabBytes <= smMax;
     if (big) win = winBig;
     const size_t sm = win + tabBytes;
     const int threads = perSm == 1 ? 1024 : perSm <= 3 ? 512 : 256;
@@ -1140,28 +1135,19 @@ cudaError_t launch_deflate_staged(const StagedArgs& a, int smCount, cudaStream_t
     static std::atomic<uint64_t> attrW{0};
     ea = once_per_device(attrW, [] {
       const int cap = 227 * 1024 - 2048;
-      cudaError_t e1 = cudaFuncSetAttribute(deflate_match_window_kernel<128, 1920, 1, 1024, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
-      if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(deflate_match_window_kernel<128, 1920, 1, 512, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
-      if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(deflate_match_window_kernel<128, 1408, 2, 1024, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
-      if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(deflate_match_window_kernel<128, 896, 2, 1024, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
-      if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(deflate_match_window_kernel<4096, 2048, 1, 1024, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
+      cudaError_t e1 = cudaFuncSetAttribute(deflate_match_window_kernel<1920, 1, 512, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
+      if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(deflate_match_window_kernel<1408, 2, 1024, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
+      if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(deflate_match_window_kernel<896, 2, 1024, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
       return e1;
     });
     if (ea != cudaSuccess) return ea;
     const uint32_t cap32 = uint32_t(tabBytes / 4);
-    if (deep) deflate_match_window_kernel<4096, 2048, 1, 1024, 1><<<ctas, threads, sm, s>>>(a, cap32);
-    else if (big) deflate_match_window_kernel<128, 1408, 2, 1024, 1><<<ctas, threads, sm, s>>>(a, cap32);
-    else if (threads == 1024 && !oneGroup) deflate_match_window_kernel<128, 896, 2, 1024, 1><<<ctas, threads, sm, s>>>(a, cap32);
-    else if (threads == 1024) deflate_match_window_kernel<128, 1920, 1, 1024, 1><<<ctas, threads, sm, s>>>(a, cap32);
-    else deflate_match_window_kernel<128, 1920, 1, 512, 3><<<ctas, threads, sm, s>>>(a, cap32);
-  }
-  e = cudaGetLastError();
-  if (e != cudaSuccess) return e;
-  static const int decLanes = getenv("G4_DECIDE_LANES") ? atoi(getenv("G4_DECIDE_LANES")) : 32;
-  if (decLanes >= 32) deflate_decide_ring_kernel<32><<<(nChunk + 31) / 32, 32, 0, s>>>(a);
-  else if (decLanes >= 16) deflate_decide_ring_kernel<16><<<(nChunk + 15) / 16, 32, 0, s>>>(a);
-  else if (decLanes >= 8) deflate_decide_ring_kernel<8><<<(nChunk + 7) / 8, 32, 0, s>>>(a);
-  else deflate_decide_ring_kernel<4><<<(nChunk + 3) / 4, 32, 0, s>>>(a);
+    if (big) deflate_match_window_kernel<1408, 2, 1024, 1><<<ctas, threads, sm, s>>>(a, cap32);
+    else if (threads == 1024) deflate_match_window_kernel<896, 2, 1024, 1><<<ctas, threads, sm, s>>>(a, cap32);
+    else deflate_match_window_kernel<1920, 1, 512, 3><<<ctas, threads, sm, s>>>(a, cap32);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    deflate_decide_ring_kernel<<<(nChunk + 31) / 32, 32, 0, s>>>(a);
   }
   e = cudaGetLastError();
   if (e != cudaSuccess) return e;

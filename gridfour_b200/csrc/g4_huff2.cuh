@@ -57,6 +57,8 @@ constexpr int kH2TreeBytes = 2048 + 1024 + 16;
 struct Huff2Geom {
   uint32_t stageBytes;  // staging area of the packing (also holds the band of the Triangle pass)
   uint32_t m32Cap;      // byte buffer of the M32 codes
+  // kH2SubBits / kH2Lookback, passed as kernel arguments: compiled in as constants, the kernel measured 0.2 % slower
+  // (B200, 1000 W)
   uint32_t subBits;     // target sub-sequence size
   uint32_t lookback;    // the first pass starts this many bits before a sub-sequence limit
 };

@@ -586,17 +586,14 @@ static cudaError_t launch_huffman2(const DecodeArgs& a, const Huff2Geom& g, size
 size_t huffman2_spill_bytes(int smCount) { return size_t(smCount) * 4 * kH2MaxSub * kH2SpillWords * sizeof(uint32_t); }
 size_t huffman2_tree_bytes(int nTiles) { return size_t(nTiles) * kH2TreeBytes; }
 
-// fused: scratch of the fast path (spill of huffman2_spill_bytes, defer list of nTilesUpper ints, two zeroed counters), or null
-cudaError_t launch_huffman_decode(const DecodeArgs& a, int nCtas, cudaStream_t s, const HuffFusedScratch* fused, int* launches) {
+// fused: scratch of the fast path (spill of huffman2_spill_bytes, defer list of nTilesUpper ints, two zeroed counters)
+cudaError_t launch_huffman_decode(const DecodeArgs& a, int nCtas, cudaStream_t s, const HuffFusedScratch& fused, int* launches) {
   // staging capacity of the fast decoder: 6 bits per sample of the tile (legacy Huffman over M32 bytes takes 4-5 bits
   // per sample on terrain), at most 160 KB (one CTA per SM)
   uint64_t bytes = uint64_t(a.band.tile_rows) * uint64_t(a.band.tile_cols) * 6 / 8 + 64;
   if (bytes > 160u * 1024u) bytes = 160u * 1024u;
   uint32_t stageWords = uint32_t((bytes + 3) / 4);
   if (stageWords < uint32_t(kHfStageWordsMin)) stageWords = kHfStageWordsMin;
-  static const bool fastOn = !(getenv("G4_HUFF_FAST") && atoi(getenv("G4_HUFF_FAST")) == 0);
-  static const bool fusedOn = !(getenv("G4_HUFF_FUSED") && atoi(getenv("G4_HUFF_FUSED")) == 0);
-  if (!fastOn) stageWords = 0;
   size_t smem = huff_fast_smem_bytes(stageWords);
   if (smem < sizeof(HuffDecShared)) smem = sizeof(HuffDecShared);
   static std::atomic<uint64_t> attr{0};
@@ -606,7 +603,7 @@ cudaError_t launch_huffman_decode(const DecodeArgs& a, int nCtas, cudaStream_t s
   });
   if (ea != cudaSuccess) return ea;
   DecodeArgs rest = a;
-  if (fused && fastOn && fusedOn && a.band.elem_type == G4_ELEM_I32) {
+  if (a.band.elem_type == G4_ELEM_I32) {
     const uint32_t n = uint32_t(a.band.tile_rows) * uint32_t(a.band.tile_cols);
     Huff2Geom g;
     uint32_t stage = (n * 6u / 8u + 256u + 15u) & ~15u;
@@ -614,26 +611,25 @@ cudaError_t launch_huffman_decode(const DecodeArgs& a, int nCtas, cudaStream_t s
     if (stage < bandBytes) stage = (bandBytes + 15u) & ~15u;
     g.stageBytes = stage;
     g.m32Cap = (n + n / 16u + 48u + 15u) & ~15u;  // room for some codes longer than one byte
-    static const int subEnv = getenv("G4_H2_SUBBITS") ? atoi(getenv("G4_H2_SUBBITS")) : 0, lbEnv = getenv("G4_H2_LOOKBACK") ? atoi(getenv("G4_H2_LOOKBACK")) : 0;
-    g.subBits = subEnv > 0 ? uint32_t(subEnv) : kH2SubBits;
-    g.lookback = lbEnv > 0 ? uint32_t(lbEnv) : kH2Lookback;
+    g.subBits = kH2SubBits;
+    g.lookback = kH2Lookback;
     const size_t smem2 = ((sizeof(Huff2Shared) + 127) & ~size_t(127)) + g.stageBytes + 16 + g.m32Cap;
     if (smem2 <= 112u * 1024u) {  // two 512-thread CTAs (or four 256-thread CTAs) per SM
       const int nTilesUpper = a.band.tiles_down * a.band.tiles_across;
-      huffman2_tree_kernel<<<(nTilesUpper + 63) / 64, 64, 0, s>>>(a, fused->trees);
+      huffman2_tree_kernel<<<(nTilesUpper + 63) / 64, 64, 0, s>>>(a, fused.trees);
       cudaError_t e = cudaGetLastError();
       if (e != cudaSuccess) return e;
-      e = n <= 16384u ? launch_huffman2<256>(a, g, smem2, fused->smCount, nTilesUpper, fused->spill, fused->trees, fused->defer, fused->counters, s)
-                      : launch_huffman2<512>(a, g, smem2, fused->smCount, nTilesUpper, fused->spill, fused->trees, fused->defer, fused->counters, s);
+      e = n <= 16384u ? launch_huffman2<256>(a, g, smem2, fused.smCount, nTilesUpper, fused.spill, fused.trees, fused.defer, fused.counters, s)
+                      : launch_huffman2<512>(a, g, smem2, fused.smCount, nTilesUpper, fused.spill, fused.trees, fused.defer, fused.counters, s);
       if (e != cudaSuccess) return e;
-      if (launches) (*launches) += 2;
-      rest.list = fused->defer;
-      rest.listCount = fused->counters;
-      rest.counter = fused->counters + 1;
+      *launches += 2;
+      rest.list = fused.defer;
+      rest.listCount = fused.counters;
+      rest.counter = fused.counters + 1;
     }
   }
   huffman_decode_kernel<<<nCtas, kThreads, smem, s>>>(rest, stageWords);
-  if (launches) (*launches)++;
+  (*launches)++;
   return cudaGetLastError();
 }
 

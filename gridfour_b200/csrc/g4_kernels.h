@@ -162,7 +162,7 @@ struct HuffFusedScratch {
 };
 size_t huffman2_spill_bytes(int smCount);
 size_t huffman2_tree_bytes(int nTiles);
-cudaError_t launch_huffman_decode(const DecodeArgs& a, int nCtas, cudaStream_t s, const HuffFusedScratch* fused = nullptr, int* launches = nullptr);
+cudaError_t launch_huffman_decode(const DecodeArgs& a, int nCtas, cudaStream_t s, const HuffFusedScratch& fused, int* launches);
 cudaError_t launch_canon_decode(const DecodeArgs& a, int nCtas, cudaStream_t s);
 cudaError_t launch_canon_encode(const EncodeArgs& a, int nCtas, cudaStream_t s);  // needs 32 KB scratch per CTA
 cudaError_t launch_lsop_encode(const EncodeArgs& a, int nCtas, cudaStream_t s);   // needs 32 KB scratch per CTA
@@ -172,8 +172,8 @@ cudaError_t launch_deflate_decode(const DecodeArgs& a, uint8_t* region, size_t r
 cudaError_t launch_float_decode(const DecodeArgs& a, uint8_t* region, size_t regionStride, int nCtas, int nTilesUpper,
                                 cudaStream_t s);
 // coef: [nTiles][12] floats of device scratch; nTilesUpper bounds the number of LSOP tiles in the list
-// defer: nTilesUpper ints; deferCounters: 6 zeroed ints (deferred-tile count, work counter of the general kernel, four
-// chunk counters of the text kernel); s2 / ev (5 events): second stream for the chunked overlap, or null
+// defer: nTilesUpper ints; deferCounters: 4 zeroed ints (deferred-tile count, work counters of the general kernel, of the
+// text kernel and of the fast path's wavefront kernel)
 // meta: nTilesUpper * lsop_meta_bytes() bytes (interior code lengths + text position handed from kernel H to kernel T)
 size_t lsop_meta_bytes();
 // LSOP08, the legacy 8-coefficient codec (decode only): entropy stage + initializers, then the wavefront
@@ -202,7 +202,6 @@ struct LsopFastArgs {
   uint32_t* exc;      // [nTiles][128]: residuals that are no byte
   uint8_t* resid;     // residual scratch (lsop_fast_resid_bytes)
   uint8_t* textStage; // spill words behind the staging slots of the text kernel, one area per persistent CTA (lsop_fast_stage_bytes)
-  uint32_t textLookback;  // bits before a sub-sequence limit at which the text kernel's first pass starts decoding
   int* defer;         // tiles for the general kernels
   int* deferCount;
   LsopFastGeom g;
@@ -215,8 +214,7 @@ size_t lsop_fast_resid_bytes(const LsopFastGeom& g, int nTiles);
 cudaError_t launch_lsop_decode_fast(const LsopFastArgs& A, int nTilesUpper, int smCount, int* textCounter, cudaStream_t s, int* launches);
 // fast: scratch of the fast path (side / exc / resid / g filled in), or null -> the round-1 kernels only
 cudaError_t launch_lsop_decode(const DecodeArgs& a, float* coef, uint8_t* meta, int* defer, int* deferCounters, int nCtas,
-                               int nTilesUpper, cudaStream_t s, cudaStream_t s2, cudaEvent_t* ev, int* launches,
-                               const LsopFastArgs* fast = nullptr, int smCount = 148);
+                               int nTilesUpper, cudaStream_t s, int* launches, const LsopFastArgs* fast = nullptr, int smCount = 148);
 
 // ICompressionDecoder.analyze (g4_analyze.cu): per-tile M32 statistics of CodecHuffman / CodecDeflate packings.
 struct AnalyzeArgs {

@@ -234,12 +234,12 @@ __device__ inline void lsop_warp_column_scan(const TileView& t, int col, int r0,
 }
 
 __global__ void __launch_bounds__(kThreads, 5) lsop_decode_head_kernel(DecodeArgs a, float* coefOut, uint8_t* meta, int* defer,
-                                                                    int* deferCount, uint32_t stageWords, int listBegin, int listEnd) {
+                                                                    int* deferCount, uint32_t stageWords) {
   __shared__ CanonWarpShared WS[kWarps];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   CanonWarpShared& W = WS[warp];
-  const int li = listBegin + blockIdx.x * kWarps + warp;
-  if (li >= listEnd || li >= *a.listCount) return;
+  const int li = blockIdx.x * kWarps + warp;
+  if (li >= *a.listCount) return;
   const int tIdx = a.list[li];
   uint8_t* m = meta + size_t(tIdx) * kLsopMetaBytes;
   if (lane == 0) *reinterpret_cast<uint32_t*>(m) = 0;
@@ -316,17 +316,17 @@ __global__ void __launch_bounds__(kThreads, 5) lsop_decode_head_kernel(DecodeArg
 }
 
 template <class InteriorSink>
-__global__ void __launch_bounds__(kThreads, 4) lsop_decode_text_kernel(DecodeArgs a, const uint8_t* meta, int listBegin, int listEnd) {
+__global__ void __launch_bounds__(kThreads, 4) lsop_decode_text_kernel(DecodeArgs a, const uint8_t* meta) {
   extern __shared__ __align__(16) unsigned char lsopFastSmem[];
   CanonFastShared& F = *reinterpret_cast<CanonFastShared*>(lsopFastSmem);
   __shared__ int sTile;
   const int tid = threadIdx.x;
   for (;;) {
     __syncthreads();
-    if (tid == 0) sTile = listBegin + atomicAdd(a.counter, 1);
+    if (tid == 0) sTile = atomicAdd(a.counter, 1);
     __syncthreads();
     const int li = sTile;
-    if (li >= listEnd || li >= *a.listCount) break;
+    if (li >= *a.listCount) break;
     const int tIdx = a.list[li];
     const uint8_t* m = meta + size_t(tIdx) * kLsopMetaBytes;
     const uint32_t T0 = *reinterpret_cast<const uint32_t*>(m);
@@ -673,18 +673,12 @@ __global__ void __launch_bounds__(kThreads) lsop_wavefront_kernel(DecodeArgs a, 
 // live; measured on the config-3 shard: 3 CTAs/SM 1.46 ms, 4 CTAs/SM 1.49 ms, 5 CTAs/SM (1280 lines) 18 ms -- past that
 // point the lines are evicted between iterations and every load becomes a scattered 32-byte DRAM access.  L1-bypassing
 // loads (ld.global.cg) show the same collapse at any occupancy (16-18 ms), and so does a second load in flight per lane.
-// mode 0: every tile of [listBegin, listEnd); 1: only tiles the fast text kernel decoded (meta T0 != 0); 2: only the others
-__global__ void __launch_bounds__(kThreads, 3) lsop_wavefront4_kernel(DecodeArgs a, const float* coef, const uint8_t* meta, int listBegin,
-                                                                      int listEnd, int mode) {
+__global__ void __launch_bounds__(kThreads, 3) lsop_wavefront4_kernel(DecodeArgs a, const float* coef) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int li = listBegin + blockIdx.x * kWarps + warp;
-  if (li >= listEnd || li >= *a.listCount) return;
+  const int li = blockIdx.x * kWarps + warp;
+  if (li >= *a.listCount) return;
   const int tIdx = a.list[li];
   if (a.status[tIdx] != G4_OK) return;
-  if (mode != 0) {
-    const bool fast = *reinterpret_cast<const uint32_t*>(meta + size_t(tIdx) * kLsopMetaBytes) != 0u;
-    if (fast != (mode == 1)) return;
-  }
   const TileView t = tile_view(a.band, a.grid, tIdx);
   const int R = t.R, C = t.C;
   const bool feeder = lane < 2;
@@ -1176,7 +1170,7 @@ cudaError_t launch_lsop08_decode(const DecodeArgs& a, float* coef, int nCtas, in
 }
 
 cudaError_t launch_lsop_decode(const DecodeArgs& a, float* coef, uint8_t* meta, int* defer, int* deferCounters, int nCtas,
-                               int nTilesUpper, cudaStream_t s, cudaStream_t s2, cudaEvent_t* ev, int* launches,
+                               int nTilesUpper, cudaStream_t s, int* launches,
                                const LsopFastArgs* fast, int smCount) {
   if (fast) {
     // g4_lsop_fast.cu takes every canonical-Huffman tile; what it cannot take (legacy Huffman / Deflate bodies, oversized
@@ -1222,53 +1216,26 @@ cudaError_t launch_lsop_decode(const DecodeArgs& a, float* coef, uint8_t* meta, 
   const bool aligned = (a.band.tile_cols % 4) == 0 && (a.band.grid_pitch % 4) == 0 && a.band.tile_cols >= 8 &&
                        (reinterpret_cast<uintptr_t>(a.grid) & 15) == 0;
   // deferCounters[0] = number of deferred tiles (filled by kernel H), [1] = work counter of the general kernel,
-  // [2..5] = work counters of the text kernel, one per chunk.
-  // Optional (G4_LSOP_CHUNKS=2..4, off by default): the band is cut into chunks and the wavefront of chunk k runs on a
-  // second stream beside kernel H and the text kernel of chunk k+1.  Measured on the config-3 shard it LOSES (3.63 ms
-  // with one chunk, 4.02 with two, 4.13 with four): the kernels compete for the same issue slots and registers, and
-  // the smaller launches add tails (DESIGN.md 6.1).
-  static const int chunkEnv = getenv("G4_LSOP_CHUNKS") ? atoi(getenv("G4_LSOP_CHUNKS")) : 1;
-  int nChunks = (aligned && s2 && ev && nTilesUpper >= 2048) ? chunkEnv : 1;
-  if (nChunks < 1) nChunks = 1;
-  if (nChunks > 4) nChunks = 4;
-  int nLaunch = 0;
-  cudaError_t e = cudaSuccess;
-  for (int k = 0; k < nChunks; k++) {
-    const int b = int(int64_t(nTilesUpper) * k / nChunks), en = int(int64_t(nTilesUpper) * (k + 1) / nChunks);
-    if (en <= b) continue;
-    const int n = en - b;
-    lsop_decode_head_kernel<<<(n + kWarps - 1) / kWarps, kThreads, 0, s>>>(a, coef, meta, defer, deferCounters, stageWords, b, en);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    DecodeArgs t = a;
-    t.counter = deferCounters + 2 + k;
-    const int ctas = nCtas < n ? nCtas : n;
-    if (aligned) lsop_decode_text_kernel<InteriorPackedSink><<<ctas, kThreads, textSmem, s>>>(t, meta, b, en);
-    else lsop_decode_text_kernel<InteriorRunSink><<<ctas, kThreads, textSmem, s>>>(t, meta, b, en);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    nLaunch += 2;
-    if (nChunks > 1) {
-      if ((e = cudaEventRecord(ev[k], s)) != cudaSuccess) return e;
-      if ((e = cudaStreamWaitEvent(s2, ev[k], 0)) != cudaSuccess) return e;
-      lsop_wavefront4_kernel<<<(n + kWarps - 1) / kWarps, kThreads, 0, s2>>>(a, coef, meta, b, en, 1);
-      if ((e = cudaGetLastError()) != cudaSuccess) return e;
-      nLaunch++;
-    }
-  }
+  // [2] = work counter of the text kernel
+  const int nBlocks = (nTilesUpper + kWarps - 1) / kWarps;
+  lsop_decode_head_kernel<<<nBlocks, kThreads, 0, s>>>(a, coef, meta, defer, deferCounters, stageWords);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  DecodeArgs t = a;
+  t.counter = deferCounters + 2;
+  const int ctas = nCtas < nTilesUpper ? nCtas : nTilesUpper;
+  if (aligned) lsop_decode_text_kernel<InteriorPackedSink><<<ctas, kThreads, textSmem, s>>>(t, meta);
+  else lsop_decode_text_kernel<InteriorRunSink><<<ctas, kThreads, textSmem, s>>>(t, meta);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
   DecodeArgs d = a;
   d.list = defer;
   d.listCount = deferCounters;
   d.counter = deferCounters + 1;
   lsop_decode_entropy_kernel<<<nCtas < 296 ? nCtas : 296, kThreads, 0, s>>>(d, coef);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  nLaunch++;
-  if (nChunks > 1) {
-    if ((e = cudaEventRecord(ev[4], s2)) != cudaSuccess) return e;
-    if ((e = cudaStreamWaitEvent(s, ev[4], 0)) != cudaSuccess) return e;
-    lsop_wavefront4_kernel<<<(nTilesUpper + kWarps - 1) / kWarps, kThreads, 0, s>>>(a, coef, meta, 0, nTilesUpper, 2);  // deferred tiles
-  } else if (aligned) lsop_wavefront4_kernel<<<(nTilesUpper + kWarps - 1) / kWarps, kThreads, 0, s>>>(a, coef, meta, 0, nTilesUpper, 0);
-  else lsop_wavefront_kernel<<<(nTilesUpper + kWarps - 1) / kWarps, kThreads, 0, s>>>(a, coef);
-  nLaunch++;
-  if (launches) *launches = nLaunch;
+  if (aligned) lsop_wavefront4_kernel<<<nBlocks, kThreads, 0, s>>>(a, coef);
+  else lsop_wavefront_kernel<<<nBlocks, kThreads, 0, s>>>(a, coef);
+  if (launches) *launches = 4;
   return cudaGetLastError();
 }
 

@@ -52,11 +52,7 @@ constexpr uint32_t kTextSmallTile = 16384;
 constexpr uint32_t kTextSubBits = 320;        // target sub-sequence size of the text kernel: one sub-sequence per thread for a 180x240 tile
 constexpr int kExcWords = 128;               // per tile: [0] count, [2+2i] interior index, [3+2i] value
 constexpr int kExcCap = (kExcWords - 2) / 2;  // 63 exceptions; more -> general path
-// Staged form of the text decode (lsop_text_decode below), on unless built with -DG4_TEXT_STAGED=0.
-#ifndef G4_TEXT_STAGED
-#define G4_TEXT_STAGED 1
-#endif
-constexpr bool kTextStaged = G4_TEXT_STAGED != 0;
+constexpr uint32_t kTextLookback = 96;        // first pass of the staged text decode: bits before a sub-sequence limit where it starts
 constexpr int kStageWordsPerThread = 22;  // registers that carry a thread's staged symbol bytes across the barrier
 constexpr int kSpillWords = 8;            // words behind every slot in a per-CTA global scratch (stays in L2): the slots hold only
                                           // about 7 % more than the average sub-sequence, so the longer ones spill their tail
@@ -550,7 +546,7 @@ __device__ __noinline__ void text_exceptions_sub(const CanonFastShared& S, uint3
 // Returns 0 = done, 1 = malformed stream, 2 = the tile does not suit the staged form (caller uses canon_fast_decode_text).
 template <int NT>
 __device__ int lsop_text_decode(CanonFastShared& S, uint32_t nBits, const uint32_t T0, uint32_t nInterior, uint32_t imageBytes,
-                                ByteTileSink sink, uint32_t* spillArea, uint32_t lookback) {
+                                ByteTileSink sink, uint32_t* spillArea) {
   constexpr int kRounds = kFastMaxSub / NT;
   const int tid = threadIdx.x;
   const uint32_t avail = nBits - T0;
@@ -567,14 +563,14 @@ __device__ int lsop_text_decode(CanonFastShared& S, uint32_t nBits, const uint32
   if (uint64_t(slotWords + uint32_t(kSpillWords)) * 4u * uint64_t(nSub) * 3u < uint64_t(nInterior) * 4u) return 2;
   uint32_t* const image32 = reinterpret_cast<uint32_t*>(sink.tile);
   if (tid == 0) S.firstEot = nSub;
-  // pass 0: only the END of every sub-sequence matters here, so start kFastLookback bits before the limit and rely on
+  // pass 0: only the END of every sub-sequence matters here, so start kTextLookback bits before the limit and rely on
   // self-synchronisation (sub-sequence 0 as well: every thread does the same amount)
 #pragma unroll 1
   for (int i = tid; i < nSub; i += NT) {
     uint32_t limit = T0 + uint32_t(i + 1) * B;
     if (limit > nBits) limit = nBits;
     uint32_t from = T0 + uint32_t(i) * B;
-    if (limit - from > lookback) from = limit - lookback;
+    if (limit - from > kTextLookback) from = limit - kTextLookback;
     uint32_t e, c;
     int f;
     canon_fast_count(S, nBits, from, limit, &e, &c, &f);
@@ -770,10 +766,8 @@ __global__ void __launch_bounds__(NT, NT == 512 ? 2 : 4) lsop2_text_kernel(LsopF
       sink.init(tileImg, A.exc + size_t(tIdx) * kExcWords, A.g);
       // the previous tile's image has left shared memory (a barrier follows before the image is written again)
       if (tid == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-      if (kTextStaged)
-        rc = lsop_text_decode<NT>(F, span * 8u, T0 + 8u * delta, nInterior, uint32_t(A.g.tileBytes), sink,
-                              reinterpret_cast<uint32_t*>(A.textStage) + size_t(blockIdx.x) * (kFastMaxSub * kSpillWords), A.textLookback);
-      else rc = 2;
+      rc = lsop_text_decode<NT>(F, span * 8u, T0 + 8u * delta, nInterior, uint32_t(A.g.tileBytes), sink,
+                                reinterpret_cast<uint32_t*>(A.textStage) + size_t(blockIdx.x) * (kFastMaxSub * kSpillWords));
       if (rc == 2) {  // (uniform) the two-pass form
         uint32_t endBit = 0, nv = 0;
         rc = (canon_fast_decode_text<ByteTileSink, NT, kTextSubBits>(F, span * 8u, T0 + 8u * delta, nInterior, 0u, sink, &endBit, &nv) &&
@@ -1115,6 +1109,8 @@ size_t lsop_fast_resid_bytes(const LsopFastGeom& g, int nTiles) { return size_t(
 
 // Kernels H, T and W over the list positions [0, nTilesUpper).  Tiles the fast path cannot take are appended to
 // A.defer / A.deferCount for the general kernels, which the caller launches AFTER this returns.
+// The kernels take that range as [listBegin, listEnd) arguments: compiled without them, kernel T keeps its shared-memory
+// addresses in vector instead of uniform registers, and the config-3 decode measured up to 0.2 % slower (B200, 1000 W).
 cudaError_t launch_lsop_decode_fast(const LsopFastArgs& A, int nTilesUpper, int smCount, int* textCounter, cudaStream_t s, int* launches) {
   const LsopFastGeom& g = A.g;
   // dynamic shared memory opt-in: per device and per geometry, so simply set before every launch set (host-side only)

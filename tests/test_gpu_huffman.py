@@ -116,25 +116,59 @@ def test_terrain_generator_matches_cpu(g4, oracle):
     assert np.array_equal(f.cpu().numpy(), oracle.terrain_f32(5, 7, 33, 65))
 
 
-def test_general_decoder_still_decodes(oracle):
-    """The staged fast path (g4_huff_fast.cuh) takes every packing that fits its staging buffer; the general decoder over
-    HBM (g4_huffdec.cuh) stays for the rest.  G4_HUFF_FAST=0 sends everything through it (read once per process, hence
-    the subprocess): same bit-exact result."""
-    import os
-    import subprocess
-    import sys
+def test_general_decoder_unaligned_packings(g4, oracle):
+    """huffman_decode_kernel stages a packing in shared memory (g4_huff_fast.cuh) only when it starts on a 4-byte
+    boundary; any other packing goes through the general decoder over HBM (g4_huffdec.cuh).  Every parity grid's packing
+    sits at arena offsets 1, 2 and 3 (mod 4) of one tile-list call and decodes bit-exact at each.  Triangle tiles take
+    the fused kernel (g4_huff2.cuh) whatever their alignment; the oversized packings below send them to the general one."""
+    spec = g4.CodecSpecification(default=False)
+    spec.addCompressionCodec("GvrsHuffman", g4.CodecHuffman)
+    master = g4.CodecMaster(spec)
+    longer_than_raw = []
+    for name, grid in parity_grids(oracle).items():
+        R, C = grid.shape
+        packing, _ = oracle.codec_encode_i32(oracle.CODEC_HUFFMAN, 0, grid)
+        if len(packing) >= 4 * grid.size:  # a tile list reads such a payload as a raw tile or rejects it (CodecMaster never writes one)
+            longer_than_raw.append(name)
+            continue
+        arena = np.zeros(3 * (len(packing) + 32), np.uint8)
+        offsets, pos = [], 0
+        for mis in (1, 2, 3):
+            pos = (pos + 15) // 16 * 16 + mis
+            arena[pos:pos + len(packing)] = np.frombuffer(packing, np.uint8)
+            offsets.append(pos)
+            pos += len(packing)
+        out = np.full(3 * grid.size, -7, np.int32)
+        refs = [(k * grid.size, C) for k in range(3)]
+        master.decodeTileList(arena, np.array(offsets, np.uint64), np.full(3, len(packing), np.uint32), out, refs, R, C)
+        assert not master.lastStatus.any(), (name, master.lastStatus)
+        for k, mis in enumerate((1, 2, 3)):
+            got = out[k * grid.size:(k + 1) * grid.size].reshape(R, C)
+            assert np.array_equal(got, grid), "%s at offset %d mod 4: %s" % (name, mis, first_diff(got, grid))
+    assert longer_than_raw == ["noise"]  # its kind of content (multi-byte M32 codes) is among the oversized grids below
 
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = (
-        "import sys; sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
-        "import numpy as np, gridfour_b200 as g4\n"
-        "from oracle import g4oracle as o\n"
-        "from gpu_common import parity_grids\n"
-        "c = g4.CodecHuffman()\n"
-        "for name, grid in parity_grids(o).items():\n"
-        "    p, _ = o.codec_encode_i32(o.CODEC_HUFFMAN, 0, grid)\n"
-        "    assert np.array_equal(c.decode(grid.shape[0], grid.shape[1], p), grid), name\n"
-        "print('general ok')\n" % (root, os.path.join(root, "tests")))
-    env = dict(os.environ, G4_HUFF_FAST="0")
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, timeout=600)
-    assert r.returncode == 0 and "general ok" in r.stdout, r.stderr[-2000:]
+
+@pytest.mark.parametrize("pred", [3, 1, 2])
+def test_general_decoder_oversized_packings(g4, oracle, pred):
+    """A packing larger than both staging buffers -- the fused Triangle kernel's (n*6/8 + 256 bytes, at least 32 rows of
+    the tile) and huffman_decode_kernel's (n*6/8 + 64 bytes, at least 8 KB) -- goes through the general decoder over HBM,
+    whatever the predictor.  One grid per predictor: the noise is the predictor's residual, 1 % of it full-range (the
+    multi-byte M32 codes of a random raster)."""
+    R, C = 180, 240
+    rng = np.random.default_rng(5 + pred)
+    noise = rng.integers(-300, 301, (R, C), dtype=np.int64)
+    tail = rng.random((R, C)) < 0.01
+    noise[tail] = rng.integers(-(2 ** 31), 2 ** 31, int(tail.sum()), dtype=np.int64)
+    if pred == 3:  # Triangle: a 2-D cumulative sum
+        grid = noise.cumsum(axis=0).cumsum(axis=1)
+    elif pred == 1:  # Differencing: a row cumulative sum
+        grid = noise.cumsum(axis=1)
+    else:  # Linear: a second row cumulative sum
+        grid = noise.cumsum(axis=1).cumsum(axis=1)
+    grid = grid.astype(np.int32)  # wraps like the codec's 32-bit arithmetic
+    packing, best = oracle.codec_encode_i32(oracle.CODEC_HUFFMAN, 0, grid)
+    assert best == pred
+    n = grid.size
+    assert len(packing) > max(n * 6 // 8 + 256, 32 * C * 4, 8192 + 8), len(packing)
+    out = g4.CodecHuffman().decode(R, C, packing)
+    assert np.array_equal(out, grid), first_diff(out, grid)
