@@ -26,6 +26,7 @@ EXPORTS = [
     "g4_fill_terrain", "g4_launch_count", "g4_context_set_timing", "g4_context_set_async", "g4_kernel_time_ms", "g4_codec_supported",
     "g4_crc32c", "g4_tile_records_bound", "g4_pack_tile_records", "g4_unpack_tile_records", "g4_context_order_stream", "g4_decode_tiles_bounded", "g4_predictor_encode", "g4_predictor_encode_int", "g4_predictor_decode",
     "g4_predictor_decode_int", "g4_predictor_tiles", "g4_encode_tile_list", "g4_decode_tile_list", "g4_analyze_tiles",
+    "g4_tile_records_bound_multi", "g4_pack_tile_records_multi", "g4_unpack_tile_records_multi",
 ]
 
 
@@ -106,6 +107,12 @@ def lib():
                                            C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint64)]
         L.g4_unpack_tile_records.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
                                              C.c_void_p, C.c_void_p]
+        L.g4_tile_records_bound_multi.argtypes = [C.c_int, C.c_int, C.c_uint64]
+        L.g4_tile_records_bound_multi.restype = C.c_uint64
+        L.g4_pack_tile_records_multi.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                                 C.c_int, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint64)]
+        L.g4_unpack_tile_records_multi.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_int, C.c_int,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 

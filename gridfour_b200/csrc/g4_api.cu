@@ -99,6 +99,7 @@ struct g4_context {
   DevBuf stSorted, stRank, stTable, stWork, stCounters;
   // GVRS tile records (g4_records.cu): layout arrays and host-space staging
   DevBuf rcPos, rcOff, rcLen, rcCrc, rcStored, rcTotal, rcData, rcOffsets, rcLens, rcIndex, rcStatus, rcOut;
+  DevBuf rcChain, rcDesc;  // multi-element records: per-tile chain lengths, element descriptors (RecordElement)
   std::vector<uint64_t> hostOff;   // jobOff / jobLen mirrored on the host (chunking of the staged encode)
   std::vector<uint32_t> hostLen;
   uint64_t hostTotal = 0;
@@ -704,7 +705,7 @@ void g4_context_destroy(g4_context* ctx) {
                     &ctx->total, &ctx->coef, &ctx->defer, &ctx->lsopMeta, &ctx->lsopSide, &ctx->lsopExc, &ctx->lsopResid, &ctx->lsopStage, &ctx->tileRefs, &ctx->lsopCks, &ctx->wide, &ctx->encScratch, &ctx->region, &ctx->jobLen, &ctx->jobOff, &ctx->jobOut, &ctx->jobTotal,
                     &ctx->streamIn, &ctx->streamOut, &ctx->deflateWork, &ctx->stSorted, &ctx->stRank, &ctx->stTable,
                     &ctx->stWork, &ctx->stCounters, &ctx->rcPos, &ctx->rcOff, &ctx->rcLen, &ctx->rcCrc, &ctx->rcStored, &ctx->rcTotal,
-                    &ctx->rcData, &ctx->rcOffsets, &ctx->rcLens, &ctx->rcIndex, &ctx->rcStatus, &ctx->rcOut, &ctx->sGrid, &ctx->sArena, &ctx->sOffsets, &ctx->sLens, &ctx->sCodec, &ctx->sPred, &ctx->sStatus};
+                    &ctx->rcData, &ctx->rcOffsets, &ctx->rcLens, &ctx->rcIndex, &ctx->rcStatus, &ctx->rcOut, &ctx->rcChain, &ctx->rcDesc, &ctx->sGrid, &ctx->sArena, &ctx->sOffsets, &ctx->sLens, &ctx->sCodec, &ctx->sPred, &ctx->sStatus};
   for (DevBuf* b : bufs) b->release();
   if (ctx->ownStream) cudaStreamDestroy(ctx->stream);
   delete ctx;
@@ -897,6 +898,144 @@ int g4_unpack_tile_records(g4_context* ctx, int mem_space, const uint8_t* image,
   if (mem_space == G4_MEM_HOST) {
     CK(cudaMemcpyAsync(payload_offsets, dPay, size_t(n) * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(lens, dLens, size_t(n) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(status, dStatus, size_t(n) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+  }
+  return G4_OK;
+}
+
+uint64_t g4_tile_records_bound_multi(int n_tiles, int n_elements, uint64_t payload_bytes) {
+  if (n_tiles < 0 || n_elements < 1 || n_elements > G4_MAX_ELEMENTS) return 0;
+  // 8 header + 4 index + 4 length per element + 4 checksum + at most 7 padding
+  return payload_bytes + uint64_t(n_tiles) * (23ull + 4ull * uint64_t(n_elements));
+}
+
+int g4_pack_tile_records_multi(g4_context* ctx, int mem_space, int n_elements, const uint8_t* const* arenas,
+                               const uint64_t* const* offsets, const uint32_t* const* lens, const int32_t* tile_index,
+                               int first_tile_index, int n_tiles, int checksum, uint64_t base_pos, uint8_t* records,
+                               uint64_t records_cap, uint64_t* content_pos, uint64_t* total_bytes) {
+  if (!ctx || !arenas || !offsets || !lens || !records || !content_pos || !total_bytes || n_tiles < 0 || (base_pos & 7)) return G4_ERR_ARG;
+  if (n_elements < 1 || n_elements > G4_MAX_ELEMENTS) return G4_ERR_UNSUPPORTED;
+  if (mem_space != G4_MEM_DEVICE && mem_space != G4_MEM_HOST) return G4_ERR_ARG;
+  for (int e = 0; e < n_elements; e++)
+    if (!arenas[e] || !offsets[e] || !lens[e]) return G4_ERR_ARG;
+  *total_bytes = 0;
+  if (n_tiles == 0) return G4_OK;
+  ENTER(ctx);
+  const int n = n_tiles, E = n_elements;
+  std::vector<RecordElement> desc(static_cast<size_t>(E));
+  const int32_t* dIndex = tile_index;
+  uint64_t* dPos = content_pos;
+  uint8_t* dRecords = records;
+  if (mem_space == G4_MEM_HOST) {
+    // every element's used arena range, back to back (16-byte aligned) in rcData; offsets and lengths element-major
+    std::vector<uint64_t> base(size_t(E) + 1, 0), used(size_t(E), 0);
+    for (int e = 0; e < E; e++) {
+      for (int t = 0; t < n; t++) {
+        const uint64_t end = offsets[e][t] + lens[e][t];
+        if (end > used[size_t(e)]) used[size_t(e)] = end;
+      }
+      base[size_t(e) + 1] = round_up(base[size_t(e)] + used[size_t(e)], 16);
+    }
+    CK(ctx->rcData.ensure(base[size_t(E)] + 16));
+    CK(ctx->rcOffsets.ensure(size_t(E) * n * 8));
+    CK(ctx->rcLens.ensure(size_t(E) * n * 4));
+    CK(ctx->rcPos.ensure(size_t(n) * 8));
+    CK(ctx->rcOut.ensure(records_cap + 16));
+    for (int e = 0; e < E; e++) {
+      uint8_t* a = ctx->rcData.as<uint8_t>() + base[size_t(e)];
+      uint64_t* o = ctx->rcOffsets.as<uint64_t>() + size_t(e) * n;
+      uint32_t* l = ctx->rcLens.as<uint32_t>() + size_t(e) * n;
+      if (used[size_t(e)]) CK(cudaMemcpyAsync(a, arenas[e], used[size_t(e)], cudaMemcpyHostToDevice, ctx->stream));
+      CK(cudaMemcpyAsync(o, offsets[e], size_t(n) * 8, cudaMemcpyHostToDevice, ctx->stream));
+      CK(cudaMemcpyAsync(l, lens[e], size_t(n) * 4, cudaMemcpyHostToDevice, ctx->stream));
+      desc[size_t(e)] = RecordElement{a, o, l};
+    }
+    if (tile_index) {
+      CK(ctx->rcIndex.ensure(size_t(n) * 4));
+      CK(cudaMemcpyAsync(ctx->rcIndex.p, tile_index, size_t(n) * 4, cudaMemcpyHostToDevice, ctx->stream));
+      dIndex = ctx->rcIndex.as<int32_t>();
+    }
+    dPos = ctx->rcPos.as<uint64_t>();
+    dRecords = ctx->rcOut.as<uint8_t>();
+  } else {
+    for (int e = 0; e < E; e++) desc[size_t(e)] = RecordElement{arenas[e], offsets[e], lens[e]};
+  }
+  CK(ctx->rcDesc.ensure(size_t(E) * sizeof(RecordElement)));
+  CK(cudaMemcpyAsync(ctx->rcDesc.p, desc.data(), size_t(E) * sizeof(RecordElement), cudaMemcpyHostToDevice, ctx->stream));
+  const RecordElement* dDesc = ctx->rcDesc.as<RecordElement>();
+  CK(ctx->rcChain.ensure(size_t(n) * 4));
+  CK(ctx->rcOff.ensure(size_t(n) * 8));
+  CK(ctx->rcLen.ensure(size_t(n) * 4));
+  CK(ctx->rcTotal.ensure(8));
+  CK(launch_record_chain_lens(dDesc, E, n, ctx->rcChain.as<uint32_t>(), ctx->stream));
+  CK(launch_record_layout(ctx->rcChain.as<uint32_t>(), n, base_pos, dPos, ctx->rcOff.as<uint64_t>(), ctx->rcLen.as<uint32_t>(),
+                          ctx->rcTotal.as<uint64_t>(), ctx->stream));
+  uint64_t total = 0;
+  CK(cudaMemcpyAsync(&total, ctx->rcTotal.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));  // (also the end of `desc`'s copy)
+  ctx->launches += 2;
+  *total_bytes = total;
+  if (total > records_cap) return G4_ERR_CAPACITY;
+  CK(launch_record_pack_multi(dDesc, E, dIndex, first_tile_index, n, ctx->rcOff.as<uint64_t>(), ctx->rcLen.as<uint32_t>(), dRecords,
+                              persistent_ctas(ctx, n, 8), ctx->stream));
+  ctx->launches++;
+  if (checksum) {
+    CK(launch_crc32c(dRecords, ctx->rcOff.as<uint64_t>(), ctx->rcLen.as<uint32_t>(), n, nullptr, 1, ctx->stream));
+    ctx->launches++;
+  }
+  if (mem_space == G4_MEM_HOST) {
+    CK(cudaMemcpyAsync(records, dRecords, total, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(content_pos, dPos, size_t(n) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+  }
+  return G4_OK;
+}
+
+int g4_unpack_tile_records_multi(g4_context* ctx, int mem_space, int n_elements, const uint8_t* image, uint64_t image_len,
+                                 const uint64_t* content_pos, int n_tiles, int checksum, uint64_t* payload_offsets,
+                                 uint32_t* lens, int32_t* status) {
+  if (!ctx || !image || !content_pos || !payload_offsets || !lens || !status || n_tiles < 0) return G4_ERR_ARG;
+  if (n_elements < 1 || n_elements > G4_MAX_ELEMENTS) return G4_ERR_UNSUPPORTED;
+  if (mem_space != G4_MEM_DEVICE && mem_space != G4_MEM_HOST) return G4_ERR_ARG;
+  if (n_tiles == 0) return G4_OK;
+  ENTER(ctx);
+  const int n = n_tiles, E = n_elements;
+  const uint8_t* dImage = image;
+  const uint64_t* dPos = content_pos;
+  uint64_t* dPay = payload_offsets;
+  uint32_t* dLens = lens;
+  int32_t* dStatus = status;
+  if (mem_space == G4_MEM_HOST) {
+    CK(ctx->rcData.ensure(image_len + 16));
+    CK(ctx->rcPos.ensure(size_t(n) * 8));
+    CK(ctx->rcOffsets.ensure(size_t(E) * n * 8));
+    CK(ctx->rcLens.ensure(size_t(E) * n * 4));
+    CK(ctx->rcStatus.ensure(size_t(n) * 4));
+    CK(cudaMemcpyAsync(ctx->rcData.p, image, image_len, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->rcPos.p, content_pos, size_t(n) * 8, cudaMemcpyHostToDevice, ctx->stream));
+    dImage = ctx->rcData.as<uint8_t>();
+    dPos = ctx->rcPos.as<uint64_t>();
+    dPay = ctx->rcOffsets.as<uint64_t>();
+    dLens = ctx->rcLens.as<uint32_t>();
+    dStatus = ctx->rcStatus.as<int32_t>();
+  }
+  if (reinterpret_cast<uintptr_t>(dImage) & 7) return G4_ERR_ARG;
+  CK(ctx->rcOff.ensure(size_t(n) * 8));
+  CK(ctx->rcLen.ensure(size_t(n) * 4));
+  CK(ctx->rcCrc.ensure(size_t(n) * 4));
+  CK(ctx->rcStored.ensure(size_t(n) * 4));
+  CK(launch_record_unpack_multi(dImage, image_len, dPos, n, E, dPay, dLens, ctx->rcOff.as<uint64_t>(), ctx->rcLen.as<uint32_t>(),
+                                ctx->rcStored.as<uint32_t>(), dStatus, ctx->stream));
+  ctx->launches++;
+  if (checksum) {
+    CK(launch_crc32c(dImage, ctx->rcOff.as<uint64_t>(), ctx->rcLen.as<uint32_t>(), n, ctx->rcCrc.as<uint32_t>(), 0, ctx->stream));
+    CK(launch_record_verify_multi(ctx->rcCrc.as<uint32_t>(), ctx->rcStored.as<uint32_t>(), n, E, dPay, dLens, dStatus, ctx->stream));
+    ctx->launches += 2;
+  }
+  if (mem_space == G4_MEM_HOST) {
+    CK(cudaMemcpyAsync(payload_offsets, dPay, size_t(E) * n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(lens, dLens, size_t(E) * n * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(status, dStatus, size_t(n) * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
   }

@@ -284,5 +284,23 @@ cudaError_t launch_record_unpack(const uint8_t* image, uint64_t imageLen, const 
 // stored value; a mismatch leaves status G4_CHECKSUM_MISMATCH (the values stay delivered: the reference only prints).
 cudaError_t launch_lsop_value_checksum(const DecodeArgs& a, int nTilesUpper, cudaStream_t s);
 cudaError_t launch_record_verify(const uint32_t* computed, const uint32_t* stored, int n, int32_t* status, cudaStream_t s);
+// Tile records of rasters with several elements per tile.  elems: device array of nElements descriptors; element e of tile t
+// is elems[e].arena[elems[e].offsets[t] .. + elems[e].lens[t]).
+struct RecordElement {
+  const uint8_t* arena;
+  const uint64_t* offsets;
+  const uint32_t* lens;
+};
+// chainLens[t] = sum_e(4 + len_e) - 4: the `lens` argument of launch_record_layout for multi-element records
+cudaError_t launch_record_chain_lens(const RecordElement* elems, int nElements, int n, uint32_t* chainLens, cudaStream_t s);
+cudaError_t launch_record_pack_multi(const RecordElement* elems, int nElements, const int32_t* tileIndex, int firstTileIndex, int n,
+                                     const uint64_t* crcOff, const uint32_t* crcLen, uint8_t* records, int nCtas, cudaStream_t s);
+// payloadOff / lens: nElements x n, element-major
+cudaError_t launch_record_unpack_multi(const uint8_t* image, uint64_t imageLen, const uint64_t* contentPos, int n, int nElements,
+                                       uint64_t* payloadOff, uint32_t* lens, uint64_t* crcOff, uint32_t* crcLen, uint32_t* storedCrc,
+                                       int32_t* status, cudaStream_t s);
+// a sound record whose CRC differs: status G4_CHECKSUM_MISMATCH, every element's offset and length 0
+cudaError_t launch_record_verify_multi(const uint32_t* computed, const uint32_t* stored, int n, int nElements, uint64_t* payloadOff,
+                                       uint32_t* lens, int32_t* status, cudaStream_t s);
 
 }  // namespace g4

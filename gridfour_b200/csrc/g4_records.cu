@@ -11,8 +11,11 @@
 //   gvrs/RecordType.java:43-51         Tile = 2
 //   util/GridfourCRC32C.java:156-163   CRC-32C (Castagnoli, reflected, init/final xor 0xffffffff), byte-wise table form
 //
-// The batched codec entry points work on rasters with ONE element per tile, and so do the pack / unpack kernels here
-// (content = [tileIndex][len][payload]); g4_crc32c is general and serves every record type.
+// record_pack_kernel / record_unpack_kernel frame and read the records of rasters with ONE element per tile
+// (content = [tileIndex][len][payload], payload 8-byte aligned on both sides).  record_pack_multi_kernel /
+// record_unpack_multi_kernel do the same for any number of elements ([tileIndex] then [len_e][payload_e] per element, every
+// payload after the first at any byte offset); both reuse record_layout_kernel and crc32c_kernel.  g4_crc32c is general
+// and serves every record type.
 #include "g4_kernels.h"
 #include "g4_device.cuh"
 
@@ -314,6 +317,181 @@ __global__ void __launch_bounds__(kThreads) record_verify_kernel(const uint32_t*
   const int t = blockIdx.x * kThreads + threadIdx.x;
   if (t >= n) return;
   if (status[t] == G4_OK && computed[t] != stored[t]) status[t] = G4_ERR_FORMAT;
+}
+
+// ---- tile records of rasters with several elements per tile -----------------------------------------------------------
+// content = [tileIndex] then, per element e, [len_e][len_e bytes]; size = multipleOf8(12 + 4 + sum_e(4 + len_e)).
+// record_layout_kernel computes that size from chainLens[t] = sum_e(4 + len_e) - 4 (its own rounding adds the 20 bytes of
+// header, tile index, first length field and checksum field).
+
+// Four bytes from any address: the two aligned words around it joined by a funnel shift.  The second word is read only
+// when p is misaligned, and then it holds p[3], so it never leaves the granule of a byte the caller owns.
+__device__ inline uint32_t load_u32_funnel(const uint8_t* p) {
+  const uint32_t sh = uint32_t(reinterpret_cast<uintptr_t>(p) & 3u);
+  const uint32_t* a = reinterpret_cast<const uint32_t*>(p - sh);
+  const uint32_t lo = a[0];
+  return sh ? __funnelshift_r(lo, a[1], 8u * sh) : lo;
+}
+
+// One thread per tile.
+__global__ void __launch_bounds__(kThreads) record_chain_lens_kernel(const RecordElement* elems, int nElements, int n,
+                                                                     uint32_t* chainLens) {
+  const int t = blockIdx.x * kThreads + threadIdx.x;
+  if (t >= n) return;
+  uint32_t sum = 0;
+  for (int e = 0; e < nElements; e++) sum += 4u + elems[e].lens[t];
+  chainLens[t] = sum - 4u;
+}
+
+// One CTA per tile (persistent).  The record is written as aligned 32-bit words.  Shared memory holds the tile's segment
+// table: segment e is element e's [len] field followed by its payload, starting at record offset segStart[e].  Word i
+// belongs to the segment its first byte lies in; a word that lies wholly inside a payload is one funnel-shifted load
+// from the source arena (whose alignment is arbitrary), a word across a segment boundary is put together byte by byte.
+__global__ void __launch_bounds__(kThreads) record_pack_multi_kernel(const RecordElement* elems, int nElements, const int32_t* tileIndex,
+                                                                     int firstTileIndex, int n, const uint64_t* crcOff,
+                                                                     const uint32_t* crcLen, uint8_t* records) {
+  __shared__ uint32_t segStart[G4_MAX_ELEMENTS + 1];  // [nElements] = end of the chain
+  __shared__ uint32_t segLen[G4_MAX_ELEMENTS];
+  __shared__ const uint8_t* segSrc[G4_MAX_ELEMENTS];
+  const int E = nElements;
+  for (int t = blockIdx.x; t < n; t += gridDim.x) {
+    if (threadIdx.x < E) {
+      const RecordElement el = elems[threadIdx.x];
+      segLen[threadIdx.x] = el.lens[t];
+      segSrc[threadIdx.x] = el.arena + el.offsets[t];
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      uint32_t p = 12;
+      for (int e = 0; e < E; e++) {
+        segStart[e] = p;
+        p += 4u + segLen[e];
+      }
+      segStart[E] = p;
+    }
+    __syncthreads();
+    uint32_t* w = reinterpret_cast<uint32_t*>(records + crcOff[t]);
+    const uint32_t size = crcLen[t] + 4u;
+    if (threadIdx.x == 0) {
+      w[0] = size;
+      w[1] = 2u;  // RecordType.Tile, three reserved zero bytes
+      w[2] = uint32_t(tileIndex ? tileIndex[t] : firstTileIndex + t);
+    }
+    for (int e = 0; e < E; e++) {
+      const uint32_t s0 = segStart[e], s1 = segStart[e + 1], p0 = s0 + 4u;
+      const uint8_t* src = segSrc[e];
+      for (uint32_t i = (s0 + 3u) / 4u + threadIdx.x; i < (s1 + 3u) / 4u; i += kThreads) {
+        const uint32_t b = 4u * i;
+        uint32_t v = 0;
+        if (b >= p0 && b + 4u <= s1) {
+          v = load_u32_funnel(src + (b - p0));
+        } else {
+          int k = e;
+          for (uint32_t j = 0; j < 4; j++) {
+            const uint32_t q = b + j;
+            while (k < E && q >= segStart[k + 1]) k++;
+            if (k == E) break;  // past the chain: padding
+            const uint32_t r = q - segStart[k];
+            const uint32_t byte = r < 4u ? (segLen[k] >> (8u * r)) & 0xffu : segSrc[k][r - 4u];
+            v |= byte << (8u * j);
+          }
+        }
+        w[i] = v;
+      }
+    }
+    // zero padding and a zero checksum field (crc32c_kernel fills it in when checksums are enabled)
+    for (uint32_t i = (segStart[E] + 3u) / 4u + threadIdx.x; i < size / 4u; i += kThreads) w[i] = 0u;
+    __syncthreads();  // the segment table is rewritten for the next tile
+  }
+}
+
+// One thread per tile: the checks of record_unpack_kernel, then the [len] chain of the nElements elements, which has to
+// end at or before the checksum field.  payloadOff / lens are element-major (element e of tile t at e * n + t); a tile
+// whose status is not G4_OK gets 0 / 0 for every element.
+__global__ void __launch_bounds__(kThreads) record_unpack_multi_kernel(const uint8_t* image, uint64_t imageLen, const uint64_t* contentPos,
+                                                                       int n, int nElements, uint64_t* payloadOff, uint32_t* lens,
+                                                                       uint64_t* crcOff, uint32_t* crcLen, uint32_t* storedCrc,
+                                                                       int32_t* status) {
+  const int t = blockIdx.x * kThreads + threadIdx.x;
+  if (t >= n) return;
+  const uint64_t cp = contentPos[t];
+  int st = G4_OK;
+  uint32_t cl = 0, sc = 0;
+  uint64_t co = 0;
+  if (cp == 0) st = G4_DECLINED;  // tile not present in the file
+  else if ((cp & 7) || cp < 8 || cp + 8 > imageLen) st = G4_ERR_FORMAT;
+  else {
+    const uint32_t* h = reinterpret_cast<const uint32_t*>(image + cp - 8);
+    const uint32_t size = h[0];
+    const uint32_t type = h[1] & 0xffu;
+    if (type != 2u || size < 24u || (size & 7u) || cp - 8 + size > imageLen) st = G4_ERR_FORMAT;
+    else {
+      const uint64_t limit = cp - 8 + size - 4;  // the checksum field
+      uint64_t q = cp + 4;                       // element 0's [len]
+      for (int e = 0; e < nElements; e++) {
+        if (q + 4 > limit) { st = G4_ERR_FORMAT; break; }
+        const uint32_t ln = load_u32_funnel(image + q);
+        if ((ln >> 31) || q + 4 + ln > limit) { st = G4_ERR_FORMAT; break; }
+        payloadOff[size_t(e) * n + t] = q + 4;
+        lens[size_t(e) * n + t] = ln;
+        q += 4ull + ln;
+      }
+      if (st == G4_OK) {
+        co = cp - 8;
+        cl = size - 4u;
+        sc = *reinterpret_cast<const uint32_t*>(image + limit);
+      }
+    }
+  }
+  if (st != G4_OK) {
+    for (int e = 0; e < nElements; e++) {
+      payloadOff[size_t(e) * n + t] = 0;
+      lens[size_t(e) * n + t] = 0;
+    }
+  }
+  crcOff[t] = co;
+  crcLen[t] = cl;
+  storedCrc[t] = sc;
+  status[t] = st;
+}
+
+__global__ void __launch_bounds__(kThreads) record_verify_multi_kernel(const uint32_t* computed, const uint32_t* stored, int n,
+                                                                       int nElements, uint64_t* payloadOff, uint32_t* lens,
+                                                                       int32_t* status) {
+  const int t = blockIdx.x * kThreads + threadIdx.x;
+  if (t >= n) return;
+  if (status[t] != G4_OK || computed[t] == stored[t]) return;
+  status[t] = G4_CHECKSUM_MISMATCH;
+  for (int e = 0; e < nElements; e++) {
+    payloadOff[size_t(e) * n + t] = 0;
+    lens[size_t(e) * n + t] = 0;
+  }
+}
+
+cudaError_t launch_record_chain_lens(const RecordElement* elems, int nElements, int n, uint32_t* chainLens, cudaStream_t s) {
+  if (n <= 0) return cudaSuccess;
+  record_chain_lens_kernel<<<(n + kThreads - 1) / kThreads, kThreads, 0, s>>>(elems, nElements, n, chainLens);
+  return cudaGetLastError();
+}
+cudaError_t launch_record_pack_multi(const RecordElement* elems, int nElements, const int32_t* tileIndex, int firstTileIndex, int n,
+                                     const uint64_t* crcOff, const uint32_t* crcLen, uint8_t* records, int nCtas, cudaStream_t s) {
+  if (n <= 0) return cudaSuccess;
+  record_pack_multi_kernel<<<nCtas, kThreads, 0, s>>>(elems, nElements, tileIndex, firstTileIndex, n, crcOff, crcLen, records);
+  return cudaGetLastError();
+}
+cudaError_t launch_record_unpack_multi(const uint8_t* image, uint64_t imageLen, const uint64_t* contentPos, int n, int nElements,
+                                       uint64_t* payloadOff, uint32_t* lens, uint64_t* crcOff, uint32_t* crcLen, uint32_t* storedCrc,
+                                       int32_t* status, cudaStream_t s) {
+  if (n <= 0) return cudaSuccess;
+  record_unpack_multi_kernel<<<(n + kThreads - 1) / kThreads, kThreads, 0, s>>>(image, imageLen, contentPos, n, nElements, payloadOff, lens,
+                                                                               crcOff, crcLen, storedCrc, status);
+  return cudaGetLastError();
+}
+cudaError_t launch_record_verify_multi(const uint32_t* computed, const uint32_t* stored, int n, int nElements, uint64_t* payloadOff,
+                                       uint32_t* lens, int32_t* status, cudaStream_t s) {
+  if (n <= 0) return cudaSuccess;
+  record_verify_multi_kernel<<<(n + kThreads - 1) / kThreads, kThreads, 0, s>>>(computed, stored, n, nElements, payloadOff, lens, status);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_crc32c(const uint8_t* data, const uint64_t* offsets, const uint32_t* sizes, int n, uint32_t* out, int storeAtEnd,

@@ -11,10 +11,11 @@ Host-side mirror of the reference's file layout -- pure offset arithmetic, no sa
 
 Everything that walks sample bytes runs on the GPU through the C ABI: record checksums (g4_crc32c), tile-record framing
 (g4_pack_tile_records), record validation + payload location (g4_unpack_tile_records) and the codecs themselves
-(g4_encode_tiles / g4_decode_tiles with the file image as the arena).  The batched tile entry points serve rasters with
-one element per tile (the BASELINE configurations); files with several elements are parsed and re-framed record by
-record with the GPU computing the checksums, and read element by element (read_raster walks the [len][bytes] chains
-on the host and hands the payload offsets to g4_decode_tiles).
+(g4_encode_tiles / g4_decode_tiles with the file image as the arena).  Rasters with several elements per tile take the
+same path: one g4_encode_tiles call per element, then g4_pack_tile_records_multi frames [tileIndex] and a [len][bytes]
+pair per element into each record; g4_unpack_tile_records_multi validates the records and locates every element's payload
+in one call, and each element is decoded straight from the image (GvrsWriter.add_rasters, GvrsImage.read_rasters).
+add_tile_record_host frames one record on the host, for records whose size the caller dictates.
 """
 import ctypes as C
 import struct
@@ -27,6 +28,7 @@ from ._lib import G4_MEM_HOST, check
 RECORD_FREESPACE, RECORD_METADATA, RECORD_TILE, RECORD_FREESPACE_DIR, RECORD_METADATA_DIR, RECORD_TILE_DIR, RECORD_HEADER = range(7)
 ELEM_INTEGER, ELEM_INT_CODED_FLOAT, ELEM_FLOAT, ELEM_SHORT = 0, 1, 2, 3  # GvrsElementType.java:50-64
 _ELEM_BYTES = {ELEM_INTEGER: 4, ELEM_INT_CODED_FLOAT: 4, ELEM_FLOAT: 4, ELEM_SHORT: 2}
+_ELEM_DTYPE = {ELEM_INTEGER: np.int32, ELEM_INT_CODED_FLOAT: np.int32, ELEM_FLOAT: np.float32, ELEM_SHORT: np.int16}
 FILEPOS_HEADER_RECORD = 16
 FILEPOS_FREESPACE_DIR, FILEPOS_METADATA_DIR, FILEPOS_TILE_DIR = 56, 64, 80
 METADATA_TYPE_STRING = 9  # GvrsMetadataType.STRING (the type byte of the two codec metadata records in every sample file)
@@ -253,65 +255,59 @@ class GvrsImage:
             raise IOError("Checksum mismatch in record at file position %d" % int(off[bad[0]]))
         return len(off)
 
-    def locate_payloads(self, ctx, element=0, verify=True):
-        """(payload offsets, lengths, status) of one element of every tile, as g4_decode_tiles takes them with the file image
-        as its arena; status G4_DECLINED marks tiles the file does not hold."""
-        from ._lib import G4_DECLINED
+    def _locate_all(self, ctx, verify):
+        """(payload offsets [E, n], lengths [E, n], status [n]) of every element of every tile, in one GPU call; raises
+        IOError for a damaged tile record or, with verify, a record whose checksum differs."""
+        from ._lib import G4_CHECKSUM_MISMATCH
 
         spec = self.spec
-        if not 0 <= element < len(spec.elements):
-            raise ValueError("no such element")
         n_tiles = spec.tiles_down * spec.tiles_across
-        directory = self.tile_directory()
         pos = np.zeros(n_tiles, dtype=np.uint64)
-        for t, p in directory.items():
+        for t, p in self.tile_directory().items():
             pos[t] = p
+        checksum = verify and spec.checksum
         if len(spec.elements) == 1:
-            payload_off, lens, status = unpack_tile_records(ctx, self.image, pos, checksum=verify and spec.checksum)
-            bad = np.nonzero(status < 0)[0]
-            if len(bad):
-                raise IOError("damaged tile record for tile %d" % int(bad[0]))
+            payload_off, lens, status = unpack_tile_records(ctx, self.image, pos, checksum=checksum)
+            payload_off, lens = payload_off[None], lens[None]
         else:
-            b = self.image
-            payload_off = np.zeros(n_tiles, dtype=np.uint64)
-            lens = np.zeros(n_tiles, dtype=np.uint32)
-            status = np.full(n_tiles, G4_DECLINED, dtype=np.int32)
-            rec_off, rec_len, rec_crc = [], [], []
-            for t, p in directory.items():
-                size, type_code = struct.unpack_from("<iB", b, p - 8)
-                if type_code != RECORD_TILE or size < 24 or (size & 7) or p - 8 + size > len(b):
-                    raise IOError("damaged tile record for tile %d" % t)
-                q = p + 4
-                for k in range(len(spec.elements)):
-                    ln = struct.unpack_from("<i", b, q)[0]
-                    if ln < 0 or q + 4 + ln > p - 8 + size - 4:
-                        raise IOError("damaged tile record for tile %d" % t)
-                    if k == element:
-                        payload_off[t], lens[t], status[t] = q + 4, ln, 0
-                    q += 4 + ln
-                rec_off.append(p - 8)
-                rec_len.append(size - 4)
-                rec_crc.append(struct.unpack_from("<I", b, p - 8 + size - 4)[0])
-            if verify and spec.checksum and rec_off:
-                crc = crc32c_ranges(ctx, b, rec_off, rec_len)
-                if np.any(crc != np.array(rec_crc, dtype=np.uint32)):
-                    raise IOError("Checksum mismatch in a tile record")
+            payload_off, lens, status = unpack_tile_records_multi(ctx, self.image, pos, len(spec.elements), checksum=checksum)
+        bad = np.nonzero(status < 0)[0]
+        if len(bad):
+            raise IOError("damaged tile record for tile %d" % int(bad[0]))
+        if np.any(status == G4_CHECKSUM_MISMATCH):
+            raise IOError("Checksum mismatch in a tile record")
         return payload_off, lens, status
+
+    def locate_payloads(self, ctx, element=0, verify=True):
+        """(payload offsets, lengths, status) of one element of every tile, as g4_decode_tiles takes them with the file image
+        as its arena; status G4_DECLINED marks tiles the file does not hold.  The records are validated, their checksums
+        checked and their payloads located on the GPU (g4_unpack_tile_records, or g4_unpack_tile_records_multi for rasters
+        with several elements per tile)."""
+        if not 0 <= element < len(self.spec.elements):
+            raise ValueError("no such element")
+        payload_off, lens, status = self._locate_all(ctx, verify)
+        return payload_off[element], lens[element], status
+
+    def _decode_element(self, master, element, payload_off, lens, status, crop):
+        spec = self.spec
+        e = spec.elements[element]
+        grid = master.decodeImageTiles(self.image, payload_off, lens, status, spec.tiles_down, spec.tiles_across, spec.tile_rows,
+                                       spec.tile_cols, _ELEM_DTYPE[e.type_code], e.fill_value)
+        return grid[:spec.n_rows, :spec.n_cols] if crop else grid
 
     def read_raster(self, master, element=0, verify=True, crop=False):
         """crop=True returns the n_rows x n_cols raster without the fill-valued margin of the edge tiles.
         Decodes every tile of one element of the raster on the GPU straight from the file image: the image is the arena
-        of g4_decode_tiles.  One-element rasters: record validation, checksum check and payload location by
-        g4_unpack_tile_records.  Rasters with several elements per tile: the [len][bytes] chain of every tile record is
-        walked on the host (structure only) and the record checksums are checked by g4_crc32c.  Tiles that are absent from
-        the file come back filled with the element's fill value (RasterTile.setToNullState)."""
-        spec = self.spec
-        e = spec.elements[element] if 0 <= element < len(spec.elements) else None
+        of g4_decode_tiles; locate_payloads finds the payloads.  Tiles that are absent from the file come back filled with
+        the element's fill value (RasterTile.setToNullState)."""
         payload_off, lens, status = self.locate_payloads(master._context(), element, verify)
-        dtype = {ELEM_INTEGER: np.int32, ELEM_INT_CODED_FLOAT: np.int32, ELEM_FLOAT: np.float32, ELEM_SHORT: np.int16}[e.type_code]
-        grid = master.decodeImageTiles(self.image, payload_off, lens, status, spec.tiles_down, spec.tiles_across, spec.tile_rows,
-                                       spec.tile_cols, dtype, e.fill_value)
-        return grid[:spec.n_rows, :spec.n_cols] if crop else grid
+        return self._decode_element(master, element, payload_off, lens, status, crop)
+
+    def read_rasters(self, master, verify=True, crop=False):
+        """Every element's raster, in specification order, from one validation + location call (read_raster per element
+        would repeat it)."""
+        payload_off, lens, status = self._locate_all(master._context(), verify)
+        return [self._decode_element(master, k, payload_off[k], lens[k], status, crop) for k in range(len(self.spec.elements))]
 
 
 # ---- GPU-backed primitives -------------------------------------------------------------------------------------------
@@ -401,6 +397,89 @@ def unpack_tile_records_device(context, image, content_pos, checksum):
     check(_lib.lib().g4_unpack_tile_records(context._h, G4_MEM_DEVICE, image.data_ptr(), int(image.numel()), content_pos.data_ptr(), n,
                                             1 if checksum else 0, payload.data_ptr(), lens.data_ptr(), status.data_ptr()),
           "g4_unpack_tile_records")
+    return payload, lens, status
+
+
+def _pointers(buffers):
+    return (C.c_void_p * len(buffers))(*buffers)
+
+
+def pack_tile_records_multi(context, arenas, offsets, lens, base_pos, checksum, tile_index=None, first_tile_index=0):
+    """RecordManager.writeTile framing of a batch of tiles with len(arenas) elements: element e of tile t is
+    arenas[e][offsets[e][t] : + lens[e][t]].  Returns (record bytes, content positions)."""
+    a = [_u8(x) for x in arenas]
+    off = [np.ascontiguousarray(o, dtype=np.uint64) for o in offsets]
+    ln = [np.ascontiguousarray(x, dtype=np.uint32) for x in lens]
+    n = len(off[0]) if off else 0
+    if len(off) != len(a) or len(ln) != len(a) or any(len(o) != n for o in off) or any(len(x) != n for x in ln):
+        raise ValueError("pack_tile_records_multi: one offset and one length array of the same length per arena")
+    L = _lib.lib()
+    cap = int(L.g4_tile_records_bound_multi(n, len(a), sum(int(x.sum()) for x in ln)))
+    out = np.zeros(cap + 16, dtype=np.uint8)
+    pos = np.zeros(n, dtype=np.uint64)
+    total = C.c_uint64(0)
+    idx = None if tile_index is None else np.ascontiguousarray(tile_index, dtype=np.int32)
+    check(L.g4_pack_tile_records_multi(context._h, G4_MEM_HOST, len(a), _pointers([x.ctypes.data for x in a]),
+                                       _pointers([x.ctypes.data for x in off]), _pointers([x.ctypes.data for x in ln]),
+                                       None if idx is None else idx.ctypes.data, int(first_tile_index), n, 1 if checksum else 0,
+                                       int(base_pos), out.ctypes.data, cap, pos.ctypes.data, C.byref(total)), "g4_pack_tile_records_multi")
+    return out[:total.value].tobytes(), pos
+
+
+def unpack_tile_records_multi(context, image, content_pos, n_elements, checksum):
+    """Inverse of pack_tile_records_multi.  Returns (payload offsets [E, n], lengths [E, n], status [n]); row e is what
+    g4_decode_tiles takes for element e with the image as its arena."""
+    a = _u8(image)
+    pos = np.ascontiguousarray(content_pos, dtype=np.uint64)
+    n = len(pos)
+    payload = np.zeros((n_elements, n), dtype=np.uint64)
+    lens = np.zeros((n_elements, n), dtype=np.uint32)
+    status = np.zeros(n, dtype=np.int32)
+    check(_lib.lib().g4_unpack_tile_records_multi(context._h, G4_MEM_HOST, int(n_elements), a.ctypes.data, a.size, pos.ctypes.data, n,
+                                                  1 if checksum else 0, payload.ctypes.data, lens.ctypes.data, status.ctypes.data),
+          "g4_unpack_tile_records_multi")
+    return payload, lens, status
+
+
+def pack_tile_records_multi_device(context, batches, base_pos, checksum, first_tile_index=0):
+    """Device-resident form: `batches` holds one TileBatch of CodecMaster.encodeTiles on a CUDA tensor per element, all of
+    the same tiles.  Returns (records, content positions) as torch CUDA tensors; nothing crosses PCIe except the 8-byte
+    total."""
+    import torch
+
+    from ._lib import G4_MEM_DEVICE
+
+    L = _lib.lib()
+    n = int(batches[0].lens.numel()) if batches else 0
+    if any(int(b.lens.numel()) != n for b in batches):
+        raise ValueError("pack_tile_records_multi_device: every element's batch holds the same tiles")
+    cap = int(L.g4_tile_records_bound_multi(n, len(batches), sum(int(b.total_bytes) for b in batches)))
+    dev = batches[0].arena.device if batches else None
+    out = torch.empty(cap + 16, dtype=torch.uint8, device=dev)
+    pos = torch.empty(n, dtype=torch.int64, device=dev)
+    total = C.c_uint64(0)
+    check(L.g4_pack_tile_records_multi(context._h, G4_MEM_DEVICE, len(batches), _pointers([b.arena.data_ptr() for b in batches]),
+                                       _pointers([b.offsets.data_ptr() for b in batches]), _pointers([b.lens.data_ptr() for b in batches]),
+                                       None, int(first_tile_index), n, 1 if checksum else 0, int(base_pos), out.data_ptr(), cap,
+                                       pos.data_ptr(), C.byref(total)), "g4_pack_tile_records_multi")
+    return out[:total.value], pos
+
+
+def unpack_tile_records_multi_device(context, image, content_pos, n_elements, checksum):
+    """Device-resident form of unpack_tile_records_multi: image and content_pos are torch CUDA tensors (uint8 / int64).
+    Returns [E, n] int64 offsets, [E, n] int32 lengths and [n] int32 status on the device."""
+    import torch
+
+    from ._lib import G4_MEM_DEVICE
+
+    n = int(content_pos.numel())
+    dev = image.device
+    payload = torch.empty((n_elements, n), dtype=torch.int64, device=dev)
+    lens = torch.empty((n_elements, n), dtype=torch.int32, device=dev)
+    status = torch.empty(n, dtype=torch.int32, device=dev)
+    check(_lib.lib().g4_unpack_tile_records_multi(context._h, G4_MEM_DEVICE, int(n_elements), image.data_ptr(), int(image.numel()),
+                                                  content_pos.data_ptr(), n, 1 if checksum else 0, payload.data_ptr(), lens.data_ptr(),
+                                                  status.data_ptr()), "g4_unpack_tile_records_multi")
     return payload, lens, status
 
 
@@ -510,24 +589,50 @@ class GvrsWriter:
             self.tile_positions[int(t)] = int(p)
         return pos
 
+    def add_tile_records_multi(self, context, arenas, offsets, lens, tile_index=None, first_tile_index=0):
+        """Tile records of a batch with one arena per element (pack_tile_records_multi), framed and checksummed on the GPU."""
+        base = len(self.buf)
+        recs, pos = pack_tile_records_multi(context, arenas, offsets, lens, base, self.spec.checksum, tile_index, first_tile_index)
+        self.buf += recs
+        idx = range(first_tile_index, first_tile_index + len(pos)) if tile_index is None else tile_index
+        for t, p in zip(idx, pos):
+            self.tile_positions[int(t)] = int(p)
+        return pos
+
+    def _encode_element(self, master, e, grid):
+        """encodeTiles of one element's raster (numpy, n_rows x n_cols): the cells of the edge tiles that lie outside the
+        raster hold the element's fill value, as a RasterTile that was never written there does (TileElementInt/Float/Short
+        constructors fill the tile)."""
+        spec = self.spec
+        full = np.full((spec.tiles_down * spec.tile_rows, spec.tiles_across * spec.tile_cols), e.fill_value, dtype=_ELEM_DTYPE[e.type_code])
+        full[:spec.n_rows, :spec.n_cols] = grid
+        return master.encodeTiles(full, spec.tile_rows, spec.tile_cols, fillValue=e.fill_value if e.type_code == ELEM_SHORT else None)
+
     def add_raster(self, master, grid):
-        """A whole one-element raster (numpy, n_rows x n_cols): the cells of the edge tiles that lie outside the raster hold
-        the element's fill value, as a RasterTile that was never written there does (TileElementInt/Float/Short
-        constructors fill the tile); encodeTiles on the GPU, then the tile records.  Returns the TileBatch."""
+        """A whole one-element raster (numpy, n_rows x n_cols): encodeTiles on the GPU, then the tile records.  Returns the
+        TileBatch."""
         spec = self.spec
         if len(spec.elements) != 1 or grid.shape != (spec.n_rows, spec.n_cols):
             raise ValueError("add_raster: a one-element raster of the specified dimensions")
-        e = spec.elements[0]
-        dtype = {ELEM_INTEGER: np.int32, ELEM_INT_CODED_FLOAT: np.int32, ELEM_FLOAT: np.float32, ELEM_SHORT: np.int16}[e.type_code]
-        full = np.full((spec.tiles_down * spec.tile_rows, spec.tiles_across * spec.tile_cols), e.fill_value, dtype=dtype)
-        full[:spec.n_rows, :spec.n_cols] = grid
-        batch = master.encodeTiles(full, spec.tile_rows, spec.tile_cols,
-                                   fillValue=e.fill_value if e.type_code == ELEM_SHORT else None)
+        batch = self._encode_element(master, spec.elements[0], grid)
         self.add_tile_records(master._context(), batch.arena, batch.offsets, batch.lens)
         return batch
 
+    def add_rasters(self, master, grids):
+        """Every element of a raster: grids[k] (numpy, n_rows x n_cols) is element k in specification order -- int32 for
+        integer and integer-coded-float elements, float32, int16 for short elements.  One encodeTiles per element, then one
+        multi-element framing call.  Returns the TileBatch of every element."""
+        spec = self.spec
+        if len(grids) != len(spec.elements) or any(np.shape(g) != (spec.n_rows, spec.n_cols) for g in grids):
+            raise ValueError("add_rasters: one raster of the specified dimensions per element")
+        batches = [self._encode_element(master, e, g) for e, g in zip(spec.elements, grids)]
+        self.add_tile_records_multi(master._context(), [b.arena for b in batches], [b.offsets for b in batches],
+                                    [b.lens for b in batches])
+        return batches
+
     def add_tile_record_host(self, tile_index, element_payloads, size=None):
-        """One tile record with any number of elements: [tileIndex] then [len][bytes] per element (multi-element files)."""
+        """One tile record with any number of elements, framed on the host: [tileIndex] then [len][bytes] per element;
+        `size` may make the record larger than the content needs (as a reused file region leaves it)."""
         content = struct.pack("<i", tile_index) + b"".join(struct.pack("<i", len(p)) + bytes(p) for p in element_payloads)
         pos = self.add_record(RECORD_TILE, content, size)
         self.tile_positions[int(tile_index)] = pos

@@ -245,9 +245,36 @@ int g4_pack_tile_records(g4_context* ctx, int mem_space, const uint8_t* arena, c
 /* Inverse: image is a GVRS file (or a part of one: content_pos is relative to image) of image_len bytes, content_pos[t]
  * the directory position of tile t (0 = tile absent -> status G4_DECLINED, len 0).  Checks every record (type, sizes,
  * bounds and, with checksum != 0, the CRC-32C) and returns payload_offsets / lens in the form g4_decode_tiles takes with
- * `image` as its arena.  A damaged record gives status G4_ERR_FORMAT for that tile; the call itself still succeeds. */
+ * `image` as its arena.  A damaged record gives status G4_ERR_FORMAT for that tile; the call itself still succeeds.  A record
+ * whose CRC differs also gets G4_ERR_FORMAT here (g4_unpack_tile_records_multi tells it apart as G4_CHECKSUM_MISMATCH). */
 int g4_unpack_tile_records(g4_context* ctx, int mem_space, const uint8_t* image, uint64_t image_len, const uint64_t* content_pos,
                            int n_tiles, int checksum, uint64_t* payload_offsets, uint32_t* lens, int32_t* status);
+
+/* ---- tile records of rasters with several elements per tile (RecordManager.writeTile / readTile :386-516) ------------------
+ * content = [tileIndex:int32] then, for each element e in specification order, [len_e:int32][len_e bytes]; the record size
+ * is multipleOf8(12 + 4 + sum_e(4 + len_e)).  Element e's payload is what g4_encode_tiles returned for that element (a codec
+ * packing, or the raw tile at the element's standard size).  With n_elements == 1 these calls write and read exactly the
+ * records of g4_pack_tile_records / g4_unpack_tile_records.  n_elements outside 1..G4_MAX_ELEMENTS: G4_ERR_UNSUPPORTED. */
+#define G4_MAX_ELEMENTS 64
+/* Upper bound of the record bytes g4_pack_tile_records_multi writes for n_tiles tiles with payload_bytes in total (0 for
+ * arguments out of range). */
+uint64_t g4_tile_records_bound_multi(int n_tiles, int n_elements, uint64_t payload_bytes);
+/* arenas / offsets / lens: HOST arrays of n_elements pointers (like g4_tile_ref); the buffers they point to live in mem_space.
+ * Element e of tile t is arenas[e][offsets[e][t] .. + lens[e][t]), at any alignment.  Host buffers are staged: for each
+ * element its range [0, max_t(offsets[e][t] + lens[e][t])) is copied.  The other arguments and results are those of
+ * g4_pack_tile_records, including G4_ERR_CAPACITY with the needed size in *total_bytes. */
+int g4_pack_tile_records_multi(g4_context* ctx, int mem_space, int n_elements, const uint8_t* const* arenas,
+                               const uint64_t* const* offsets, const uint32_t* const* lens, const int32_t* tile_index,
+                               int first_tile_index, int n_tiles, int checksum, uint64_t base_pos, uint8_t* records,
+                               uint64_t records_cap, uint64_t* content_pos, uint64_t* total_bytes);
+/* Inverse.  payload_offsets / lens: n_elements x n_tiles, ELEMENT-major (element e of tile t at e * n_tiles + t), so that row e
+ * feeds g4_decode_tiles directly with `image` as the arena.  status[t]: G4_OK; G4_DECLINED for content_pos 0 (tile absent);
+ * G4_ERR_FORMAT for a damaged record (misaligned or out-of-image position, type, size, a len with bit 31 set, or a chain
+ * that runs into the checksum field); G4_CHECKSUM_MISMATCH, with checksum != 0, for a sound record whose CRC differs.  Every
+ * tile whose status is not G4_OK gets offset 0 and length 0 for every element.  The call itself still succeeds. */
+int g4_unpack_tile_records_multi(g4_context* ctx, int mem_space, int n_elements, const uint8_t* image, uint64_t image_len,
+                                 const uint64_t* content_pos, int n_tiles, int checksum, uint64_t* payload_offsets,
+                                 uint32_t* lens, int32_t* status);
 
 /* ---- benchmark support --------------------------------------------------------------------------
  * Fills a device raster with the synthetic fractal terrain of include/g4terrain.h
