@@ -185,10 +185,14 @@ struct LsopFastGeom {
   int R, C;
   int W;          // strip width in columns: 4, 8 or 16 (C is a multiple of W)
   int logW;
-  int nStrips;    // lanes of a wavefront warp in use: strip k = columns 2 + k W .. 2 + k W + W - 1; ceil((C - 2) / W) <= 32
+  int tilesPerWarp;  // wavefront tiles per warp: 2 when nStrips <= 16 (each 16-lane half of the warp decodes its own
+                     // tile), else 1
+  int nStrips;    // lanes of a wavefront tile in use: strip k = columns 2 + k W .. 2 + k W + W - 1; ceil((C - 2) / W) <= 32
+                  // (<= 16 with two tiles per warp)
   int P;          // bytes per row of the residual image = nStrips * W
   int nSteps;     // wavefront steps = R - 2 + nStrips - 1 (lane k works on row s - k + 2 at step s)
-  int chunkRows;  // image rows per bulk copy of the wavefront kernel = 128 / W (chunk = chunkRows * P <= 4096 bytes)
+  int chunkRows;  // image rows per bulk copy of the wavefront kernel = 128 / W (chunk = chunkRows * P <= 4096 bytes;
+                  // <= 2048 with two tiles per warp, which share one 4096-byte ring stage)
   int nChunks;
   int tileBytes;  // nChunks * chunkRows * P: the image one tile writes
   int tilePitch;  // bytes between the images of consecutive tiles (a multiple of 128)

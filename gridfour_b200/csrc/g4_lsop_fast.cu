@@ -15,7 +15,10 @@
 //      leave as ONE BYTE each (symbol = residual + 128) into a shared-memory image of the tile's residual scratch,
 //      which goes to HBM with one bulk-async store.  Residuals that do not fit a byte (escapes, nulls) are written as
 //      byte 0 plus an entry in a small per-tile exception list.
-//   W  lsop3_wave_kernel   one warp per tile.  The causal 12-tap float32 stencil as a wavefront over COLUMN STRIPS:
+//   W  lsop3_wave_kernel   one warp per tile, or one 16-lane half-warp per tile when the tile's columns fit 16 strips
+//      (LsopFastGeom::tilesPerWarp; the two tiles of a warp share only its instruction stream and ring: wider strips
+//      give fewer ramp steps and spread the fixed cost of a step over more cells).  The causal 12-tap float32 stencil as
+//      a wavefront over COLUMN STRIPS:
 //      lane k owns the W columns 2 + k W .. (W = 4, 8 or 16), walks down the rows and is one ROW behind lane k - 1
 //      (row r of strip k needs row r of strip k - 1 and rows r - 1, r - 2 of strip k + 1).  Every lane is at the same
 //      cell of its strip at the same time, so the control flow is uniform: no per-lane row ends, no wrap blocks; the
@@ -805,93 +808,140 @@ constexpr int kWaveWarps = G4_WAVE_WARPS;  // warps (= tiles) per CTA of the wav
 constexpr int kWaveChunkBytes = 4096;  // ring stage: one bulk copy of 128 / W image rows (<= 32 strips x W bytes each)
 
 // The value of an exceptional cell (byte 0 in the scratch): its list entry, or -128 when the byte was genuine.
-__device__ __noinline__ int32_t wave_exception(const uint32_t* exc, int n, int k) {
+// exc: the tile's list, which holds at most kExcCap entries (the wavefront skips tiles with more).
+__device__ __noinline__ int32_t wave_exception(const uint32_t* exc, int k) {
+  const int n = int(exc[0]);
   for (int i = 0; i < n; i++)
     if (int(exc[2 + 2 * i]) == k) return int32_t(exc[3 + 2 * i]);
   return -128;
 }
 
-// floats of rows 0 and 1 of the tile (written by kernel H), columns 0 .. C + 3 (zeros past C - 1), per warp
+// floats of rows 0 and 1 of the tile (written by kernel H), columns 0 .. C + 3 (zeros past C - 1), per tile of a warp
 __device__ __forceinline__ int wave_rowbuf_floats(int C) { return (C + 4 + 3) & ~3; }
 
-template <int W, bool WIDE>
+// PAIR: two tiles per warp (LsopFastGeom::tilesPerWarp), one per 16-lane half; lane & 15 is the strip, and the halves
+// share nothing but the instruction stream and the warp's ring (each takes half of every stage).
+template <int W, bool WIDE, bool PAIR>
 __global__ void __launch_bounds__(32 * kWaveWarps, G4_WAVE_CTAS) lsop3_wave_kernel(LsopFastArgs A, int* tileCounter, int listBegin, int listEnd) {
   extern __shared__ __align__(128) unsigned char waveSmem[];
   constexpr int CR = 128 / W;   // image rows per chunk
   constexpr int NW = W / 4;     // residual words per lane and step
   constexpr int E = W - 4;      // the last strip: cells E, E + 1 are the row's last two columns (C a multiple of W)
+  constexpr int TPW = PAIR ? 2 : 1;  // tiles per warp
+  constexpr int HL = 32 / TPW;       // lanes per tile (the width of every shuffle)
+  constexpr uint32_t kHalfStage = uint32_t(kWaveChunkBytes) / 2;
+  // W 16 stores the first 8 columns of a strip row as soon as they are done: with the row's 14 outputs held to the end
+  // of the step, pairs need more than 128 registers
+  constexpr bool kEarlyLo = W == 16;
   const DecodeArgs& a = A.a;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int half = PAIR ? lane >> 4 : 0, ks = PAIR ? lane & 15 : lane;  // this lane's tile of the warp, its strip in it
   const LsopFastGeom& G = A.g;
   const int R = G.R, C = G.C, nS = G.nStrips, P = G.P;
   const int rbFloats = wave_rowbuf_floats(C);
   unsigned char* ring = waveSmem + size_t(warp) * (2 * kWaveChunkBytes);
-  float* rowbuf = reinterpret_cast<float*>(waveSmem + size_t(kWaveWarps) * (2 * kWaveChunkBytes)) + size_t(warp) * (2 * rbFloats);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(waveSmem + size_t(kWaveWarps) * (2 * kWaveChunkBytes) + size_t(kWaveWarps) * (2 * rbFloats) * sizeof(float)) + 2 * warp;
-  const uint32_t bar0 = smem_u32(bars), ring0 = smem_u32(ring);
-  const bool active = lane < nS, isFirst = lane == 0, isLast = lane == nS - 1;
+  // rows 0 and 1 of this lane's tile (shared-memory address)
+  const uint32_t rowbuf = smem_u32(waveSmem + size_t(kWaveWarps) * (2 * kWaveChunkBytes)) + uint32_t(warp * TPW + half) * uint32_t(2 * rbFloats) * 4u;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(waveSmem + size_t(kWaveWarps) * (2 * kWaveChunkBytes) +
+                                               size_t(kWaveWarps * TPW) * (2 * rbFloats) * sizeof(float)) + 2 * warp;
+  const uint32_t bar0 = smem_u32(bars);
+  // this lane's residual bytes in ring stage 0 (lane 0: the start of the warp's ring)
+  const uint32_t ringLane = smem_u32(ring) + uint32_t(half) * kHalfStage + uint32_t(ks * W);
+  const bool isFirst = ks == 0, isLast = ks == nS - 1;
   if (lane == 0) {
     mbar_init(bar0, 1);
     mbar_init(bar0 + 8, 1);
     asm volatile("fence.mbarrier_init.release.cluster;");
   }
   __syncwarp();
-  // persistent warps: every warp fetches its next tile when it is through with one (no wave quantisation of a static grid);
-  // gchunk counts the chunks this warp has fetched so far -- ring stage and mbarrier parity follow from it across tiles
+  // persistent warps: every warp fetches its next tile (pair of tiles) when it is through with one (no wave quantisation
+  // of a static grid); gchunk counts the chunks this warp has fetched so far -- ring stage and mbarrier parity follow
+  // from it across tiles
   uint32_t gchunk = 0;
   for (;;) {
   int li = 0;
-  if (lane == 0) li = listBegin + atomicAdd(tileCounter, 1);
+  if (lane == 0) li = listBegin + atomicAdd(tileCounter, TPW);
   li = __shfl_sync(0xffffffffu, li, 0);
   if (li >= listEnd || li >= *a.listCount) break;
-  const int tIdx = a.list[li];
-  if (a.status[tIdx] != G4_OK) continue;
-  if (*reinterpret_cast<const uint32_t*>(A.meta + size_t(tIdx) * kLsopMetaBytes) == 0u) continue;  // general path
-  const uint32_t* exc = A.exc + size_t(tIdx) * kExcWords;
-  const int nExc = int(exc[0]);
-  if (nExc > kExcCap) continue;  // deferred by kernel T
+  // a tile that failed in kernel H, goes to the general path or was deferred by kernel T is skipped; so is the second
+  // half of a pair at the end of the list.  A half without a tile stays idle while the other one works.
+  li += half;
+  int tIdx = 0, nExc = 0;
+  bool live = false;
+  if (!PAIR || (li < listEnd && li < *a.listCount)) {
+    tIdx = a.list[li];
+    if (a.status[tIdx] == G4_OK && *reinterpret_cast<const uint32_t*>(A.meta + size_t(tIdx) * kLsopMetaBytes) != 0u) {  // else general path
+      nExc = int(A.exc[size_t(tIdx) * kExcWords]);
+      live = nExc <= kExcCap;  // else deferred by kernel T
+    }
+  }
+  const uint32_t liveMask = __ballot_sync(0xffffffffu, live);
+  if (liveMask == 0u) continue;
+  const bool anyExc = PAIR ? __any_sync(0xffffffffu, live && nExc > 0) : nExc > 0;  // (uniform)
+  const bool active = live && ks < nS;
   const TileView t = tile_view(a.band, a.grid, tIdx);
-  const uint8_t* img = A.resid + kResidGuard + size_t(tIdx) * size_t(G.tilePitch);
   const uint32_t chunkBytes = uint32_t(CR * P);
   const int nChunks = G.nChunks;
-  auto issue = [&](int chunk) {  // lane 0: image rows CR chunk .. CR chunk + CR - 1 into the next ring stage
+  // image rows CR chunk .. CR chunk + CR - 1 into the next ring stage: lane 0 issues one copy per live tile (a skipped
+  // tile may have no image) and one expect_tx for all of them.  Called by the whole warp; the second tile and the live
+  // mask are fetched here rather than kept in registers across the steps.
+  auto issue = [&](int chunk) {
     const uint32_t g = gchunk + uint32_t(chunk);
-    const uint32_t bar = bar0 + 8u * (g & 1u), dst = ring0 + uint32_t(kWaveChunkBytes) * (g & 1u);
-    mbar_expect_tx(bar, chunkBytes);
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                 "l"(img + size_t(chunk) * chunkBytes), "r"(chunkBytes), "r"(bar)
-                 : "memory");
+    const uint32_t bar = bar0 + 8u * (g & 1u), dst = ringLane + uint32_t(kWaveChunkBytes) * (g & 1u);  // (lane 0)
+    const size_t off = size_t(chunk) * chunkBytes + kResidGuard;
+    if constexpr (PAIR) {
+      const int t1 = __shfl_sync(0xffffffffu, tIdx, 16);
+      const uint32_t lm = __ballot_sync(0xffffffffu, live);
+      if (lane == 0) {
+        const bool l0 = (lm & 1u) != 0u, l1 = (lm >> 16) != 0u;
+        mbar_expect_tx(bar, chunkBytes * uint32_t(int(l0) + int(l1)));
+        if (l0)
+          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
+                       "l"(A.resid + size_t(tIdx) * size_t(G.tilePitch) + off), "r"(chunkBytes), "r"(bar)
+                       : "memory");
+        if (l1)
+          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst + kHalfStage),
+                       "l"(A.resid + size_t(t1) * size_t(G.tilePitch) + off), "r"(chunkBytes), "r"(bar)
+                       : "memory");
+      }
+    } else if (lane == 0) {
+      mbar_expect_tx(bar, chunkBytes);
+      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
+                   "l"(A.resid + size_t(tIdx) * size_t(G.tilePitch) + off), "r"(chunkBytes), "r"(bar)
+                   : "memory");
+    }
   };
-  if (lane == 0) issue(0);
+  issue(0);
 
   float u[12];
 #pragma unroll
   for (int i = 0; i < 12; i++) u[i] = active ? A.coef[size_t(tIdx) * 12 + i] : 0.f;
   // rows 0 and 1 as floats (int -> float exactly as the reference converts them)
-  for (int c = lane; c < rbFloats; c += 32) {
-    rowbuf[c] = c < C ? float(t.row(0)[c]) : 0.f;
-    rowbuf[rbFloats + c] = c < C ? float(t.row(1)[c]) : 0.f;
-  }
-  const int4* side = A.side + size_t(tIdx) * R;
+  if (live)
+    for (int c = ks; c < rbFloats; c += HL) {
+      const float x = c < C ? float(t.row(0)[c]) : 0.f, y = c < C ? float(t.row(1)[c]) : 0.f;
+      asm volatile("st.shared.f32 [%0], %1;" ::"r"(rowbuf + 4u * uint32_t(c)), "f"(x) : "memory");
+      asm volatile("st.shared.f32 [%0], %1;" ::"r"(rowbuf + 4u * uint32_t(rbFloats + c)), "f"(y) : "memory");
+    }
+  // side records: the first lane needs {v[r][0], v[r][1]} of each, the last lane {D2[r], D1[r]} (nStrips >= 2)
+  const int2* side = reinterpret_cast<const int2*>(A.side + size_t(tIdx) * R) + (isLast ? 1 : 0);
   const bool needSide = active && (isFirst || isLast);
   // rr = (row this lane works on in the coming step) - 2; lanes that hold no strip never become valid
-  uint32_t rr = active ? uint32_t(-lane) : 0x40000000u;
+  uint32_t rr = active ? uint32_t(-ks) : 0x40000000u;
   const uint32_t nRowsIn = uint32_t(R - 2);
-  int4 sideCur = make_int4(0, 0, 0, 0), sideNext = make_int4(0, 0, 0, 0);
-  if (needSide && rr < nRowsIn) sideNext = side[2 + rr];   // (lane 0; the last lane fetches when its rows begin)
-  const int4* sideAt = side + 3 - lane;                   // record of the row after the coming step's (dereferenced for valid rows)
-  char* rowp = reinterpret_cast<char*>(t.base + int64_t(2 - lane) * t.pitch + lane * W);  // dereferenced only for valid rows
+  int2 sideCur = make_int2(0, 0), sideNext = make_int2(0, 0);
+  if (needSide && rr < nRowsIn) sideNext = side[2 * (2 + rr)];  // (first lane; the last lane fetches when its rows begin)
+  const int2* sideAt = side + 2 * (3 - ks);                      // record of the row after the coming step's (dereferenced for valid rows)
+  char* rowp = reinterpret_cast<char*>(t.base + int64_t(2 - ks) * t.pitch + ks * W);  // dereferenced only for valid rows
   const int64_t rowStep = int64_t(t.pitch) * 4;
-  const uint32_t ringLane = ring0 + uint32_t(lane * W);
   uint32_t ringAt = ringLane;                             // this lane's residual bytes of the coming step
-  const uint32_t rb0 = smem_u32(rowbuf) + uint32_t(lane * W) * 4u, rb1 = rb0 + uint32_t(rbFloats) * 4u;
+  const uint32_t rb0 = rowbuf + uint32_t(ks * W) * 4u, rb1 = rb0 + uint32_t(rbFloats) * 4u;
   const int wInterior = C - 4;
   uint32_t badBits = 0;  // nonzero: some cell left the range of the fast arithmetic
   float a0[W + 4], a1[W + 4], a2[W + 4];  // three rows of the strip, columns 2 + kW - 2 .. 2 + kW + W + 1, rotating roles
 #pragma unroll
   for (int i = 0; i < W + 4; i++) { a0[i] = 0.f; a1[i] = 0.f; a2[i] = 0.f; }
   int32_t pa = 0, pb = 0;        // own outputs of cells W - 2, W - 1 of the previous step (the right neighbour's left values)
-  float h0 = 0.f, h1 = 0.f;      // row 1 right of the strip, used in the lane's first step instead of the shuffle
   __syncwarp();
 
   // one step: row r of the strip into cur[]; am1 / am2 hold rows r - 1 / r - 2
@@ -899,7 +949,7 @@ __global__ void __launch_bounds__(32 * kWaveWarps, G4_WAVE_CTAS) lsop3_wave_kern
     if ((s & (CR - 1)) == 0) {  // (uniform) next chunk of the residual image
       const int chunk = s / CR;
       if (chunk < nChunks) {
-        if (lane == 0 && chunk + 1 < nChunks) issue(chunk + 1);
+        if (chunk + 1 < nChunks) issue(chunk + 1);
         const uint32_t g = gchunk + uint32_t(chunk);
         mbar_wait(bar0 + 8u * (g & 1u), (g >> 1) & 1u);
       }
@@ -917,14 +967,12 @@ __global__ void __launch_bounds__(32 * kWaveWarps, G4_WAVE_CTAS) lsop3_wave_kern
         am2[i] = x.x; am2[i + 1] = x.y; am2[i + 2] = x.z; am2[i + 3] = x.w;
         am1[i] = y.x; am1[i + 1] = y.y; am1[i + 2] = y.z; am1[i + 3] = y.w;
       }
-      h0 = am1[W + 2];
-      h1 = am1[W + 3];
      }
     }
-    // side record of this row (lane 0: columns 0,1; last lane: D2, D1), the next row's fetched now
+    // side record of this row (first lane: columns 0,1; last lane: D2, D1), the next row's fetched now
     sideCur = sideNext;
     if (needSide && rr + 1u < nRowsIn) sideNext = *sideAt;
-    sideAt++;
+    sideAt += 2;
     // residual bytes of the strip
     uint32_t rw[NW];
     {
@@ -935,20 +983,32 @@ __global__ void __launch_bounds__(32 * kWaveWarps, G4_WAVE_CTAS) lsop3_wave_kern
       else asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(rw[0]), "=r"(rw[1]), "=r"(rw[2]), "=r"(rw[3]) : "r"(at));
     }
     // left values: cells W-2, W-1 of row r in the strip to the left (finished one step ago: its am1), or columns 0,1
-    float l2 = __shfl_up_sync(0xffffffffu, am1[W], 1), l1 = __shfl_up_sync(0xffffffffu, am1[W + 1], 1);
-    int32_t li2 = __shfl_up_sync(0xffffffffu, pa, 1), li1 = __shfl_up_sync(0xffffffffu, pb, 1);
+    float l2 = __shfl_up_sync(0xffffffffu, am1[W], 1, HL), l1 = __shfl_up_sync(0xffffffffu, am1[W + 1], 1, HL);
+    int32_t li2 = __shfl_up_sync(0xffffffffu, pa, 1, HL), li1 = __shfl_up_sync(0xffffffffu, pb, 1, HL);
     if (isFirst) { li2 = sideCur.x; li1 = sideCur.y; l2 = float(li2); l1 = float(li1); }
     cur[0] = l2;
     cur[1] = l1;
-    // exceptions: a zero byte in a tile that has an exception list -> the general form of the step
+    // exceptions: a zero byte in a tile that has an exception list -> the general form of the step (for the whole warp)
     bool general = false;
-    if (nExc > 0) {
+    if (anyExc) {
       bool z = false;
 #pragma unroll
       for (int i = 0; i < NW; i++) z = z || ((rw[i] - 0x01010101u) & ~rw[i] & 0x80808080u) != 0u;
       general = __any_sync(0xffffffffu, z && valid);
     }
     int32_t oi[W];
+    auto store_lo = [&](const int32_t (&o)[W]) {  // columns k W .. k W + 7 of the raster row: {left2, left1, cells 0 .. 5}
+      if constexpr (W >= 8) {
+        if (WIDE) {
+          asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(rowp), "r"(li2), "r"(li1), "r"(o[0]), "r"(o[1]), "r"(o[2]),
+                       "r"(o[3]), "r"(o[4]), "r"(o[5])
+                       : "memory");
+        } else {
+          *reinterpret_cast<int4*>(rowp) = make_int4(li2, li1, o[0], o[1]);
+          *reinterpret_cast<int4*>(rowp + 16) = make_int4(o[2], o[3], o[4], o[5]);
+        }
+      }
+    };
     uint32_t accLo = 0, accHi = 0;  // exponent bits of t1 that differ from those of [2^22, 2^23): nonzero <=> p outside [-2^21, 2^21) or NaN
     auto cells = [&](auto genTag) {
       constexpr bool GEN = decltype(genTag)::value;
@@ -958,9 +1018,11 @@ __global__ void __launch_bounds__(32 * kWaveWarps, G4_WAVE_CTAS) lsop3_wave_kern
         (void)dummy;
         const int c = j + 2;
         if (j == 2) {  // cells 0,1 of row r - 1 in the strip to the right were computed a moment ago (its cur[2], cur[3])
-          const float s0 = __shfl_down_sync(0xffffffffu, cur[2], 1), s1 = __shfl_down_sync(0xffffffffu, cur[3], 1);
-          am1[W + 2] = first ? h0 : s0;
-          am1[W + 3] = first ? h1 : s1;
+          const float s0 = __shfl_down_sync(0xffffffffu, cur[2], 1, HL), s1 = __shfl_down_sync(0xffffffffu, cur[3], 1, HL);
+          if (!first) {  // (in its first step the lane has row 1 right of the strip from the row buffer)
+            am1[W + 2] = s0;
+            am1[W + 3] = s1;
+          }
         }
         // LsDecoder12.java:424-438 -- evaluated left to right in float32, no fused multiply-add
         float p = u[0] * cur[c - 1];
@@ -986,17 +1048,18 @@ __global__ void __launch_bounds__(32 * kWaveWarps, G4_WAVE_CTAS) lsop3_wave_kern
         if constexpr (GEN) {
           const uint32_t byte = (word >> (8 * (j & 3))) & 0xffu;
           int32_t ex = int32_t(byte) - 128;
-          if (byte == 0u && valid) ex = wave_exception(exc, nExc, int(rr) * wInterior + lane * W + j);
+          if (byte == 0u && valid) ex = wave_exception(A.exc + size_t(tIdx) * kExcWords, int(rr) * wInterior + ks * W + j);
           iv = int32_t(uint32_t(__float_as_int(t2)) - 0x4B400000u + uint32_t(ex));
           fv = float(iv);
         } else iv = int32_t(uint32_t(__float_as_int(t2)) + __float_as_uint(xj) - 0x96800080u);  // round(p) + byte - 128
         if (j == E || j == E + 1) {  // the last strip: Triangle predictor folded into D2 / D1 by kernel H (LsDecoder12.java:459-468)
           const int32_t prev = j == 0 ? li1 : oi[j > 0 ? j - 1 : 0];
-          const int32_t sv = int32_t(uint32_t(prev) + uint32_t(j == E ? sideCur.z : sideCur.w));
+          const int32_t sv = int32_t(uint32_t(prev) + uint32_t(j == E ? sideCur.x : sideCur.y));
           if (isLast) { iv = sv; fv = float(sv); }
         }
         oi[j] = iv;
         cur[c] = fv;
+        if (kEarlyLo && j == 5 && valid) store_lo(oi);  // (frees oi[0 .. 5] for the second half of the strip)
       }
     };
     if (general) cells(std::true_type{});
@@ -1006,18 +1069,13 @@ __global__ void __launch_bounds__(32 * kWaveWarps, G4_WAVE_CTAS) lsop3_wave_kern
     if (valid) {
       if constexpr (W == 4) *reinterpret_cast<int4*>(rowp) = make_int4(li2, li1, oi[0], oi[1]);
       else {
-        if (WIDE) {
-          asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(rowp), "r"(li2), "r"(li1), "r"(oi[0]), "r"(oi[1]), "r"(oi[2]),
-                       "r"(oi[3]), "r"(oi[4]), "r"(oi[5])
-                       : "memory");
-          if constexpr (W == 16)
+        if constexpr (!kEarlyLo) store_lo(oi);
+        if constexpr (W == 16) {
+          if (WIDE) {
             asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(rowp + 32), "r"(oi[6]), "r"(oi[7]), "r"(oi[8]), "r"(oi[9]),
                          "r"(oi[10]), "r"(oi[11]), "r"(oi[12]), "r"(oi[13])
                          : "memory");
-        } else {
-          *reinterpret_cast<int4*>(rowp) = make_int4(li2, li1, oi[0], oi[1]);
-          *reinterpret_cast<int4*>(rowp + 16) = make_int4(oi[2], oi[3], oi[4], oi[5]);
-          if constexpr (W == 16) {
+          } else {
             *reinterpret_cast<int4*>(rowp + 32) = make_int4(oi[6], oi[7], oi[8], oi[9]);
             *reinterpret_cast<int4*>(rowp + 48) = make_int4(oi[10], oi[11], oi[12], oi[13]);
           }
@@ -1038,9 +1096,9 @@ __global__ void __launch_bounds__(32 * kWaveWarps, G4_WAVE_CTAS) lsop3_wave_kern
     step(a1, a2, a0, s + 1);
     step(a2, a0, a1, s + 2);
   }
-  if (__any_sync(0xffffffffu, badBits != 0u)) {  // outside the fast arithmetic's range: the general kernels redo the tile
-    if (lane == 0) A.defer[atomicAdd(A.deferCount, 1)] = tIdx;
-  }
+  // outside the fast arithmetic's range: the general kernels redo the tile
+  const uint32_t bad = __ballot_sync(0xffffffffu, badBits != 0u);
+  if (isFirst && (PAIR ? (bad >> (16 * half)) & 0xffffu : bad) != 0u) A.defer[atomicAdd(A.deferCount, 1)] = tIdx;
   gchunk += uint32_t(nChunks);
   }
 }
@@ -1059,21 +1117,25 @@ size_t text_smem_bytes(const LsopFastGeom& g) { return text_fast_bytes(text_stag
 bool text_small(const LsopFastGeom& g) { return uint32_t(g.R) * uint32_t(g.C) <= kTextSmallTile; }
 size_t wave_smem_bytes(const LsopFastGeom& g) {
   const size_t rbFloats = size_t((g.C + 4 + 3) & ~3);
-  return size_t(kWaveWarps) * (2 * kWaveChunkBytes) + size_t(kWaveWarps) * (2 * rbFloats) * sizeof(float) + size_t(kWaveWarps) * 16;
+  return size_t(kWaveWarps) * (2 * kWaveChunkBytes) + size_t(kWaveWarps * g.tilesPerWarp) * (2 * rbFloats) * sizeof(float) +
+         size_t(kWaveWarps) * 16;
 }
 
+template <int W, bool WIDE, bool PAIR>
+cudaError_t launch_wave_kernel(const LsopFastArgs& A, int nCtas, int nTilesUpper, int* tileCounter, cudaStream_t s) {
+  const size_t smem = wave_smem_bytes(A.g);
+  cudaError_t e = cudaFuncSetAttribute(lsop3_wave_kernel<W, WIDE, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+  if (e != cudaSuccess) return e;
+  lsop3_wave_kernel<W, WIDE, PAIR><<<nCtas, 32 * kWaveWarps, smem, s>>>(A, tileCounter, 0, nTilesUpper);
+  return cudaGetLastError();
+}
 template <int W>
 cudaError_t launch_wave(const LsopFastArgs& A, int nCtas, int nTilesUpper, int* tileCounter, cudaStream_t s) {
-  const size_t smem = wave_smem_bytes(A.g);
-  cudaError_t e;
-  if (A.g.wide) {
-    if ((e = cudaFuncSetAttribute(lsop3_wave_kernel<W, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem))) != cudaSuccess) return e;
-    lsop3_wave_kernel<W, true><<<nCtas, 32 * kWaveWarps, smem, s>>>(A, tileCounter, 0, nTilesUpper);
-  } else {
-    if ((e = cudaFuncSetAttribute(lsop3_wave_kernel<W, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem))) != cudaSuccess) return e;
-    lsop3_wave_kernel<W, false><<<nCtas, 32 * kWaveWarps, smem, s>>>(A, tileCounter, 0, nTilesUpper);
-  }
-  return cudaGetLastError();
+  if (A.g.tilesPerWarp == 2)
+    return A.g.wide ? launch_wave_kernel<W, true, true>(A, nCtas, nTilesUpper, tileCounter, s)
+                    : launch_wave_kernel<W, false, true>(A, nCtas, nTilesUpper, tileCounter, s);
+  return A.g.wide ? launch_wave_kernel<W, true, false>(A, nCtas, nTilesUpper, tileCounter, s)
+                  : launch_wave_kernel<W, false, false>(A, nCtas, nTilesUpper, tileCounter, s);
 }
 
 }  // namespace
@@ -1083,12 +1145,23 @@ bool lsop_fast_geometry(const g4_band_desc& band, const void* grid, LsopFastGeom
   g.R = band.tile_rows;
   g.C = band.tile_cols;
   if (g.R < 6 || g.C < 16 || (g.C & 3) != 0 || (band.grid_pitch & 3) != 0 || (reinterpret_cast<uintptr_t>(grid) & 15) != 0) return false;
-  // strip width: the narrowest that covers the columns with 32 lanes; C has to be a multiple of it (the last strip then
-  // ends with the row's last two columns)
-  if (g.C <= 128) g.W = 4;
-  else if (g.C <= 256 && (g.C & 7) == 0) g.W = 8;
-  else if (g.C <= 512 && (g.C & 15) == 0) g.W = 16;
-  else return false;
+  // strip width: C has to be a multiple of it (the last strip then ends with the row's last two columns).  The narrowest
+  // that covers the columns with 16 lanes, two tiles per warp: fewer ramp steps per tile, more cells per step to share
+  // the fixed cost of a step, and 30 of 32 lanes busy at 240 columns instead of 30 (W 8, 207 steps for 178 rows) or
+  // 15 (W 16 single).  Otherwise the narrowest that covers them with 32 lanes, one tile per warp.
+  g.tilesPerWarp = 1;
+  for (int w = 4; w <= 16; w *= 2)
+    if (g.C % w == 0 && (g.C - 2 + w - 1) / w <= 16) {
+      g.W = w;
+      g.tilesPerWarp = 2;
+      break;
+    }
+  if (g.tilesPerWarp == 1) {
+    if (g.C <= 128) g.W = 4;
+    else if (g.C <= 256 && (g.C & 7) == 0) g.W = 8;
+    else if (g.C <= 512 && (g.C & 15) == 0) g.W = 16;
+    else return false;
+  }
   g.logW = g.W == 4 ? 2 : g.W == 8 ? 3 : 4;
   g.nStrips = (g.C - 2 + g.W - 1) / g.W;
   g.P = g.nStrips * g.W;
@@ -1138,7 +1211,8 @@ cudaError_t launch_lsop_decode_fast(const LsopFastArgs& A, int nTilesUpper, int 
   if (text_small(g)) lsop2_text_kernel<kTextThreadsSmall><<<ctas, kTextThreadsSmall, textSmem, s>>>(T, stageWords, 0, nTilesUpper);
   else lsop2_text_kernel<kTextThreads><<<ctas, kTextThreads, textSmem, s>>>(T, stageWords, 0, nTilesUpper);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  int nCtasWave = (nTilesUpper + kWaveWarps - 1) / kWaveWarps;
+  const int nWarpsWave = (nTilesUpper + g.tilesPerWarp - 1) / g.tilesPerWarp;
+  int nCtasWave = (nWarpsWave + kWaveWarps - 1) / kWaveWarps;
   if (nCtasWave > smCount * G4_WAVE_CTAS) nCtasWave = smCount * G4_WAVE_CTAS;  // persistent: one resident set of CTAs
   int* waveCounter = textCounter + 1;
   e = g.W == 4 ? launch_wave<4>(A, nCtasWave, nTilesUpper, waveCounter, s) : g.W == 8 ? launch_wave<8>(A, nCtasWave, nTilesUpper, waveCounter, s)
