@@ -6,7 +6,8 @@ CodecMaster, plus the new batched encodeTiles / decodeTiles entry.  See DESIGN.m
 """
 from .codecs import (  # noqa: F401
     CodecCanonHuffman, CodecDeflate, CodecFloat, CodecHuffman, CodecMaster, CodecSpecification, Context,
-    ICompressionDecoder, ICompressionEncoder, LsDecoder08, LsDecoder12, LsEncoder08, LsEncoder12, TileBatch, INT4_NULL_CODE,
+    ICompressionDecoder, ICompressionEncoder, IntCodedFloat, LsDecoder08, LsDecoder12, LsEncoder08, LsEncoder12, TileBatch,
+    INT4_NULL_CODE,
 )
 from ._lib import FormatError, G4Error, ValueChecksumWarning  # noqa: F401
 from . import gvrs  # noqa: F401

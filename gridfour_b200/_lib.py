@@ -13,7 +13,7 @@ G4_OK, G4_DECLINED, G4_CHECKSUM_MISMATCH = 0, 1, 2
 G4_ERR_ARG, G4_ERR_FORMAT, G4_ERR_CAPACITY, G4_ERR_CUDA, G4_ERR_UNSUPPORTED = -1, -2, -3, -4, -5
 G4_CODEC_HUFFMAN, G4_CODEC_DEFLATE, G4_CODEC_FLOAT, G4_CODEC_CANON_HUFFMAN, G4_CODEC_LSOP12 = 0, 1, 2, 3, 4
 G4_CODEC_LSOP08 = 5
-G4_ELEM_I32, G4_ELEM_F32, G4_ELEM_I16 = 0, 1, 2
+G4_ELEM_I32, G4_ELEM_F32, G4_ELEM_I16, G4_ELEM_ICF = 0, 1, 2, 3
 G4_MEM_HOST, G4_MEM_DEVICE = 0, 1
 G4_MAX_CODECS = 16
 G4_CODEC_RAW = 255
@@ -27,6 +27,7 @@ EXPORTS = [
     "g4_crc32c", "g4_tile_records_bound", "g4_pack_tile_records", "g4_unpack_tile_records", "g4_context_order_stream", "g4_decode_tiles_bounded", "g4_predictor_encode", "g4_predictor_encode_int", "g4_predictor_decode",
     "g4_predictor_decode_int", "g4_predictor_tiles", "g4_encode_tile_list", "g4_decode_tile_list", "g4_analyze_tiles",
     "g4_tile_records_bound_multi", "g4_pack_tile_records_multi", "g4_unpack_tile_records_multi",
+    "g4_icf_map", "g4_encode_tiles_icf", "g4_decode_tiles_icf",
 ]
 
 
@@ -43,6 +44,11 @@ class BandDesc(C.Structure):
     _fields_ = [("elem_type", C.c_int32), ("tile_rows", C.c_int32), ("tile_cols", C.c_int32),
                 ("tiles_down", C.c_int32), ("tiles_across", C.c_int32), ("grid_pitch", C.c_int64),
                 ("fill_value", C.c_int32), ("reserved", C.c_int32)]
+
+
+class IcfDesc(C.Structure):
+    """g4_icf_desc: the mapping of an integer-coded float element (code = floor((v - offset) * scale + 0.5))."""
+    _fields_ = [("scale", C.c_float), ("offset", C.c_float), ("fill_int", C.c_int32), ("fill_value", C.c_float)]
 
 
 _lib = None
@@ -95,6 +101,13 @@ def lib():
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.g4_analyze_tiles.argtypes = [C.c_void_p, C.POINTER(CodecList), C.POINTER(BandDesc), C.c_int, C.c_void_p, C.c_uint64, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p]
+        L.g4_icf_map.argtypes = [C.c_void_p, C.c_int, C.POINTER(IcfDesc), C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,
+                                 C.c_int64]
+        L.g4_encode_tiles_icf.argtypes = [C.c_void_p, C.POINTER(CodecList), C.POINTER(BandDesc), C.POINTER(IcfDesc), C.c_int, C.c_void_p,
+                                          C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.POINTER(C.c_uint64)]
+        L.g4_decode_tiles_icf.argtypes = [C.c_void_p, C.POINTER(CodecList), C.POINTER(BandDesc), C.POINTER(IcfDesc), C.c_int, C.c_void_p,
+                                          C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.g4_fill_terrain.argtypes = [C.c_void_p, C.c_int, C.c_uint64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]
         L.g4_context_set_timing.argtypes = [C.c_void_p, C.c_int]
         L.g4_context_set_async.argtypes = [C.c_void_p, C.c_int]

@@ -13,7 +13,8 @@ import numpy as np
 
 from . import _lib
 from ._lib import (G4_CODEC_CANON_HUFFMAN, G4_CODEC_DEFLATE, G4_CODEC_FLOAT, G4_CODEC_HUFFMAN, G4_CODEC_LSOP08, G4_CODEC_LSOP12, G4_DECLINED,
-                   G4_ELEM_F32, G4_ELEM_I16, G4_ELEM_I32, G4_MEM_DEVICE, G4_MEM_HOST, G4_OK, BandDesc, CodecList, check)
+                   G4_ELEM_F32, G4_ELEM_I16, G4_ELEM_I32, G4_ELEM_ICF, G4_MEM_DEVICE, G4_MEM_HOST, G4_OK, BandDesc, CodecList, IcfDesc,
+                   check)
 
 from .stats import AnalysisMixin  # noqa: E402
 
@@ -300,13 +301,86 @@ class CodecSpecification:
         return cl
 
 
-class TileBatch:
-    """Result of CodecMaster.encodeTiles: payloads packed back to back (8-byte aligned) in `arena`."""
+class IntCodedFloat:
+    """The mapping of an integer-coded float element (GvrsElementIntCodedFloat): float values are stored as int codes,
+    code = floor((v - offset) * scale + 0.5), and read back as code / scale + offset; NaN <-> fill_int <-> fill_value.
+    The exact arithmetic is that of g4_icf_desc (include/g4codec.h).  The maps run on the GPU (g4_icf_map)."""
 
-    def __init__(self, arena, offsets, lens, codec, predictor, status, total_bytes, band):
+    def __init__(self, scale, offset=0.0, fill_int=INT4_NULL_CODE, fill_value=float("nan")):
+        self.scale, self.offset, self.fill_value = np.float32(scale), np.float32(offset), np.float32(fill_value)
+        self.fill_int = int(fill_int)
+        if not np.isfinite(self.scale) or self.scale == 0:
+            raise ValueError("integer-coded float: the scale must be finite and not zero")
+
+    def desc(self):
+        d = IcfDesc()
+        d.scale, d.offset, d.fill_int, d.fill_value = float(self.scale), float(self.offset), self.fill_int, float(self.fill_value)
+        return d
+
+    def __eq__(self, other):
+        return isinstance(other, IntCodedFloat) and (self.scale, self.offset, self.fill_int) == (other.scale, other.offset, other.fill_int) \
+            and self.fill_value.tobytes() == other.fill_value.tobytes()
+
+    def __repr__(self):
+        return "IntCodedFloat(scale=%r, offset=%r, fill_int=%d, fill_value=%r)" % (float(self.scale), float(self.offset), self.fill_int,
+                                                                                  float(self.fill_value))
+
+    def to_float(self, codes, out=None, context=None):
+        """int32 codes -> float32 values (numpy, or a torch CUDA tensor); `out` may be `codes` viewed as float32."""
+        return self._map(1, codes, out, np.int32, np.float32, context)
+
+    def to_int(self, values, out=None, context=None):
+        """float32 values -> int32 codes (numpy, or a torch CUDA tensor)."""
+        return self._map(0, values, out, np.float32, np.int32, context)
+
+    def _map(self, to_float, src, out, src_dt, dst_dt, context):
+        ctx = context or Context.default()
+        d = self.desc()
+        if isinstance(src, np.ndarray):
+            src = np.asarray(src, dtype=src_dt)
+            if src.ndim == 1:
+                src = src.reshape(1, -1)
+            out = np.empty(src.shape, dst_dt) if out is None else out
+            if out.dtype != dst_dt or out.shape != src.shape:
+                raise ValueError("out: %s of shape %s" % (np.dtype(dst_dt).name, src.shape))
+            sp, dp = _pitch(src.strides, src.itemsize), _pitch(out.strides, out.itemsize)
+            if src.size:
+                check(_lib.lib().g4_icf_map(ctx._h, to_float, C.byref(d), G4_MEM_HOST, src.shape[0], src.shape[1], src.ctypes.data, sp,
+                                            out.ctypes.data, dp), "g4_icf_map")
+            return out
+        import torch
+
+        tdt = {np.int32: torch.int32, np.float32: torch.float32}
+        if not (isinstance(src, torch.Tensor) and src.is_cuda and src.dtype == tdt[src_dt] and src.dim() == 2):
+            raise ValueError("a 2-D %s numpy array or CUDA tensor" % np.dtype(src_dt).name)
+        out = torch.empty(src.shape, dtype=tdt[dst_dt], device=src.device) if out is None else out
+        if out.dtype != tdt[dst_dt] or tuple(out.shape) != tuple(src.shape):
+            raise ValueError("out: %s of shape %s" % (np.dtype(dst_dt).name, tuple(src.shape)))
+        sp, dp = _pitch(tuple(4 * x for x in src.stride()), 4), _pitch(tuple(4 * x for x in out.stride()), 4)
+        if src.numel():
+            ctx.after_torch_stream(src.device)
+            st = _lib.lib().g4_icf_map(ctx._h, to_float, C.byref(d), G4_MEM_DEVICE, src.shape[0], src.shape[1], src.data_ptr(), sp,
+                                       out.data_ptr(), dp)
+            ctx.before_torch_stream(src.device)
+            check(st, "g4_icf_map")
+        return out
+
+
+def _pitch(strides, itemsize):
+    """Samples per row of a 2-D array whose rows are contiguous."""
+    if strides[1] != itemsize or strides[0] % itemsize or strides[0] < 0:
+        raise ValueError("rows must be contiguous, with a non-negative pitch that is a whole number of samples")
+    return strides[0] // itemsize
+
+
+class TileBatch:
+    """Result of CodecMaster.encodeTiles: payloads packed back to back (8-byte aligned) in `arena`.  `icf` is the
+    IntCodedFloat of a batch of integer-coded float tiles (its payloads hold the codes; decodeTiles returns float32)."""
+
+    def __init__(self, arena, offsets, lens, codec, predictor, status, total_bytes, band, icf=None):
         self.arena, self.offsets, self.lens = arena, offsets, lens
         self.codec, self.predictor, self.status = codec, predictor, status
-        self.total_bytes, self.band = total_bytes, band
+        self.total_bytes, self.band, self.icf = total_bytes, band, icf
 
     def payload(self, t):
         o, n = int(self.offsets[t]), int(self.lens[t])
@@ -373,17 +447,30 @@ class CodecMaster:
         b.grid_pitch = pitch or cols
         return b
 
-    def encodeTiles(self, grid, tileRows, tileCols, fillValue=None):
+    def _encode_call(self, icf):
+        """g4_encode_tiles, or g4_encode_tiles_icf with the descriptor of `icf` bound in."""
+        L = _lib.lib()
+        if icf is None:
+            return L.g4_encode_tiles, "g4_encode_tiles"
+        d = icf.desc()
+        return (lambda ctx, cl, band, *rest: L.g4_encode_tiles_icf(ctx, cl, band, C.byref(d), *rest)), "g4_encode_tiles_icf"
+
+    def encodeTiles(self, grid, tileRows, tileCols, fillValue=None, icf=None):
         """grid: 2-D numpy array (host path) or torch CUDA tensor (device path); int32, float32, or int16 (a short
-        element, TileElementShort: `fillValue` is coded as null, raw tiles take 2 bytes per sample)."""
+        element, TileElementShort: `fillValue` is coded as null, raw tiles take 2 bytes per sample).  With `icf` (an
+        IntCodedFloat) the float32 grid is an integer-coded float element: it is mapped to codes on the GPU and the codes are
+        encoded with the integer codecs; the batch remembers the mapping."""
         L = _lib.lib()
         cl = self.spec.native_list()
         total = C.c_uint64(0)
+        encode, name = self._encode_call(icf)
         if isinstance(grid, np.ndarray):
             g = np.ascontiguousarray(grid)
-            if g.dtype not in (np.int32, np.float32, np.int16):
-                raise ValueError("int32, float32 or int16 rasters only")
+            if g.dtype not in (np.int32, np.float32, np.int16) or (icf is not None and g.dtype != np.float32):
+                raise ValueError("int32, float32 or int16 rasters only (float32 for an integer-coded float element)")
             band = self._band(g.shape, g.dtype, tileRows, tileCols, fillValue=fillValue)
+            if icf is not None:
+                band.elem_type = G4_ELEM_ICF
             nT = band.tiles_down * band.tiles_across
             cap = int(L.g4_encode_arena_bound(C.byref(band)))
             arena = np.empty(cap, np.uint8)
@@ -392,17 +479,20 @@ class CodecMaster:
             codec = np.empty(nT, np.uint8)
             pred = np.empty(nT, np.uint8)
             status = np.empty(nT, np.int32)
-            st = L.g4_encode_tiles(self._context()._h, C.byref(cl), C.byref(band), G4_MEM_HOST, g.ctypes.data, arena.ctypes.data, cap,
-                                   offsets.ctypes.data, lens.ctypes.data, codec.ctypes.data, pred.ctypes.data, status.ctypes.data,
-                                   C.byref(total))
-            check(st, "g4_encode_tiles")
-            return TileBatch(arena[: total.value], offsets, lens, codec, pred, status, total.value, band)
+            st = encode(self._context()._h, C.byref(cl), C.byref(band), G4_MEM_HOST, g.ctypes.data, arena.ctypes.data, cap,
+                        offsets.ctypes.data, lens.ctypes.data, codec.ctypes.data, pred.ctypes.data, status.ctypes.data, C.byref(total))
+            check(st, name)
+            return TileBatch(arena[: total.value], offsets, lens, codec, pred, status, total.value, band, icf)
         import torch
 
         if not (isinstance(grid, torch.Tensor) and grid.is_cuda and grid.dim() == 2 and grid.is_contiguous()):
             raise ValueError("expected a contiguous 2-D CUDA tensor")
+        if icf is not None and grid.dtype != torch.float32:
+            raise ValueError("an integer-coded float element is encoded from a float32 tensor")
         npdt = np.float32 if grid.dtype == torch.float32 else np.int16 if grid.dtype == torch.int16 else np.int32
         band = self._band(tuple(grid.shape), npdt, tileRows, tileCols, fillValue=fillValue)
+        if icf is not None:
+            band.elem_type = G4_ELEM_ICF
         nT = band.tiles_down * band.tiles_across
         cap = int(L.g4_encode_arena_bound(C.byref(band)))
         dev = grid.device
@@ -414,12 +504,11 @@ class CodecMaster:
         status = torch.empty(nT, dtype=torch.int32, device=dev)
         ctx = self._context()
         ctx.after_torch_stream(dev)  # `grid` may come from kernels still queued on torch's stream
-        st = L.g4_encode_tiles(ctx._h, C.byref(cl), C.byref(band), G4_MEM_DEVICE, grid.data_ptr(), arena.data_ptr(), cap,
-                               offsets.data_ptr(), lens.data_ptr(), codec.data_ptr(), pred.data_ptr(), status.data_ptr(),
-                               C.byref(total))
+        st = encode(ctx._h, C.byref(cl), C.byref(band), G4_MEM_DEVICE, grid.data_ptr(), arena.data_ptr(), cap, offsets.data_ptr(),
+                    lens.data_ptr(), codec.data_ptr(), pred.data_ptr(), status.data_ptr(), C.byref(total))
         ctx.before_torch_stream(dev)
-        check(st, "g4_encode_tiles")
-        return TileBatch(arena, offsets, lens, codec, pred, status, total.value, band)
+        check(st, name)
+        return TileBatch(arena, offsets, lens, codec, pred, status, total.value, band, icf)
 
     # -- tile lists (new): scattered tiles of one size, each with its own {offset, pitch} -- the tile cache's calls -----
     @staticmethod
@@ -507,14 +596,18 @@ class CodecMaster:
         check(st, "g4_decode_tile_list")
         return base
 
-    def decodeImageTiles(self, image, payload_offsets, lens, status, tilesDown, tilesAcross, tileRows, tileCols, dtype, fillValue):
+    def decodeImageTiles(self, image, payload_offsets, lens, status, tilesDown, tilesAcross, tileRows, tileCols, dtype, fillValue,
+                         icf=None):
         """Decodes the tiles of a one-element raster whose payloads sit inside a GVRS file image (gvrs.GvrsImage.read_raster):
         the image is the arena of g4_decode_tiles.  Tiles the file does not hold (status G4_DECLINED) are pointed at one
-        raw tile of fill values appended to the arena (RasterTile.setToNullState)."""
+        raw tile of fill values appended to the arena (RasterTile.setToNullState).  With `icf` (an IntCodedFloat; dtype
+        int32, fillValue its fill_int) the codes are mapped and the raster comes back as float32."""
         from ._lib import G4_DECLINED
 
         band = self._band((tilesDown * tileRows, tilesAcross * tileCols), dtype, tileRows, tileCols,
                           fillValue=fillValue if np.dtype(dtype) == np.int16 else None)
+        if icf is not None:
+            band.elem_type = G4_ELEM_ICF
         arena = np.frombuffer(image, dtype=np.uint8) if not isinstance(image, np.ndarray) else image
         offsets = np.array(payload_offsets, dtype=np.uint64)
         lens = np.array(lens, dtype=np.uint32)
@@ -526,36 +619,46 @@ class CodecMaster:
             arena = np.concatenate([arena, np.zeros(base - arena.size, np.uint8), np.frombuffer(fill, dtype=np.uint8)])
             offsets[absent] = base
             lens[absent] = len(fill)
-        return self.decodeTiles(TileBatch(arena, offsets, lens, None, None, None, int(arena.size), band))
+        return self.decodeTiles(TileBatch(arena, offsets, lens, None, None, None, int(arena.size), band, icf))
+
+    def _decode_call(self, icf):
+        """g4_decode_tiles_bounded, or g4_decode_tiles_icf with the descriptor of `icf` bound in."""
+        L = _lib.lib()
+        if icf is None:
+            return L.g4_decode_tiles_bounded, "g4_decode_tiles"
+        d = icf.desc()
+        return (lambda ctx, cl, band, *rest: L.g4_decode_tiles_icf(ctx, cl, band, C.byref(d), *rest)), "g4_decode_tiles_icf"
 
     def decodeTiles(self, batch, out=None):
-        """Inverse of encodeTiles.  Returns the raster (numpy for host batches, torch for device batches)."""
-        L = _lib.lib()
+        """Inverse of encodeTiles.  Returns the raster (numpy for host batches, torch for device batches); float32 for a
+        batch of integer-coded float tiles (batch.icf)."""
         cl = self.spec.native_list()
         band = batch.band
         rows, cols = band.tiles_down * band.tile_rows, band.tiles_across * band.tile_cols
+        decode, name = self._decode_call(batch.icf)
+        f32 = band.elem_type in (G4_ELEM_F32, G4_ELEM_ICF)
         if isinstance(batch.arena, np.ndarray):
-            dt = np.float32 if band.elem_type == G4_ELEM_F32 else np.int16 if band.elem_type == G4_ELEM_I16 else np.int32
+            dt = np.float32 if f32 else np.int16 if band.elem_type == G4_ELEM_I16 else np.int32
             grid = out if out is not None else np.empty((rows, cols), dt)
             status = np.empty(band.tiles_down * band.tiles_across, np.int32)
             arena = np.ascontiguousarray(batch.arena)
             offsets = np.ascontiguousarray(batch.offsets, dtype=np.uint64)
             lens = np.ascontiguousarray(batch.lens, dtype=np.uint32)
-            st = L.g4_decode_tiles_bounded(self._context()._h, C.byref(cl), C.byref(band), G4_MEM_HOST, arena.ctypes.data, int(arena.size),
-                                           offsets.ctypes.data, lens.ctypes.data, grid.ctypes.data, status.ctypes.data)
+            st = decode(self._context()._h, C.byref(cl), C.byref(band), G4_MEM_HOST, arena.ctypes.data, int(arena.size), offsets.ctypes.data,
+                        lens.ctypes.data, grid.ctypes.data, status.ctypes.data)
             self.lastStatus = status
-            check(st, "g4_decode_tiles")
+            check(st, name)
             return grid
         import torch
 
-        dt = torch.float32 if band.elem_type == G4_ELEM_F32 else torch.int16 if band.elem_type == G4_ELEM_I16 else torch.int32
+        dt = torch.float32 if f32 else torch.int16 if band.elem_type == G4_ELEM_I16 else torch.int32
         grid = out if out is not None else torch.empty((rows, cols), dtype=dt, device=batch.arena.device)
         status = torch.empty(band.tiles_down * band.tiles_across, dtype=torch.int32, device=batch.arena.device)
         ctx = self._context()
         ctx.after_torch_stream(batch.arena.device)  # the payloads and `out` may still be in use on torch's stream
-        st = L.g4_decode_tiles_bounded(ctx._h, C.byref(cl), C.byref(band), G4_MEM_DEVICE, batch.arena.data_ptr(), int(batch.arena.numel()),
-                                       batch.offsets.data_ptr(), batch.lens.data_ptr(), grid.data_ptr(), status.data_ptr())
+        st = decode(ctx._h, C.byref(cl), C.byref(band), G4_MEM_DEVICE, batch.arena.data_ptr(), int(batch.arena.numel()),
+                    batch.offsets.data_ptr(), batch.lens.data_ptr(), grid.data_ptr(), status.data_ptr())
         ctx.before_torch_stream(batch.arena.device)
         self.lastStatus = status
-        check(st, "g4_decode_tiles")
+        check(st, name)
         return grid

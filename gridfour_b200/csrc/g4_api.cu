@@ -5,6 +5,7 @@
 //   TileElementInt.encode / decode            gvrs/TileElementInt.java:196-219
 // (paths under /root/reference/core/src/main/java/org/gridfour/).  No CPU compute path exists here:
 // every entry point launches CUDA kernels and fails with G4_ERR_CUDA when that is impossible.
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -109,6 +110,8 @@ struct g4_context {
   const int64_t* curTilePitch = nullptr;
   DevBuf tileRefs;      // device copy of the tile references of a tile-list call
   uint64_t arenaLimit = ~0ull;  // g4_decode_tiles_bounded: bytes addressable behind the arena of the running call
+  bool icfOn = false;           // g4_encode_tiles_icf / g4_decode_tiles_icf: the running call's band is G4_ELEM_ICF ...
+  g4::IcfMap icf{};             // ... mapped with this descriptor
   bool lsopDeflate = true;  // LsEncoder12.deflateEnabled (lsop/LsEncoder12.java:78)
   // staging used by the host-memory entry points
   DevBuf sGrid, sArena, sOffsets, sLens, sCodec, sPred, sStatus;
@@ -385,9 +388,10 @@ int launch_encoder(g4_context* ctx, int codecId, EncodeArgs& a, int nTiles) {
   return launch_encoder_impl(ctx, codecId, a, nTiles);
 }
 
-int check_band(const g4_band_desc* b) {
+int check_band(const g4_band_desc* b, bool icf = false) {  // icf: the band of a g4_*_tiles_icf call
   if (!b) return G4_ERR_ARG;
-  if (b->elem_type != G4_ELEM_I32 && b->elem_type != G4_ELEM_F32 && b->elem_type != G4_ELEM_I16) return G4_ERR_ARG;
+  if (icf ? b->elem_type != G4_ELEM_ICF : b->elem_type != G4_ELEM_I32 && b->elem_type != G4_ELEM_F32 && b->elem_type != G4_ELEM_I16)
+    return G4_ERR_ARG;
   if (b->tile_rows < 2 || b->tile_cols < 2) return G4_ERR_UNSUPPORTED;
   if (b->tiles_down < 1 || b->tiles_across < 1) return G4_ERR_ARG;
   if (int64_t(b->tile_rows) * b->tile_cols > (1 << 20)) return G4_ERR_UNSUPPORTED;
@@ -560,6 +564,15 @@ g4_band_desc widened(const g4_band_desc& b) {
 int encode_device(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, void* grid, uint8_t* arena,
                   uint64_t arenaCap, uint64_t* offsets, uint32_t* lens, uint8_t* codecOut, uint8_t* predOut, int32_t* status,
                   uint64_t* totalHost, size_t slotBytes) {
+  if (band->elem_type == G4_ELEM_ICF) {  // the float band is mapped to codes in the staging raster, which is then encoded
+    const g4_band_desc w = widened(*band);
+    const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = w.grid_pitch;
+    CK(ctx->wide.ensure(size_t(rows) * size_t(cols) * 4));
+    CK(launch_icf_map(0, grid, band->grid_pitch, ctx->wide.p, cols, rows, cols, ctx->icf, ctx->stream));
+    ctx->launches++;
+    return encode_device_i32(ctx, codecs, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
+                             nullptr, 0);
+  }
   if (band->elem_type != G4_ELEM_I16)
     return encode_device_i32(ctx, codecs, band, grid, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
                              nullptr, 0);
@@ -575,6 +588,16 @@ int encode_device(g4_context* ctx, const g4_codec_list* codecs, const g4_band_de
 
 int decode_device(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, const uint8_t* arena,
                   const uint64_t* offsets, const uint32_t* lens, void* grid, int32_t* status) {
+  if (band->elem_type == G4_ELEM_ICF) {  // codes are decoded into the caller's float raster (4 bytes per sample), then mapped in place
+    g4_band_desc w = *band;
+    w.elem_type = G4_ELEM_I32;
+    int rc = decode_device_i32(ctx, codecs, &w, arena, offsets, lens, grid, status, false);
+    if (rc != G4_OK) return rc;
+    const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = int64_t(band->tiles_across) * band->tile_cols;
+    CK(launch_icf_map(1, grid, band->grid_pitch, grid, band->grid_pitch, rows, cols, ctx->icf, ctx->stream));
+    ctx->launches++;
+    return G4_OK;
+  }
   if (band->elem_type != G4_ELEM_I16) return decode_device_i32(ctx, codecs, band, arena, offsets, lens, grid, status, false);
   const g4_band_desc w = widened(*band);
   const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = w.grid_pitch;
@@ -1079,7 +1102,7 @@ static int encode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
                              const g4_tile_ref* refs, uint8_t* arena, uint64_t arena_cap, uint64_t* offsets, uint32_t* lens,
                              uint8_t* codec_out, uint8_t* predictor_out, int32_t* status, uint64_t* total_bytes) {
   if (!ctx || !codecs || !grid || !arena || !offsets || !lens || !codec_out || !predictor_out || !status) return G4_ERR_ARG;
-  int rc = check_band(band);
+  int rc = check_band(band, ctx->icfOn);
   if (rc != G4_OK) return rc;
   if (codecs->n_codecs < 0 || codecs->n_codecs > G4_MAX_CODECS) return G4_ERR_ARG;
   ENTER(ctx);
@@ -1179,7 +1202,7 @@ int g4_encode_tile_list(g4_context* ctx, const g4_codec_list* codecs, int elem_t
 static int decode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, int mem_space, const uint8_t* arena,
                              const uint64_t* offsets, const uint32_t* lens, void* grid, const g4_tile_ref* refs, int32_t* status) {
   if (!ctx || !codecs || !grid || !arena || !offsets || !lens || !status) return G4_ERR_ARG;
-  int rc = check_band(band);
+  int rc = check_band(band, ctx->icfOn);
   if (rc != G4_OK) return rc;
   if (codecs->n_codecs < 0 || codecs->n_codecs > G4_MAX_CODECS) return G4_ERR_ARG;
   ENTER(ctx);
@@ -1324,6 +1347,53 @@ int g4_decode_tiles_bounded(g4_context* ctx, const g4_codec_list* codecs, const 
   const int rc = g4_decode_tiles(ctx, codecs, band, mem_space, arena, offsets, lens, grid, status);
   ctx->arenaLimit = ~0ull;
   return rc;
+}
+
+// ---- integer-coded float elements ------------------------------------------------------------------------------------
+static bool icf_valid(const g4_icf_desc* icf) { return icf && icf->scale != 0.0f && std::isfinite(icf->scale); }
+static g4::IcfMap icf_of(const g4_icf_desc* icf) { return g4::IcfMap{icf->scale, icf->offset, icf->fill_int, icf->fill_value}; }
+struct IcfScope {  // the descriptor is valid for one call only
+  g4_context* c;
+  IcfScope(g4_context* ctx, const g4_icf_desc* icf) : c(ctx) { c->icfOn = true; c->icf = icf_of(icf); }
+  ~IcfScope() { c->icfOn = false; c->icf = g4::IcfMap{}; }
+};
+
+int g4_icf_map(g4_context* ctx, int to_float, const g4_icf_desc* icf, int mem_space, int64_t n_rows, int64_t n_cols, const void* src,
+               int64_t src_pitch, void* dst, int64_t dst_pitch) {
+  if (!ctx || !icf_valid(icf) || !src || !dst || n_rows < 1 || n_cols < 1 || src_pitch < n_cols || dst_pitch < n_cols) return G4_ERR_ARG;
+  ENTER(ctx);
+  const g4::IcfMap m = icf_of(icf);
+  if (mem_space == G4_MEM_DEVICE) {
+    CK(launch_icf_map(to_float, src, src_pitch, dst, dst_pitch, n_rows, n_cols, m, ctx->stream));
+    ctx->launches++;
+    return G4_OK;
+  }
+  if (mem_space != G4_MEM_HOST) return G4_ERR_ARG;
+  const size_t rowBytes = size_t(n_cols) * 4;
+  CK(ctx->sGrid.ensure(rowBytes * size_t(n_rows)));
+  CK(cudaMemcpy2DAsync(ctx->sGrid.p, rowBytes, src, size_t(src_pitch) * 4, rowBytes, size_t(n_rows), cudaMemcpyHostToDevice, ctx->stream));
+  CK(launch_icf_map(to_float, ctx->sGrid.p, n_cols, ctx->sGrid.p, n_cols, n_rows, n_cols, m, ctx->stream));
+  ctx->launches++;
+  CK(cudaMemcpy2DAsync(dst, size_t(dst_pitch) * 4, ctx->sGrid.p, rowBytes, rowBytes, size_t(n_rows), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return G4_OK;
+}
+
+int g4_encode_tiles_icf(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, const g4_icf_desc* icf, int mem_space,
+                        const float* grid, uint8_t* arena, uint64_t arena_cap, uint64_t* offsets, uint32_t* lens, uint8_t* codec_out,
+                        uint8_t* predictor_out, int32_t* status, uint64_t* total_bytes) {
+  if (!ctx || !band || band->elem_type != G4_ELEM_ICF || !icf_valid(icf)) return G4_ERR_ARG;
+  IcfScope scope(ctx, icf);
+  return encode_tiles_impl(ctx, codecs, band, mem_space, grid, nullptr, arena, arena_cap, offsets, lens, codec_out, predictor_out, status,
+                           total_bytes);
+}
+
+int g4_decode_tiles_icf(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, const g4_icf_desc* icf, int mem_space,
+                        const uint8_t* arena, uint64_t arena_len, const uint64_t* offsets, const uint32_t* lens, float* grid,
+                        int32_t* status) {
+  if (!ctx || !band || band->elem_type != G4_ELEM_ICF || !icf_valid(icf)) return G4_ERR_ARG;
+  IcfScope scope(ctx, icf);
+  return g4_decode_tiles_bounded(ctx, codecs, band, mem_space, arena, arena_len, offsets, lens, grid, status);
 }
 
 // ---- per-tile entry points: one-tile bands through the same kernels --------------------------------

@@ -198,6 +198,58 @@ __global__ void narrow_i16_kernel(const int32_t* src, int16_t* dst, int64_t dstP
   }
 }
 
+// Integer-coded float elements (GvrsElementSpecificationIntCodedFloat / GvrsElementIntCodedFloat).  The reference source
+// is not in this tree; these are the formulas as the ICF feature request restates them (the oracle's g4o_icf.cpp states
+// them once more).  No reference fixture pins them beyond exactly representable values.
+//   float -> code: NaN -> fillInt; else (int) Math.floor((double)((v - offset) * scale) + 0.5): float32 subtract and multiply,
+//                  correctly rounded and not fused, + 0.5 and floor in double, Java's saturating (int) cast (NaN -> 0),
+//                  which is what PTX cvt.rzi.s32.f64 does.
+//   code -> float: fillInt -> fillValue; else (float) code / scale + offset in float32, with a true IEEE division.
+__device__ __forceinline__ int32_t icf_code(float v, const IcfMap& m) {
+  if (v != v) return m.fillInt;
+  return __double2int_rz(floor(__dadd_rn(double(__fmul_rn(__fsub_rn(v, m.offset), m.scale)), 0.5)));
+}
+__device__ __forceinline__ float icf_value(int32_t k, const IcfMap& m) {
+  return k == m.fillInt ? m.fillValue : __fadd_rn(__fdiv_rn(__int2float_rn(k), m.scale), m.offset);
+}
+__device__ __forceinline__ int32_t icf_apply(float v, const IcfMap& m) { return icf_code(v, m); }
+__device__ __forceinline__ float icf_apply(int32_t k, const IcfMap& m) { return icf_value(k, m); }
+
+// One pass over a pitched rows x cols rectangle (pitches in samples); src and dst may be the same buffer.  Each thread maps
+// four consecutive cells of a row: with one 16-byte load and store where both row starts are 16-byte aligned, cell by cell
+// otherwise (pitches or offsets that are not multiples of 4, and the last partial quad of a row).  blockDim = (bx, 256 / bx)
+// with bx sized to the row, so that narrow rectangles keep the threads busy; no division per cell.
+template <class S, class D, class S4, class D4>
+__device__ __forceinline__ void icf_map_rect(const S* src, int64_t srcPitch, D* dst, int64_t dstPitch, int64_t rows, int64_t cols,
+                                             const IcfMap& m) {
+  const int64_t c = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) * 4;
+  if (c >= cols) return;
+  for (int64_t r = int64_t(blockIdx.y) * blockDim.y + threadIdx.y; r < rows; r += int64_t(gridDim.y) * blockDim.y) {
+    const S* s = src + r * srcPitch + c;
+    D* d = dst + r * dstPitch + c;
+    if (c + 4 <= cols && ((reinterpret_cast<uintptr_t>(s) | reinterpret_cast<uintptr_t>(d)) & 15) == 0) {
+      const S4 x = *reinterpret_cast<const S4*>(s);
+      D4 y;
+      y.x = icf_apply(x.x, m);
+      y.y = icf_apply(x.y, m);
+      y.z = icf_apply(x.z, m);
+      y.w = icf_apply(x.w, m);
+      *reinterpret_cast<D4*>(d) = y;
+    } else {
+      const int k = cols - c < 4 ? int(cols - c) : 4;
+      for (int i = 0; i < k; i++) d[i] = icf_apply(s[i], m);
+    }
+  }
+}
+__global__ void __launch_bounds__(256) icf_to_int_kernel(const float* src, int64_t srcPitch, int32_t* dst, int64_t dstPitch, int64_t rows,
+                                                         int64_t cols, IcfMap m) {
+  icf_map_rect<float, int32_t, float4, int4>(src, srcPitch, dst, dstPitch, rows, cols, m);
+}
+__global__ void __launch_bounds__(256) icf_to_float_kernel(const int32_t* src, int64_t srcPitch, float* dst, int64_t dstPitch,
+                                                           int64_t rows, int64_t cols, IcfMap m) {
+  icf_map_rect<int32_t, float, int4, float4>(src, srcPitch, dst, dstPitch, rows, cols, m);
+}
+
 cudaError_t launch_fill_terrain(int elemType, uint64_t seed, int64_t row0, int64_t col0, int64_t nRows, int64_t nCols, void* out,
                                 cudaStream_t s) {
   fill_terrain_kernel<<<148 * 8, 256, 0, s>>>(elemType, seed, row0, col0, nRows, nCols, out);
@@ -209,6 +261,21 @@ cudaError_t launch_widen_i16(const int16_t* src, int64_t srcPitch, int32_t* dst,
 }
 cudaError_t launch_narrow_i16(const int32_t* src, int16_t* dst, int64_t dstPitch, int64_t rows, int64_t cols, cudaStream_t s) {
   narrow_i16_kernel<<<148 * 8, 256, 0, s>>>(src, dst, dstPitch, rows, cols);
+  return cudaGetLastError();
+}
+cudaError_t launch_icf_map(int toFloat, const void* src, int64_t srcPitch, void* dst, int64_t dstPitch, int64_t rows, int64_t cols,
+                           const IcfMap& m, cudaStream_t s) {
+  const int64_t quads = (cols + 3) / 4;
+  int bx = 1;
+  while (bx < 256 && bx < quads) bx <<= 1;
+  const dim3 block(bx, 256 / bx);
+  const int64_t gx = (quads + bx - 1) / bx, gy = (rows + block.y - 1) / block.y;
+  if (gx > 0x7fffffff) return cudaErrorInvalidValue;
+  const dim3 grid(unsigned(gx), unsigned(gy < 65535 ? gy : 65535));
+  if (toFloat)
+    icf_to_float_kernel<<<grid, block, 0, s>>>(static_cast<const int32_t*>(src), srcPitch, static_cast<float*>(dst), dstPitch, rows, cols, m);
+  else
+    icf_to_int_kernel<<<grid, block, 0, s>>>(static_cast<const float*>(src), srcPitch, static_cast<int32_t*>(dst), dstPitch, rows, cols, m);
   return cudaGetLastError();
 }
 cudaError_t launch_select(const SelectArgs& a, cudaStream_t s) {

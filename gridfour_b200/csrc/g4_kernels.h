@@ -148,6 +148,15 @@ cudaError_t launch_raw_decode(const DecodeArgs& a, int nTiles, cudaStream_t s);
 // TileElementShort (gvrs/TileElementShort.java:211-248): int16 raster <-> the int32 raster the codecs work on
 cudaError_t launch_widen_i16(const int16_t* src, int64_t srcPitch, int32_t* dst, int64_t rows, int64_t cols, int32_t fill, cudaStream_t s);
 cudaError_t launch_narrow_i16(const int32_t* src, int16_t* dst, int64_t dstPitch, int64_t rows, int64_t cols, cudaStream_t s);
+// Integer-coded float elements: float32 <-> int32 codes over a pitched rectangle (pitches in samples; src may equal dst).
+// toFloat != 0 runs icf_to_float_kernel (codes -> values), else icf_to_int_kernel (values -> codes).
+struct IcfMap {
+  float scale, offset;
+  int32_t fillInt;
+  float fillValue;
+};
+cudaError_t launch_icf_map(int toFloat, const void* src, int64_t srcPitch, void* dst, int64_t dstPitch, int64_t rows, int64_t cols,
+                           const IcfMap& m, cudaStream_t s);
 
 // ---- codec kernels -----------------------------------------------------------------------------
 // Host-side launchers (defined next to their kernels).  nCtas persistent CTAs of kThreads threads.

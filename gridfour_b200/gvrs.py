@@ -91,6 +91,46 @@ class ElementSpec:
     def floating(name, min_value=-3.4028235e38, max_value=3.4028235e38, fill_value=float("nan"), **kw):
         return ElementSpec(ELEM_FLOAT, name, range_block=struct.pack("<fff", min_value, max_value, fill_value), **kw)
 
+    @staticmethod
+    def int_coded_float(name, scale, offset=0.0, min_value=None, max_value=None, fill_value=float("nan"), **kw):
+        """GvrsElementSpecificationIntCodedFloat.  The range block is [min f32][max f32][fill f32][scale f32][offset f32]
+        [iMin][iMax][iFill]: with min and max given, the int bounds are their codes; without them, the int bounds are
+        +-(2^31 - 1) and the float bounds are the values of those codes.  A NaN fill is coded as INT4_NULL_CODE.  (Header
+        metadata computed with numpy float32 / float64 in the arithmetic of g4_icf_desc; sample data is mapped on the GPU.)"""
+        f32 = np.float32
+        scale, offset, fill = f32(scale), f32(offset), f32(fill_value)
+        if not np.isfinite(scale) or scale == 0:
+            raise ValueError("integer-coded float: the scale must be finite and not zero")
+
+        def code(v):
+            with np.errstate(invalid="ignore", over="ignore"):
+                d = np.floor(np.float64((f32(v) - offset) * scale) + 0.5)
+            return 0 if np.isnan(d) else int(min(max(d, -2.0 ** 31), 2.0 ** 31 - 1))
+
+        def value(k):
+            return (f32(k) / scale) + offset
+
+        if (min_value is None) != (max_value is None):
+            raise ValueError("integer-coded float: give both min_value and max_value, or neither")
+        if min_value is None:
+            i_min, i_max = -(2 ** 31) + 1, 2 ** 31 - 1
+            min_value, max_value = value(i_min), value(i_max)
+        else:
+            i_min, i_max = code(min_value), code(max_value)
+        i_fill = -(2 ** 31) if np.isnan(fill) else code(fill)
+        block = np.array([min_value, max_value, fill, scale, offset], "<f4").tobytes() + struct.pack("<iii", i_min, i_max, i_fill)
+        return ElementSpec(ELEM_INT_CODED_FLOAT, name, range_block=block, **kw)
+
+    @property
+    def icf(self):
+        """The IntCodedFloat of an integer-coded float element (None for the other types)."""
+        if self.type_code != ELEM_INT_CODED_FLOAT:
+            return None
+        from .codecs import IntCodedFloat
+
+        fill, scale, offset = np.frombuffer(self.range_block, "<f4", 3, 8)
+        return IntCodedFloat(scale, offset, struct.unpack_from("<i", self.range_block, 28)[0], fill)
+
     def standard_size(self, n_cells):
         n = n_cells * _ELEM_BYTES[self.type_code]
         return (n + 3) & ~3  # TileElement.java:89-93: the 2-byte form is padded to a multiple of 4
@@ -288,26 +328,27 @@ class GvrsImage:
         payload_off, lens, status = self._locate_all(ctx, verify)
         return payload_off[element], lens[element], status
 
-    def _decode_element(self, master, element, payload_off, lens, status, crop):
+    def _decode_element(self, master, element, payload_off, lens, status, crop, as_float):
         spec = self.spec
         e = spec.elements[element]
         grid = master.decodeImageTiles(self.image, payload_off, lens, status, spec.tiles_down, spec.tiles_across, spec.tile_rows,
-                                       spec.tile_cols, _ELEM_DTYPE[e.type_code], e.fill_value)
+                                       spec.tile_cols, _ELEM_DTYPE[e.type_code], e.fill_value, icf=e.icf if as_float else None)
         return grid[:spec.n_rows, :spec.n_cols] if crop else grid
 
-    def read_raster(self, master, element=0, verify=True, crop=False):
+    def read_raster(self, master, element=0, verify=True, crop=False, as_float=False):
         """crop=True returns the n_rows x n_cols raster without the fill-valued margin of the edge tiles.
         Decodes every tile of one element of the raster on the GPU straight from the file image: the image is the arena
         of g4_decode_tiles; locate_payloads finds the payloads.  Tiles that are absent from the file come back filled with
-        the element's fill value (RasterTile.setToNullState)."""
+        the element's fill value (RasterTile.setToNullState).  An integer-coded float element comes back as its int codes,
+        or with as_float=True as float32 values (g4_decode_tiles_icf); as_float changes nothing for the other types."""
         payload_off, lens, status = self.locate_payloads(master._context(), element, verify)
-        return self._decode_element(master, element, payload_off, lens, status, crop)
+        return self._decode_element(master, element, payload_off, lens, status, crop, as_float)
 
-    def read_rasters(self, master, verify=True, crop=False):
+    def read_rasters(self, master, verify=True, crop=False, as_float=False):
         """Every element's raster, in specification order, from one validation + location call (read_raster per element
         would repeat it)."""
         payload_off, lens, status = self._locate_all(master._context(), verify)
-        return [self._decode_element(master, k, payload_off[k], lens[k], status, crop) for k in range(len(self.spec.elements))]
+        return [self._decode_element(master, k, payload_off[k], lens[k], status, crop, as_float) for k in range(len(self.spec.elements))]
 
 
 # ---- GPU-backed primitives -------------------------------------------------------------------------------------------
@@ -602,15 +643,22 @@ class GvrsWriter:
     def _encode_element(self, master, e, grid):
         """encodeTiles of one element's raster (numpy, n_rows x n_cols): the cells of the edge tiles that lie outside the
         raster hold the element's fill value, as a RasterTile that was never written there does (TileElementInt/Float/Short
-        constructors fill the tile)."""
+        constructors fill the tile).  A float32 raster of an integer-coded float element holds values, which are mapped to
+        codes on the GPU (the margin is filled with the float fill value first); an int32 raster holds the codes."""
         spec = self.spec
-        full = np.full((spec.tiles_down * spec.tile_rows, spec.tiles_across * spec.tile_cols), e.fill_value, dtype=_ELEM_DTYPE[e.type_code])
+        shape = (spec.tiles_down * spec.tile_rows, spec.tiles_across * spec.tile_cols)
+        if e.type_code == ELEM_INT_CODED_FLOAT and np.asarray(grid).dtype == np.float32:
+            icf = e.icf
+            full = np.full(shape, icf.fill_value, dtype=np.float32)
+            full[:spec.n_rows, :spec.n_cols] = grid
+            return master.encodeTiles(full, spec.tile_rows, spec.tile_cols, icf=icf)
+        full = np.full(shape, e.fill_value, dtype=_ELEM_DTYPE[e.type_code])
         full[:spec.n_rows, :spec.n_cols] = grid
         return master.encodeTiles(full, spec.tile_rows, spec.tile_cols, fillValue=e.fill_value if e.type_code == ELEM_SHORT else None)
 
     def add_raster(self, master, grid):
         """A whole one-element raster (numpy, n_rows x n_cols): encodeTiles on the GPU, then the tile records.  Returns the
-        TileBatch."""
+        TileBatch.  For an integer-coded float element, a float32 raster holds values and an int32 raster holds codes."""
         spec = self.spec
         if len(spec.elements) != 1 or grid.shape != (spec.n_rows, spec.n_cols):
             raise ValueError("add_raster: a one-element raster of the specified dimensions")
@@ -620,8 +668,9 @@ class GvrsWriter:
 
     def add_rasters(self, master, grids):
         """Every element of a raster: grids[k] (numpy, n_rows x n_cols) is element k in specification order -- int32 for
-        integer and integer-coded-float elements, float32, int16 for short elements.  One encodeTiles per element, then one
-        multi-element framing call.  Returns the TileBatch of every element."""
+        integer elements, float32 for float elements, int16 for short elements, and for integer-coded float elements float32
+        values or int32 codes.  One encodeTiles per element, then one multi-element framing call.  Returns the TileBatch of
+        every element."""
         spec = self.spec
         if len(grids) != len(spec.elements) or any(np.shape(g) != (spec.n_rows, spec.n_cols) for g in grids):
             raise ValueError("add_rasters: one raster of the specified dimensions per element")

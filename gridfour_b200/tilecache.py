@@ -8,7 +8,9 @@ Reference call pattern (paths under /root/reference/core/src/main/java/org/gridf
 Here a block read first works out which tiles of the window are missing and decodes ALL of them with one
 g4_decode_tile_list call, straight into their cache slots (each slot is its own small raster: the {offset, pitch} tile
 references exist for exactly this); flush() encodes all dirty slots with one g4_encode_tile_list call.  The read-ahead
-thread of the reference has no counterpart: a whole window costs one launch set."""
+thread of the reference has no counterpart: a whole window costs one launch set.
+Integer-coded float elements keep their int codes in the slots, as TileElementIntCodedFloat does; readBlockFloat /
+writeBlockFloat map a block at the accessor with g4_icf_map."""
 from collections import OrderedDict
 
 import numpy as np
@@ -26,6 +28,7 @@ class RasterTileCache:
         if e.type_code == ELEM_SHORT:
             raise ValueError("short elements: use GvrsImage.read_raster (their widening pass works on a rectangle)")
         self.fill = e.fill_value
+        self.icf = e.icf   # IntCodedFloat of an integer-coded float element, else None
         self.dtype = np.float32 if e.type_code == ELEM_FLOAT else np.int32
         self.R, self.C = spec.tile_rows, spec.tile_cols
         self.max_tiles = int(max_tiles)
@@ -104,6 +107,19 @@ class RasterTileCache:
     def readValue(self, row, col):
         return self.readBlock(row, col, 1, 1)[0, 0]
 
+    def _icf(self):
+        if self.icf is None:
+            raise ValueError("readBlockFloat / writeBlockFloat: an integer-coded float element")
+        return self.icf
+
+    def readBlockFloat(self, row, col, nRows, nColumns):
+        """The values of an integer-coded float element (float32): readBlock's codes mapped on the GPU."""
+        icf = self._icf()
+        return icf.to_float(self.readBlock(row, col, nRows, nColumns), context=self.master._context())
+
+    def readValueFloat(self, row, col):
+        return self.readBlockFloat(row, col, 1, 1)[0, 0]
+
     # ---- writes: GvrsElement.writeBlock / writeValue, RasterTileCache.flush (:286-294) -----------------------------------
     def writeBlock(self, row, col, block):
         block = np.asarray(block, dtype=self.dtype)
@@ -119,6 +135,11 @@ class RasterTileCache:
 
     def writeValue(self, row, col, value):
         self.writeBlock(row, col, np.array([[value]], dtype=self.dtype))
+
+    def writeBlockFloat(self, row, col, block):
+        """Values of an integer-coded float element: mapped to codes on the GPU, then written as writeBlock does."""
+        icf = self._icf()
+        self.writeBlock(row, col, icf.to_int(np.asarray(block, dtype=np.float32), context=self.master._context()))
 
     def flush(self):
         """Encodes every dirty tile with ONE batched call (best-of over the codec list, raw fallback) and remembers the

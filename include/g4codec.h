@@ -63,7 +63,7 @@ enum { G4_PRED_NONE = 0, G4_PRED_DIFFERENCING = 1, G4_PRED_LINEAR = 2, G4_PRED_T
 /* Sample types of a raster.  G4_ELEM_I16 mirrors TileElementShort (C/gvrs/TileElementShort.java:211-248): samples are
  * widened to int for the codecs with fill_value -> INT4_NULL_CODE, a decoded INT4_NULL_CODE comes back as
  * SHORT_NULL_CODE (-32768), and the raw form is 2 bytes per sample rounded up to a multiple of 4 (TileElement.java:85-93). */
-enum { G4_ELEM_I32 = 0, G4_ELEM_F32 = 1, G4_ELEM_I16 = 2 };
+enum { G4_ELEM_I32 = 0, G4_ELEM_F32 = 1, G4_ELEM_I16 = 2, G4_ELEM_ICF = 3 };
 enum { G4_MEM_HOST = 0, G4_MEM_DEVICE = 1 };
 
 #define G4_MAX_CODECS 16
@@ -82,7 +82,7 @@ typedef struct {
  * Tile t = tr * tiles_across + tc covers rows [tr*tile_rows, ...) and cols [tc*tile_cols, ...) of the
  * buffer passed as `grid` (whose first sample is the band's upper-left cell). */
 typedef struct {
-  int32_t elem_type; /* G4_ELEM_I32, G4_ELEM_F32 or G4_ELEM_I16 */
+  int32_t elem_type; /* G4_ELEM_I32, G4_ELEM_F32 or G4_ELEM_I16 (G4_ELEM_ICF: the *_icf calls only) */
   int32_t tile_rows, tile_cols;
   int32_t tiles_down, tiles_across;
   int64_t grid_pitch; /* samples per raster row (>= tiles_across*tile_cols); a band may sit inside a wider raster:
@@ -170,6 +170,37 @@ int g4_decode_tiles(g4_context* ctx, const g4_codec_list* codecs, const g4_band_
 int g4_decode_tiles_bounded(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, int mem_space,
                             const uint8_t* arena, uint64_t arena_len, const uint64_t* offsets, const uint32_t* lens,
                             void* grid, int32_t* status);
+
+/* ---- integer-coded float elements (GvrsElementSpecificationIntCodedFloat / GvrsElementIntCodedFloat) -------------------
+ * An ICF element stores float values as int codes and its tiles go through the integer codecs untouched, like
+ * TileElementInt: raw tiles are the int32 codes (4 bytes per sample), and a fill_int of INT4_NULL_CODE is the null code the
+ * predictors know.  The mapping (no reference fixture pins it beyond exactly representable values):
+ *   float -> code: NaN -> fill_int; else (int) Math.floor((double)((v - offset) * scale) + 0.5) -- the subtraction and the
+ *                  multiplication in float32, correctly rounded and not fused, + 0.5 and floor in double, Java's saturating
+ *                  (int) cast.  A finite value whose code is fill_int (-inf with the default fill) reads back as fill_value.
+ *   code -> float: fill_int -> fill_value; else (float) code / scale + offset in float32 (a true IEEE division).
+ * A NULL descriptor, or a scale that is 0 or not finite: G4_ERR_ARG. */
+typedef struct {
+  float scale;
+  float offset;
+  int32_t fill_int;
+  float fill_value;
+} g4_icf_desc;
+/* One rectangle of n_rows x n_cols samples, pitches in samples; to_float != 0 maps codes (int32) to values (float32), else
+ * values to codes.  src and dst may be the same buffer.  G4_MEM_DEVICE: one kernel on the context's stream (the result is
+ * complete on that stream); G4_MEM_HOST: staged through the device, complete on return. */
+int g4_icf_map(g4_context* ctx, int to_float, const g4_icf_desc* icf, int mem_space, int64_t n_rows, int64_t n_cols, const void* src,
+               int64_t src_pitch, void* dst, int64_t dst_pitch);
+/* g4_encode_tiles / g4_decode_tiles_bounded of an ICF band (band->elem_type == G4_ELEM_ICF; band->fill_value is ignored).
+ * Encode maps the float32 band to codes and encodes those (the integer codecs; GvrsFloat in the list is skipped).  Decode
+ * decodes the codes into `grid` and maps them to float32 in place, the band's columns only; with g4_context_set_async it
+ * only enqueues, as g4_decode_tiles does.  The other band calls reject G4_ELEM_ICF with G4_ERR_ARG. */
+int g4_encode_tiles_icf(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, const g4_icf_desc* icf, int mem_space,
+                        const float* grid, uint8_t* arena, uint64_t arena_cap, uint64_t* offsets, uint32_t* lens, uint8_t* codec_out,
+                        uint8_t* predictor_out, int32_t* status, uint64_t* total_bytes);
+int g4_decode_tiles_icf(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, const g4_icf_desc* icf, int mem_space,
+                        const uint8_t* arena, uint64_t arena_len, const uint64_t* offsets, const uint32_t* lens, float* grid,
+                        int32_t* status);
 
 /* ---- tile LISTS: scattered tiles of one size (the tile cache's callers) -------------------------------------------------
  * The band calls above take one rectangle of one raster.  A tile cache flushes whatever tiles are dirty, each in its own
