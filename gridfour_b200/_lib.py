@@ -13,6 +13,7 @@ G4_OK, G4_DECLINED, G4_CHECKSUM_MISMATCH = 0, 1, 2
 G4_ERR_ARG, G4_ERR_FORMAT, G4_ERR_CAPACITY, G4_ERR_CUDA, G4_ERR_UNSUPPORTED = -1, -2, -3, -4, -5
 G4_CODEC_HUFFMAN, G4_CODEC_DEFLATE, G4_CODEC_FLOAT, G4_CODEC_CANON_HUFFMAN, G4_CODEC_LSOP12 = 0, 1, 2, 3, 4
 G4_CODEC_LSOP08 = 5
+G4_LSOP12_NO_DEFLATE, G4_LSOP12_VALUE_CHECKSUM = 1 << 8, 1 << 9  # option bits of an LSOP12 codec entry
 G4_ELEM_I32, G4_ELEM_F32, G4_ELEM_I16, G4_ELEM_ICF = 0, 1, 2, 3
 G4_MEM_HOST, G4_MEM_DEVICE = 0, 1
 G4_MAX_CODECS = 16

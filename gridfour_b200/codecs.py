@@ -13,8 +13,8 @@ import numpy as np
 
 from . import _lib
 from ._lib import (G4_CODEC_CANON_HUFFMAN, G4_CODEC_DEFLATE, G4_CODEC_FLOAT, G4_CODEC_HUFFMAN, G4_CODEC_LSOP08, G4_CODEC_LSOP12, G4_DECLINED,
-                   G4_ELEM_F32, G4_ELEM_I16, G4_ELEM_I32, G4_ELEM_ICF, G4_MEM_DEVICE, G4_MEM_HOST, G4_OK, BandDesc, CodecList, IcfDesc,
-                   check)
+                   G4_ELEM_F32, G4_ELEM_I16, G4_ELEM_I32, G4_ELEM_ICF, G4_LSOP12_NO_DEFLATE, G4_LSOP12_VALUE_CHECKSUM, G4_MEM_DEVICE,
+                   G4_MEM_HOST, G4_OK, BandDesc, CodecList, IcfDesc, check)
 
 from .stats import AnalysisMixin  # noqa: E402
 
@@ -105,6 +105,10 @@ class ICompressionEncoder:
     def _context(self):
         return self._ctx or Context.default()
 
+    def native_id(self):
+        """The codec id this instance passes to the library, with its option bits (include/g4codec.h)."""
+        return self.codec_id
+
     def implementsIntegerEncoding(self):
         return self.codec_id != G4_CODEC_FLOAT
 
@@ -122,7 +126,7 @@ class ICompressionEncoder:
         out = np.empty(cap, np.uint8)
         n = C.c_size_t(0)
         pred = C.c_int(0)
-        st = _lib.lib().g4_encode_i32(self._context()._h, self.codec_id, int(codecIndex), int(nRows), int(nCols), v.ctypes.data,
+        st = _lib.lib().g4_encode_i32(self._context()._h, self.native_id(), int(codecIndex), int(nRows), int(nCols), v.ctypes.data,
                                       out.ctypes.data, cap, C.byref(n), C.byref(pred))
         if st == G4_DECLINED:
             return None
@@ -224,8 +228,32 @@ class CodecCanonHuffman(_Codec):
 
 
 class LsEncoder12(ICompressionEncoder):
-    """lsop/LsEncoder12.java"""
+    """lsop/LsEncoder12.java, with its two switches (:93-119): the Deflate alternative (on by default) and the value
+    checksum (off by default)."""
     codec_id = G4_CODEC_LSOP12
+
+    def __init__(self, context=None):
+        super().__init__(context)
+        self.deflateEnabled = True
+        self.valueChecksumEnabled = False
+
+    def setDeflateEnabled(self, deflateEnabled):
+        """False: every packing is the canonical-Huffman form; the Deflate alternative is not tried."""
+        self.deflateEnabled = bool(deflateEnabled)
+
+    def isDeflateEnabled(self):
+        return self.deflateEnabled
+
+    def setValueChecksumEnabled(self, valueChecksumEnabled):
+        """True: every packing carries the CRC-32C of the tile's values, which the decoder checks."""
+        self.valueChecksumEnabled = bool(valueChecksumEnabled)
+
+    def isValueChecksumEnabled(self):
+        return self.valueChecksumEnabled
+
+    def native_id(self):
+        return self.codec_id | (0 if self.deflateEnabled else G4_LSOP12_NO_DEFLATE) | (
+            G4_LSOP12_VALUE_CHECKSUM if self.valueChecksumEnabled else 0)
 
 
 class LsDecoder12(ICompressionDecoder):
@@ -399,6 +427,22 @@ class CodecMaster:
     def _context(self):
         return self._ctx or Context.default()
 
+    def getEncoder(self, codecID):
+        """The encoder instance this master encodes with for the codec named codecID (e.g. "LSOP12"), so that its options
+        can be set; None when the list has no such codec."""
+        for (cid, _e, _d), enc in zip(self.spec.codecList, self._enc):
+            if cid == codecID:
+                return enc
+        return None
+
+    def _native_list(self):
+        """The codec list of the native calls, taken from this master's encoder instances (with their option bits)."""
+        cl = CodecList()
+        cl.n_codecs = len(self._enc)
+        for k, enc in enumerate(self._enc):
+            cl.codec_ids[k] = enc.native_id()
+        return cl
+
     # -- per tile, exactly CodecMaster.encodeSingleThread / decode ---------------------------------------
     def encode(self, nRows, nCols, values):
         result = None
@@ -461,7 +505,7 @@ class CodecMaster:
         IntCodedFloat) the float32 grid is an integer-coded float element: it is mapped to codes on the GPU and the codes are
         encoded with the integer codecs; the batch remembers the mapping."""
         L = _lib.lib()
-        cl = self.spec.native_list()
+        cl = self._native_list()
         total = C.c_uint64(0)
         encode, name = self._encode_call(icf)
         if isinstance(grid, np.ndarray):
@@ -525,7 +569,7 @@ class CodecMaster:
         first element (RasterTileCache.flush: whatever tiles are dirty, gvrs/RasterTileCache.java:286-294).  Returns a
         TileBatch whose tile t is list position t."""
         L = _lib.lib()
-        cl = self.spec.native_list()
+        cl = self._native_list()
         n = len(refs)
         total = C.c_uint64(0)
         tiles = self._refs(refs)
@@ -567,7 +611,7 @@ class CodecMaster:
         buffers in the same memory space).  RasterTileCache.readTileUsingAssistant / a bulk readBlock
         (gvrs/RasterTileCache.java:339-426, gvrs/GvrsElement.java:298-404): every missing tile of a window in one call."""
         L = _lib.lib()
-        cl = self.spec.native_list()
+        cl = self._native_list()
         n = len(refs)
         tiles = self._refs(refs)
         if isinstance(base, np.ndarray):
@@ -632,7 +676,7 @@ class CodecMaster:
     def decodeTiles(self, batch, out=None):
         """Inverse of encodeTiles.  Returns the raster (numpy for host batches, torch for device batches); float32 for a
         batch of integer-coded float tiles (batch.icf)."""
-        cl = self.spec.native_list()
+        cl = self._native_list()
         band = batch.band
         rows, cols = band.tiles_down * band.tile_rows, band.tiles_across * band.tile_cols
         decode, name = self._decode_call(batch.icf)

@@ -94,6 +94,7 @@ struct g4_context {
   DevBuf lsopMeta;     // LSOP12 decode: interior code lengths + text position, kernel H -> kernel T
   DevBuf lsopSide, lsopExc, lsopResid, lsopStage, lsopCks;  // LSOP12 decode, fast path (g4_lsop_fast.cu): side records, exception lists, residual bytes
   DevBuf wide;         // TileElementShort: int32 staging raster around the integer codecs
+  DevBuf lsopValueCrc; // LSOP12 encode with G4_LSOP12_VALUE_CHECKSUM: one CRC-32C per tile
   // zlib-stream encode stages (CodecDeflate, CodecFloat, LSOP12 Deflate alternative)
   DevBuf jobLen, jobOff, jobOut, jobTotal, streamIn, streamOut, deflateWork;
   // staged zlib encode (streams <= deflate_staged_max() bytes): sorted positions, bucket ranks, match table, sort tables
@@ -112,7 +113,6 @@ struct g4_context {
   uint64_t arenaLimit = ~0ull;  // g4_decode_tiles_bounded: bytes addressable behind the arena of the running call
   bool icfOn = false;           // g4_encode_tiles_icf / g4_decode_tiles_icf: the running call's band is G4_ELEM_ICF ...
   g4::IcfMap icf{};             // ... mapped with this descriptor
-  bool lsopDeflate = true;  // LsEncoder12.deflateEnabled (lsop/LsEncoder12.java:78)
   // staging used by the host-memory entry points
   DevBuf sGrid, sArena, sOffsets, sLens, sCodec, sPred, sStatus;
   // host-buffer decode pipeline: payload H2D / kernels / raster D2H of consecutive chunks overlap
@@ -227,9 +227,9 @@ int run_streams(g4_context* ctx, int nStreams, int capExtra, int level, int* cou
   return G4_OK;
 }
 
-// Launch one candidate encoder over every tile of the band.
+// Launch one candidate encoder over every tile of the band.  opts: the G4_LSOP12_* option bits of the codec's list entry.
 struct KernelTimer;
-int launch_encoder_impl(g4_context* ctx, int codecId, EncodeArgs& a, int nTiles) {
+int launch_encoder_impl(g4_context* ctx, int codecId, int opts, EncodeArgs& a, int nTiles) {
   const int nGrid = persistent_ctas(ctx, nTiles, 8);
   uint32_t* jl = nullptr;
   uint64_t* jo = nullptr;
@@ -274,10 +274,16 @@ int launch_encoder_impl(g4_context* ctx, int codecId, EncodeArgs& a, int nTiles)
       CK(ctx->encScratch.ensure(stride * n));
       a.scratch = ctx->encScratch.as<uint8_t>();
       a.scratchStride = stride;
+      if (codecId == G4_CODEC_LSOP12 && (opts & G4_LSOP12_VALUE_CHECKSUM)) {  // LsEncoder12.java:128-131
+        CK(ctx->lsopValueCrc.ensure(size_t(nTiles) * 4));
+        CK(launch_lsop_value_crc(a, ctx->lsopValueCrc.as<uint32_t>(), nTiles, ctx->stream));
+        ctx->launches++;
+        a.valueCrc = ctx->lsopValueCrc.as<uint32_t>();
+      }
       if (codecId == G4_CODEC_CANON_HUFFMAN) CK(launch_canon_encode(a, n, ctx->stream));
       else CK(launch_lsop_encode(a, n, ctx->stream));
       ctx->launches++;
-      if (codecId == G4_CODEC_LSOP12 && ctx->lsopDeflate) {  // LsEncoder12.java:170-218
+      if (codecId == G4_CODEC_LSOP12 && !(opts & G4_LSOP12_NO_DEFLATE)) {  // LsEncoder12.java:170-218
         const int nStreams = 2 * nTiles;
         int rc = ensure_jobs(ctx, nStreams);
         if (rc != G4_OK) return rc;
@@ -383,9 +389,30 @@ int launch_decoder(g4_context* ctx, int codecId, DecodeArgs& a, int nCtas) {
   }
 }
 
-int launch_encoder(g4_context* ctx, int codecId, EncodeArgs& a, int nTiles) {
+int launch_encoder(g4_context* ctx, int codecId, int opts, EncodeArgs& a, int nTiles) {
   KernelTimer timer(ctx, 1, codecId);
-  return launch_encoder_impl(ctx, codecId, a, nTiles);
+  return launch_encoder_impl(ctx, codecId, opts, a, nTiles);
+}
+
+// A codec-list entry or codec_id argument is a codec id, with the G4_LSOP12_* option bits OR-ed into an LSOP12 entry.
+// Splits it into the plain id (what the kernels and every switch on codec ids see) and the bits; G4_ERR_ARG for unknown
+// bits or bits on another codec.  Negative entries pass unchanged, for the callers' own checks.
+constexpr int32_t kLsop12Options = G4_LSOP12_NO_DEFLATE | G4_LSOP12_VALUE_CHECKSUM;
+int split_codec_id(int32_t entry, int32_t* id, int* opts) {
+  *id = entry;
+  *opts = 0;
+  if (entry < 0 || entry <= 0xff) return G4_OK;
+  if ((entry & 0xff) != G4_CODEC_LSOP12 || (entry & ~0xff & ~kLsop12Options) != 0) return G4_ERR_ARG;
+  *id = G4_CODEC_LSOP12;
+  *opts = entry & kLsop12Options;
+  return G4_OK;
+}
+int split_codec_list(const g4_codec_list* in, g4_codec_list* ids, int* opts) {
+  if (in->n_codecs < 0 || in->n_codecs > G4_MAX_CODECS) return G4_ERR_ARG;
+  *ids = *in;
+  for (int k = 0; k < in->n_codecs; k++)
+    if (split_codec_id(in->codec_ids[k], &ids->codec_ids[k], &opts[k]) != G4_OK) return G4_ERR_ARG;
+  return G4_OK;
 }
 
 int check_band(const g4_band_desc* b, bool icf = false) {  // icf: the band of a g4_*_tiles_icf call
@@ -413,7 +440,7 @@ size_t band_samples(const g4_band_desc& b) {
 
 // Encode with every applicable codec of `codecs`, select, compact.  All pointers are device pointers.
 // slotBytes: capacity of each candidate slot.
-int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, void* grid, uint8_t* arena,
+int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const int* opts, const g4_band_desc* band, void* grid, uint8_t* arena,
                       uint64_t arenaCap, uint64_t* offsets, uint32_t* lens, uint8_t* codecOut, uint8_t* predOut, int32_t* status,
                       uint64_t* totalHost, size_t slotBytes, const int16_t* raw16, int64_t raw16Pitch) {
   const int nTiles = band->tiles_down * band->tiles_across;
@@ -451,7 +478,7 @@ int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const g4_ban
     a.codecIndex = cand[c];
     a.scratch = nullptr;
     a.scratchStride = 0;
-    int rc = launch_encoder(ctx, codecs->codec_ids[cand[c]], a, nTiles);
+    int rc = launch_encoder(ctx, codecs->codec_ids[cand[c]], opts[cand[c]], a, nTiles);
     if (rc != G4_OK) return rc;
     sel.candIndex[c] = cand[c];
     cmp.slots[c] = a.slots;
@@ -561,7 +588,7 @@ g4_band_desc widened(const g4_band_desc& b) {
   return w;
 }
 
-int encode_device(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, void* grid, uint8_t* arena,
+int encode_device(g4_context* ctx, const g4_codec_list* codecs, const int* opts, const g4_band_desc* band, void* grid, uint8_t* arena,
                   uint64_t arenaCap, uint64_t* offsets, uint32_t* lens, uint8_t* codecOut, uint8_t* predOut, int32_t* status,
                   uint64_t* totalHost, size_t slotBytes) {
   if (band->elem_type == G4_ELEM_ICF) {  // the float band is mapped to codes in the staging raster, which is then encoded
@@ -570,11 +597,11 @@ int encode_device(g4_context* ctx, const g4_codec_list* codecs, const g4_band_de
     CK(ctx->wide.ensure(size_t(rows) * size_t(cols) * 4));
     CK(launch_icf_map(0, grid, band->grid_pitch, ctx->wide.p, cols, rows, cols, ctx->icf, ctx->stream));
     ctx->launches++;
-    return encode_device_i32(ctx, codecs, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
+    return encode_device_i32(ctx, codecs, opts, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
                              nullptr, 0);
   }
   if (band->elem_type != G4_ELEM_I16)
-    return encode_device_i32(ctx, codecs, band, grid, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
+    return encode_device_i32(ctx, codecs, opts, band, grid, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
                              nullptr, 0);
   const g4_band_desc w = widened(*band);
   const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = w.grid_pitch;
@@ -582,7 +609,7 @@ int encode_device(g4_context* ctx, const g4_codec_list* codecs, const g4_band_de
   CK(launch_widen_i16(static_cast<const int16_t*>(grid), band->grid_pitch, ctx->wide.as<int32_t>(), rows, cols, band->fill_value,
                       ctx->stream));
   ctx->launches++;
-  return encode_device_i32(ctx, codecs, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
+  return encode_device_i32(ctx, codecs, opts, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
                            static_cast<const int16_t*>(grid), band->grid_pitch);
 }
 
@@ -1104,7 +1131,10 @@ static int encode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
   if (!ctx || !codecs || !grid || !arena || !offsets || !lens || !codec_out || !predictor_out || !status) return G4_ERR_ARG;
   int rc = check_band(band, ctx->icfOn);
   if (rc != G4_OK) return rc;
-  if (codecs->n_codecs < 0 || codecs->n_codecs > G4_MAX_CODECS) return G4_ERR_ARG;
+  g4_codec_list ids;
+  int opts[G4_MAX_CODECS];
+  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
+  codecs = &ids;
   ENTER(ctx);
   const int nTiles = band->tiles_down * band->tiles_across;
   const size_t n = size_t(band->tile_rows) * band->tile_cols;
@@ -1115,7 +1145,7 @@ static int encode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
   TileRefScope scope{ctx};
   if (mem_space == G4_MEM_DEVICE) {
     if (refs && (rc = upload_tile_refs(ctx, refs, nTiles)) != G4_OK) return rc;
-    rc = encode_device(ctx, codecs, band, const_cast<void*>(grid), arena, arena_cap, offsets, lens, codec_out, predictor_out,
+    rc = encode_device(ctx, codecs, opts, band, const_cast<void*>(grid), arena, arena_cap, offsets, lens, codec_out, predictor_out,
                        status, &total, slotBytes);
     if (rc != G4_OK) return rc;
     CK(cudaMemcpyAsync(st.data(), status, size_t(nTiles) * 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1143,7 +1173,7 @@ static int encode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
                              size_t(band->tile_cols) * eb, size_t(band->tile_rows), cudaMemcpyHostToDevice, ctx->stream));
     } else CK(cudaMemcpyAsync(ctx->sGrid.p, grid, gridBytes, cudaMemcpyHostToDevice, ctx->stream));
     band = &staged;
-    rc = encode_device(ctx, codecs, band, ctx->sGrid.p, ctx->sArena.as<uint8_t>(), bound, ctx->sOffsets.as<uint64_t>(),
+    rc = encode_device(ctx, codecs, opts, band, ctx->sGrid.p, ctx->sArena.as<uint8_t>(), bound, ctx->sOffsets.as<uint64_t>(),
                        ctx->sLens.as<uint32_t>(), ctx->sCodec.as<uint8_t>(), ctx->sPred.as<uint8_t>(), ctx->sStatus.as<int32_t>(),
                        &total, slotBytes);
     if (rc != G4_OK) return rc;
@@ -1204,7 +1234,10 @@ static int decode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
   if (!ctx || !codecs || !grid || !arena || !offsets || !lens || !status) return G4_ERR_ARG;
   int rc = check_band(band, ctx->icfOn);
   if (rc != G4_OK) return rc;
-  if (codecs->n_codecs < 0 || codecs->n_codecs > G4_MAX_CODECS) return G4_ERR_ARG;
+  g4_codec_list ids;  // decode ignores the option bits: they describe how to encode, the packings say the rest
+  int opts[G4_MAX_CODECS];
+  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
+  codecs = &ids;
   ENTER(ctx);
   const int nTiles = band->tiles_down * band->tiles_across;
   std::vector<int32_t> st(nTiles);
@@ -1401,6 +1434,8 @@ int g4_decode_tiles_icf(g4_context* ctx, const g4_codec_list* codecs, const g4_b
 static int encode_one(g4_context* ctx, int codec_id, int codec_index, int elem, int n_rows, int n_cols, const void* values,
                       uint8_t* out, size_t out_cap, size_t* out_len, int* predictor) {
   if (!ctx || !values || !out || !out_len) return G4_ERR_ARG;
+  int opts = 0;
+  if (split_codec_id(codec_id, &codec_id, &opts) != G4_OK) return G4_ERR_ARG;
   if (codec_id < 0 || codec_id >= G4_CODEC_COUNT || codec_index < 0 || codec_index > 255) return G4_ERR_ARG;
   if (codec_is_float(codec_id) != (elem == G4_ELEM_F32)) return G4_DECLINED;  // e.g. CodecHuffman.encodeFloats -> null
   if (codec_id == G4_CODEC_LSOP08) return G4_DECLINED;  // decode-only legacy codec (include/g4codec.h)
@@ -1431,7 +1466,7 @@ static int encode_one(g4_context* ctx, int codec_id, int codec_index, int elem, 
   a.status = ctx->candStatus.as<int32_t>();
   a.counter = ctx->counters.as<int>();
   a.codecIndex = codec_index;
-  rc = launch_encoder(ctx, codec_id, a, 1);
+  rc = launch_encoder(ctx, codec_id, opts, a, 1);
   if (rc != G4_OK) return rc;
   uint32_t len = 0;
   int32_t st = 0;
@@ -1452,6 +1487,8 @@ static int encode_one(g4_context* ctx, int codec_id, int codec_index, int elem, 
 
 static int decode_one(g4_context* ctx, int codec_id, int elem, int n_rows, int n_cols, const uint8_t* packing, size_t len, void* out) {
   if (!ctx || !packing || !out || len == 0 || len > 0xffffffffull) return G4_ERR_ARG;
+  int opts = 0;  // ignored, as in g4_decode_tiles
+  if (split_codec_id(codec_id, &codec_id, &opts) != G4_OK) return G4_ERR_ARG;
   if (codec_id < 0 || codec_id >= G4_CODEC_COUNT) return G4_ERR_ARG;
   if (codec_is_float(codec_id) != (elem == G4_ELEM_F32)) return G4_DECLINED;  // decodeFloats on an int codec -> null
   g4_band_desc band{elem, n_rows, n_cols, 1, 1, n_cols};
@@ -1507,7 +1544,10 @@ int g4_analyze_tiles(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   if (!ctx || !codecs || !band || !arena || !offsets || !lens || !stats) return G4_ERR_ARG;
   int rc = check_band(band);
   if (rc != G4_OK) return rc;
-  if (codecs->n_codecs < 0 || codecs->n_codecs > G4_MAX_CODECS) return G4_ERR_ARG;
+  g4_codec_list ids;  // the option bits are ignored, as in decode
+  int opts[G4_MAX_CODECS];
+  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
+  codecs = &ids;
   ENTER(ctx);
   const int nTiles = band->tiles_down * band->tiles_across;
   const size_t n = size_t(band->tile_rows) * band->tile_cols;

@@ -38,6 +38,7 @@ struct EncodeArgs {
   int codecIndex;       // list position of this codec == packing[0]
   uint8_t* scratch;     // per-CTA scratch (codec specific)
   size_t scratchStride;
+  const uint32_t* valueCrc;  // LSOP12: per-tile value checksum to store in the header (launch_lsop_value_crc), or null
 };
 
 // One decoder launch over the tiles of one codec kind: list[0..*listCount) are tile indices.
@@ -296,6 +297,8 @@ cudaError_t launch_record_unpack(const uint8_t* image, uint64_t imageLen, const 
 // LSOP12 value checksum (LsDecoder12.java:153-158): CRC-32C of every decoded tile whose packing carries one, compared with the
 // stored value; a mismatch leaves status G4_CHECKSUM_MISMATCH (the values stay delivered: the reference only prints).
 cudaError_t launch_lsop_value_checksum(const DecodeArgs& a, int nTilesUpper, cudaStream_t s);
+// LSOP12 encode with the value checksum: crc[t] = CRC-32C of tile t's values, every tile of a.band
+cudaError_t launch_lsop_value_crc(const EncodeArgs& a, uint32_t* crc, int nTiles, cudaStream_t s);
 cudaError_t launch_record_verify(const uint32_t* computed, const uint32_t* stored, int n, int32_t* status, cudaStream_t s);
 // Tile records of rasters with several elements per tile.  elems: device array of nElements descriptors; element e of tile t
 // is elems[e].arena[elems[e].offsets[t] .. + elems[e].lens[t]).

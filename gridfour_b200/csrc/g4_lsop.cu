@@ -807,6 +807,9 @@ __device__ __forceinline__ void moment_accumulate(const double (&z)[13], double 
   moment_accumulate_seq<ROLE>(z, acc, std::make_integer_sequence<int, kMomentPerRole>{});
 }
 
+// Header bytes of the canonical-Huffman packing: 55, or 59 with the value checksum behind the coefficients.
+__device__ __forceinline__ uint32_t lsop_canon_header_bytes(const EncodeArgs& a) { return a.valueCrc ? 59u : 55u; }
+
 struct LsopEncShared {
   CanonEncShared E;
   BitWindow W;
@@ -1018,12 +1021,13 @@ __global__ void __launch_bounds__(kThreads) lsop_encode_kernel(EncodeArgs a) {
     if (tid == 0) {
       WinSink sink{S.W.win, 0};
       sink.put(uint32_t(a.codecIndex) & 0xffu, 8);
-      sink.put(0x40u | 2u, 8);  // revision flag | COMPRESSION_TYPE_CANON_HUFFMAN
+      sink.put((a.valueCrc ? 0x80u : 0u) | 0x40u | 2u, 8);  // checksum flag | revision flag | COMPRESSION_TYPE_CANON_HUFFMAN
       sink.put(12, 8);
       sink.put(uint32_t(t.at(0, 0)), 32);
       for (int i = 0; i < 12; i++) sink.put(__float_as_uint(S.u[i]), 32);
+      if (a.valueCrc) sink.put(a.valueCrc[tIdx], 32);
     }
-    o.bitPos = 55u * 8u;
+    o.bitPos = lsop_canon_header_bytes(a) * 8u;
     __syncthreads();
     LsInitGet g1{t};
     LsInteriorGet g2{t, S.u};
@@ -1058,6 +1062,7 @@ __global__ void __launch_bounds__(kThreads) lsop_encode_kernel(EncodeArgs a) {
 // deflated at level 6 by the stream workers, and the packing is replaced by the type-1 form when
 // insideN < canonLength and initN + insideN < canonLength (the reference compares bodies only, headers excluded).
 namespace {
+// The coefficients sit at bytes 7..54 of both header forms; only what follows them depends on the value checksum.
 __device__ __forceinline__ void load_slot_coefficients(const uint8_t* slot, float* u) {
   if (threadIdx.x < 12) u[threadIdx.x] = __uint_as_float(load_le32(slot + 7 + 4 * threadIdx.x));
   __syncthreads();
@@ -1070,7 +1075,7 @@ __global__ void __launch_bounds__(kThreads) lsop_m32_size_kernel(EncodeArgs a, u
   const int nTiles = a.band.tiles_down * a.band.tiles_across;
   for (int tIdx = blockIdx.x; tIdx < nTiles; tIdx += gridDim.x) {
     __syncthreads();
-    if (a.status[tIdx] != G4_OK || a.lens[tIdx] < 55) {  // declined (too small / singular): nothing to deflate
+    if (a.status[tIdx] != G4_OK || a.lens[tIdx] < lsop_canon_header_bytes(a)) {  // declined (too small / singular): nothing to deflate
       if (threadIdx.x == 0) inLen[2 * tIdx] = inLen[2 * tIdx + 1] = 0;
       continue;
     }
@@ -1110,27 +1115,30 @@ __global__ void __launch_bounds__(kThreads) lsop_pick_kernel(EncodeArgs a, const
   const int nTiles = a.band.tiles_down * a.band.tiles_across;
   for (int tIdx = blockIdx.x; tIdx < nTiles; tIdx += gridDim.x) {
     if (inLen[2 * tIdx + 1] == 0) continue;
-    const uint32_t canonLength = a.lens[tIdx] - 55u;
+    const uint32_t canonLength = a.lens[tIdx] - lsop_canon_header_bytes(a);  // bodies only (Appendix C quirk 11)
     const uint32_t initN = outLen[2 * tIdx], insideN = outLen[2 * tIdx + 1];
     if (insideN == 0 || insideN >= canonLength) continue;         // LsEncoder12.java:185-190
     if (initN == 0 || initN + insideN >= canonLength) continue;   // :197-201
-    const uint32_t len = 63u + initN + insideN;
+    const uint32_t body = lsop_canon_header_bytes(a) + 8u;       // [nInit][nInterior] then the checksum, if any
+    const uint32_t len = body + initN + insideN;
     if (len > a.slotBytes) {
       if (tid == 0) a.status[tIdx] = G4_ERR_CAPACITY;
       continue;
     }
     uint8_t* slot = a.slots + size_t(tIdx) * a.slotBytes;
     if (tid == 0) {
-      slot[1] = uint8_t(0x40u | 1u);  // revision flag | COMPRESSION_TYPE_DEFLATE (LsHeader.java:220-245)
+      slot[1] = uint8_t((a.valueCrc ? 0x80u : 0u) | 0x40u | 1u);  // checksum flag | revision flag | COMPRESSION_TYPE_DEFLATE (LsHeader.java:220-245)
       const uint32_t n0 = inLen[2 * tIdx], n1 = inLen[2 * tIdx + 1];
       for (int k = 0; k < 4; k++) { slot[55 + k] = uint8_t(n0 >> (8 * k)); slot[59 + k] = uint8_t(n1 >> (8 * k)); }
+      if (a.valueCrc)
+        for (int k = 0; k < 4; k++) slot[63 + k] = uint8_t(a.valueCrc[tIdx] >> (8 * k));
       a.lens[tIdx] = len;
       a.preds[tIdx] = 1;
     }
     const uint8_t* s0 = outBuf + inOff[2 * tIdx] + 112ull * uint64_t(2 * tIdx);
     const uint8_t* s1 = outBuf + inOff[2 * tIdx + 1] + 112ull * uint64_t(2 * tIdx + 1);
-    for (uint32_t i = tid; i < initN; i += kThreads) slot[63 + i] = s0[i];
-    for (uint32_t i = tid; i < insideN; i += kThreads) slot[63 + initN + i] = s1[i];
+    for (uint32_t i = tid; i < initN; i += kThreads) slot[body + i] = s0[i];
+    for (uint32_t i = tid; i < insideN; i += kThreads) slot[body + initN + i] = s1[i];
   }
 }
 

@@ -135,23 +135,8 @@ __global__ void __launch_bounds__(kCrcThreads) crc32c_kernel(const uint8_t* data
   }
 }
 
-// LSOP12 value checksum (LsHeader.computeChecksum :391-406, checked in LsDecoder12.decode :153-158): CRC-32C of the tile's
-// nRows x nColumns values as little-endian int32, row-major.  One WARP per tile of the list whose packing carries the
-// checksum; every lane takes a contiguous run of values (an even number: the slice-by-8 step eats two), the 32 pieces are
-// joined like in crc32c_kernel.  The tile is a strided window of the raster, so the values are read cell by cell.
-__global__ void __launch_bounds__(kCrcThreads) lsop_value_checksum_kernel(DecodeArgs a) {
-  __shared__ uint32_t T[8][256];
-  __shared__ uint32_t x2n[32];
-  const int lane = threadIdx.x & 31;
-  const int li = (blockIdx.x * kCrcThreads + threadIdx.x) >> 5;
-  // (uniform per warp) does this warp's tile carry a checksum at all?  Most files do not: leave before building the tables.
-  bool need = false;
-  int tIdx = 0;
-  if (li < *a.listCount) {
-    tIdx = a.list[li];
-    need = a.lsopCks[2 * tIdx] != 0u && a.status[tIdx] == G4_OK;
-  }
-  if (!__syncthreads_or(need ? 1 : 0)) return;
+// The slice-by-8 tables and the table of x^(2^i) mod P that the joins of the kernels below need, in shared memory.
+__device__ inline void crc_build_join_tables(uint32_t (*T)[256], uint32_t* x2n) {
   crc_build_tables(T);
   if (threadIdx.x == 0) {
     uint32_t p = 1u << 30;  // x^1
@@ -159,8 +144,13 @@ __global__ void __launch_bounds__(kCrcThreads) lsop_value_checksum_kernel(Decode
     for (int i = 1; i < 32; i++) x2n[i] = p = crc_multmodp(p, p);
   }
   __syncthreads();
-  if (!need) return;
-  const TileView t = tile_view(a.band, a.grid, tIdx);
+}
+
+// LSOP12 value checksum (LsHeader.computeChecksum :391-406): CRC-32C of the tile's nRows x nColumns values as little-endian
+// int32, row-major.  One WARP per tile: every lane takes a contiguous run of values (an even number: the slice-by-8 step
+// eats two), the 32 pieces are joined like in crc32c_kernel.  The tile is a strided window of the raster, so the values
+// are read cell by cell.  All 32 lanes call; lane 0 returns the CRC.
+__device__ uint32_t lsop_tile_value_crc(const uint32_t (*T)[256], const uint32_t* x2n, const TileView& t, int lane) {
   const uint32_t n = uint32_t(t.R) * uint32_t(t.C);
   uint32_t piece = ((n + 31u) / 32u + 1u) & ~1u;
   if (piece < 16u) piece = 16u;
@@ -197,12 +187,50 @@ __global__ void __launch_bounds__(kCrcThreads) lsop_value_checksum_kernel(Decode
       myLen += rl;
     }
   }
+  return c;
+}
+
+// Decode: checked in LsDecoder12.decode :153-158 for every tile of the list whose packing carries the checksum.
+__global__ void __launch_bounds__(kCrcThreads) lsop_value_checksum_kernel(DecodeArgs a) {
+  __shared__ uint32_t T[8][256];
+  __shared__ uint32_t x2n[32];
+  const int lane = threadIdx.x & 31;
+  const int li = (blockIdx.x * kCrcThreads + threadIdx.x) >> 5;
+  // (uniform per warp) does this warp's tile carry a checksum at all?  Most files do not: leave before building the tables.
+  bool need = false;
+  int tIdx = 0;
+  if (li < *a.listCount) {
+    tIdx = a.list[li];
+    need = a.lsopCks[2 * tIdx] != 0u && a.status[tIdx] == G4_OK;
+  }
+  if (!__syncthreads_or(need ? 1 : 0)) return;
+  crc_build_join_tables(T, x2n);
+  if (!need) return;
+  const uint32_t c = lsop_tile_value_crc(T, x2n, tile_view(a.band, a.grid, tIdx), lane);
   if (lane == 0 && c != a.lsopCks[2 * tIdx + 1]) a.status[tIdx] = G4_CHECKSUM_MISMATCH;
+}
+
+// Encode with the value checksum enabled (LsEncoder12.java:128-131): crc[t] for every tile of the band, which
+// lsop_encode_kernel and lsop_pick_kernel then store in the header.
+__global__ void __launch_bounds__(kCrcThreads) lsop_value_crc_kernel(EncodeArgs a, uint32_t* crc) {
+  __shared__ uint32_t T[8][256];
+  __shared__ uint32_t x2n[32];
+  crc_build_join_tables(T, x2n);
+  const int tIdx = (blockIdx.x * kCrcThreads + threadIdx.x) >> 5;
+  if (tIdx >= a.band.tiles_down * a.band.tiles_across) return;
+  const uint32_t c = lsop_tile_value_crc(T, x2n, tile_view(a.band, a.grid, tIdx), threadIdx.x & 31);
+  if ((threadIdx.x & 31) == 0) crc[tIdx] = c;
 }
 
 cudaError_t launch_lsop_value_checksum(const DecodeArgs& a, int nTilesUpper, cudaStream_t s) {
   const int warpsPerCta = kCrcThreads / 32;
   lsop_value_checksum_kernel<<<(nTilesUpper + warpsPerCta - 1) / warpsPerCta, kCrcThreads, 0, s>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_lsop_value_crc(const EncodeArgs& a, uint32_t* crc, int nTiles, cudaStream_t s) {
+  const int warpsPerCta = kCrcThreads / 32;
+  lsop_value_crc_kernel<<<(nTiles + warpsPerCta - 1) / warpsPerCta, kCrcThreads, 0, s>>>(a, crc);
   return cudaGetLastError();
 }
 

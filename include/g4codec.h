@@ -57,6 +57,21 @@ enum {
   G4_CODEC_COUNT = 6
 };
 
+/* Options of the LSOP12 encoder (C/lsop/LsEncoder12.java:93-119), OR-ed into a G4_CODEC_LSOP12 entry of a g4_codec_list or
+ * into the codec_id of g4_encode_i32, as they belong to the encoder instance in the reference.  Without them LSOP12 encodes
+ * as the reference's defaults do: the Deflate alternative on, no value checksum.
+ *   G4_LSOP12_NO_DEFLATE      setDeflateEnabled(false): every packing is the canonical-Huffman form (type 2); the Deflate
+ *                             alternative (type 1: M32 streams deflated at level 6, kept when its bodies are smaller) is not run.
+ *   G4_LSOP12_VALUE_CHECKSUM  setValueChecksumEnabled(true): bit 0x80 of packing[1] is set and the CRC-32C of the tile's values
+ *                             (little-endian int32, row-major; for short elements the widened ints, for ICF elements the codes)
+ *                             follows the coefficients (type 2, body at byte 59) or [nInit][nInterior] (type 1, body at byte 67).
+ * The encode entry points (g4_encode_i32, g4_encode_tiles, g4_encode_tiles_icf, g4_encode_tile_list) honour them; the decode
+ * and analyze entry points accept them and ignore them, so that one list serves both directions.  Other bits above the low
+ * byte, or option bits on another codec: G4_ERR_ARG.  g4_codec_name and g4_codec_supported take plain ids (an id with option
+ * bits has no name and is not supported there). */
+#define G4_LSOP12_NO_DEFLATE (1 << 8)
+#define G4_LSOP12_VALUE_CHECKSUM (1 << 9)
+
 /* Predictor codes stored in packing[1] (C/compress/PredictorModelType.java:46-63). */
 enum { G4_PRED_NONE = 0, G4_PRED_DIFFERENCING = 1, G4_PRED_LINEAR = 2, G4_PRED_TRIANGLE = 3, G4_PRED_DIFF_NULLS = 4 };
 

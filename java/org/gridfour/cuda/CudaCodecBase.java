@@ -22,6 +22,11 @@ abstract class CudaCodecBase {
     this.codecId = codecId;
   }
 
+  /** The codec id passed to g4_encode_i32: the plain id, with the option bits of an encoder that has options. */
+  int encodeId() {
+    return codecId;
+  }
+
   public byte[] encode(int codecIndex, int nRows, int nCols, int[] values) {
     if (codecId == G4Native.CODEC_FLOAT) {
       throw new IllegalArgumentException("Integer encoding not supported");  // CodecFloat.java:116-125
@@ -31,7 +36,7 @@ abstract class CudaCodecBase {
       MemorySegment in = a.allocateFrom(JAVA_INT, values);
       MemorySegment out = a.allocate(cap);
       MemorySegment len = a.allocate(JAVA_LONG);
-      int rc = (int) G4Native.ENCODE_I32.invokeExact(G4Native.CONTEXT.get(), codecId, codecIndex, nRows, nCols, in, out, cap, len,
+      int rc = (int) G4Native.ENCODE_I32.invokeExact(G4Native.CONTEXT.get(), encodeId(), codecIndex, nRows, nCols, in, out, cap, len,
         MemorySegment.NULL);
       if (rc == G4Native.G4_DECLINED) {
         return null;

@@ -21,6 +21,7 @@ final class G4Native {
 
   static final int G4_OK = 0, G4_DECLINED = 1, G4_ERR_FORMAT = -2;
   static final int CODEC_HUFFMAN = 0, CODEC_DEFLATE = 1, CODEC_FLOAT = 2, CODEC_CANON_HUFFMAN = 3, CODEC_LSOP12 = 4;
+  static final int LSOP12_NO_DEFLATE = 1 << 8, LSOP12_VALUE_CHECKSUM = 1 << 9;  // option bits of an LSOP12 codec id
   static final int MEM_HOST = 0;
 
   private static final Linker LINKER = Linker.nativeLinker();
