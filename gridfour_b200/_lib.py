@@ -28,7 +28,7 @@ EXPORTS = [
     "g4_crc32c", "g4_tile_records_bound", "g4_pack_tile_records", "g4_unpack_tile_records", "g4_context_order_stream", "g4_decode_tiles_bounded", "g4_predictor_encode", "g4_predictor_encode_int", "g4_predictor_decode",
     "g4_predictor_decode_int", "g4_predictor_tiles", "g4_encode_tile_list", "g4_decode_tile_list", "g4_analyze_tiles",
     "g4_tile_records_bound_multi", "g4_pack_tile_records_multi", "g4_unpack_tile_records_multi",
-    "g4_icf_map", "g4_encode_tiles_icf", "g4_decode_tiles_icf",
+    "g4_icf_map", "g4_encode_tiles_icf", "g4_decode_tiles_icf", "g4_decode_window",
 ]
 
 
@@ -109,7 +109,10 @@ def lib():
                                           C.POINTER(C.c_uint64)]
         L.g4_decode_tiles_icf.argtypes = [C.c_void_p, C.POINTER(CodecList), C.POINTER(BandDesc), C.POINTER(IcfDesc), C.c_int, C.c_void_p,
                                           C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
-        L.g4_fill_terrain.argtypes = [C.c_void_p, C.c_int, C.c_uint64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]
+        L.g4_decode_window.argtypes = [C.c_void_p, C.POINTER(CodecList), C.POINTER(BandDesc), C.POINTER(IcfDesc), C.c_void_p, C.c_uint64,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
+                                       C.c_void_p, C.c_int64, C.c_void_p]
+        L.g4_fill_terrain.argtypes =[C.c_void_p, C.c_int, C.c_uint64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]
         L.g4_context_set_timing.argtypes = [C.c_void_p, C.c_int]
         L.g4_context_set_async.argtypes = [C.c_void_p, C.c_int]
         L.g4_kernel_time_ms.argtypes = [C.c_void_p, C.c_int, C.c_int]

@@ -115,6 +115,8 @@ struct g4_context {
   g4::IcfMap icf{};             // ... mapped with this descriptor
   // staging used by the host-memory entry points
   DevBuf sGrid, sArena, sOffsets, sLens, sCodec, sPred, sStatus;
+  // g4_decode_window: payload locations of the window tiles, absent-tile flags, int32 staging band of unaligned windows
+  DevBuf winOff, winLen, winAbsent, winStage;
   // host-buffer decode pipeline: payload H2D / kernels / raster D2H of consecutive chunks overlap
   cudaStream_t copyIn = nullptr, copyOut = nullptr;
   cudaEvent_t evIn[16] = {}, evDone[16] = {}, evStart = nullptr, evOrder = nullptr;
@@ -755,7 +757,8 @@ void g4_context_destroy(g4_context* ctx) {
                     &ctx->total, &ctx->coef, &ctx->defer, &ctx->lsopMeta, &ctx->lsopSide, &ctx->lsopExc, &ctx->lsopResid, &ctx->lsopStage, &ctx->tileRefs, &ctx->lsopCks, &ctx->wide, &ctx->encScratch, &ctx->region, &ctx->jobLen, &ctx->jobOff, &ctx->jobOut, &ctx->jobTotal,
                     &ctx->streamIn, &ctx->streamOut, &ctx->deflateWork, &ctx->stSorted, &ctx->stRank, &ctx->stTable,
                     &ctx->stWork, &ctx->stCounters, &ctx->rcPos, &ctx->rcOff, &ctx->rcLen, &ctx->rcCrc, &ctx->rcStored, &ctx->rcTotal,
-                    &ctx->rcData, &ctx->rcOffsets, &ctx->rcLens, &ctx->rcIndex, &ctx->rcStatus, &ctx->rcOut, &ctx->rcChain, &ctx->rcDesc, &ctx->sGrid, &ctx->sArena, &ctx->sOffsets, &ctx->sLens, &ctx->sCodec, &ctx->sPred, &ctx->sStatus};
+                    &ctx->rcData, &ctx->rcOffsets, &ctx->rcLens, &ctx->rcIndex, &ctx->rcStatus, &ctx->rcOut, &ctx->rcChain, &ctx->rcDesc, &ctx->sGrid, &ctx->sArena, &ctx->sOffsets, &ctx->sLens, &ctx->sCodec, &ctx->sPred, &ctx->sStatus,
+                    &ctx->winOff, &ctx->winLen, &ctx->winAbsent, &ctx->winStage};
   for (DevBuf* b : bufs) b->release();
   if (ctx->ownStream) cudaStreamDestroy(ctx->stream);
   delete ctx;
@@ -1427,6 +1430,89 @@ int g4_decode_tiles_icf(g4_context* ctx, const g4_codec_list* codecs, const g4_b
   if (!ctx || !band || band->elem_type != G4_ELEM_ICF || !icf_valid(icf)) return G4_ERR_ARG;
   IcfScope scope(ctx, icf);
   return g4_decode_tiles_bounded(ctx, codecs, band, mem_space, arena, arena_len, offsets, lens, grid, status);
+}
+
+// ---- window reads: GvrsElement.readBlock (gvrs/GvrsElement.java:298-404) on the device ----------------------------------
+// gather (window tiles' payload locations) -> classify + decoders -> store.  A tile-aligned window is decoded straight into
+// `out` and the store launch only fills absent tiles; any other window is decoded into an int32 staging band of its covering
+// tiles (4 bytes per sample) and the store launch crops, converts and fills in one pass.  Launches beyond those of
+// g4_decode_tiles_bounded on the same tiles: exactly two (gather, store).
+int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf, const uint8_t* image,
+                     uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens, const int32_t* tile_status, uint32_t fill_bits,
+                     int64_t row0, int64_t col0, int64_t n_rows, int64_t n_cols, void* out, int64_t out_pitch, int32_t* status) {
+  if (!ctx || !codecs || !image || !payload_offsets || !lens || !tile_status || !out || !status) return G4_ERR_ARG;
+  int rc = check_band(raster, icf != nullptr);
+  if (rc != G4_OK) return rc;
+  if (icf && !icf_valid(icf)) return G4_ERR_ARG;
+  const int R = raster->tile_rows, Cc = raster->tile_cols;
+  const int64_t gridRows = int64_t(raster->tiles_down) * R, gridCols = int64_t(raster->tiles_across) * Cc;
+  if (n_rows < 1 || n_cols < 1 || row0 < 0 || col0 < 0 || row0 > gridRows - n_rows || col0 > gridCols - n_cols) return G4_ERR_ARG;
+  if (out_pitch < n_cols) return G4_ERR_ARG;
+  g4_codec_list ids;
+  int opts[G4_MAX_CODECS];
+  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
+  codecs = &ids;
+  ENTER(ctx);
+  const int tr0 = int(row0 / R), tc0 = int(col0 / Cc);
+  const int nTd = int((row0 + n_rows - 1) / R) - tr0 + 1, nTa = int((col0 + n_cols - 1) / Cc) - tc0 + 1;
+  const int nW = nTd * nTa;
+  CK(ctx->winOff.ensure(size_t(nW) * 8));
+  CK(ctx->winLen.ensure(size_t(nW) * 4));
+  CK(ctx->winAbsent.ensure(size_t(nW)));
+  CK(launch_window_gather(payload_offsets, lens, tile_status, raster->tiles_across, tr0, tc0, nTd, nTa, ctx->winOff.as<uint64_t>(),
+                          ctx->winLen.as<uint32_t>(), ctx->winAbsent.as<uint8_t>(), ctx->stream));
+  ctx->launches++;
+  struct ArenaScope {  // payloads that leave the image are G4_ERR_FORMAT, as in g4_decode_tiles_bounded
+    g4_context* c;
+    ~ArenaScope() { c->arenaLimit = ~0ull; }
+  } arenaScope{ctx};
+  ctx->arenaLimit = image_len;
+  WindowStore ws{};
+  ws.rows = n_rows;
+  ws.cols = n_cols;
+  ws.out = out;
+  ws.outPitch = out_pitch;
+  ws.R = R;
+  ws.C = Cc;
+  ws.nTa = nTa;
+  ws.nW = nW;
+  ws.absent = ctx->winAbsent.as<uint8_t>();
+  ws.status = status;
+  ws.fillBits = fill_bits;
+  ws.mode = raster->elem_type == G4_ELEM_I16 ? kWindowNarrow16 : icf ? kWindowIcfFloat : kWindowCopy32;
+  if (icf) ws.icf = icf_of(icf);
+  g4_band_desc b = *raster;
+  b.tiles_down = nTd;
+  b.tiles_across = nTa;
+  if (row0 % R == 0 && col0 % Cc == 0 && n_rows == int64_t(nTd) * R && n_cols == int64_t(nTa) * Cc) {
+    b.grid_pitch = out_pitch;
+    if (icf) {
+      IcfScope scope(ctx, icf);
+      rc = decode_device(ctx, codecs, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), out, status);
+    } else {
+      rc = decode_device(ctx, codecs, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), out, status);
+    }
+  } else {
+    b = widened(b);  // int32 samples, pitch = the covering tiles' width
+    if (raster->elem_type == G4_ELEM_F32) b.elem_type = G4_ELEM_F32;
+    CK(ctx->winStage.ensure(band_samples(b) * 4));
+    rc = decode_device_i32(ctx, codecs, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), ctx->winStage.p, status,
+                           raster->elem_type == G4_ELEM_I16);
+    ws.stage = ctx->winStage.as<int32_t>();
+    ws.stagePitch = b.grid_pitch;
+    ws.sr0 = row0 - int64_t(tr0) * R;
+    ws.sc0 = col0 - int64_t(tc0) * Cc;
+  }
+  if (rc != G4_OK) return rc;
+  CK(launch_window_store(ws, ctx->smCount, ctx->stream));
+  ctx->launches++;
+  if (ctx->asyncDevice) return G4_OK;  // enqueued; status[] is read by the caller after g4_context_synchronize
+  std::vector<int32_t> st(nW);
+  CK(cudaMemcpyAsync(st.data(), status, size_t(nW) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  for (int32_t& s : st)
+    if (s == G4_DECLINED) s = G4_OK;  // absent tiles read as fill values; they are neither errors nor notes
+  return first_bad_status(st);
 }
 
 // ---- per-tile entry points: one-tile bands through the same kernels --------------------------------

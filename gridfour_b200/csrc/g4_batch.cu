@@ -250,6 +250,137 @@ __global__ void __launch_bounds__(256) icf_to_float_kernel(const int32_t* src, i
   icf_map_rect<int32_t, float, int4, float4>(src, srcPitch, dst, dstPitch, rows, cols, m);
 }
 
+// ---- window reads (g4_decode_window, GvrsElement.readBlock :298-404) ------------------------------------------------------
+// One thread per window tile: the tile's payload location in window order.  Tiles the file does not hold (G4_DECLINED) and
+// damaged records (< 0) get a zero-length payload, which classify_kernel puts in no decoder list.
+__global__ void window_gather_kernel(const uint64_t* offsets, const uint32_t* lens, const int32_t* tileStatus, int tilesAcross, int tr0,
+                                     int tc0, int nTd, int nTa, uint64_t* offW, uint32_t* lenW, uint8_t* absentW) {
+  const int w = blockIdx.x * blockDim.x + threadIdx.x;
+  if (w >= nTd * nTa) return;
+  const int wr = w / nTa, wc = w - wr * nTa;
+  const int64_t t = int64_t(tr0 + wr) * tilesAcross + (tc0 + wc);
+  const int32_t st = tileStatus[t];
+  offW[w] = st == G4_OK ? offsets[t] : 0;
+  lenW[w] = st == G4_OK ? lens[t] : 0u;
+  absentW[w] = st == G4_DECLINED ? 1 : 0;
+}
+
+// classify_kernel reported the zero-length payloads of absent tiles as G4_ERR_FORMAT; they are G4_DECLINED, not errors.
+__device__ __forceinline__ void window_mark_absent(const WindowStore& a) {
+  const int64_t nThreads = int64_t(gridDim.x) * gridDim.y * blockDim.x * blockDim.y;
+  const int64_t id = (int64_t(blockIdx.y) * gridDim.x + blockIdx.x) * (blockDim.x * blockDim.y) + threadIdx.y * blockDim.x + threadIdx.x;
+  for (int64_t w = id; w < a.nW; w += nThreads)
+    if (a.absent[w]) a.status[w] = G4_DECLINED;
+}
+
+template <int Mode> struct WindowOut { using T = int32_t; using V = int4; };
+template <> struct WindowOut<kWindowNarrow16> { using T = int16_t; using V = short4; };
+template <> struct WindowOut<kWindowIcfFloat> { using T = float; using V = float4; };
+
+template <int Mode>
+__device__ __forceinline__ typename WindowOut<Mode>::T window_sample(int32_t v, const WindowStore& a) {
+  if constexpr (Mode == kWindowNarrow16) return v == kNull ? int16_t(-32768) : int16_t(v);  // as narrow_i16_kernel
+  else if constexpr (Mode == kWindowIcfFloat) return icf_value(v, a.icf);
+  else return v;
+}
+template <int Mode>
+__device__ __forceinline__ typename WindowOut<Mode>::T window_fill(const WindowStore& a) {
+  if constexpr (Mode == kWindowNarrow16) return int16_t(uint16_t(a.fillBits));
+  else if constexpr (Mode == kWindowIcfFloat) return __uint_as_float(a.fillBits);
+  else return int32_t(a.fillBits);
+}
+
+// The store pass of an unaligned window: staging band -> the caller's rectangle, cropped, converted, absent tiles filled.
+// Threads take four consecutive cells of a row as icf_map_rect does: one 16-byte load where the staging address is 16-byte
+// aligned, one 16-byte (8-byte for shorts) store where the output address is, cell by cell otherwise.
+template <int Mode>
+__global__ void __launch_bounds__(256) window_store_kernel(WindowStore a) {
+  using T = typename WindowOut<Mode>::T;
+  using V = typename WindowOut<Mode>::V;
+  window_mark_absent(a);
+  const int64_t c = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) * 4;
+  if (c >= a.cols) return;
+  const int k = a.cols - c < 4 ? int(a.cols - c) : 4;
+  const int64_t sc = a.sc0 + c;
+  const int tcA = int(sc / a.C), tcB = int((sc + k - 1) / a.C);  // window tile columns of the first and last cell
+  const T fill = window_fill<Mode>(a);
+  for (int64_t r = int64_t(blockIdx.y) * blockDim.y + threadIdx.y; r < a.rows; r += int64_t(gridDim.y) * blockDim.y) {
+    const int64_t sr = a.sr0 + r;
+    const uint8_t* absentRow = a.absent + (sr / a.R) * a.nTa;
+    const int32_t* s = a.stage + sr * a.stagePitch + sc;
+    T* d = static_cast<T*>(a.out) + r * a.outPitch + c;
+    int32_t v[4] = {0, 0, 0, 0};
+    if (k == 4 && (reinterpret_cast<uintptr_t>(s) & 15) == 0) {
+      const int4 x = *reinterpret_cast<const int4*>(s);
+      v[0] = x.x; v[1] = x.y; v[2] = x.z; v[3] = x.w;
+    } else {
+#pragma unroll
+      for (int i = 0; i < 4; i++)
+        if (i < k) v[i] = s[i];
+    }
+    T y[4];
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      const bool gone = i < k && absentRow[tcA == tcB ? tcA : int((sc + i) / a.C)];
+      y[i] = gone ? fill : window_sample<Mode>(v[i], a);
+    }
+    if (k == 4 && (reinterpret_cast<uintptr_t>(d) & (sizeof(V) - 1)) == 0) {
+      V z;
+      z.x = y[0]; z.y = y[1]; z.z = y[2]; z.w = y[3];
+      *reinterpret_cast<V*>(d) = z;
+    } else {
+#pragma unroll
+      for (int i = 0; i < 4; i++)
+        if (i < k) d[i] = y[i];
+    }
+  }
+}
+
+// A tile-aligned window decoded straight into the caller's rectangle: only absent tiles are written, with the fill sample.
+template <class T>
+__global__ void __launch_bounds__(256) window_fill_kernel(WindowStore a) {
+  const T fill = T(a.fillBits);
+  for (int w = blockIdx.x; w < a.nW; w += gridDim.x) {
+    if (!a.absent[w]) continue;
+    if (threadIdx.x == 0 && threadIdx.y == 0) a.status[w] = G4_DECLINED;
+    const int wr = w / a.nTa, wc = w - wr * a.nTa;
+    T* base = static_cast<T*>(a.out) + int64_t(wr) * a.R * a.outPitch + int64_t(wc) * a.C;
+    for (int r = threadIdx.y; r < a.R; r += blockDim.y)
+      for (int c = threadIdx.x; c < a.C; c += blockDim.x) base[int64_t(r) * a.outPitch + c] = fill;
+  }
+}
+
+cudaError_t launch_window_gather(const uint64_t* offsets, const uint32_t* lens, const int32_t* tileStatus, int tilesAcross, int tr0,
+                                 int tc0, int nTd, int nTa, uint64_t* offW, uint32_t* lenW, uint8_t* absentW, cudaStream_t s) {
+  const int n = nTd * nTa;
+  window_gather_kernel<<<(n + 255) / 256, 256, 0, s>>>(offsets, lens, tileStatus, tilesAcross, tr0, tc0, nTd, nTa, offW, lenW, absentW);
+  return cudaGetLastError();
+}
+cudaError_t launch_window_store(const WindowStore& a, int smCount, cudaStream_t s) {
+  if (!a.stage) {
+    const int n = a.nW < smCount * 8 ? a.nW : smCount * 8;
+    int bx = 32;
+    while (bx < 256 && bx < a.C) bx <<= 1;
+    const dim3 block(bx, 256 / bx);
+    if (a.mode == kWindowNarrow16) window_fill_kernel<uint16_t><<<n, block, 0, s>>>(a);
+    else window_fill_kernel<uint32_t><<<n, block, 0, s>>>(a);
+    return cudaGetLastError();
+  }
+  const int64_t quads = (a.cols + 3) / 4;
+  int bx = 1;
+  while (bx < 256 && bx < quads) bx <<= 1;
+  const dim3 block(bx, 256 / bx);
+  const int64_t gx = (quads + bx - 1) / bx, gy = (a.rows + block.y - 1) / block.y;
+  if (gx > 0x7fffffff) return cudaErrorInvalidValue;
+  const dim3 grid(unsigned(gx), unsigned(gy < 65535 ? gy : 65535));
+  switch (a.mode) {
+    case kWindowNarrow16: window_store_kernel<kWindowNarrow16><<<grid, block, 0, s>>>(a); break;
+    case kWindowIcfFloat: window_store_kernel<kWindowIcfFloat><<<grid, block, 0, s>>>(a); break;
+    default: window_store_kernel<kWindowCopy32><<<grid, block, 0, s>>>(a); break;
+  }
+  return cudaGetLastError();
+}
+
 cudaError_t launch_fill_terrain(int elemType, uint64_t seed, int64_t row0, int64_t col0, int64_t nRows, int64_t nCols, void* out,
                                 cudaStream_t s) {
   fill_terrain_kernel<<<148 * 8, 256, 0, s>>>(elemType, seed, row0, col0, nRows, nCols, out);

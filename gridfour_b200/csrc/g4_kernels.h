@@ -159,6 +159,31 @@ struct IcfMap {
 cudaError_t launch_icf_map(int toFloat, const void* src, int64_t srcPitch, void* dst, int64_t dstPitch, int64_t rows, int64_t cols,
                            const IcfMap& m, cudaStream_t s);
 
+// Window reads (g4_decode_window): the tiles tr0.. x tc0.. (nTd x nTa, "window tiles" w = wr * nTa + wc) of a raster whose
+// per-tile arrays are in tile-index order.  The gather copies the window tiles' payload locations into window order; a tile
+// whose status is not G4_OK gets offset 0 and length 0 (classify_kernel then keeps it out of every decoder list) and, when
+// it is G4_DECLINED, absent[w] = 1.
+cudaError_t launch_window_gather(const uint64_t* offsets, const uint32_t* lens, const int32_t* tileStatus, int tilesAcross, int tr0,
+                                 int tc0, int nTd, int nTa, uint64_t* offW, uint32_t* lenW, uint8_t* absentW, cudaStream_t s);
+enum { kWindowCopy32 = 0, kWindowNarrow16 = 1, kWindowIcfFloat = 2 };  // how a decoded int32 sample becomes an output sample
+struct WindowStore {
+  const int32_t* stage;   // the decoded window tiles (int32 / float32 bits / ICF codes); null: decoded in place (tile-aligned)
+  int64_t stagePitch;     // samples per staging row
+  int64_t sr0, sc0;       // staging cell of output cell (0, 0)
+  int64_t rows, cols;     // output rectangle
+  void* out;
+  int64_t outPitch;       // samples per output row
+  int R, C, nTa, nW;      // tile size, window tiles across, window tiles
+  const uint8_t* absent;  // [nW] from launch_window_gather
+  int32_t* status;        // [nW]: absent tiles get G4_DECLINED
+  uint32_t fillBits;      // output sample of absent tiles (the low 16 bits for kWindowNarrow16)
+  int mode;               // kWindow*
+  IcfMap icf;             // kWindowIcfFloat
+};
+// stage != null: one pass stage -> out (crop, narrow / ICF map, fill of absent tiles).  stage == null: the window tiles were
+// decoded straight into out; only the absent ones are filled.
+cudaError_t launch_window_store(const WindowStore& a, int smCount, cudaStream_t s);
+
 // ---- codec kernels -----------------------------------------------------------------------------
 // Host-side launchers (defined next to their kernels).  nCtas persistent CTAs of kThreads threads.
 cudaError_t launch_huffman_encode(const EncodeArgs& a, int nCtas, cudaStream_t s);

@@ -350,6 +350,137 @@ class GvrsImage:
         payload_off, lens, status = self._locate_all(master._context(), verify)
         return [self._decode_element(master, k, payload_off[k], lens[k], status, crop, as_float) for k in range(len(self.spec.elements))]
 
+    def to_device(self, context=None, device=None, verify=True):
+        """The image resident on a GPU, for reads that leave their results there (GvrsDeviceImage).  Uploads the image
+        once, then validates every tile record and locates every element's payloads on the device; raises IOError for a
+        damaged tile record or, with verify, a record whose checksum differs, as read_raster does."""
+        import warnings
+
+        import torch
+
+        from ._lib import G4_CHECKSUM_MISMATCH
+        from .codecs import Context
+
+        if device is None:
+            device = context.device if context is not None else torch.cuda.current_device()
+        dev = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
+        if dev.index is None:
+            dev = torch.device("cuda", torch.cuda.current_device())
+        ctx = context or Context.default(dev.index)
+        spec = self.spec
+        n_tiles = spec.tiles_down * spec.tiles_across
+        n = len(self.image)
+        buf = torch.empty(multiple_of_8(n) + 8, dtype=torch.uint8, device=dev)  # the unpack calls take an 8-byte aligned image
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore", UserWarning)  # the bytes are only read: torch warns about any read-only buffer
+            host = torch.from_numpy(np.frombuffer(self.image, dtype=np.uint8))
+        buf[:n].copy_(host)
+        image = buf[:n]
+        pos = np.zeros(n_tiles, dtype=np.int64)
+        for t, p in self.tile_directory().items():
+            pos[t] = p
+        content_pos = torch.from_numpy(pos).to(dev)
+        checksum = verify and spec.checksum
+        ctx.after_torch_stream(dev)
+        if len(spec.elements) == 1:
+            payload_off, lens, status = unpack_tile_records_device(ctx, image, content_pos, checksum)
+            payload_off, lens = payload_off[None], lens[None]
+        else:
+            payload_off, lens, status = unpack_tile_records_multi_device(ctx, image, content_pos, len(spec.elements), checksum)
+        ctx.before_torch_stream(dev)
+        st = status.cpu().numpy()
+        bad = np.nonzero(st < 0)[0]
+        if len(bad):
+            raise IOError("damaged tile record for tile %d" % int(bad[0]))
+        if np.any(st == G4_CHECKSUM_MISMATCH):
+            raise IOError("Checksum mismatch in a tile record")
+        return GvrsDeviceImage(self, image, payload_off, lens, status, ctx)
+
+
+class GvrsDeviceImage:
+    """A GVRS file image resident in device memory with its payloads located (GvrsImage.to_device).  Reads decode only the
+    tiles a request touches, straight from the resident image, and return torch CUDA tensors (g4_decode_window):
+    per read, nothing crosses PCIe but the status of the tiles read.  The reads run on the context the image was made
+    with; `master` gives the codec list."""
+
+    def __init__(self, host, image, payload_off, lens, status, context):
+        self.host, self.spec = host, host.spec
+        self.image, self.payload_off, self.lens, self.status = image, payload_off, lens, status  # [n] / [E, n] / [E, n] / [n]
+        self.context = context
+        self.device = image.device
+        self.lastStatus = None  # per covering tile of the latest read, window-tile order (device tensor)
+
+    def _element(self, element):
+        if not 0 <= element < len(self.spec.elements):
+            raise ValueError("no such element")
+        return self.spec.elements[element]
+
+    def read_block(self, master, row, col, n_rows, n_cols, element=0, as_float=False, out=None):
+        """GvrsElement.readBlock: the n_rows x n_cols cells from (row, col), which must lie inside the raster (ValueError
+        otherwise).  Returns a CUDA tensor: int32 for integer elements and the codes of integer-coded float elements,
+        float32 for float elements and, with as_float, for integer-coded float values, int16 for short elements.  Tiles
+        absent from the file read as the element's fill value.  `out` may be any 2-D CUDA tensor of that dtype and shape
+        whose rows are contiguous, e.g. a slice of a larger mosaic; its other cells are left as they are."""
+        spec = self.spec
+        self._element(element)
+        if row < 0 or col < 0 or row + n_rows > spec.n_rows or col + n_cols > spec.n_cols or n_rows < 1 or n_cols < 1:
+            raise ValueError("block outside the raster")
+        return self._read(master, row, col, n_rows, n_cols, element, as_float, out)
+
+    def read_raster(self, master, element=0, crop=False, as_float=False):
+        """The values GvrsImage.read_raster returns, as a CUDA tensor: the whole tile grid, or with crop the n_rows x n_cols
+        raster."""
+        spec = self.spec
+        self._element(element)
+        if crop:
+            return self._read(master, 0, 0, spec.n_rows, spec.n_cols, element, as_float, None)
+        return self._read(master, 0, 0, spec.tiles_down * spec.tile_rows, spec.tiles_across * spec.tile_cols, element, as_float, None)
+
+    def _read(self, master, row, col, n_rows, n_cols, element, as_float, out):
+        import torch
+
+        from ._lib import G4_ELEM_F32, G4_ELEM_I16, G4_ELEM_I32, G4_ELEM_ICF, BandDesc
+
+        spec = self.spec
+        e = spec.elements[element]
+        icf = e.icf if as_float else None
+        band = BandDesc()
+        band.tile_rows, band.tile_cols = spec.tile_rows, spec.tile_cols
+        band.tiles_down, band.tiles_across = spec.tiles_down, spec.tiles_across
+        band.grid_pitch = spec.tiles_across * spec.tile_cols
+        if icf is not None:
+            band.elem_type, dtype = G4_ELEM_ICF, torch.float32
+            fill = struct.unpack("<I", bytes(C.c_float(float(icf.fill_value))))[0]  # the float g4_icf_desc carries
+        elif e.type_code == ELEM_FLOAT:
+            band.elem_type, dtype = G4_ELEM_F32, torch.float32
+            fill = int(np.float32(e.fill_value).view(np.uint32))
+        elif e.type_code == ELEM_SHORT:
+            band.elem_type, dtype = G4_ELEM_I16, torch.int16
+            fill = e.fill_value & 0xffff
+        else:
+            band.elem_type, dtype = G4_ELEM_I32, torch.int32
+            fill = e.fill_value & 0xffffffff
+        if out is None:
+            out = torch.empty((n_rows, n_cols), dtype=dtype, device=self.device)
+        elif not (isinstance(out, torch.Tensor) and out.device == self.device and out.dtype == dtype and out.dim() == 2
+                  and tuple(out.shape) == (n_rows, n_cols) and (n_rows == 1 or out.stride(0) >= n_cols) and (n_cols == 1 or out.stride(1) == 1)):
+            raise ValueError("out: a 2-D %s tensor of shape (%d, %d) on %s with contiguous rows" % (dtype, n_rows, n_cols, self.device))
+        pitch = out.stride(0) if n_rows > 1 else n_cols
+        t_down = (row + n_rows - 1) // spec.tile_rows - row // spec.tile_rows + 1
+        t_across = (col + n_cols - 1) // spec.tile_cols - col // spec.tile_cols + 1
+        status = torch.empty(t_down * t_across, dtype=torch.int32, device=self.device)
+        d = icf.desc() if icf is not None else None
+        ctx = self.context
+        ctx.after_torch_stream(self.device)  # `out` may still be in use on torch's stream
+        st = _lib.lib().g4_decode_window(ctx._h, C.byref(master._native_list()), C.byref(band), None if d is None else C.byref(d),
+                                         self.image.data_ptr(), int(self.image.numel()), self.payload_off[element].data_ptr(),
+                                         self.lens[element].data_ptr(), self.status.data_ptr(), fill, int(row), int(col), int(n_rows),
+                                         int(n_cols), out.data_ptr(), int(pitch), status.data_ptr())
+        ctx.before_torch_stream(self.device)
+        self.lastStatus = status
+        check(st, "g4_decode_window")
+        return out
+
 
 # ---- GPU-backed primitives -------------------------------------------------------------------------------------------
 def _u8(buf):

@@ -217,6 +217,33 @@ int g4_decode_tiles_icf(g4_context* ctx, const g4_codec_list* codecs, const g4_b
                         const uint8_t* arena, uint64_t arena_len, const uint64_t* offsets, const uint32_t* lens, float* grid,
                         int32_t* status);
 
+/* ---- window reads: GvrsElement.readBlock on the device (C/gvrs/GvrsElement.java:298-404) --------------------------------
+ * The cells [row0, row0 + n_rows) x [col0, col0 + n_cols) of one element of a raster whose file image is resident on the
+ * device, written to out[r * out_pitch + c] (pitch in samples).  Every pointer is a device pointer (host readers keep
+ * g4_decode_tiles).  Only the tiles the window touches are decoded.
+ *   raster       element type and tile geometry of the WHOLE tile grid (tiles_down x tiles_across tiles; grid_pitch is not
+ *                used beyond check_band's rule, tiles_across * tile_cols will do).  G4_ELEM_I32 / F32 / I16, or G4_ELEM_ICF
+ *                together with `icf`: the codes are then mapped to float32 values.  To read the codes of an ICF element, pass
+ *                G4_ELEM_I32 and no descriptor.
+ *   image, image_len, payload_offsets, lens, tile_status
+ *                the file image and, in tile-index order, what g4_unpack_tile_records(_multi) returns for the element (one
+ *                row of the element-major arrays).  Payloads that leave image_len get G4_ERR_FORMAT, as in
+ *                g4_decode_tiles_bounded.
+ *   fill_bits    the sample written into the cells of tiles with tile_status G4_DECLINED (absent from the file), as a 32-bit
+ *                pattern: float bits for float32 output, the int16 value in the low half for G4_ELEM_I16.
+ *   status       one entry per covering tile, in window-tile order (the tile rows and columns the window touches, row-major):
+ *                G4_DECLINED for absent tiles (not an error), G4_ERR_FORMAT for a tile whose tile_status is an error or
+ *                whose payload is malformed, G4_CHECKSUM_MISMATCH for an LSOP12 value checksum that differs.
+ * Returns the first bad status as g4_decode_tiles does, absent tiles not counted (a window of tiles that are all sound or
+ * absent returns G4_OK); with g4_context_set_async it only enqueues and returns G4_OK.
+ * G4_ERR_ARG for a window that is empty or leaves the tile grid, out_pitch < n_cols, a bad `raster`, or an `icf` for a
+ * non-ICF element or with an invalid scale.  A window whose edges lie on tile boundaries is decoded straight into `out`; any
+ * other window stages its covering tiles at 4 bytes per sample in device memory the context keeps. */
+int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf,
+                     const uint8_t* image, uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens,
+                     const int32_t* tile_status, uint32_t fill_bits, int64_t row0, int64_t col0, int64_t n_rows, int64_t n_cols,
+                     void* out, int64_t out_pitch, int32_t* status);
+
 /* ---- tile LISTS: scattered tiles of one size (the tile cache's callers) -------------------------------------------------
  * The band calls above take one rectangle of one raster.  A tile cache flushes whatever tiles are dirty, each in its own
  * int[] (gvrs/RasterTileCache.java:253-294, RasterTile.getCompressedPacking :234-256), and a block read lands tiles in a
