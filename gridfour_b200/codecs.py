@@ -499,11 +499,18 @@ class CodecMaster:
         d = icf.desc()
         return (lambda ctx, cl, band, *rest: L.g4_encode_tiles_icf(ctx, cl, band, C.byref(d), *rest)), "g4_encode_tiles_icf"
 
-    def encodeTiles(self, grid, tileRows, tileCols, fillValue=None, icf=None):
+    def encodeTiles(self, grid, tileRows, tileCols, fillValue=None, icf=None, padValue=None):
         """grid: 2-D numpy array (host path) or torch CUDA tensor (device path); int32, float32, or int16 (a short
         element, TileElementShort: `fillValue` is coded as null, raw tiles take 2 bytes per sample).  With `icf` (an
         IntCodedFloat) the float32 grid is an integer-coded float element: it is mapped to codes on the GPU and the codes are
-        encoded with the integer codecs; the batch remembers the mapping."""
+        encoded with the integer codecs; the batch remembers the mapping.
+        With `padValue` (CUDA tensors only) the grid may have any dimensions and any row pitch, as long as its rows are
+        contiguous: it covers ceil(rows / tileRows) x ceil(cols / tileCols) tiles, whose cells outside the grid encode as
+        padValue does (g4_encode_window; the padding happens on the device)."""
+        if padValue is not None:
+            if isinstance(grid, np.ndarray):
+                raise ValueError("padValue: CUDA tensors only (a numpy grid is padded by the caller)")
+            return self._encode_window(grid, tileRows, tileCols, fillValue, icf, padValue)
         L = _lib.lib()
         cl = self._native_list()
         total = C.c_uint64(0)
@@ -553,6 +560,53 @@ class CodecMaster:
         ctx.before_torch_stream(dev)
         check(st, name)
         return TileBatch(arena, offsets, lens, codec, pred, status, total.value, band, icf)
+
+    def _encode_window(self, grid, tileRows, tileCols, fillValue, icf, padValue):
+        """encodeTiles of a CUDA tensor of any dimensions, padded with padValue on the device (g4_encode_window)."""
+        import torch
+
+        L = _lib.lib()
+        dtypes = {torch.int32: np.int32, torch.float32: np.float32, torch.int16: np.int16}
+        if not (isinstance(grid, torch.Tensor) and grid.is_cuda and grid.dim() == 2 and grid.dtype in dtypes):
+            raise ValueError("expected a 2-D int32, float32 or int16 CUDA tensor")
+        if icf is not None and grid.dtype != torch.float32:
+            raise ValueError("an integer-coded float element is encoded from a float32 tensor")
+        rows, cols = grid.shape
+        if rows < 1 or cols < 1:
+            raise ValueError("an empty grid")
+        if (cols > 1 and grid.stride(1) != 1) or (rows > 1 and grid.stride(0) < cols):
+            raise ValueError("the grid's rows must be contiguous")
+        pitch = grid.stride(0) if rows > 1 else cols
+        npdt = dtypes[grid.dtype]
+        b = BandDesc()
+        b.elem_type = G4_ELEM_F32 if npdt == np.float32 else G4_ELEM_I16 if npdt == np.int16 else G4_ELEM_I32
+        if icf is not None:
+            b.elem_type = G4_ELEM_ICF
+        b.fill_value = int(fillValue) if fillValue is not None else -32768
+        b.tile_rows, b.tile_cols = tileRows, tileCols
+        b.tiles_down, b.tiles_across = -(-rows // tileRows), -(-cols // tileCols)
+        b.grid_pitch = b.tiles_across * tileCols
+        # the margin sample as a 32-bit pattern of the source type (int16: the low half)
+        fill_bits = int(np.array(padValue, dtype=npdt).view(np.uint16 if npdt == np.int16 else np.uint32))
+        nT = b.tiles_down * b.tiles_across
+        cap = int(L.g4_encode_arena_bound(C.byref(b)))
+        dev = grid.device
+        arena = torch.empty(cap, dtype=torch.uint8, device=dev)
+        offsets = torch.empty(nT, dtype=torch.int64, device=dev)
+        lens = torch.empty(nT, dtype=torch.int32, device=dev)
+        codec = torch.empty(nT, dtype=torch.uint8, device=dev)
+        pred = torch.empty(nT, dtype=torch.uint8, device=dev)
+        status = torch.empty(nT, dtype=torch.int32, device=dev)
+        d = icf.desc() if icf is not None else None
+        total = C.c_uint64(0)
+        ctx = self._context()
+        ctx.after_torch_stream(dev)  # `grid` may come from kernels still queued on torch's stream
+        st = L.g4_encode_window(ctx._h, C.byref(self._native_list()), C.byref(b), None if d is None else C.byref(d), rows, cols,
+                                grid.data_ptr(), pitch, fill_bits, arena.data_ptr(), cap, offsets.data_ptr(), lens.data_ptr(),
+                                codec.data_ptr(), pred.data_ptr(), status.data_ptr(), C.byref(total))
+        ctx.before_torch_stream(dev)
+        check(st, "g4_encode_window")
+        return TileBatch(arena, offsets, lens, codec, pred, status, total.value, b, icf)
 
     # -- tile lists (new): scattered tiles of one size, each with its own {offset, pitch} -- the tile cache's calls -----
     @staticmethod

@@ -444,7 +444,7 @@ size_t band_samples(const g4_band_desc& b) {
 // slotBytes: capacity of each candidate slot.
 int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const int* opts, const g4_band_desc* band, void* grid, uint8_t* arena,
                       uint64_t arenaCap, uint64_t* offsets, uint32_t* lens, uint8_t* codecOut, uint8_t* predOut, int32_t* status,
-                      uint64_t* totalHost, size_t slotBytes, const int16_t* raw16, int64_t raw16Pitch) {
+                      uint64_t* totalHost, size_t slotBytes, bool rawShorts, int32_t fill16) {
   const int nTiles = band->tiles_down * band->tiles_across;
   const int n = band->tile_rows * band->tile_cols;
   const bool isFloat = band->elem_type == G4_ELEM_F32;
@@ -487,7 +487,7 @@ int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const int* o
   }
   sel.nTiles = nTiles;
   sel.nCand = nCand;
-  sel.rawLen = raw16 ? ((2u * uint32_t(n) + 3u) & ~3u) : uint32_t(n) * 4u;
+  sel.rawLen = rawShorts ? ((2u * uint32_t(n) + 3u) & ~3u) : uint32_t(n) * 4u;
   sel.candLens = ctx->candLens.as<uint32_t>();
   sel.candPreds = ctx->candPreds.as<uint8_t>();
   sel.candStatus = ctx->candStatus.as<int32_t>();
@@ -509,8 +509,8 @@ int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const int* o
   cmp.arena = arena;
   cmp.arenaCap = arenaCap;
   cmp.status = status;
-  cmp.raw16 = raw16;
-  cmp.raw16Pitch = raw16Pitch;
+  cmp.rawShorts = rawShorts ? 1 : 0;
+  cmp.fill16 = fill16;
   CK(launch_compact(cmp, nTiles, ctx->stream));
   ctx->launches += 3;
   uint64_t total = 0;
@@ -590,6 +590,30 @@ g4_band_desc widened(const g4_band_desc& b) {
   return w;
 }
 
+// The load pass into ctx->wide: the nRows x nCols source raster, the rest of the band's tile grid filled with the margin
+// sample fillBits.  The staging raster is 4 bytes per sample of the tile grid.
+int stage_window(g4_context* ctx, const g4_band_desc& band, int mode, const void* src, int64_t srcPitch, int64_t nRows, int64_t nCols,
+                 uint32_t fillBits, const g4::IcfMap& icf) {
+  const g4_band_desc w = widened(band);
+  WindowLoad ld{};
+  ld.src = src;
+  ld.srcPitch = srcPitch;
+  ld.nRows = nRows;
+  ld.nCols = nCols;
+  ld.rows = int64_t(band.tiles_down) * band.tile_rows;
+  ld.cols = w.grid_pitch;
+  ld.dstPitch = w.grid_pitch;
+  CK(ctx->wide.ensure(size_t(ld.rows) * size_t(ld.cols) * 4));
+  ld.dst = ctx->wide.as<int32_t>();
+  ld.fillBits = fillBits;
+  ld.fill16 = band.fill_value;
+  ld.mode = mode;
+  ld.icf = icf;
+  CK(launch_window_load(ld, ctx->stream));
+  ctx->launches++;
+  return G4_OK;
+}
+
 int encode_device(g4_context* ctx, const g4_codec_list* codecs, const int* opts, const g4_band_desc* band, void* grid, uint8_t* arena,
                   uint64_t arenaCap, uint64_t* offsets, uint32_t* lens, uint8_t* codecOut, uint8_t* predOut, int32_t* status,
                   uint64_t* totalHost, size_t slotBytes) {
@@ -600,19 +624,18 @@ int encode_device(g4_context* ctx, const g4_codec_list* codecs, const int* opts,
     CK(launch_icf_map(0, grid, band->grid_pitch, ctx->wide.p, cols, rows, cols, ctx->icf, ctx->stream));
     ctx->launches++;
     return encode_device_i32(ctx, codecs, opts, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
-                             nullptr, 0);
+                             false, 0);
   }
   if (band->elem_type != G4_ELEM_I16)
     return encode_device_i32(ctx, codecs, opts, band, grid, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
-                             nullptr, 0);
+                             false, 0);
+  // the widening is the load pass of g4_encode_window over the whole band, with no margin
+  const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = int64_t(band->tiles_across) * band->tile_cols;
+  int rc = stage_window(ctx, *band, kLoadWiden16, grid, band->grid_pitch, rows, cols, 0, g4::IcfMap{});
+  if (rc != G4_OK) return rc;
   const g4_band_desc w = widened(*band);
-  const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = w.grid_pitch;
-  CK(ctx->wide.ensure(size_t(rows) * size_t(cols) * 4));
-  CK(launch_widen_i16(static_cast<const int16_t*>(grid), band->grid_pitch, ctx->wide.as<int32_t>(), rows, cols, band->fill_value,
-                      ctx->stream));
-  ctx->launches++;
   return encode_device_i32(ctx, codecs, opts, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
-                           static_cast<const int16_t*>(grid), band->grid_pitch);
+                           true, band->fill_value);
 }
 
 int decode_device(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, const uint8_t* arena,
@@ -1512,6 +1535,51 @@ int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   CK(cudaStreamSynchronize(ctx->stream));
   for (int32_t& s : st)
     if (s == G4_DECLINED) s = G4_OK;  // absent tiles read as fill values; they are neither errors nor notes
+  return first_bad_status(st);
+}
+
+// ---- window writes: a raster of any dimensions and pitch, padded to whole tiles on the device -----------------------------
+// A tile-aligned int32 / float32 raster is encoded straight from `src`, exactly as g4_encode_tiles.  Every other raster goes
+// through one window_load_kernel pass into the context's int32 staging raster (4 bytes per sample of the tile grid), which
+// for short and ICF elements stands in for the widening / mapping launch of g4_encode_tiles(_icf), and is then encoded.
+int g4_encode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf, int64_t n_rows,
+                     int64_t n_cols, const void* src, int64_t src_pitch, uint32_t fill_bits, uint8_t* arena, uint64_t arena_cap,
+                     uint64_t* offsets, uint32_t* lens, uint8_t* codec_out, uint8_t* predictor_out, int32_t* status, uint64_t* total_bytes) {
+  if (!ctx || !codecs || !src || !arena || !offsets || !lens || !codec_out || !predictor_out || !status) return G4_ERR_ARG;
+  int rc = check_band(raster, icf != nullptr);
+  if (rc != G4_OK) return rc;
+  if (icf && !icf_valid(icf)) return G4_ERR_ARG;
+  const int R = raster->tile_rows, Cc = raster->tile_cols;
+  if (n_rows < 1 || n_cols < 1 || src_pitch < n_cols) return G4_ERR_ARG;
+  if ((n_rows + R - 1) / R != raster->tiles_down || (n_cols + Cc - 1) / Cc != raster->tiles_across) return G4_ERR_ARG;
+  g4_codec_list ids;
+  int opts[G4_MAX_CODECS];
+  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
+  codecs = &ids;
+  ENTER(ctx);
+  const int nTiles = raster->tiles_down * raster->tiles_across;
+  const size_t slotBytes = round_up(size_t(R) * Cc * 4 + 64, 16);
+  const bool wide32 = raster->elem_type == G4_ELEM_I32 || raster->elem_type == G4_ELEM_F32;
+  uint64_t total = 0;
+  if (wide32 && n_rows == int64_t(raster->tiles_down) * R && n_cols == int64_t(raster->tiles_across) * Cc) {
+    g4_band_desc b = *raster;
+    b.grid_pitch = src_pitch;
+    rc = encode_device_i32(ctx, codecs, opts, &b, const_cast<void*>(src), arena, arena_cap, offsets, lens, codec_out, predictor_out,
+                           status, &total, slotBytes, false, 0);
+  } else {
+    const int mode = raster->elem_type == G4_ELEM_I16 ? kLoadWiden16 : icf ? kLoadIcfCode : kLoadCopy32;
+    rc = stage_window(ctx, *raster, mode, src, src_pitch, n_rows, n_cols, fill_bits, icf ? icf_of(icf) : g4::IcfMap{});
+    if (rc != G4_OK) return rc;
+    g4_band_desc w = widened(*raster);
+    if (raster->elem_type == G4_ELEM_F32) w.elem_type = G4_ELEM_F32;  // the float codecs see float32 bits
+    rc = encode_device_i32(ctx, codecs, opts, &w, ctx->wide.p, arena, arena_cap, offsets, lens, codec_out, predictor_out, status, &total,
+                           slotBytes, raster->elem_type == G4_ELEM_I16, raster->fill_value);
+  }
+  if (rc != G4_OK) return rc;
+  std::vector<int32_t> st(nTiles);
+  CK(cudaMemcpyAsync(st.data(), status, size_t(nTiles) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (total_bytes) *total_bytes = total;
   return first_bad_status(st);
 }
 

@@ -89,17 +89,20 @@ __global__ void __launch_bounds__(kThreads) compact_kernel(CompactArgs a) {
   }
   uint8_t* dst = a.arena + off;
   const int src = a.src[t];
-  if (src < 0 && a.raw16) {  // TileElementShort raw form: little-endian shorts, zero padded to a multiple of 4 bytes
-    const int R = a.band.tile_rows, C = a.band.tile_cols, n = R * C;
-    const int tr = t / a.band.tiles_across, tc = t - tr * a.band.tiles_across;
-    const int16_t* base = a.raw16 + int64_t(tr) * R * a.raw16Pitch + int64_t(tc) * C;
+  if (src < 0 && a.rawShorts) {  // TileElementShort raw form: little-endian shorts, zero padded to a multiple of 4 bytes
+    const TileView tv = tile_view(a.band, a.grid, t);
+    const int C = tv.C, n = tv.R * C;
     uint32_t* d32 = reinterpret_cast<uint32_t*>(dst);
     const int nWords = int((len + 3u) >> 2);
     for (int i = threadIdx.x; i < ((nWords + 1) & ~1); i += kThreads) {
       uint32_t w = 0;
       for (int h = 0; h < 2; h++) {
         int k = 2 * i + h;
-        if (k < n) { int r = k / C, c = k - r * C; w |= uint32_t(uint16_t(base[int64_t(r) * a.raw16Pitch + c])) << (16 * h); }
+        if (k < n) {
+          int r = k / C, c = k - r * C;
+          const int32_t v = tv.at(r, c);  // the staged int32: INT4_NULL_CODE only where the short was the fill value
+          w |= uint32_t(uint16_t(v == kNull ? int16_t(a.fill16) : int16_t(v))) << (16 * h);
+        }
       }
       d32[i] = w;
     }
@@ -179,15 +182,6 @@ __global__ void __launch_bounds__(kThreads) raw_decode_kernel(DecodeArgs a) {
   }
 }
 
-// TileElementShort.encode (:213-220): widen, fill value -> INT4_NULL_CODE
-__global__ void widen_i16_kernel(const int16_t* src, int64_t srcPitch, int32_t* dst, int64_t rows, int64_t cols, int32_t fill) {
-  const int64_t total = rows * cols;
-  for (int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; i < total; i += int64_t(gridDim.x) * blockDim.x) {
-    int64_t r = i / cols, c = i - r * cols;
-    int32_t v = src[r * srcPitch + c];
-    dst[i] = v == fill ? kNull : v;
-  }
-}
 // TileElementShort.decode (:236-245): INT4_NULL_CODE -> SHORT_NULL_CODE, everything else narrowed with a (short) cast
 __global__ void narrow_i16_kernel(const int32_t* src, int16_t* dst, int64_t dstPitch, int64_t rows, int64_t cols) {
   const int64_t total = rows * cols;
@@ -248,6 +242,64 @@ __global__ void __launch_bounds__(256) icf_to_int_kernel(const float* src, int64
 __global__ void __launch_bounds__(256) icf_to_float_kernel(const int32_t* src, int64_t srcPitch, float* dst, int64_t dstPitch,
                                                            int64_t rows, int64_t cols, IcfMap m) {
   icf_map_rect<int32_t, float, int4, float4>(src, srcPitch, dst, dstPitch, rows, cols, m);
+}
+
+// ---- window writes (g4_encode_window; the staging of every short encode) ------------------------------------------------
+template <int Mode> struct LoadIn { using T = int32_t; using V = int4; };
+template <> struct LoadIn<kLoadWiden16> { using T = int16_t; using V = short4; };
+template <> struct LoadIn<kLoadIcfCode> { using T = float; using V = float4; };
+
+template <int Mode>
+__device__ __forceinline__ int32_t load_sample(typename LoadIn<Mode>::T v, const WindowLoad& a) {
+  if constexpr (Mode == kLoadWiden16) return int32_t(v) == a.fill16 ? kNull : int32_t(v);  // TileElementShort.encode (:213-220)
+  else if constexpr (Mode == kLoadIcfCode) return icf_code(v, a.icf);
+  else return v;
+}
+template <int Mode>
+__device__ __forceinline__ typename LoadIn<Mode>::T load_fill(const WindowLoad& a) {
+  if constexpr (Mode == kLoadWiden16) return int16_t(uint16_t(a.fillBits));
+  else if constexpr (Mode == kLoadIcfCode) return __uint_as_float(a.fillBits);
+  else return int32_t(a.fillBits);
+}
+
+// The caller's raster -> the staging raster of its covering tiles, converted, the margin filled: the mirror of
+// window_store_kernel.  Threads take four consecutive staging cells of a row as icf_map_rect does: one 16-byte (8-byte for
+// shorts) load where all four cells lie inside the raster and the source address is aligned, one 16-byte store where the
+// staging address is, cell by cell otherwise.  Rows below the raster are margin only.  No division.
+template <int Mode>
+__global__ void __launch_bounds__(256) window_load_kernel(WindowLoad a) {
+  using T = typename LoadIn<Mode>::T;
+  using V = typename LoadIn<Mode>::V;
+  const int64_t c = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) * 4;
+  if (c >= a.cols) return;
+  const int k = a.cols - c < 4 ? int(a.cols - c) : 4;                        // staged cells of this quad
+  const int kin = a.nCols - c >= 4 ? 4 : a.nCols > c ? int(a.nCols - c) : 0;  // ... of which inside the raster
+  const int32_t margin = load_sample<Mode>(load_fill<Mode>(a), a);
+  for (int64_t r = int64_t(blockIdx.y) * blockDim.y + threadIdx.y; r < a.rows; r += int64_t(gridDim.y) * blockDim.y) {
+    int32_t y[4] = {margin, margin, margin, margin};
+    if (r < a.nRows && kin > 0) {
+      const T* s = static_cast<const T*>(a.src) + r * a.srcPitch + c;
+      if (kin == 4 && (reinterpret_cast<uintptr_t>(s) & (sizeof(V) - 1)) == 0) {
+        const V x = *reinterpret_cast<const V*>(s);
+        y[0] = load_sample<Mode>(x.x, a);
+        y[1] = load_sample<Mode>(x.y, a);
+        y[2] = load_sample<Mode>(x.z, a);
+        y[3] = load_sample<Mode>(x.w, a);
+      } else {
+#pragma unroll
+        for (int i = 0; i < 4; i++)
+          if (i < kin) y[i] = load_sample<Mode>(s[i], a);
+      }
+    }
+    int32_t* d = a.dst + r * a.dstPitch + c;
+    if (k == 4 && (reinterpret_cast<uintptr_t>(d) & 15) == 0) {
+      *reinterpret_cast<int4*>(d) = make_int4(y[0], y[1], y[2], y[3]);
+    } else {
+#pragma unroll
+      for (int i = 0; i < 4; i++)
+        if (i < k) d[i] = y[i];
+    }
+  }
 }
 
 // ---- window reads (g4_decode_window, GvrsElement.readBlock :298-404) ------------------------------------------------------
@@ -386,8 +438,19 @@ cudaError_t launch_fill_terrain(int elemType, uint64_t seed, int64_t row0, int64
   fill_terrain_kernel<<<148 * 8, 256, 0, s>>>(elemType, seed, row0, col0, nRows, nCols, out);
   return cudaGetLastError();
 }
-cudaError_t launch_widen_i16(const int16_t* src, int64_t srcPitch, int32_t* dst, int64_t rows, int64_t cols, int32_t fill, cudaStream_t s) {
-  widen_i16_kernel<<<148 * 8, 256, 0, s>>>(src, srcPitch, dst, rows, cols, fill);
+cudaError_t launch_window_load(const WindowLoad& a, cudaStream_t s) {
+  const int64_t quads = (a.cols + 3) / 4;
+  int bx = 1;
+  while (bx < 256 && bx < quads) bx <<= 1;
+  const dim3 block(bx, 256 / bx);
+  const int64_t gx = (quads + bx - 1) / bx, gy = (a.rows + block.y - 1) / block.y;
+  if (gx > 0x7fffffff) return cudaErrorInvalidValue;
+  const dim3 grid(unsigned(gx), unsigned(gy < 65535 ? gy : 65535));
+  switch (a.mode) {
+    case kLoadWiden16: window_load_kernel<kLoadWiden16><<<grid, block, 0, s>>>(a); break;
+    case kLoadIcfCode: window_load_kernel<kLoadIcfCode><<<grid, block, 0, s>>>(a); break;
+    default: window_load_kernel<kLoadCopy32><<<grid, block, 0, s>>>(a); break;
+  }
   return cudaGetLastError();
 }
 cudaError_t launch_narrow_i16(const int32_t* src, int16_t* dst, int64_t dstPitch, int64_t rows, int64_t cols, cudaStream_t s) {

@@ -83,8 +83,8 @@ struct CompactArgs {
   uint8_t* arena;
   uint64_t arenaCap;
   int32_t* status;
-  const int16_t* raw16;   // TileElementShort: raw tiles are copied from this 2-byte raster (pitch raw16Pitch), else nullptr
-  int64_t raw16Pitch;
+  int rawShorts;          // TileElementShort: raw tiles take 2 bytes per sample, narrowed from the int32 staging raster `grid`
+  int32_t fill16;         // ... with INT4_NULL_CODE -> the element's fill value (the inverse of window_load_kernel's widening)
 };
 
 struct ClassifyArgs {
@@ -146,8 +146,8 @@ cudaError_t launch_offsets(const uint32_t* lens, uint64_t* offsets, int nTiles, 
 cudaError_t launch_compact(const CompactArgs& a, int nTiles, cudaStream_t s);
 cudaError_t launch_classify(const ClassifyArgs& a, cudaStream_t s);
 cudaError_t launch_raw_decode(const DecodeArgs& a, int nTiles, cudaStream_t s);
-// TileElementShort (gvrs/TileElementShort.java:211-248): int16 raster <-> the int32 raster the codecs work on
-cudaError_t launch_widen_i16(const int16_t* src, int64_t srcPitch, int32_t* dst, int64_t rows, int64_t cols, int32_t fill, cudaStream_t s);
+// TileElementShort (gvrs/TileElementShort.java:236-248): the decoded int32 raster -> int16 (the encode side widens in
+// window_load_kernel)
 cudaError_t launch_narrow_i16(const int32_t* src, int16_t* dst, int64_t dstPitch, int64_t rows, int64_t cols, cudaStream_t s);
 // Integer-coded float elements: float32 <-> int32 codes over a pitched rectangle (pitches in samples; src may equal dst).
 // toFloat != 0 runs icf_to_float_kernel (codes -> values), else icf_to_int_kernel (values -> codes).
@@ -158,6 +158,25 @@ struct IcfMap {
 };
 cudaError_t launch_icf_map(int toFloat, const void* src, int64_t srcPitch, void* dst, int64_t dstPitch, int64_t rows, int64_t cols,
                            const IcfMap& m, cudaStream_t s);
+
+// Window writes (g4_encode_window, and the staging of every short encode): one pass from the caller's n_rows x n_cols raster
+// (any pitch) into the int32 staging raster of the covering tile grid (rows x cols cells, pitch dstPitch).  Cells inside the
+// raster are converted by `mode`, the cells outside it get the margin sample fillBits converted by the same rule, so that a
+// margin cell encodes exactly as if the caller had padded the raster with that sample.
+enum { kLoadCopy32 = 0, kLoadWiden16 = 1, kLoadIcfCode = 2 };  // how a source sample becomes a staged int32
+struct WindowLoad {
+  const void* src;        // int32 / float32 / int16 samples
+  int64_t srcPitch;       // samples per source row
+  int64_t nRows, nCols;   // the source raster
+  int32_t* dst;           // staging raster
+  int64_t dstPitch;       // samples per staging row
+  int64_t rows, cols;     // staged cells (rows >= nRows, cols >= nCols)
+  uint32_t fillBits;      // margin sample as a 32-bit pattern of the source type (the int16 in the low half for kLoadWiden16)
+  int32_t fill16;         // kLoadWiden16: the element's fill value, staged as INT4_NULL_CODE (TileElementShort.java:213-220)
+  int mode;               // kLoad*
+  IcfMap icf;             // kLoadIcfCode
+};
+cudaError_t launch_window_load(const WindowLoad& a, cudaStream_t s);
 
 // Window reads (g4_decode_window): the tiles tr0.. x tc0.. (nTd x nTa, "window tiles" w = wr * nTa + wc) of a raster whose
 // per-tile arrays are in tile-index order.  The gather copies the window tiles' payload locations into window order; a tile

@@ -483,6 +483,14 @@ class GvrsDeviceImage:
 
 
 # ---- GPU-backed primitives -------------------------------------------------------------------------------------------
+def _is_tensor(x):
+    """True for a torch tensor (torch is not imported for numpy callers)."""
+    import sys
+
+    torch = sys.modules.get("torch")
+    return torch is not None and isinstance(x, torch.Tensor)
+
+
 def _u8(buf):
     a = np.frombuffer(buf, dtype=np.uint8) if not isinstance(buf, np.ndarray) else buf
     return np.ascontiguousarray(a)
@@ -787,10 +795,54 @@ class GvrsWriter:
         full[:spec.n_rows, :spec.n_cols] = grid
         return master.encodeTiles(full, spec.tile_rows, spec.tile_cols, fillValue=e.fill_value if e.type_code == ELEM_SHORT else None)
 
-    def add_raster(self, master, grid):
-        """A whole one-element raster (numpy, n_rows x n_cols): encodeTiles on the GPU, then the tile records.  Returns the
-        TileBatch.  For an integer-coded float element, a float32 raster holds values and an int32 raster holds codes."""
+    def _encode_element_device(self, master, e, grid):
+        """encodeTiles of one element's raster held in a CUDA tensor: the tile grid is padded on the device with the sample
+        the host writer pads with (_encode_element), so the payloads are the same bytes."""
+        import torch
+
         spec = self.spec
+        dtypes = {ELEM_INTEGER: (torch.int32,), ELEM_FLOAT: (torch.float32,), ELEM_SHORT: (torch.int16,),
+                  ELEM_INT_CODED_FLOAT: (torch.float32, torch.int32)}[e.type_code]
+        if not grid.is_cuda or grid.device.index != master._context().device:
+            raise ValueError("a CUDA tensor on the device of the master's context")
+        if tuple(grid.shape) != (spec.n_rows, spec.n_cols):
+            raise ValueError("a raster of the specified dimensions (%d, %d)" % (spec.n_rows, spec.n_cols))
+        if grid.dtype not in dtypes:
+            raise ValueError("element %r takes %s tensors" % (e.name, " or ".join(str(d) for d in dtypes)))
+        if e.type_code == ELEM_INT_CODED_FLOAT and grid.dtype == torch.float32:
+            icf = e.icf
+            return master.encodeTiles(grid, spec.tile_rows, spec.tile_cols, icf=icf, padValue=icf.fill_value)
+        return master.encodeTiles(grid, spec.tile_rows, spec.tile_cols, fillValue=e.fill_value if e.type_code == ELEM_SHORT else None,
+                                  padValue=e.fill_value)
+
+    def _add_device_records(self, master, batches, multi):
+        """Tile records of device batches, framed and checksummed on the device; the records and their content positions
+        cross to the host once and are appended."""
+        ctx = master._context()
+        dev = batches[0].arena.device
+        ctx.after_torch_stream(dev)
+        if multi:
+            recs, pos = pack_tile_records_multi_device(ctx, batches, len(self.buf), self.spec.checksum)
+        else:
+            recs, pos = pack_tile_records_device(ctx, batches[0], len(self.buf), self.spec.checksum)
+        ctx.before_torch_stream(dev)
+        self.buf += memoryview(recs.cpu().numpy())
+        for t, p in enumerate(pos.cpu().tolist()):
+            self.tile_positions[t] = p
+        return pos
+
+    def add_raster(self, master, grid):
+        """A whole one-element raster (numpy or a CUDA tensor, n_rows x n_cols): encodeTiles on the GPU, then the tile
+        records.  Returns the TileBatch.  For an integer-coded float element, a float32 raster holds values and an int32
+        raster holds codes.  A CUDA tensor (rows contiguous, any pitch) is padded, encoded and framed on the device; only the
+        records come to the host, and the returned batch stays on the device."""
+        spec = self.spec
+        if _is_tensor(grid):
+            if len(spec.elements) != 1:
+                raise ValueError("add_raster: a one-element raster of the specified dimensions")
+            batch = self._encode_element_device(master, spec.elements[0], grid)
+            self._add_device_records(master, [batch], multi=False)
+            return batch
         if len(spec.elements) != 1 or grid.shape != (spec.n_rows, spec.n_cols):
             raise ValueError("add_raster: a one-element raster of the specified dimensions")
         batch = self._encode_element(master, spec.elements[0], grid)
@@ -801,8 +853,19 @@ class GvrsWriter:
         """Every element of a raster: grids[k] (numpy, n_rows x n_cols) is element k in specification order -- int32 for
         integer elements, float32 for float elements, int16 for short elements, and for integer-coded float elements float32
         values or int32 codes.  One encodeTiles per element, then one multi-element framing call.  Returns the TileBatch of
-        every element."""
+        every element.  The grids may instead all be CUDA tensors on one device, which take the device path of add_raster."""
         spec = self.spec
+        tensors = [_is_tensor(g) for g in grids]
+        if any(tensors):
+            if not all(tensors):
+                raise ValueError("add_rasters: numpy arrays and tensors cannot be mixed")
+            if len({g.device for g in grids}) != 1:
+                raise ValueError("add_rasters: every tensor on the same device")
+            if len(grids) != len(spec.elements):
+                raise ValueError("add_rasters: one raster of the specified dimensions per element")
+            batches = [self._encode_element_device(master, e, g) for e, g in zip(spec.elements, grids)]
+            self._add_device_records(master, batches, multi=True)
+            return batches
         if len(grids) != len(spec.elements) or any(np.shape(g) != (spec.n_rows, spec.n_cols) for g in grids):
             raise ValueError("add_rasters: one raster of the specified dimensions per element")
         batches = [self._encode_element(master, e, g) for e, g in zip(spec.elements, grids)]
@@ -830,9 +893,13 @@ class GvrsWriter:
         struct.pack_into("<qq", self.buf, FILEPOS_FREESPACE_DIR, 0, md_pos)
         struct.pack_into("<q", self.buf, FILEPOS_TILE_DIR, td_pos)
         if self.spec.checksum and context is not None:
-            off = np.array([p for p, _ in self.record_spans], dtype=np.uint64)
+            # the records framed here (header, metadata, directories) are a few kilobytes: checksum a compact copy of them,
+            # not the whole image (the tile records carry the checksums the GPU framing computed)
             size = np.array([s - 4 for _, s in self.record_spans], dtype=np.uint32)
-            crc = crc32c_ranges(context, self.buf, off, size)
+            off = np.concatenate([[0], np.cumsum(size, dtype=np.uint64)[:-1]]).astype(np.uint64)
+            with memoryview(self.buf) as mv:
+                spans = b"".join(mv[p:p + s - 4] for p, s in self.record_spans)
+            crc = crc32c_ranges(context, spans, off, size)
             for (p, s), c in zip(self.record_spans, crc):
                 struct.pack_into("<I", self.buf, p + s - 4, int(c))
         return bytes(self.buf)

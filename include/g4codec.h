@@ -244,6 +244,30 @@ int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
                      const int32_t* tile_status, uint32_t fill_bits, int64_t row0, int64_t col0, int64_t n_rows, int64_t n_cols,
                      void* out, int64_t out_pitch, int32_t* status);
 
+/* ---- window writes: a raster of any dimensions on the device, padded to whole tiles there --------------------------------
+ * g4_encode_tiles (or g4_encode_tiles_icf) of the n_rows x n_cols raster at src (row pitch src_pitch samples) padded to the
+ * tile grid with the margin sample fill_bits: the same arena bytes, offsets, lengths, codec and predictor bytes, statuses
+ * and total, and the LSOP12 option bits act as there (a value checksum covers the padded tile).  Every pointer is a device
+ * pointer (host writers keep g4_encode_tiles).
+ *   raster     element type and tile geometry of the whole tile grid: tiles_down == ceil(n_rows / tile_rows) and
+ *              tiles_across == ceil(n_cols / tile_cols).  grid_pitch is not used beyond check_band's rule (tiles_across *
+ *              tile_cols will do); fill_value is the short element's fill, coded as null, as in g4_encode_tiles.
+ *              G4_ELEM_I32 / F32 / I16, or G4_ELEM_ICF together with `icf`: src then holds float32 values, mapped to codes.
+ *              To write an ICF element's codes, pass G4_ELEM_I32 and no descriptor.
+ *   fill_bits  the margin sample as a 32-bit pattern of the source type: float bits for float32 and ICF values, the int
+ *              for int32, the int16 in the low half for G4_ELEM_I16 (the convention of g4_decode_window).  A margin cell
+ *              is converted as a raster cell is: a short equal to fill_value becomes null, an ICF value is mapped.
+ * A tile-aligned int32 / float32 raster is encoded straight from src with the launches of g4_encode_tiles.  Any other raster
+ * takes one load pass into an int32 staging raster of 4 bytes per sample of the tile grid, in device memory the context
+ * keeps; for short and ICF elements that pass replaces the widening / mapping launch, so the launch count is that of
+ * g4_encode_tiles(_icf), and for an unaligned int32 / float32 raster it is one more.
+ * G4_ERR_ARG for an empty raster, tile counts that do not cover it exactly, src_pitch < n_cols, a bad `raster`, or an `icf`
+ * for a non-ICF element or with an invalid scale; tiles thinner than 2 x 2 are G4_ERR_UNSUPPORTED as in g4_encode_tiles. */
+int g4_encode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf, int64_t n_rows,
+                     int64_t n_cols, const void* src, int64_t src_pitch, uint32_t fill_bits, uint8_t* arena, uint64_t arena_cap,
+                     uint64_t* offsets, uint32_t* lens, uint8_t* codec_out, uint8_t* predictor_out, int32_t* status,
+                     uint64_t* total_bytes);
+
 /* ---- tile LISTS: scattered tiles of one size (the tile cache's callers) -------------------------------------------------
  * The band calls above take one rectangle of one raster.  A tile cache flushes whatever tiles are dirty, each in its own
  * int[] (gvrs/RasterTileCache.java:253-294, RasterTile.getCompressedPacking :234-256), and a block read lands tiles in a
