@@ -117,6 +117,8 @@ struct g4_context {
   DevBuf sGrid, sArena, sOffsets, sLens, sCodec, sPred, sStatus;
   // g4_decode_window: payload locations of the window tiles, absent-tile flags, int32 staging band of unaligned windows
   DevBuf winOff, winLen, winAbsent, winStage;
+  // g4_decode_points: per-tile touched flags (zero between calls), per-tile slots, {bad point, K} (bad point zero between calls)
+  DevBuf ptFlag, ptSlot, ptInfo;
   // host-buffer decode pipeline: payload H2D / kernels / raster D2H of consecutive chunks overlap
   cudaStream_t copyIn = nullptr, copyOut = nullptr;
   cudaEvent_t evIn[16] = {}, evDone[16] = {}, evStart = nullptr, evOrder = nullptr;
@@ -781,7 +783,7 @@ void g4_context_destroy(g4_context* ctx) {
                     &ctx->streamIn, &ctx->streamOut, &ctx->deflateWork, &ctx->stSorted, &ctx->stRank, &ctx->stTable,
                     &ctx->stWork, &ctx->stCounters, &ctx->rcPos, &ctx->rcOff, &ctx->rcLen, &ctx->rcCrc, &ctx->rcStored, &ctx->rcTotal,
                     &ctx->rcData, &ctx->rcOffsets, &ctx->rcLens, &ctx->rcIndex, &ctx->rcStatus, &ctx->rcOut, &ctx->rcChain, &ctx->rcDesc, &ctx->sGrid, &ctx->sArena, &ctx->sOffsets, &ctx->sLens, &ctx->sCodec, &ctx->sPred, &ctx->sStatus,
-                    &ctx->winOff, &ctx->winLen, &ctx->winAbsent, &ctx->winStage};
+                    &ctx->winOff, &ctx->winLen, &ctx->winAbsent, &ctx->winStage, &ctx->ptFlag, &ctx->ptSlot, &ctx->ptInfo};
   for (DevBuf* b : bufs) b->release();
   if (ctx->ownStream) cudaStreamDestroy(ctx->stream);
   delete ctx;
@@ -1532,6 +1534,121 @@ int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   if (ctx->asyncDevice) return G4_OK;  // enqueued; status[] is read by the caller after g4_context_synchronize
   std::vector<int32_t> st(nW);
   CK(cudaMemcpyAsync(st.data(), status, size_t(nW) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  for (int32_t& s : st)
+    if (s == G4_DECLINED) s = G4_OK;  // absent tiles read as fill values; they are neither errors nor notes
+  return first_bad_status(st);
+}
+
+// ---- point reads: GvrsElement.readValue / readValueInt (gvrs/GvrsElementInt.java:85-95) on the device -----------------------
+// mark (touched tiles) -> compact (their payload locations in tile order) -> one readback of {bad point, K} -> classify +
+// decoders on the K touched tiles as a K x 1 band in the int32 staging buffer of g4_decode_window -> store (one thread per
+// point).  Launches beyond those of g4_decode_tiles_bounded on the same K tiles: exactly three (mark, compact, store).
+static bool device_pointer(const g4_context* ctx, const void* p) {  // a host or another GPU's array is refused, not faulted on
+  cudaPointerAttributes at{};
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+    cudaGetLastError();  // not left for the next launch check to find
+    return false;
+  }
+  return (at.type == cudaMemoryTypeDevice && at.device == ctx->device) || at.type == cudaMemoryTypeManaged;
+}
+
+int g4_decode_points(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf, const uint8_t* image,
+                     uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens, const int32_t* tile_status, uint32_t fill_bits,
+                     int64_t raster_rows, int64_t raster_cols, int64_t n_points, const int64_t* rows, const int64_t* cols, void* out,
+                     int32_t* tiles_out, int32_t* status, int32_t* n_tiles_out) {
+  if (!ctx || !codecs || !image || !payload_offsets || !lens || !tile_status || !n_tiles_out) return G4_ERR_ARG;
+  *n_tiles_out = 0;
+  if (n_points < 0 || (n_points > 0 && (!rows || !cols || !out || !tiles_out || !status))) return G4_ERR_ARG;
+  int rc = check_band(raster, icf != nullptr);
+  if (rc != G4_OK) return rc;
+  if (icf && !icf_valid(icf)) return G4_ERR_ARG;
+  const int R = raster->tile_rows, Cc = raster->tile_cols;
+  if (raster_rows < 1 || raster_cols < 1 || raster_rows > int64_t(raster->tiles_down) * R || raster_cols > int64_t(raster->tiles_across) * Cc)
+    return G4_ERR_ARG;
+  g4_codec_list ids;
+  int opts[G4_MAX_CODECS];
+  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
+  codecs = &ids;
+  if (n_points == 0) return G4_OK;
+  ENTER(ctx);
+  for (const void* p : {(const void*)rows, (const void*)cols, (const void*)out, (const void*)tiles_out, (const void*)status})
+    if (!device_pointer(ctx, p)) return G4_ERR_ARG;
+  const int nTiles = raster->tiles_down * raster->tiles_across;
+  const int kMax = int(std::min<int64_t>(n_points, nTiles));
+  const size_t flagCap = ctx->ptFlag.cap, infoCap = ctx->ptInfo.cap;
+  CK(ctx->ptFlag.ensure(round_up(size_t(nTiles), 16)));
+  CK(ctx->ptInfo.ensure(8));
+  if (ctx->ptFlag.cap != flagCap) CK(cudaMemsetAsync(ctx->ptFlag.p, 0, ctx->ptFlag.cap, ctx->stream));
+  if (ctx->ptInfo.cap != infoCap) CK(cudaMemsetAsync(ctx->ptInfo.p, 0, ctx->ptInfo.cap, ctx->stream));
+  CK(ctx->ptSlot.ensure(size_t(nTiles) * 4));
+  CK(ctx->winOff.ensure(size_t(kMax) * 8));
+  CK(ctx->winLen.ensure(size_t(kMax) * 4));
+  CK(ctx->winAbsent.ensure(size_t(kMax)));
+  PointArgs pa{};
+  pa.rows = rows;
+  pa.cols = cols;
+  pa.n = n_points;
+  pa.rasterRows = raster_rows;
+  pa.rasterCols = raster_cols;
+  pa.R = R;
+  pa.C = Cc;
+  pa.tilesAcross = raster->tiles_across;
+  pa.nTiles = nTiles;
+  pa.flag = ctx->ptFlag.as<uint8_t>();
+  pa.info = ctx->ptInfo.as<int32_t>();
+  pa.slot = ctx->ptSlot.as<int32_t>();
+  pa.offsets = payload_offsets;
+  pa.lens = lens;
+  pa.tileStatus = tile_status;
+  pa.tilesOut = tiles_out;
+  pa.offK = ctx->winOff.as<uint64_t>();
+  pa.lenK = ctx->winLen.as<uint32_t>();
+  pa.absentK = ctx->winAbsent.as<uint8_t>();
+  CK(launch_point_mark(pa, ctx->smCount, ctx->stream));
+  ctx->launches++;
+  CK(launch_point_compact(pa, ctx->stream));
+  ctx->launches++;
+  int32_t info[2] = {0, 0};  // the decoder launches are sized on the host: this call waits here even under g4_context_set_async
+  CK(cudaMemcpyAsync(info, ctx->ptInfo.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (info[0]) {
+    CK(cudaMemsetAsync(ctx->ptInfo.p, 0, 4, ctx->stream));
+    return G4_ERR_ARG;
+  }
+  const int K = info[1];
+  *n_tiles_out = K;
+  struct ArenaScope {  // payloads that leave the image are G4_ERR_FORMAT, as in g4_decode_tiles_bounded
+    g4_context* c;
+    ~ArenaScope() { c->arenaLimit = ~0ull; }
+  } arenaScope{ctx};
+  ctx->arenaLimit = image_len;
+  g4_band_desc b = *raster;  // the touched tiles one under the other: tile k at k * R * C, int32 samples
+  b.tiles_down = K;
+  b.tiles_across = 1;
+  b = widened(b);
+  if (raster->elem_type == G4_ELEM_F32) b.elem_type = G4_ELEM_F32;
+  CK(ctx->winStage.ensure(band_samples(b) * 4));
+  rc = decode_device_i32(ctx, codecs, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), ctx->winStage.p, status,
+                         raster->elem_type == G4_ELEM_I16);
+  if (rc != G4_OK) return rc;
+  WindowStore ws{};
+  ws.stage = ctx->winStage.as<int32_t>();
+  ws.out = out;
+  ws.R = R;
+  ws.C = Cc;
+  ws.nTa = 1;
+  ws.nW = K;
+  ws.absent = ctx->winAbsent.as<uint8_t>();
+  ws.status = status;
+  ws.fillBits = fill_bits;
+  ws.mode = raster->elem_type == G4_ELEM_I16 ? kWindowNarrow16 : icf ? kWindowIcfFloat : kWindowCopy32;
+  if (icf) ws.icf = icf_of(icf);
+  CK(launch_point_store(pa, ws, ctx->smCount, ctx->stream));
+  ctx->launches++;
+  if (ctx->asyncDevice) return G4_OK;  // enqueued; status[] is read by the caller after g4_context_synchronize
+  std::vector<int32_t> st(K);
+  CK(cudaMemcpyAsync(st.data(), status, size_t(K) * 4, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   for (int32_t& s : st)
     if (s == G4_DECLINED) s = G4_OK;  // absent tiles read as fill values; they are neither errors nor notes

@@ -433,6 +433,115 @@ cudaError_t launch_window_store(const WindowStore& a, int smCount, cudaStream_t 
   return cudaGetLastError();
 }
 
+// ---- point reads (g4_decode_points, GvrsElement.readValue / readValueInt) ------------------------------------------------
+// One thread per point.  Every thread that flags a tile stores the same 1, and every out-of-range point the same error.
+// (Loading the flag first and storing only a 0 measured slower: the loads queue on the same few L2 lines, DESIGN §6.2.6.)
+__global__ void __launch_bounds__(256) point_mark_kernel(PointArgs a) {
+  for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < a.n; i += int64_t(gridDim.x) * blockDim.x) {
+    const int64_t r = a.rows[i], c = a.cols[i];
+    if (r < 0 || c < 0 || r >= a.rasterRows || c >= a.rasterCols) {
+      a.info[0] = 1;
+      continue;
+    }
+    a.flag[(r / a.R) * a.tilesAcross + c / a.C] = 1;
+  }
+}
+
+// One CTA scans the whole flag array, 16 flags (one 16-byte load) per thread and 16,384 per round, so that any tile count
+// is covered; a touched tile is written out at its rank and its flags are cleared.
+constexpr int kCompactThreads = 1024;
+__global__ void __launch_bounds__(kCompactThreads) point_compact_kernel(PointArgs a) {
+  __shared__ int warpSum[kCompactThreads / 32];
+  __shared__ int carry;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (threadIdx.x == 0) carry = 0;
+  __syncthreads();
+  for (int base = 0; base < a.nTiles; base += 16 * kCompactThreads) {
+    const int t0 = base + 16 * int(threadIdx.x);
+    uint4 f = make_uint4(0, 0, 0, 0);
+    if (t0 < a.nTiles) f = *reinterpret_cast<const uint4*>(a.flag + t0);
+    const int cnt = __popc(f.x) + __popc(f.y) + __popc(f.z) + __popc(f.w);  // flags are 0 / 1 bytes
+    int inc = cnt;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, inc, d);
+      if (lane >= d) inc += y;
+    }
+    if (lane == 31) warpSum[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+      int v = warpSum[lane];
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const int y = __shfl_up_sync(0xffffffffu, v, d);
+        if (lane >= d) v += y;
+      }
+      warpSum[lane] = v;
+    }
+    __syncthreads();
+    if (cnt) {
+      int k = carry + (warp ? warpSum[warp - 1] : 0) + inc - cnt;
+      const uint32_t words[4] = {f.x, f.y, f.z, f.w};
+#pragma unroll
+      for (int j = 0; j < 4; j++)
+#pragma unroll
+        for (int b = 0; b < 4; b++) {
+          if (!((words[j] >> (8 * b)) & 0xffu)) continue;
+          const int t = t0 + 4 * j + b;
+          const int32_t st = a.tileStatus[t];
+          a.slot[t] = k;
+          a.tilesOut[k] = t;
+          a.offK[k] = st == G4_OK ? a.offsets[t] : 0;
+          a.lenK[k] = st == G4_OK ? a.lens[t] : 0u;
+          a.absentK[k] = st == G4_DECLINED ? 1 : 0;
+          k++;
+        }
+      *reinterpret_cast<uint4*>(a.flag + t0) = make_uint4(0, 0, 0, 0);
+    }
+    __syncthreads();
+    // the last thread alone reads warpSum[31] here, and it is also the only thread that writes it in the next round
+    if (threadIdx.x == kCompactThreads - 1) carry += warpSum[kCompactThreads / 32 - 1];
+  }
+  if (threadIdx.x == kCompactThreads - 1) a.info[1] = carry;
+}
+
+template <int Mode>
+__global__ void __launch_bounds__(256) point_store_kernel(PointArgs p, WindowStore a) {
+  using T = typename WindowOut<Mode>::T;
+  window_mark_absent(a);
+  const T fill = window_fill<Mode>(a);
+  const int64_t tileCells = int64_t(a.R) * a.C;
+  for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < p.n; i += int64_t(gridDim.x) * blockDim.x) {
+    const int64_t r = p.rows[i], c = p.cols[i];
+    const int64_t tr = r / a.R, tc = c / a.C;
+    const int k = p.slot[tr * p.tilesAcross + tc];
+    const int32_t v = a.stage[k * tileCells + (r - tr * a.R) * a.C + (c - tc * a.C)];
+    static_cast<T*>(a.out)[i] = a.absent[k] ? fill : window_sample<Mode>(v, a);
+  }
+}
+
+static unsigned point_blocks(int64_t n, int smCount) {
+  const int64_t b = (n + 255) / 256, cap = int64_t(smCount) * 32;
+  return unsigned(b < cap ? b : cap);
+}
+cudaError_t launch_point_mark(const PointArgs& a, int smCount, cudaStream_t s) {
+  point_mark_kernel<<<point_blocks(a.n, smCount), 256, 0, s>>>(a);
+  return cudaGetLastError();
+}
+cudaError_t launch_point_compact(const PointArgs& a, cudaStream_t s) {
+  point_compact_kernel<<<1, kCompactThreads, 0, s>>>(a);
+  return cudaGetLastError();
+}
+cudaError_t launch_point_store(const PointArgs& p, const WindowStore& w, int smCount, cudaStream_t s) {
+  const unsigned nb = point_blocks(p.n, smCount);
+  switch (w.mode) {
+    case kWindowNarrow16: point_store_kernel<kWindowNarrow16><<<nb, 256, 0, s>>>(p, w); break;
+    case kWindowIcfFloat: point_store_kernel<kWindowIcfFloat><<<nb, 256, 0, s>>>(p, w); break;
+    default: point_store_kernel<kWindowCopy32><<<nb, 256, 0, s>>>(p, w); break;
+  }
+  return cudaGetLastError();
+}
+
 cudaError_t launch_fill_terrain(int elemType, uint64_t seed, int64_t row0, int64_t col0, int64_t nRows, int64_t nCols, void* out,
                                 cudaStream_t s) {
   fill_terrain_kernel<<<148 * 8, 256, 0, s>>>(elemType, seed, row0, col0, nRows, nCols, out);

@@ -203,6 +203,35 @@ struct WindowStore {
 // decoded straight into out; only the absent ones are filled.
 cudaError_t launch_window_store(const WindowStore& a, int smCount, cudaStream_t s);
 
+// Point reads (g4_decode_points): cell (rows[i], cols[i]) of the raster for each of n points.  The mark pass sets flag[t]
+// for every tile a point falls in (info[0] = 1 for a point outside the raster); the compaction pass, one CTA, scans the
+// flags in tile-index order: the k-th touched tile t gets slot[t] = k, tilesOut[k] = t, its payload location and absent flag
+// as launch_window_gather gives them, and info[1] = K.  The compaction leaves every flag zero again, so the flag array
+// (nTiles rounded up to 16 bytes, zero padded) is zero between calls; info[0] is cleared by the caller that reads it set.
+struct PointArgs {
+  const int64_t* rows;
+  const int64_t* cols;
+  int64_t n;
+  int64_t rasterRows, rasterCols;  // points must lie in [0, rasterRows) x [0, rasterCols)
+  int R, C, tilesAcross, nTiles;
+  uint8_t* flag;                   // [nTiles rounded up to 16]
+  int32_t* info;                   // [0] a point outside the raster, [1] K
+  int32_t* slot;                   // [nTiles]: valid for touched tiles
+  const uint64_t* offsets;         // per tile of the raster, tile-index order
+  const uint32_t* lens;
+  const int32_t* tileStatus;
+  int32_t* tilesOut;               // [K] touched tiles, ascending
+  uint64_t* offK;                  // [K] payload locations in slot order (zero-length for tiles not G4_OK)
+  uint32_t* lenK;
+  uint8_t* absentK;                // [K] 1 for G4_DECLINED
+};
+cudaError_t launch_point_mark(const PointArgs& a, int smCount, cudaStream_t s);
+cudaError_t launch_point_compact(const PointArgs& a, cudaStream_t s);
+// w.stage holds the K touched tiles decoded as a K x 1 band (tile k at k * R * C, pitch C); w.absent / w.status are in slot
+// order (w.nW = K).  out[i] = the converted sample of point i, or the fill sample for an absent tile; absent tiles' status
+// becomes G4_DECLINED.
+cudaError_t launch_point_store(const PointArgs& p, const WindowStore& w, int smCount, cudaStream_t s);
+
 // ---- codec kernels -----------------------------------------------------------------------------
 // Host-side launchers (defined next to their kernels).  nCtas persistent CTAs of kThreads threads.
 cudaError_t launch_huffman_encode(const EncodeArgs& a, int nCtas, cudaStream_t s);

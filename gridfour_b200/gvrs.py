@@ -408,7 +408,8 @@ class GvrsDeviceImage:
         self.image, self.payload_off, self.lens, self.status = image, payload_off, lens, status  # [n] / [E, n] / [E, n] / [n]
         self.context = context
         self.device = image.device
-        self.lastStatus = None  # per covering tile of the latest read, window-tile order (device tensor)
+        self.lastStatus = None  # per covering tile of the latest read, window-tile order (device tensor); read_values: per lastTiles
+        self.lastTiles = None   # read_values: the tiles the latest point read touched, ascending tile index (device tensor)
 
     def _element(self, element):
         if not 0 <= element < len(self.spec.elements):
@@ -436,7 +437,51 @@ class GvrsDeviceImage:
             return self._read(master, 0, 0, spec.n_rows, spec.n_cols, element, as_float, None)
         return self._read(master, 0, 0, spec.tiles_down * spec.tile_rows, spec.tiles_across * spec.tile_cols, element, as_float, None)
 
-    def _read(self, master, row, col, n_rows, n_cols, element, as_float, out):
+    def read_values(self, master, rows, cols, element=0, as_float=False, out=None):
+        """GvrsElement.readValueInt / readValue for many cells at once: the values at (rows[i], cols[i]), with the dtype
+        read_block gives the element.  rows and cols are integer CUDA tensors (int32 or int64) of one shape on the image's
+        device; the result has that shape.  Points may repeat and come in any order; each tile they touch is decoded once
+        (g4_decode_points).  A point outside the raster raises ValueError.  `out`, if given, is a contiguous tensor of that
+        dtype and shape.  Afterwards lastTiles holds the touched tile indices (ascending) and lastStatus their statuses."""
+        import torch
+
+        self._element(element)
+        for name, x in (("rows", rows), ("cols", cols)):
+            if not (isinstance(x, torch.Tensor) and x.device == self.device and x.dtype in (torch.int32, torch.int64)):
+                raise ValueError("%s: an int32 or int64 tensor on %s" % (name, self.device))
+        if rows.shape != cols.shape:
+            raise ValueError("rows and cols differ in shape")
+        band, dtype, fill, icf = self._layout(element, as_float)
+        shape = tuple(rows.shape)
+        if out is None:
+            out = torch.empty(shape, dtype=dtype, device=self.device)
+        elif not (isinstance(out, torch.Tensor) and out.device == self.device and out.dtype == dtype and tuple(out.shape) == shape
+                  and out.is_contiguous()):
+            raise ValueError("out: a contiguous %s tensor of shape %s on %s" % (dtype, shape, self.device))
+        r = rows.to(torch.int64).contiguous()
+        c = cols.to(torch.int64).contiguous()
+        spec = self.spec
+        k_max = min(r.numel(), spec.tiles_down * spec.tiles_across)
+        tiles = torch.empty(k_max, dtype=torch.int32, device=self.device)
+        status = torch.empty(k_max, dtype=torch.int32, device=self.device)
+        k = C.c_int32(0)
+        d = icf.desc() if icf is not None else None
+        ctx = self.context
+        ctx.after_torch_stream(self.device)  # the index copies above and `out` are on torch's stream
+        st = _lib.lib().g4_decode_points(ctx._h, C.byref(master._native_list()), C.byref(band), None if d is None else C.byref(d),
+                                         self.image.data_ptr(), int(self.image.numel()), self.payload_off[element].data_ptr(),
+                                         self.lens[element].data_ptr(), self.status.data_ptr(), fill, spec.n_rows, spec.n_cols,
+                                         r.numel(), r.data_ptr(), c.data_ptr(), out.data_ptr(), tiles.data_ptr(), status.data_ptr(),
+                                         C.byref(k))
+        ctx.before_torch_stream(self.device)
+        self.lastTiles, self.lastStatus = tiles[:k.value], status[:k.value]
+        if st == _lib.G4_ERR_ARG:
+            raise ValueError("a point outside the raster")
+        check(st, "g4_decode_points")
+        return out
+
+    def _layout(self, element, as_float):
+        """The band descriptor, output dtype, fill-sample bits and ICF mapping (or None) of one element's reads."""
         import torch
 
         from ._lib import G4_ELEM_F32, G4_ELEM_I16, G4_ELEM_I32, G4_ELEM_ICF, BandDesc
@@ -460,6 +505,13 @@ class GvrsDeviceImage:
         else:
             band.elem_type, dtype = G4_ELEM_I32, torch.int32
             fill = e.fill_value & 0xffffffff
+        return band, dtype, fill, icf
+
+    def _read(self, master, row, col, n_rows, n_cols, element, as_float, out):
+        import torch
+
+        spec = self.spec
+        band, dtype, fill, icf = self._layout(element, as_float)
         if out is None:
             out = torch.empty((n_rows, n_cols), dtype=dtype, device=self.device)
         elif not (isinstance(out, torch.Tensor) and out.device == self.device and out.dtype == dtype and out.dim() == 2

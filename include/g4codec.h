@@ -244,6 +244,35 @@ int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
                      const int32_t* tile_status, uint32_t fill_bits, int64_t row0, int64_t col0, int64_t n_rows, int64_t n_cols,
                      void* out, int64_t out_pitch, int32_t* status);
 
+/* ---- point reads: GvrsElement.readValueInt / readValue on the device, batched (C/gvrs/GvrsElementInt.java:85-95) ---------
+ * out[i] = the value at cell (rows[i], cols[i]) of one element of a raster whose file image is resident on the device, for
+ * i < n_points.  Every pointer except n_tiles_out is a device pointer; rows, cols, out, tiles_out or status in host memory
+ * or on another device are refused.
+ * Each tile that points fall in is decoded once, however many points it holds; points may repeat and come in any order.
+ *   raster, icf, image, image_len, payload_offsets, lens, tile_status, fill_bits
+ *                as in g4_decode_window; a cell is converted exactly as there (int32 / float32 bits copied, G4_ELEM_I16
+ *                narrowed with null -> -32768, G4_ELEM_ICF with `icf` mapped to float32, cells of absent tiles = fill_bits).
+ *   raster_rows, raster_cols
+ *                the raster's extent, at most the tile grid's: a point must lie in [0, raster_rows) x [0, raster_cols), so
+ *                cells in the fill margin of the edge tiles are refused, as g4_decode_window's callers refuse them.
+ *   tiles_out    the K distinct touched tiles, ascending tile index; *n_tiles_out = K (host pointer).
+ *   status       status[k] of tiles_out[k], with the meanings of g4_decode_window's status.
+ *                Size tiles_out and status as min(n_points, tiles_down * tiles_across).
+ * Returns the first bad status, absent tiles not counted, as g4_decode_window does; with g4_context_set_async the decode is
+ * only enqueued and G4_OK returned, but the call always waits once first: the touched-tile count and a flag for points
+ * outside the raster come back to the host in one small copy, since the decoder launches are sized from them.
+ * G4_ERR_ARG, with nothing decoded and `out` not written, for n_points < 0, a bad `raster` or `icf` (as g4_decode_window),
+ * a raster extent larger than the tile grid, or any point outside the raster.  n_points == 0 returns G4_OK with K = 0 and
+ * launches nothing; rows, cols, out, tiles_out and status may then be null.
+ * The K touched tiles are decoded into an int32 staging buffer of 4 * K * tile_rows * tile_cols bytes, in device memory the
+ * context keeps (that of g4_decode_window); with every tile touched this is the bound of a whole-raster unaligned window.
+ * Launches: those of g4_decode_tiles_bounded on the K tiles, plus three (mark, compact, store). */
+int g4_decode_points(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf,
+                     const uint8_t* image, uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens,
+                     const int32_t* tile_status, uint32_t fill_bits, int64_t raster_rows, int64_t raster_cols,
+                     int64_t n_points, const int64_t* rows, const int64_t* cols, void* out,
+                     int32_t* tiles_out, int32_t* status, int32_t* n_tiles_out);
+
 /* ---- window writes: a raster of any dimensions on the device, padded to whole tiles there --------------------------------
  * g4_encode_tiles (or g4_encode_tiles_icf) of the n_rows x n_cols raster at src (row pitch src_pitch samples) padded to the
  * tile grid with the margin sample fill_bits: the same arena bytes, offsets, lengths, codec and predictor bytes, statuses
