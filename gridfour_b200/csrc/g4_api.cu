@@ -32,9 +32,15 @@ int cuda_fail(cudaError_t e, const char* what) {
     if (e_ != cudaSuccess) return cuda_fail(e_, #call);    \
   } while (0)
 
-struct DevBuf {
+struct DevBuf {  // a device allocation that grows on demand and is freed with its owner
   void* p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() {
+    if (p) cudaFree(p);
+  }
   cudaError_t ensure(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
     if (p) cudaFree(p);
@@ -44,11 +50,6 @@ struct DevBuf {
     cudaError_t e = cudaMalloc(&p, want);
     if (e == cudaSuccess) cap = want;
     return e;
-  }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
   }
   template <class T>
   T* as() const { return static_cast<T*>(p); }
@@ -107,12 +108,7 @@ struct g4_context {
   uint64_t hostTotal = 0;
   int deflateWorkers = 0;   // resident stream-worker threads (0 = default, see g4_context_create)
   uint64_t stagedChunkBytes = 2ull << 30;  // staged zlib encode: input bytes per chunk (scratch = 12x)
-  const int64_t* curTileOffset = nullptr;  // tile-list calls: device {offset, pitch} tables of the running call
-  const int64_t* curTilePitch = nullptr;
   DevBuf tileRefs;      // device copy of the tile references of a tile-list call
-  uint64_t arenaLimit = ~0ull;  // g4_decode_tiles_bounded: bytes addressable behind the arena of the running call
-  bool icfOn = false;           // g4_encode_tiles_icf / g4_decode_tiles_icf: the running call's band is G4_ELEM_ICF ...
-  g4::IcfMap icf{};             // ... mapped with this descriptor
   // staging used by the host-memory entry points
   DevBuf sGrid, sArena, sOffsets, sLens, sCodec, sPred, sStatus;
   // g4_decode_window: payload locations of the window tiles, absent-tile flags, int32 staging band of unaligned windows
@@ -127,6 +123,20 @@ struct g4_context {
   bool asyncDevice = false;  // g4_context_set_async: device batches are enqueued, not awaited
   cudaEvent_t ev[2][G4_CODEC_COUNT + 1][2] = {};
   bool evUsed[2][G4_CODEC_COUNT + 1] = {};
+
+  // Runs on the context's device with its streams idle (g4_context_destroy); the DevBuf members free themselves after it.
+  ~g4_context() {
+    if (copyIn) cudaStreamDestroy(copyIn);
+    if (copyOut) cudaStreamDestroy(copyOut);
+    for (cudaEvent_t e : evIn) if (e) cudaEventDestroy(e);
+    for (cudaEvent_t e : evDone) if (e) cudaEventDestroy(e);
+    if (evStart) cudaEventDestroy(evStart);
+    if (evOrder) cudaEventDestroy(evOrder);
+    for (auto& dir : ev)
+      for (auto& kind : dir)
+        for (cudaEvent_t e : kind) if (e) cudaEventDestroy(e);
+    if (ownStream) cudaStreamDestroy(stream);
+  }
 };
 
 namespace {
@@ -411,15 +421,30 @@ int split_codec_id(int32_t entry, int32_t* id, int* opts) {
   *opts = entry & kLsop12Options;
   return G4_OK;
 }
-int split_codec_list(const g4_codec_list* in, g4_codec_list* ids, int* opts) {
+struct CodecList {
+  g4_codec_list ids;
+  int opts[G4_MAX_CODECS];  // decode ignores them: they describe how to encode, the packings say the rest
+};
+int split_codec_list(const g4_codec_list* in, CodecList* out) {
   if (in->n_codecs < 0 || in->n_codecs > G4_MAX_CODECS) return G4_ERR_ARG;
-  *ids = *in;
+  out->ids = *in;
   for (int k = 0; k < in->n_codecs; k++)
-    if (split_codec_id(in->codec_ids[k], &ids->codec_ids[k], &opts[k]) != G4_OK) return G4_ERR_ARG;
+    if (split_codec_id(in->codec_ids[k], &out->ids.codec_ids[k], &out->opts[k]) != G4_OK) return G4_ERR_ARG;
   return G4_OK;
 }
 
-int check_band(const g4_band_desc* b, bool icf = false) {  // icf: the band of a g4_*_tiles_icf call
+// What one call of an entry point adds to its band and codec list; the entry point builds it, the helpers take it along.
+struct CallSettings {
+  uint64_t arenaLen = ~0ull;          // bytes addressable behind the arena (~0: the caller vouches for the directory)
+  const g4_icf_desc* icf = nullptr;   // the G4_ELEM_ICF band's descriptor, null for every other band
+  const int64_t* tileOffset = nullptr;  // tile-list calls on device memory: per-tile {offset, pitch} tables on the device
+  const int64_t* tilePitch = nullptr;
+};
+
+bool icf_valid(const g4_icf_desc* icf) { return icf && icf->scale != 0.0f && std::isfinite(icf->scale); }
+g4::IcfMap icf_of(const g4_icf_desc* icf) { return g4::IcfMap{icf->scale, icf->offset, icf->fill_int, icf->fill_value}; }
+
+int check_band(const g4_band_desc* b, bool icf = false) {  // icf: the band of a call that carries a g4_icf_desc
   if (!b) return G4_ERR_ARG;
   if (icf ? b->elem_type != G4_ELEM_ICF : b->elem_type != G4_ELEM_I32 && b->elem_type != G4_ELEM_F32 && b->elem_type != G4_ELEM_I16)
     return G4_ERR_ARG;
@@ -432,6 +457,13 @@ int check_band(const g4_band_desc* b, bool icf = false) {  // icf: the band of a
 }
 
 size_t elem_bytes(const g4_band_desc& b) { return b.elem_type == G4_ELEM_I16 ? 2 : 4; }
+// The raster of a resident-image call (g4_decode_window, g4_decode_points, g4_encode_window) and its optional ICF descriptor.
+int check_raster(const g4_band_desc* raster, const g4_icf_desc* icf) {
+  const int rc = check_band(raster, icf != nullptr);
+  if (rc != G4_OK) return rc;
+  return icf && !icf_valid(icf) ? G4_ERR_ARG : G4_OK;
+}
+
 // TileElement.standardSizeInBytes (gvrs/TileElement.java:85-93): 4n, or 2n rounded up to a multiple of 4 for shorts
 uint32_t standard_size(const g4_band_desc& b) {
   const uint32_t n = uint32_t(b.tile_rows) * uint32_t(b.tile_cols);
@@ -444,15 +476,15 @@ size_t band_samples(const g4_band_desc& b) {
 
 // Encode with every applicable codec of `codecs`, select, compact.  All pointers are device pointers.
 // slotBytes: capacity of each candidate slot.
-int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const int* opts, const g4_band_desc* band, void* grid, uint8_t* arena,
-                      uint64_t arenaCap, uint64_t* offsets, uint32_t* lens, uint8_t* codecOut, uint8_t* predOut, int32_t* status,
-                      uint64_t* totalHost, size_t slotBytes, bool rawShorts, int32_t fill16) {
+int encode_device_i32(g4_context* ctx, const CodecList& codecs, const g4_band_desc* band, void* grid, uint8_t* arena, uint64_t arenaCap,
+                      uint64_t* offsets, uint32_t* lens, uint8_t* codecOut, uint8_t* predOut, int32_t* status, uint64_t* totalHost,
+                      size_t slotBytes, bool rawShorts, int32_t fill16, const CallSettings& set) {
   const int nTiles = band->tiles_down * band->tiles_across;
   const int n = band->tile_rows * band->tile_cols;
   const bool isFloat = band->elem_type == G4_ELEM_F32;
   int cand[G4_MAX_CODECS], nCand = 0;
-  for (int k = 0; k < codecs->n_codecs; k++) {
-    int id = codecs->codec_ids[k];
+  for (int k = 0; k < codecs.ids.n_codecs; k++) {
+    int id = codecs.ids.codec_ids[k];
     if (id < 0 || id >= G4_CODEC_COUNT) return G4_ERR_ARG;
     if (id == G4_CODEC_LSOP08) continue;  // decode-only legacy codec: its encoder declines every tile
     if (codec_is_float(id) == isFloat) cand[nCand++] = k;
@@ -470,8 +502,8 @@ int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const int* o
     CK(ctx->slots[c].ensure(size_t(nTiles) * slotBytes));
     EncodeArgs a{};
     a.band = *band;
-    a.band.tileOffset = ctx->curTileOffset;
-    a.band.tilePitch = ctx->curTilePitch;
+    a.band.tileOffset = set.tileOffset;
+    a.band.tilePitch = set.tilePitch;
     a.grid = grid;
     a.slots = ctx->slots[c].as<uint8_t>();
     a.slotBytes = slotBytes;
@@ -482,7 +514,7 @@ int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const int* o
     a.codecIndex = cand[c];
     a.scratch = nullptr;
     a.scratchStride = 0;
-    int rc = launch_encoder(ctx, codecs->codec_ids[cand[c]], opts[cand[c]], a, nTiles);
+    int rc = launch_encoder(ctx, codecs.ids.codec_ids[cand[c]], codecs.opts[cand[c]], a, nTiles);
     if (rc != G4_OK) return rc;
     sel.candIndex[c] = cand[c];
     cmp.slots[c] = a.slots;
@@ -501,8 +533,8 @@ int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const int* o
   CK(launch_select(sel, ctx->stream));
   CK(launch_offsets(lens, offsets, nTiles, ctx->total.as<uint64_t>(), ctx->stream));
   cmp.band = *band;
-  cmp.band.tileOffset = ctx->curTileOffset;
-  cmp.band.tilePitch = ctx->curTilePitch;
+  cmp.band.tileOffset = set.tileOffset;
+  cmp.band.tilePitch = set.tilePitch;
   cmp.grid = grid;
   cmp.slotBytes = slotBytes;
   cmp.lens = lens;
@@ -523,7 +555,7 @@ int encode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const int* o
 }
 
 int decode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, const uint8_t* arena,
-                      const uint64_t* offsets, const uint32_t* lens, void* grid, int32_t* status, bool rawShorts) {
+                      const uint64_t* offsets, const uint32_t* lens, void* grid, int32_t* status, bool rawShorts, const CallSettings& set) {
   const int nTiles = band->tiles_down * band->tiles_across;
   const int n = band->tile_rows * band->tile_cols;
   const int kinds = G4_CODEC_COUNT + 1;
@@ -536,7 +568,7 @@ int decode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const g4_ban
   cl.rawLen = rawShorts ? ((2u * uint32_t(n) + 3u) & ~3u) : uint32_t(n) * 4u;
   cl.codecs = *codecs;
   cl.arena = arena;
-  cl.arenaLen = ctx->arenaLimit;
+  cl.arenaLen = set.arenaLen;
   cl.offsets = offsets;
   cl.lens = lens;
   cl.lists = ctx->lists.as<int>();
@@ -557,8 +589,8 @@ int decode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const g4_ban
     if (kind < G4_CODEC_COUNT && !present[kind]) continue;
     DecodeArgs a{};
     a.band = *band;
-    a.band.tileOffset = ctx->curTileOffset;
-    a.band.tilePitch = ctx->curTilePitch;
+    a.band.tileOffset = set.tileOffset;
+    a.band.tilePitch = set.tilePitch;
     a.grid = grid;
     a.arena = arena;
     a.offsets = offsets;
@@ -585,9 +617,11 @@ int decode_device_i32(g4_context* ctx, const g4_codec_list* codecs, const g4_ban
 // TileElementShort around the integer codecs (gvrs/TileElementShort.java:211-248): the 2-byte raster is widened into an
 // int32 staging raster (fill value -> INT4_NULL_CODE) before encoding and narrowed after decoding (INT4_NULL_CODE ->
 // SHORT_NULL_CODE); raw tiles keep 2 bytes per sample.  All pointers are device pointers.
+// The staging band of `b`: 4 bytes per sample, pitch = the band's width.  float32 samples stay float32 (the float codecs
+// take float32 bits); every other element is staged as int32.
 g4_band_desc widened(const g4_band_desc& b) {
   g4_band_desc w = b;
-  w.elem_type = G4_ELEM_I32;
+  if (b.elem_type != G4_ELEM_F32) w.elem_type = G4_ELEM_I32;
   w.grid_pitch = int64_t(b.tiles_across) * b.tile_cols;
   return w;
 }
@@ -616,60 +650,97 @@ int stage_window(g4_context* ctx, const g4_band_desc& band, int mode, const void
   return G4_OK;
 }
 
-int encode_device(g4_context* ctx, const g4_codec_list* codecs, const int* opts, const g4_band_desc* band, void* grid, uint8_t* arena,
-                  uint64_t arenaCap, uint64_t* offsets, uint32_t* lens, uint8_t* codecOut, uint8_t* predOut, int32_t* status,
-                  uint64_t* totalHost, size_t slotBytes) {
+int encode_device(g4_context* ctx, const CodecList& codecs, const g4_band_desc* band, void* grid, uint8_t* arena, uint64_t arenaCap,
+                  uint64_t* offsets, uint32_t* lens, uint8_t* codecOut, uint8_t* predOut, int32_t* status, uint64_t* totalHost,
+                  size_t slotBytes, const CallSettings& set) {
   if (band->elem_type == G4_ELEM_ICF) {  // the float band is mapped to codes in the staging raster, which is then encoded
     const g4_band_desc w = widened(*band);
     const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = w.grid_pitch;
     CK(ctx->wide.ensure(size_t(rows) * size_t(cols) * 4));
-    CK(launch_icf_map(0, grid, band->grid_pitch, ctx->wide.p, cols, rows, cols, ctx->icf, ctx->stream));
+    CK(launch_icf_map(0, grid, band->grid_pitch, ctx->wide.p, cols, rows, cols, icf_of(set.icf), ctx->stream));
     ctx->launches++;
-    return encode_device_i32(ctx, codecs, opts, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
-                             false, 0);
+    return encode_device_i32(ctx, codecs, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
+                             false, 0, set);
   }
   if (band->elem_type != G4_ELEM_I16)
-    return encode_device_i32(ctx, codecs, opts, band, grid, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
-                             false, 0);
+    return encode_device_i32(ctx, codecs, band, grid, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
+                             false, 0, set);
   // the widening is the load pass of g4_encode_window over the whole band, with no margin
   const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = int64_t(band->tiles_across) * band->tile_cols;
   int rc = stage_window(ctx, *band, kLoadWiden16, grid, band->grid_pitch, rows, cols, 0, g4::IcfMap{});
   if (rc != G4_OK) return rc;
   const g4_band_desc w = widened(*band);
-  return encode_device_i32(ctx, codecs, opts, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
-                           true, band->fill_value);
+  return encode_device_i32(ctx, codecs, &w, ctx->wide.p, arena, arenaCap, offsets, lens, codecOut, predOut, status, totalHost, slotBytes,
+                           true, band->fill_value, set);
 }
 
 int decode_device(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, const uint8_t* arena,
-                  const uint64_t* offsets, const uint32_t* lens, void* grid, int32_t* status) {
+                  const uint64_t* offsets, const uint32_t* lens, void* grid, int32_t* status, const CallSettings& set) {
   if (band->elem_type == G4_ELEM_ICF) {  // codes are decoded into the caller's float raster (4 bytes per sample), then mapped in place
     g4_band_desc w = *band;
     w.elem_type = G4_ELEM_I32;
-    int rc = decode_device_i32(ctx, codecs, &w, arena, offsets, lens, grid, status, false);
+    int rc = decode_device_i32(ctx, codecs, &w, arena, offsets, lens, grid, status, false, set);
     if (rc != G4_OK) return rc;
     const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = int64_t(band->tiles_across) * band->tile_cols;
-    CK(launch_icf_map(1, grid, band->grid_pitch, grid, band->grid_pitch, rows, cols, ctx->icf, ctx->stream));
+    CK(launch_icf_map(1, grid, band->grid_pitch, grid, band->grid_pitch, rows, cols, icf_of(set.icf), ctx->stream));
     ctx->launches++;
     return G4_OK;
   }
-  if (band->elem_type != G4_ELEM_I16) return decode_device_i32(ctx, codecs, band, arena, offsets, lens, grid, status, false);
+  if (band->elem_type != G4_ELEM_I16) return decode_device_i32(ctx, codecs, band, arena, offsets, lens, grid, status, false, set);
   const g4_band_desc w = widened(*band);
   const int64_t rows = int64_t(band->tiles_down) * band->tile_rows, cols = w.grid_pitch;
   CK(ctx->wide.ensure(size_t(rows) * size_t(cols) * 4));
-  int rc = decode_device_i32(ctx, codecs, &w, arena, offsets, lens, ctx->wide.p, status, true);
+  int rc = decode_device_i32(ctx, codecs, &w, arena, offsets, lens, ctx->wide.p, status, true, set);
   if (rc != G4_OK) return rc;
   CK(launch_narrow_i16(ctx->wide.as<int32_t>(), static_cast<int16_t*>(grid), band->grid_pitch, rows, cols, ctx->stream));
   ctx->launches++;
   return G4_OK;
 }
 
-int first_bad_status(const std::vector<int32_t>& st) {  // errors before notes (G4_DECLINED, G4_CHECKSUM_MISMATCH)
+// Errors before notes (G4_DECLINED, G4_CHECKSUM_MISMATCH).  absentOk: G4_DECLINED marks a tile absent from the image, which
+// a window or point read returns as fill values; it is then neither an error nor a note.
+int first_bad_status(const int32_t* st, int n, bool absentOk) {
   int32_t note = G4_OK;
-  for (int32_t s : st) {
+  for (int i = 0; i < n; i++) {
+    const int32_t s = st[i];
     if (s < 0) return s;
-    if (s != G4_OK && note == G4_OK) note = s;
+    if (s != G4_OK && note == G4_OK && !(absentOk && s == G4_DECLINED)) note = s;
   }
   return note;
+}
+// The n statuses of a call on device memory, read back on the context's stream once the call's work is done.
+int read_status(g4_context* ctx, const int32_t* status, int n, bool absentOk) {
+  std::vector<int32_t> st(n);
+  CK(cudaMemcpyAsync(st.data(), status, size_t(n) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return first_bad_status(st.data(), n, absentOk);
+}
+
+// The WindowStore fields the window and point reads share: how a decoded sample becomes an output sample, absent tiles.
+WindowStore window_store(const g4_context* ctx, const g4_band_desc& raster, const g4_icf_desc* icf, uint32_t fillBits, int32_t* status) {
+  WindowStore ws{};
+  ws.R = raster.tile_rows;
+  ws.C = raster.tile_cols;
+  ws.absent = ctx->winAbsent.as<uint8_t>();
+  ws.status = status;
+  ws.fillBits = fillBits;
+  ws.mode = raster.elem_type == G4_ELEM_I16 ? kWindowNarrow16 : icf ? kWindowIcfFloat : kWindowCopy32;
+  if (icf) ws.icf = icf_of(icf);
+  return ws;
+}
+// Decodes nTd x nTa tiles of the raster, whose payload locations winOff / winLen hold, into the staging band winStage of
+// the window and point reads, and points the store at it.  Statuses go to ws.status.
+int decode_to_stage(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc& raster, int nTd, int nTa, const uint8_t* image,
+                    const CallSettings& set, WindowStore& ws) {
+  g4_band_desc b = raster;
+  b.tiles_down = nTd;
+  b.tiles_across = nTa;
+  b = widened(b);
+  CK(ctx->winStage.ensure(band_samples(b) * 4));
+  ws.stage = ctx->winStage.as<int32_t>();
+  ws.stagePitch = b.grid_pitch;
+  return decode_device_i32(ctx, codecs, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), ctx->winStage.p, ws.status,
+                           raster.elem_type == G4_ELEM_I16, set);
 }
 
 }  // namespace
@@ -724,7 +795,6 @@ int g4_context_create(int device, void* cuda_stream, g4_context** out) {
   g4_context* ctx = new g4_context();
   ctx->device = device;
   auto fail = [&](cudaError_t err, const char* what) {
-    if (ctx->ownStream && ctx->stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
     return cuda_fail(err, what);
   };
@@ -768,24 +838,8 @@ void g4_context_destroy(g4_context* ctx) {
   if (!ctx) return;
   DeviceGuard guard(ctx->device);
   cudaStreamSynchronize(ctx->stream);
-  if (ctx->copyIn) {
-    cudaStreamSynchronize(ctx->copyIn);
-    cudaStreamSynchronize(ctx->copyOut);
-    cudaStreamDestroy(ctx->copyIn);
-    cudaStreamDestroy(ctx->copyOut);
-    for (int k = 0; k < kMaxChunks; k++) { cudaEventDestroy(ctx->evIn[k]); cudaEventDestroy(ctx->evDone[k]); }
-  }
-  if (ctx->evStart) cudaEventDestroy(ctx->evStart);
-  if (ctx->evOrder) cudaEventDestroy(ctx->evOrder);
-  for (auto& b : ctx->slots) b.release();
-  DevBuf* bufs[] = {&ctx->candLens, &ctx->candPreds, &ctx->candStatus, &ctx->counters, &ctx->scratch, &ctx->lists, &ctx->src,
-                    &ctx->total, &ctx->coef, &ctx->defer, &ctx->lsopMeta, &ctx->lsopSide, &ctx->lsopExc, &ctx->lsopResid, &ctx->lsopStage, &ctx->tileRefs, &ctx->lsopCks, &ctx->wide, &ctx->encScratch, &ctx->region, &ctx->jobLen, &ctx->jobOff, &ctx->jobOut, &ctx->jobTotal,
-                    &ctx->streamIn, &ctx->streamOut, &ctx->deflateWork, &ctx->stSorted, &ctx->stRank, &ctx->stTable,
-                    &ctx->stWork, &ctx->stCounters, &ctx->rcPos, &ctx->rcOff, &ctx->rcLen, &ctx->rcCrc, &ctx->rcStored, &ctx->rcTotal,
-                    &ctx->rcData, &ctx->rcOffsets, &ctx->rcLens, &ctx->rcIndex, &ctx->rcStatus, &ctx->rcOut, &ctx->rcChain, &ctx->rcDesc, &ctx->sGrid, &ctx->sArena, &ctx->sOffsets, &ctx->sLens, &ctx->sCodec, &ctx->sPred, &ctx->sStatus,
-                    &ctx->winOff, &ctx->winLen, &ctx->winAbsent, &ctx->winStage, &ctx->ptFlag, &ctx->ptSlot, &ctx->ptInfo};
-  for (DevBuf* b : bufs) b->release();
-  if (ctx->ownStream) cudaStreamDestroy(ctx->stream);
+  if (ctx->copyIn) cudaStreamSynchronize(ctx->copyIn);
+  if (ctx->copyOut) cudaStreamSynchronize(ctx->copyOut);
   delete ctx;
 }
 
@@ -1138,46 +1192,37 @@ int g4_fill_terrain(g4_context* ctx, int elem_type, uint64_t seed, int64_t row0,
 // Tile-list calls: `refs` (host array, one {offset, pitch} per tile, in samples relative to `grid`) replaces the tile grid
 // of the band, which is then a list of band->tiles_across tiles.  Device rasters are addressed in place through the
 // per-tile tables of BandEx; host rasters are staged tile under tile by 2-D copies (no host gather).
-static int upload_tile_refs(g4_context* ctx, const g4_tile_ref* refs, int nTiles) {
+static int upload_tile_refs(g4_context* ctx, const g4_tile_ref* refs, int nTiles, CallSettings* set) {
   std::vector<int64_t> h(size_t(nTiles) * 2);
   for (int t = 0; t < nTiles; t++) { h[size_t(t)] = refs[t].offset; h[size_t(nTiles) + t] = refs[t].pitch; }
   CK(ctx->tileRefs.ensure(h.size() * 8));
   CK(cudaMemcpyAsync(ctx->tileRefs.p, h.data(), h.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));  // h goes out of scope
-  ctx->curTileOffset = ctx->tileRefs.as<int64_t>();
-  ctx->curTilePitch = ctx->tileRefs.as<int64_t>() + nTiles;
+  set->tileOffset = ctx->tileRefs.as<int64_t>();
+  set->tilePitch = ctx->tileRefs.as<int64_t>() + nTiles;
   return G4_OK;
 }
-struct TileRefScope {  // the tables are valid for one call only
-  g4_context* c;
-  ~TileRefScope() { c->curTileOffset = nullptr; c->curTilePitch = nullptr; }
-};
 
 static int encode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, int mem_space, const void* grid,
                              const g4_tile_ref* refs, uint8_t* arena, uint64_t arena_cap, uint64_t* offsets, uint32_t* lens,
-                             uint8_t* codec_out, uint8_t* predictor_out, int32_t* status, uint64_t* total_bytes) {
+                             uint8_t* codec_out, uint8_t* predictor_out, int32_t* status, uint64_t* total_bytes, CallSettings set) {
   if (!ctx || !codecs || !grid || !arena || !offsets || !lens || !codec_out || !predictor_out || !status) return G4_ERR_ARG;
-  int rc = check_band(band, ctx->icfOn);
+  int rc = check_band(band, set.icf != nullptr);
   if (rc != G4_OK) return rc;
-  g4_codec_list ids;
-  int opts[G4_MAX_CODECS];
-  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
-  codecs = &ids;
+  CodecList list;
+  if (split_codec_list(codecs, &list) != G4_OK) return G4_ERR_ARG;
   ENTER(ctx);
   const int nTiles = band->tiles_down * band->tiles_across;
   const size_t n = size_t(band->tile_rows) * band->tile_cols;
   const size_t slotBytes = round_up(n * 4 + 64, 16);
   const size_t eb = elem_bytes(*band);
-  std::vector<int32_t> st(nTiles);
   uint64_t total = 0;
-  TileRefScope scope{ctx};
   if (mem_space == G4_MEM_DEVICE) {
-    if (refs && (rc = upload_tile_refs(ctx, refs, nTiles)) != G4_OK) return rc;
-    rc = encode_device(ctx, codecs, opts, band, const_cast<void*>(grid), arena, arena_cap, offsets, lens, codec_out, predictor_out,
-                       status, &total, slotBytes);
+    if (refs && (rc = upload_tile_refs(ctx, refs, nTiles, &set)) != G4_OK) return rc;
+    rc = encode_device(ctx, list, band, const_cast<void*>(grid), arena, arena_cap, offsets, lens, codec_out, predictor_out, status, &total,
+                       slotBytes, set);
     if (rc != G4_OK) return rc;
-    CK(cudaMemcpyAsync(st.data(), status, size_t(nTiles) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
+    rc = read_status(ctx, status, nTiles, false);
   } else if (mem_space == G4_MEM_HOST) {
     g4_band_desc staged = *band;
     if (refs) {  // the tiles go tile under tile into one staging raster of pitch tile_cols
@@ -1201,9 +1246,9 @@ static int encode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
                              size_t(band->tile_cols) * eb, size_t(band->tile_rows), cudaMemcpyHostToDevice, ctx->stream));
     } else CK(cudaMemcpyAsync(ctx->sGrid.p, grid, gridBytes, cudaMemcpyHostToDevice, ctx->stream));
     band = &staged;
-    rc = encode_device(ctx, codecs, opts, band, ctx->sGrid.p, ctx->sArena.as<uint8_t>(), bound, ctx->sOffsets.as<uint64_t>(),
-                       ctx->sLens.as<uint32_t>(), ctx->sCodec.as<uint8_t>(), ctx->sPred.as<uint8_t>(), ctx->sStatus.as<int32_t>(),
-                       &total, slotBytes);
+    rc = encode_device(ctx, list, band, ctx->sGrid.p, ctx->sArena.as<uint8_t>(), bound, ctx->sOffsets.as<uint64_t>(),
+                       ctx->sLens.as<uint32_t>(), ctx->sCodec.as<uint8_t>(), ctx->sPred.as<uint8_t>(), ctx->sStatus.as<int32_t>(), &total,
+                       slotBytes, set);
     if (rc != G4_OK) return rc;
     if (total > arena_cap) {
       if (total_bytes) *total_bytes = total;
@@ -1216,19 +1261,19 @@ static int encode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
     CK(cudaMemcpyAsync(predictor_out, ctx->sPred.p, nTiles, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(status, ctx->sStatus.p, size_t(nTiles) * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    std::memcpy(st.data(), status, size_t(nTiles) * 4);
+    rc = first_bad_status(status, nTiles, false);
   } else {
     return G4_ERR_ARG;
   }
   if (total_bytes) *total_bytes = total;
-  return first_bad_status(st);
+  return rc;
 }
 
 int g4_encode_tiles(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, int mem_space, const void* grid,
                     uint8_t* arena, uint64_t arena_cap, uint64_t* offsets, uint32_t* lens, uint8_t* codec_out,
                     uint8_t* predictor_out, int32_t* status, uint64_t* total_bytes) {
   return encode_tiles_impl(ctx, codecs, band, mem_space, grid, nullptr, arena, arena_cap, offsets, lens, codec_out, predictor_out, status,
-                           total_bytes);
+                           total_bytes, CallSettings{});
 }
 
 // The band a tile list runs as: one row of n tiles.  grid_pitch only carries the ALIGNMENT the kernels may rely on (the
@@ -1254,29 +1299,26 @@ int g4_encode_tile_list(g4_context* ctx, const g4_codec_list* codecs, int elem_t
   const int rc = tile_list_band(elem_type, tile_rows, tile_cols, n_tiles, tiles, &band);
   if (rc != G4_OK) return rc;
   return encode_tiles_impl(ctx, codecs, &band, mem_space, base, tiles, arena, arena_cap, offsets, lens, codec_out, predictor_out, status,
-                           total_bytes);
+                           total_bytes, CallSettings{});
 }
 
 static int decode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, int mem_space, const uint8_t* arena,
-                             const uint64_t* offsets, const uint32_t* lens, void* grid, const g4_tile_ref* refs, int32_t* status) {
+                             const uint64_t* offsets, const uint32_t* lens, void* grid, const g4_tile_ref* refs, int32_t* status,
+                             CallSettings set) {
   if (!ctx || !codecs || !grid || !arena || !offsets || !lens || !status) return G4_ERR_ARG;
-  int rc = check_band(band, ctx->icfOn);
+  int rc = check_band(band, set.icf != nullptr);
   if (rc != G4_OK) return rc;
-  g4_codec_list ids;  // decode ignores the option bits: they describe how to encode, the packings say the rest
-  int opts[G4_MAX_CODECS];
-  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
-  codecs = &ids;
+  CodecList list;
+  if (split_codec_list(codecs, &list) != G4_OK) return G4_ERR_ARG;
+  codecs = &list.ids;
   ENTER(ctx);
   const int nTiles = band->tiles_down * band->tiles_across;
-  std::vector<int32_t> st(nTiles);
-  TileRefScope scope{ctx};
   if (mem_space == G4_MEM_DEVICE) {
-    if (refs && (rc = upload_tile_refs(ctx, refs, nTiles)) != G4_OK) return rc;
-    rc = decode_device(ctx, codecs, band, arena, offsets, lens, grid, status);
+    if (refs && (rc = upload_tile_refs(ctx, refs, nTiles, &set)) != G4_OK) return rc;
+    rc = decode_device(ctx, codecs, band, arena, offsets, lens, grid, status, set);
     if (rc != G4_OK) return rc;
     if (ctx->asyncDevice && !refs) return G4_OK;  // enqueued; status[] is read by the caller after g4_context_synchronize
-    CK(cudaMemcpyAsync(st.data(), status, size_t(nTiles) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
+    return read_status(ctx, status, nTiles, false);
   } else if (mem_space == G4_MEM_HOST) {
     // a directory entry that leaves the caller's arena (g4_decode_tiles_bounded) or is longer than the raw tile is never
     // staged: it reaches the device as an empty payload, which classify_kernel reports as G4_ERR_FORMAT for that tile
@@ -1284,7 +1326,7 @@ static int decode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
     std::vector<uint32_t> lenSafe;
     const uint32_t rawLen = standard_size(*band);
     for (int t = 0; t < nTiles; t++) {
-      const bool bad = lens[t] > rawLen || (ctx->arenaLimit != ~0ull && (offsets[t] > ctx->arenaLimit || lens[t] > ctx->arenaLimit - offsets[t]));
+      const bool bad = lens[t] > rawLen || (set.arenaLen != ~0ull && (offsets[t] > set.arenaLen || lens[t] > set.arenaLen - offsets[t]));
       if (bad && offSafe.empty()) {
         offSafe.assign(offsets, offsets + nTiles);
         lenSafe.assign(lens, lens + nTiles);
@@ -1334,7 +1376,7 @@ static int decode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
     if (nChunks == 1) {
       CK(cudaMemcpyAsync(ctx->sArena.p, arena, arenaBytes, cudaMemcpyHostToDevice, ctx->stream));
       rc = decode_device(ctx, codecs, band, ctx->sArena.as<uint8_t>(), ctx->sOffsets.as<uint64_t>(), ctx->sLens.as<uint32_t>(),
-                         ctx->sGrid.p, ctx->sStatus.as<int32_t>());
+                         ctx->sGrid.p, ctx->sStatus.as<int32_t>(), set);
       if (rc != G4_OK) return rc;
       if (refs) {
         const size_t eb = elem_bytes(*band), tileBytes = size_t(band->tile_rows) * band->tile_cols * eb;
@@ -1361,7 +1403,7 @@ static int decode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
         sub.tiles_down = r1 - r0;
         uint8_t* gdev = ctx->sGrid.as<uint8_t>() + size_t(r0) * band->tile_rows * rowBytes;
         rc = decode_device(ctx, codecs, &sub, ctx->sArena.as<uint8_t>(), ctx->sOffsets.as<uint64_t>() + t0, ctx->sLens.as<uint32_t>() + t0,
-                           gdev, ctx->sStatus.as<int32_t>() + t0);
+                           gdev, ctx->sStatus.as<int32_t>() + t0, set);
         if (rc != G4_OK) return rc;
         CK(cudaEventRecord(ctx->evDone[k], ctx->stream));
         CK(cudaStreamWaitEvent(ctx->copyOut, ctx->evDone[k], 0));
@@ -1376,16 +1418,14 @@ static int decode_tiles_impl(g4_context* ctx, const g4_codec_list* codecs, const
     }
     CK(cudaMemcpyAsync(status, ctx->sStatus.p, size_t(nTiles) * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    std::memcpy(st.data(), status, size_t(nTiles) * 4);
-  } else {
-    return G4_ERR_ARG;
+    return first_bad_status(status, nTiles, false);
   }
-  return first_bad_status(st);
+  return G4_ERR_ARG;
 }
 
 int g4_decode_tiles(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, int mem_space, const uint8_t* arena,
                     const uint64_t* offsets, const uint32_t* lens, void* grid, int32_t* status) {
-  return decode_tiles_impl(ctx, codecs, band, mem_space, arena, offsets, lens, grid, nullptr, status);
+  return decode_tiles_impl(ctx, codecs, band, mem_space, arena, offsets, lens, grid, nullptr, status, CallSettings{});
 }
 
 int g4_decode_tile_list(g4_context* ctx, const g4_codec_list* codecs, int elem_type, int tile_rows, int tile_cols, int n_tiles,
@@ -1394,31 +1434,15 @@ int g4_decode_tile_list(g4_context* ctx, const g4_codec_list* codecs, int elem_t
   g4_band_desc band;
   int rc = tile_list_band(elem_type, tile_rows, tile_cols, n_tiles, tiles, &band);
   if (rc != G4_OK) return rc;
-  if (!ctx) return G4_ERR_ARG;
-  ctx->arenaLimit = arena_len;
-  rc = decode_tiles_impl(ctx, codecs, &band, mem_space, arena, offsets, lens, base, tiles, status);
-  ctx->arenaLimit = ~0ull;
-  return rc;
+  return decode_tiles_impl(ctx, codecs, &band, mem_space, arena, offsets, lens, base, tiles, status, CallSettings{arena_len});
 }
 
 int g4_decode_tiles_bounded(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, int mem_space, const uint8_t* arena,
                             uint64_t arena_len, const uint64_t* offsets, const uint32_t* lens, void* grid, int32_t* status) {
-  if (!ctx) return G4_ERR_ARG;
-  ctx->arenaLimit = arena_len;
-  const int rc = g4_decode_tiles(ctx, codecs, band, mem_space, arena, offsets, lens, grid, status);
-  ctx->arenaLimit = ~0ull;
-  return rc;
+  return decode_tiles_impl(ctx, codecs, band, mem_space, arena, offsets, lens, grid, nullptr, status, CallSettings{arena_len});
 }
 
 // ---- integer-coded float elements ------------------------------------------------------------------------------------
-static bool icf_valid(const g4_icf_desc* icf) { return icf && icf->scale != 0.0f && std::isfinite(icf->scale); }
-static g4::IcfMap icf_of(const g4_icf_desc* icf) { return g4::IcfMap{icf->scale, icf->offset, icf->fill_int, icf->fill_value}; }
-struct IcfScope {  // the descriptor is valid for one call only
-  g4_context* c;
-  IcfScope(g4_context* ctx, const g4_icf_desc* icf) : c(ctx) { c->icfOn = true; c->icf = icf_of(icf); }
-  ~IcfScope() { c->icfOn = false; c->icf = g4::IcfMap{}; }
-};
-
 int g4_icf_map(g4_context* ctx, int to_float, const g4_icf_desc* icf, int mem_space, int64_t n_rows, int64_t n_cols, const void* src,
                int64_t src_pitch, void* dst, int64_t dst_pitch) {
   if (!ctx || !icf_valid(icf) || !src || !dst || n_rows < 1 || n_cols < 1 || src_pitch < n_cols || dst_pitch < n_cols) return G4_ERR_ARG;
@@ -1444,17 +1468,15 @@ int g4_encode_tiles_icf(g4_context* ctx, const g4_codec_list* codecs, const g4_b
                         const float* grid, uint8_t* arena, uint64_t arena_cap, uint64_t* offsets, uint32_t* lens, uint8_t* codec_out,
                         uint8_t* predictor_out, int32_t* status, uint64_t* total_bytes) {
   if (!ctx || !band || band->elem_type != G4_ELEM_ICF || !icf_valid(icf)) return G4_ERR_ARG;
-  IcfScope scope(ctx, icf);
   return encode_tiles_impl(ctx, codecs, band, mem_space, grid, nullptr, arena, arena_cap, offsets, lens, codec_out, predictor_out, status,
-                           total_bytes);
+                           total_bytes, CallSettings{~0ull, icf});
 }
 
 int g4_decode_tiles_icf(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* band, const g4_icf_desc* icf, int mem_space,
                         const uint8_t* arena, uint64_t arena_len, const uint64_t* offsets, const uint32_t* lens, float* grid,
                         int32_t* status) {
   if (!ctx || !band || band->elem_type != G4_ELEM_ICF || !icf_valid(icf)) return G4_ERR_ARG;
-  IcfScope scope(ctx, icf);
-  return g4_decode_tiles_bounded(ctx, codecs, band, mem_space, arena, arena_len, offsets, lens, grid, status);
+  return decode_tiles_impl(ctx, codecs, band, mem_space, arena, offsets, lens, grid, nullptr, status, CallSettings{arena_len, icf});
 }
 
 // ---- window reads: GvrsElement.readBlock (gvrs/GvrsElement.java:298-404) on the device ----------------------------------
@@ -1466,17 +1488,14 @@ int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
                      uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens, const int32_t* tile_status, uint32_t fill_bits,
                      int64_t row0, int64_t col0, int64_t n_rows, int64_t n_cols, void* out, int64_t out_pitch, int32_t* status) {
   if (!ctx || !codecs || !image || !payload_offsets || !lens || !tile_status || !out || !status) return G4_ERR_ARG;
-  int rc = check_band(raster, icf != nullptr);
+  int rc = check_raster(raster, icf);
   if (rc != G4_OK) return rc;
-  if (icf && !icf_valid(icf)) return G4_ERR_ARG;
   const int R = raster->tile_rows, Cc = raster->tile_cols;
   const int64_t gridRows = int64_t(raster->tiles_down) * R, gridCols = int64_t(raster->tiles_across) * Cc;
   if (n_rows < 1 || n_cols < 1 || row0 < 0 || col0 < 0 || row0 > gridRows - n_rows || col0 > gridCols - n_cols) return G4_ERR_ARG;
   if (out_pitch < n_cols) return G4_ERR_ARG;
-  g4_codec_list ids;
-  int opts[G4_MAX_CODECS];
-  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
-  codecs = &ids;
+  CodecList list;
+  if (split_codec_list(codecs, &list) != G4_OK) return G4_ERR_ARG;
   ENTER(ctx);
   const int tr0 = int(row0 / R), tc0 = int(col0 / Cc);
   const int nTd = int((row0 + n_rows - 1) / R) - tr0 + 1, nTa = int((col0 + n_cols - 1) / Cc) - tc0 + 1;
@@ -1487,44 +1506,22 @@ int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   CK(launch_window_gather(payload_offsets, lens, tile_status, raster->tiles_across, tr0, tc0, nTd, nTa, ctx->winOff.as<uint64_t>(),
                           ctx->winLen.as<uint32_t>(), ctx->winAbsent.as<uint8_t>(), ctx->stream));
   ctx->launches++;
-  struct ArenaScope {  // payloads that leave the image are G4_ERR_FORMAT, as in g4_decode_tiles_bounded
-    g4_context* c;
-    ~ArenaScope() { c->arenaLimit = ~0ull; }
-  } arenaScope{ctx};
-  ctx->arenaLimit = image_len;
-  WindowStore ws{};
+  const CallSettings set{image_len, icf};  // payloads that leave the image are G4_ERR_FORMAT, as in g4_decode_tiles_bounded
+  WindowStore ws = window_store(ctx, *raster, icf, fill_bits, status);
   ws.rows = n_rows;
   ws.cols = n_cols;
   ws.out = out;
   ws.outPitch = out_pitch;
-  ws.R = R;
-  ws.C = Cc;
   ws.nTa = nTa;
   ws.nW = nW;
-  ws.absent = ctx->winAbsent.as<uint8_t>();
-  ws.status = status;
-  ws.fillBits = fill_bits;
-  ws.mode = raster->elem_type == G4_ELEM_I16 ? kWindowNarrow16 : icf ? kWindowIcfFloat : kWindowCopy32;
-  if (icf) ws.icf = icf_of(icf);
-  g4_band_desc b = *raster;
-  b.tiles_down = nTd;
-  b.tiles_across = nTa;
   if (row0 % R == 0 && col0 % Cc == 0 && n_rows == int64_t(nTd) * R && n_cols == int64_t(nTa) * Cc) {
+    g4_band_desc b = *raster;
+    b.tiles_down = nTd;
+    b.tiles_across = nTa;
     b.grid_pitch = out_pitch;
-    if (icf) {
-      IcfScope scope(ctx, icf);
-      rc = decode_device(ctx, codecs, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), out, status);
-    } else {
-      rc = decode_device(ctx, codecs, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), out, status);
-    }
+    rc = decode_device(ctx, &list.ids, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), out, status, set);
   } else {
-    b = widened(b);  // int32 samples, pitch = the covering tiles' width
-    if (raster->elem_type == G4_ELEM_F32) b.elem_type = G4_ELEM_F32;
-    CK(ctx->winStage.ensure(band_samples(b) * 4));
-    rc = decode_device_i32(ctx, codecs, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), ctx->winStage.p, status,
-                           raster->elem_type == G4_ELEM_I16);
-    ws.stage = ctx->winStage.as<int32_t>();
-    ws.stagePitch = b.grid_pitch;
+    rc = decode_to_stage(ctx, &list.ids, *raster, nTd, nTa, image, set, ws);
     ws.sr0 = row0 - int64_t(tr0) * R;
     ws.sc0 = col0 - int64_t(tc0) * Cc;
   }
@@ -1532,12 +1529,7 @@ int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   CK(launch_window_store(ws, ctx->smCount, ctx->stream));
   ctx->launches++;
   if (ctx->asyncDevice) return G4_OK;  // enqueued; status[] is read by the caller after g4_context_synchronize
-  std::vector<int32_t> st(nW);
-  CK(cudaMemcpyAsync(st.data(), status, size_t(nW) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  for (int32_t& s : st)
-    if (s == G4_DECLINED) s = G4_OK;  // absent tiles read as fill values; they are neither errors nor notes
-  return first_bad_status(st);
+  return read_status(ctx, status, nW, true);
 }
 
 // ---- point reads: GvrsElement.readValue / readValueInt (gvrs/GvrsElementInt.java:85-95) on the device -----------------------
@@ -1560,16 +1552,13 @@ int g4_decode_points(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   if (!ctx || !codecs || !image || !payload_offsets || !lens || !tile_status || !n_tiles_out) return G4_ERR_ARG;
   *n_tiles_out = 0;
   if (n_points < 0 || (n_points > 0 && (!rows || !cols || !out || !tiles_out || !status))) return G4_ERR_ARG;
-  int rc = check_band(raster, icf != nullptr);
+  int rc = check_raster(raster, icf);
   if (rc != G4_OK) return rc;
-  if (icf && !icf_valid(icf)) return G4_ERR_ARG;
   const int R = raster->tile_rows, Cc = raster->tile_cols;
   if (raster_rows < 1 || raster_cols < 1 || raster_rows > int64_t(raster->tiles_down) * R || raster_cols > int64_t(raster->tiles_across) * Cc)
     return G4_ERR_ARG;
-  g4_codec_list ids;
-  int opts[G4_MAX_CODECS];
-  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
-  codecs = &ids;
+  CodecList list;
+  if (split_codec_list(codecs, &list) != G4_OK) return G4_ERR_ARG;
   if (n_points == 0) return G4_OK;
   ENTER(ctx);
   for (const void* p : {(const void*)rows, (const void*)cols, (const void*)out, (const void*)tiles_out, (const void*)status})
@@ -1618,41 +1607,17 @@ int g4_decode_points(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   }
   const int K = info[1];
   *n_tiles_out = K;
-  struct ArenaScope {  // payloads that leave the image are G4_ERR_FORMAT, as in g4_decode_tiles_bounded
-    g4_context* c;
-    ~ArenaScope() { c->arenaLimit = ~0ull; }
-  } arenaScope{ctx};
-  ctx->arenaLimit = image_len;
-  g4_band_desc b = *raster;  // the touched tiles one under the other: tile k at k * R * C, int32 samples
-  b.tiles_down = K;
-  b.tiles_across = 1;
-  b = widened(b);
-  if (raster->elem_type == G4_ELEM_F32) b.elem_type = G4_ELEM_F32;
-  CK(ctx->winStage.ensure(band_samples(b) * 4));
-  rc = decode_device_i32(ctx, codecs, &b, image, ctx->winOff.as<uint64_t>(), ctx->winLen.as<uint32_t>(), ctx->winStage.p, status,
-                         raster->elem_type == G4_ELEM_I16);
-  if (rc != G4_OK) return rc;
-  WindowStore ws{};
-  ws.stage = ctx->winStage.as<int32_t>();
+  WindowStore ws = window_store(ctx, *raster, icf, fill_bits, status);
   ws.out = out;
-  ws.R = R;
-  ws.C = Cc;
   ws.nTa = 1;
   ws.nW = K;
-  ws.absent = ctx->winAbsent.as<uint8_t>();
-  ws.status = status;
-  ws.fillBits = fill_bits;
-  ws.mode = raster->elem_type == G4_ELEM_I16 ? kWindowNarrow16 : icf ? kWindowIcfFloat : kWindowCopy32;
-  if (icf) ws.icf = icf_of(icf);
+  // the touched tiles one under the other: tile k at k * R * C; payloads that leave the image are G4_ERR_FORMAT
+  rc = decode_to_stage(ctx, &list.ids, *raster, K, 1, image, CallSettings{image_len, icf}, ws);
+  if (rc != G4_OK) return rc;
   CK(launch_point_store(pa, ws, ctx->smCount, ctx->stream));
   ctx->launches++;
   if (ctx->asyncDevice) return G4_OK;  // enqueued; status[] is read by the caller after g4_context_synchronize
-  std::vector<int32_t> st(K);
-  CK(cudaMemcpyAsync(st.data(), status, size_t(K) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  for (int32_t& s : st)
-    if (s == G4_DECLINED) s = G4_OK;  // absent tiles read as fill values; they are neither errors nor notes
-  return first_bad_status(st);
+  return read_status(ctx, status, K, true);
 }
 
 // ---- window writes: a raster of any dimensions and pitch, padded to whole tiles on the device -----------------------------
@@ -1663,16 +1628,13 @@ int g4_encode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
                      int64_t n_cols, const void* src, int64_t src_pitch, uint32_t fill_bits, uint8_t* arena, uint64_t arena_cap,
                      uint64_t* offsets, uint32_t* lens, uint8_t* codec_out, uint8_t* predictor_out, int32_t* status, uint64_t* total_bytes) {
   if (!ctx || !codecs || !src || !arena || !offsets || !lens || !codec_out || !predictor_out || !status) return G4_ERR_ARG;
-  int rc = check_band(raster, icf != nullptr);
+  int rc = check_raster(raster, icf);
   if (rc != G4_OK) return rc;
-  if (icf && !icf_valid(icf)) return G4_ERR_ARG;
   const int R = raster->tile_rows, Cc = raster->tile_cols;
   if (n_rows < 1 || n_cols < 1 || src_pitch < n_cols) return G4_ERR_ARG;
   if ((n_rows + R - 1) / R != raster->tiles_down || (n_cols + Cc - 1) / Cc != raster->tiles_across) return G4_ERR_ARG;
-  g4_codec_list ids;
-  int opts[G4_MAX_CODECS];
-  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
-  codecs = &ids;
+  CodecList list;
+  if (split_codec_list(codecs, &list) != G4_OK) return G4_ERR_ARG;
   ENTER(ctx);
   const int nTiles = raster->tiles_down * raster->tiles_across;
   const size_t slotBytes = round_up(size_t(R) * Cc * 4 + 64, 16);
@@ -1681,23 +1643,20 @@ int g4_encode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   if (wide32 && n_rows == int64_t(raster->tiles_down) * R && n_cols == int64_t(raster->tiles_across) * Cc) {
     g4_band_desc b = *raster;
     b.grid_pitch = src_pitch;
-    rc = encode_device_i32(ctx, codecs, opts, &b, const_cast<void*>(src), arena, arena_cap, offsets, lens, codec_out, predictor_out,
-                           status, &total, slotBytes, false, 0);
+    rc = encode_device_i32(ctx, list, &b, const_cast<void*>(src), arena, arena_cap, offsets, lens, codec_out, predictor_out, status,
+                           &total, slotBytes, false, 0, CallSettings{});
   } else {
     const int mode = raster->elem_type == G4_ELEM_I16 ? kLoadWiden16 : icf ? kLoadIcfCode : kLoadCopy32;
     rc = stage_window(ctx, *raster, mode, src, src_pitch, n_rows, n_cols, fill_bits, icf ? icf_of(icf) : g4::IcfMap{});
     if (rc != G4_OK) return rc;
-    g4_band_desc w = widened(*raster);
-    if (raster->elem_type == G4_ELEM_F32) w.elem_type = G4_ELEM_F32;  // the float codecs see float32 bits
-    rc = encode_device_i32(ctx, codecs, opts, &w, ctx->wide.p, arena, arena_cap, offsets, lens, codec_out, predictor_out, status, &total,
-                           slotBytes, raster->elem_type == G4_ELEM_I16, raster->fill_value);
+    const g4_band_desc w = widened(*raster);
+    rc = encode_device_i32(ctx, list, &w, ctx->wide.p, arena, arena_cap, offsets, lens, codec_out, predictor_out, status, &total,
+                           slotBytes, raster->elem_type == G4_ELEM_I16, raster->fill_value, CallSettings{});
   }
   if (rc != G4_OK) return rc;
-  std::vector<int32_t> st(nTiles);
-  CK(cudaMemcpyAsync(st.data(), status, size_t(nTiles) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
+  rc = read_status(ctx, status, nTiles, false);
   if (total_bytes) *total_bytes = total;
-  return first_bad_status(st);
+  return rc;
 }
 
 // ---- per-tile entry points: one-tile bands through the same kernels --------------------------------
@@ -1815,10 +1774,8 @@ int g4_analyze_tiles(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   if (!ctx || !codecs || !band || !arena || !offsets || !lens || !stats) return G4_ERR_ARG;
   int rc = check_band(band);
   if (rc != G4_OK) return rc;
-  g4_codec_list ids;  // the option bits are ignored, as in decode
-  int opts[G4_MAX_CODECS];
-  if (split_codec_list(codecs, &ids, opts) != G4_OK) return G4_ERR_ARG;
-  codecs = &ids;
+  CodecList list;  // the option bits are ignored, as in decode
+  if (split_codec_list(codecs, &list) != G4_OK) return G4_ERR_ARG;
   ENTER(ctx);
   const int nTiles = band->tiles_down * band->tiles_across;
   const size_t n = size_t(band->tile_rows) * band->tile_cols;
@@ -1829,7 +1786,7 @@ int g4_analyze_tiles(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   a.nTiles = nTiles;
   a.nCells = uint32_t(n);
   a.rawLen = standard_size(*band);
-  a.codecs = *codecs;
+  a.codecs = list.ids;
   a.scratch = ctx->scratch.as<uint8_t>();
   a.scratchStride = stride;
   constexpr size_t kPairBytes = size_t(2) * 5 * 65536 * 8;
