@@ -29,7 +29,7 @@ EXPORTS = [
     "g4_predictor_decode_int", "g4_predictor_tiles", "g4_encode_tile_list", "g4_decode_tile_list", "g4_analyze_tiles",
     "g4_tile_records_bound_multi", "g4_pack_tile_records_multi", "g4_unpack_tile_records_multi",
     "g4_icf_map", "g4_encode_tiles_icf", "g4_decode_tiles_icf", "g4_decode_window",
-    "g4_encode_window", "g4_decode_points",
+    "g4_encode_window", "g4_decode_points", "g4_decode_blocks",
 ]
 
 
@@ -116,6 +116,9 @@ def lib():
         L.g4_decode_points.argtypes = [C.c_void_p, C.POINTER(CodecList), C.POINTER(BandDesc), C.POINTER(IcfDesc), C.c_void_p, C.c_uint64,
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32)]
+        L.g4_decode_blocks.argtypes = [C.c_void_p, C.POINTER(CodecList), C.POINTER(BandDesc), C.POINTER(IcfDesc), C.c_void_p, C.c_uint64,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
+                                       C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32)]
         L.g4_encode_window.argtypes = [C.c_void_p, C.POINTER(CodecList), C.POINTER(BandDesc), C.POINTER(IcfDesc), C.c_int64, C.c_int64,
                                        C.c_void_p, C.c_int64, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]

@@ -1532,10 +1532,12 @@ int g4_decode_window(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   return read_status(ctx, status, nW, true);
 }
 
-// ---- point reads: GvrsElement.readValue / readValueInt (gvrs/GvrsElementInt.java:85-95) on the device -----------------------
-// mark (touched tiles) -> compact (their payload locations in tile order) -> one readback of {bad point, K} -> classify +
-// decoders on the K touched tiles as a K x 1 band in the int32 staging buffer of g4_decode_window -> store (one thread per
-// point).  Launches beyond those of g4_decode_tiles_bounded on the same K tiles: exactly three (mark, compact, store).
+// ---- point and block reads: GvrsElement.readValue / readValueInt / readBlock (gvrs/GvrsElementInt.java:85-95, ---------------
+// gvrs/GvrsElement.java:298-404) on the device, many at once.
+// mark (touched tiles) -> compact (their payload locations in tile order) -> one readback of {bad point or block, K} ->
+// classify + decoders on the K touched tiles as a K x 1 band in the int32 staging buffer of g4_decode_window -> store (one
+// thread per point, or per four cells of a block row).  Launches beyond those of g4_decode_tiles_bounded on the same K tiles:
+// exactly three (mark, compact, store).
 static bool device_pointer(const g4_context* ctx, const void* p) {  // a host or another GPU's array is refused, not faulted on
   cudaPointerAttributes at{};
   if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
@@ -1545,26 +1547,30 @@ static bool device_pointer(const g4_context* ctx, const void* p) {  // a host or
   return (at.type == cudaMemoryTypeDevice && at.device == ctx->device) || at.type == cudaMemoryTypeManaged;
 }
 
-int g4_decode_points(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf, const uint8_t* image,
-                     uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens, const int32_t* tile_status, uint32_t fill_bits,
-                     int64_t raster_rows, int64_t raster_cols, int64_t n_points, const int64_t* rows, const int64_t* cols, void* out,
-                     int32_t* tiles_out, int32_t* status, int32_t* n_tiles_out) {
-  if (!ctx || !codecs || !image || !payload_offsets || !lens || !tile_status || !n_tiles_out) return G4_ERR_ARG;
-  *n_tiles_out = 0;
-  if (n_points < 0 || (n_points > 0 && (!rows || !cols || !out || !tiles_out || !status))) return G4_ERR_ARG;
-  int rc = check_raster(raster, icf);
+// The argument checks g4_decode_points and g4_decode_blocks share, up to the device pointers.
+static int check_marked_read(const g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf,
+                             const uint8_t* image, const uint64_t* payload_offsets, const uint32_t* lens, const int32_t* tile_status,
+                             int64_t raster_rows, int64_t raster_cols, int64_t n, const int64_t* rows, const int64_t* cols,
+                             const void* out, const int32_t* tiles_out, const int32_t* status, CodecList* list) {
+  if (!ctx || !codecs || !image || !payload_offsets || !lens || !tile_status) return G4_ERR_ARG;
+  if (n < 0 || (n > 0 && (!rows || !cols || !out || !tiles_out || !status))) return G4_ERR_ARG;
+  const int rc = check_raster(raster, icf);
   if (rc != G4_OK) return rc;
-  const int R = raster->tile_rows, Cc = raster->tile_cols;
-  if (raster_rows < 1 || raster_cols < 1 || raster_rows > int64_t(raster->tiles_down) * R || raster_cols > int64_t(raster->tiles_across) * Cc)
+  if (raster_rows < 1 || raster_cols < 1 || raster_rows > int64_t(raster->tiles_down) * raster->tile_rows ||
+      raster_cols > int64_t(raster->tiles_across) * raster->tile_cols)
     return G4_ERR_ARG;
-  CodecList list;
-  if (split_codec_list(codecs, &list) != G4_OK) return G4_ERR_ARG;
-  if (n_points == 0) return G4_OK;
+  return split_codec_list(codecs, list) != G4_OK ? G4_ERR_ARG : G4_OK;
+}
+
+// pa carries the blocks (rows, cols, n, blockRows x blockCols, coverTd x coverTa); kMax bounds K.
+static int decode_marked(g4_context* ctx, const CodecList& list, const g4_band_desc* raster, const g4_icf_desc* icf, const uint8_t* image,
+                         uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens, const int32_t* tile_status,
+                         uint32_t fill_bits, int64_t raster_rows, int64_t raster_cols, PointArgs pa, int64_t kMax, bool blocks, void* out,
+                         int32_t* tiles_out, int32_t* status, int32_t* n_tiles_out) {
   ENTER(ctx);
-  for (const void* p : {(const void*)rows, (const void*)cols, (const void*)out, (const void*)tiles_out, (const void*)status})
+  for (const void* p : {(const void*)pa.rows, (const void*)pa.cols, (const void*)out, (const void*)tiles_out, (const void*)status})
     if (!device_pointer(ctx, p)) return G4_ERR_ARG;
   const int nTiles = raster->tiles_down * raster->tiles_across;
-  const int kMax = int(std::min<int64_t>(n_points, nTiles));
   const size_t flagCap = ctx->ptFlag.cap, infoCap = ctx->ptInfo.cap;
   CK(ctx->ptFlag.ensure(round_up(size_t(nTiles), 16)));
   CK(ctx->ptInfo.ensure(8));
@@ -1574,14 +1580,10 @@ int g4_decode_points(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   CK(ctx->winOff.ensure(size_t(kMax) * 8));
   CK(ctx->winLen.ensure(size_t(kMax) * 4));
   CK(ctx->winAbsent.ensure(size_t(kMax)));
-  PointArgs pa{};
-  pa.rows = rows;
-  pa.cols = cols;
-  pa.n = n_points;
   pa.rasterRows = raster_rows;
   pa.rasterCols = raster_cols;
-  pa.R = R;
-  pa.C = Cc;
+  pa.R = raster->tile_rows;
+  pa.C = raster->tile_cols;
   pa.tilesAcross = raster->tiles_across;
   pa.nTiles = nTiles;
   pa.flag = ctx->ptFlag.as<uint8_t>();
@@ -1612,12 +1614,64 @@ int g4_decode_points(g4_context* ctx, const g4_codec_list* codecs, const g4_band
   ws.nTa = 1;
   ws.nW = K;
   // the touched tiles one under the other: tile k at k * R * C; payloads that leave the image are G4_ERR_FORMAT
-  rc = decode_to_stage(ctx, &list.ids, *raster, K, 1, image, CallSettings{image_len, icf}, ws);
+  const int rc = decode_to_stage(ctx, &list.ids, *raster, K, 1, image, CallSettings{image_len, icf}, ws);
   if (rc != G4_OK) return rc;
-  CK(launch_point_store(pa, ws, ctx->smCount, ctx->stream));
+  CK(blocks ? launch_block_store(pa, ws, ctx->smCount, ctx->stream) : launch_point_store(pa, ws, ctx->smCount, ctx->stream));
   ctx->launches++;
   if (ctx->asyncDevice) return G4_OK;  // enqueued; status[] is read by the caller after g4_context_synchronize
   return read_status(ctx, status, K, true);
+}
+
+int g4_decode_points(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf, const uint8_t* image,
+                     uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens, const int32_t* tile_status, uint32_t fill_bits,
+                     int64_t raster_rows, int64_t raster_cols, int64_t n_points, const int64_t* rows, const int64_t* cols, void* out,
+                     int32_t* tiles_out, int32_t* status, int32_t* n_tiles_out) {
+  if (!n_tiles_out) return G4_ERR_ARG;
+  *n_tiles_out = 0;
+  CodecList list;
+  const int rc = check_marked_read(ctx, codecs, raster, icf, image, payload_offsets, lens, tile_status, raster_rows, raster_cols, n_points,
+                                   rows, cols, out, tiles_out, status, &list);
+  if (rc != G4_OK || n_points == 0) return rc;
+  PointArgs pa{};
+  pa.rows = rows;
+  pa.cols = cols;
+  pa.n = n_points;
+  pa.blockRows = pa.blockCols = 1;
+  pa.coverTd = pa.coverTa = 1;
+  return decode_marked(ctx, list, raster, icf, image, image_len, payload_offsets, lens, tile_status, fill_bits, raster_rows, raster_cols, pa,
+                       std::min<int64_t>(n_points, int64_t(raster->tiles_down) * raster->tiles_across), false, out, tiles_out, status,
+                       n_tiles_out);
+}
+
+int g4_decode_blocks(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf, const uint8_t* image,
+                     uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens, const int32_t* tile_status, uint32_t fill_bits,
+                     int64_t raster_rows, int64_t raster_cols, int64_t n_blocks, const int64_t* rows0, const int64_t* cols0,
+                     int64_t block_rows, int64_t block_cols, void* out, int32_t* tiles_out, int32_t* status, int32_t* n_tiles_out) {
+  if (!n_tiles_out) return G4_ERR_ARG;
+  *n_tiles_out = 0;
+  int64_t cells = 0;
+  if (block_rows < 1 || block_cols < 1 || __builtin_mul_overflow(block_rows, block_cols, &cells) ||
+      __builtin_mul_overflow(cells, n_blocks < 0 ? 0 : n_blocks, &cells))
+    return G4_ERR_ARG;
+  CodecList list;
+  const int rc = check_marked_read(ctx, codecs, raster, icf, image, payload_offsets, lens, tile_status, raster_rows, raster_cols, n_blocks,
+                                   rows0, cols0, out, tiles_out, status, &list);
+  if (rc != G4_OK || n_blocks == 0) return rc;
+  const int R = raster->tile_rows, Cc = raster->tile_cols;
+  PointArgs pa{};
+  pa.rows = rows0;
+  pa.cols = cols0;
+  pa.n = n_blocks;
+  pa.blockRows = block_rows;
+  pa.blockCols = block_cols;
+  // a block of h rows covers at most (h + R - 2) / R + 1 tile rows, and never more than the grid has (a block larger than
+  // the raster is refused by the mark pass, so h is capped at the raster's rows here only to keep the sum from overflowing)
+  pa.coverTd = int(std::min<int64_t>(raster->tiles_down, (std::min(block_rows, raster_rows) + R - 2) / R + 1));
+  pa.coverTa = int(std::min<int64_t>(raster->tiles_across, (std::min(block_cols, raster_cols) + Cc - 2) / Cc + 1));
+  // n_blocks * coverTd * coverTa <= n_blocks * block_rows * block_cols, which fits
+  return decode_marked(ctx, list, raster, icf, image, image_len, payload_offsets, lens, tile_status, fill_bits, raster_rows, raster_cols, pa,
+                       std::min<int64_t>(n_blocks * pa.coverTd * pa.coverTa, int64_t(raster->tiles_down) * raster->tiles_across), true,
+                       out, tiles_out, status, n_tiles_out);
 }
 
 // ---- window writes: a raster of any dimensions and pitch, padded to whole tiles on the device -----------------------------

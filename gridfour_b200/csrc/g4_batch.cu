@@ -433,17 +433,32 @@ cudaError_t launch_window_store(const WindowStore& a, int smCount, cudaStream_t 
   return cudaGetLastError();
 }
 
-// ---- point reads (g4_decode_points, GvrsElement.readValue / readValueInt) ------------------------------------------------
-// One thread per point.  Every thread that flags a tile stores the same 1, and every out-of-range point the same error.
-// (Loading the flag first and storing only a 0 measured slower: the loads queue on the same few L2 lines, DESIGN §6.2.6.)
+// ---- point and block reads (g4_decode_points / g4_decode_blocks, GvrsElement.readValue / readBlock) -----------------------
+// Blocks == false: one thread per point (a 1 x 1 block).  Blocks == true: one thread per (block, covered tile) pair of a
+// flat index over n x coverTd x coverTa, so that one block covering thousands of tiles does not serialise on one thread;
+// pairs past the block's last tile row or column do nothing.  Every thread that flags a tile stores the same 1, and every
+// thread of an out-of-range block the same error.  (Loading the flag first and storing only a 0 measured slower: the loads
+// queue on the same few L2 lines, DESIGN §6.2.6.)
+template <bool Blocks>
 __global__ void __launch_bounds__(256) point_mark_kernel(PointArgs a) {
-  for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < a.n; i += int64_t(gridDim.x) * blockDim.x) {
+  const int64_t n = Blocks ? a.n * a.coverTd * a.coverTa : a.n;
+  for (int64_t j = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; j < n; j += int64_t(gridDim.x) * blockDim.x) {
+    int64_t i = j, dr = 0, dc = 0;
+    if constexpr (Blocks) {
+      const int64_t box = int64_t(a.coverTd) * a.coverTa;
+      i = j / box;
+      dr = (j - i * box) / a.coverTa;
+      dc = j - i * box - dr * a.coverTa;
+    }
     const int64_t r = a.rows[i], c = a.cols[i];
-    if (r < 0 || c < 0 || r >= a.rasterRows || c >= a.rasterCols) {
+    if (r < 0 || c < 0 || r >= a.rasterRows || c >= a.rasterCols ||
+        (Blocks && (r > a.rasterRows - a.blockRows || c > a.rasterCols - a.blockCols))) {
       a.info[0] = 1;
       continue;
     }
-    a.flag[(r / a.R) * a.tilesAcross + c / a.C] = 1;
+    const int64_t tr = r / a.R + dr, tc = c / a.C + dc;
+    if (Blocks && (tr > (r + a.blockRows - 1) / a.R || tc > (c + a.blockCols - 1) / a.C)) continue;
+    a.flag[tr * a.tilesAcross + tc] = 1;
   }
 }
 
@@ -520,12 +535,71 @@ __global__ void __launch_bounds__(256) point_store_kernel(PointArgs p, WindowSto
   }
 }
 
+// One thread per quad of four consecutive cells of one block row, from a flat index over n x blockRows x ceil(blockCols / 4).
+// Where the quad lies in one tile and its staging address is 16-byte aligned, one 16-byte load; cell by cell otherwise,
+// stepping across tile edges (a quad spans up to three tiles when C < 4).  One 16-byte (8-byte for shorts) store where
+// the output address is aligned, cell by cell otherwise.
+template <int Mode>
+__global__ void __launch_bounds__(256) block_store_kernel(PointArgs p, WindowStore a) {
+  using T = typename WindowOut<Mode>::T;
+  using V = typename WindowOut<Mode>::V;
+  window_mark_absent(a);
+  const T fill = window_fill<Mode>(a);
+  const int64_t tileCells = int64_t(a.R) * a.C;
+  const int64_t qRow = (p.blockCols + 3) / 4, qBlock = p.blockRows * qRow, n = p.n * qBlock;
+  for (int64_t q = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; q < n; q += int64_t(gridDim.x) * blockDim.x) {
+    const int64_t i = q / qBlock, br = (q - i * qBlock) / qRow, bc = (q - i * qBlock - br * qRow) * 4;
+    const int k = p.blockCols - bc < 4 ? int(p.blockCols - bc) : 4;
+    const int64_t r = p.rows[i] + br, c = p.cols[i] + bc;
+    const int64_t tr = r / a.R, tc = c / a.C;
+    const int sc = int(c - tc * a.C);
+    const int32_t* slotRow = p.slot + tr * p.tilesAcross;
+    const int64_t rowOff = (r - tr * a.R) * a.C;
+    T y[4];
+    const int s0 = slotRow[tc];
+    const int32_t* s = a.stage + s0 * tileCells + rowOff + sc;
+    if (k == 4 && sc + 4 <= a.C && (reinterpret_cast<uintptr_t>(s) & 15) == 0) {
+      const int4 x = *reinterpret_cast<const int4*>(s);
+      const bool gone = a.absent[s0];
+      y[0] = gone ? fill : window_sample<Mode>(x.x, a);
+      y[1] = gone ? fill : window_sample<Mode>(x.y, a);
+      y[2] = gone ? fill : window_sample<Mode>(x.z, a);
+      y[3] = gone ? fill : window_sample<Mode>(x.w, a);
+    } else {
+      int64_t t = tc;
+      int x = sc;
+#pragma unroll
+      for (int m = 0; m < 4; m++) {
+        if (m < k) {
+          const int sm = slotRow[t];
+          y[m] = a.absent[sm] ? fill : window_sample<Mode>(a.stage[sm * tileCells + rowOff + x], a);
+        }
+        if (++x == a.C) {
+          x = 0;
+          t++;
+        }
+      }
+    }
+    T* d = static_cast<T*>(a.out) + i * p.blockRows * p.blockCols + br * p.blockCols + bc;
+    if (k == 4 && (reinterpret_cast<uintptr_t>(d) & (sizeof(V) - 1)) == 0) {
+      V z;
+      z.x = y[0]; z.y = y[1]; z.z = y[2]; z.w = y[3];
+      *reinterpret_cast<V*>(d) = z;
+    } else {
+#pragma unroll
+      for (int m = 0; m < 4; m++)
+        if (m < k) d[m] = y[m];
+    }
+  }
+}
+
 static unsigned point_blocks(int64_t n, int smCount) {
   const int64_t b = (n + 255) / 256, cap = int64_t(smCount) * 32;
   return unsigned(b < cap ? b : cap);
 }
 cudaError_t launch_point_mark(const PointArgs& a, int smCount, cudaStream_t s) {
-  point_mark_kernel<<<point_blocks(a.n, smCount), 256, 0, s>>>(a);
+  if (a.blockRows == 1 && a.blockCols == 1) point_mark_kernel<false><<<point_blocks(a.n, smCount), 256, 0, s>>>(a);
+  else point_mark_kernel<true><<<point_blocks(a.n * a.coverTd * a.coverTa, smCount), 256, 0, s>>>(a);
   return cudaGetLastError();
 }
 cudaError_t launch_point_compact(const PointArgs& a, cudaStream_t s) {
@@ -538,6 +612,15 @@ cudaError_t launch_point_store(const PointArgs& p, const WindowStore& w, int smC
     case kWindowNarrow16: point_store_kernel<kWindowNarrow16><<<nb, 256, 0, s>>>(p, w); break;
     case kWindowIcfFloat: point_store_kernel<kWindowIcfFloat><<<nb, 256, 0, s>>>(p, w); break;
     default: point_store_kernel<kWindowCopy32><<<nb, 256, 0, s>>>(p, w); break;
+  }
+  return cudaGetLastError();
+}
+cudaError_t launch_block_store(const PointArgs& p, const WindowStore& w, int smCount, cudaStream_t s) {
+  const unsigned nb = point_blocks(p.n * p.blockRows * ((p.blockCols + 3) / 4), smCount);
+  switch (w.mode) {
+    case kWindowNarrow16: block_store_kernel<kWindowNarrow16><<<nb, 256, 0, s>>>(p, w); break;
+    case kWindowIcfFloat: block_store_kernel<kWindowIcfFloat><<<nb, 256, 0, s>>>(p, w); break;
+    default: block_store_kernel<kWindowCopy32><<<nb, 256, 0, s>>>(p, w); break;
   }
   return cudaGetLastError();
 }

@@ -203,16 +203,17 @@ struct WindowStore {
 // decoded straight into out; only the absent ones are filled.
 cudaError_t launch_window_store(const WindowStore& a, int smCount, cudaStream_t s);
 
-// Point reads (g4_decode_points): cell (rows[i], cols[i]) of the raster for each of n points.  The mark pass sets flag[t]
-// for every tile a point falls in (info[0] = 1 for a point outside the raster); the compaction pass, one CTA, scans the
-// flags in tile-index order: the k-th touched tile t gets slot[t] = k, tilesOut[k] = t, its payload location and absent flag
-// as launch_window_gather gives them, and info[1] = K.  The compaction leaves every flag zero again, so the flag array
-// (nTiles rounded up to 16 bytes, zero padded) is zero between calls; info[0] is cleared by the caller that reads it set.
+// Point and block reads (g4_decode_points, g4_decode_blocks): the blockRows x blockCols block at (rows[i], cols[i]) of the
+// raster for each of n blocks; a point is a 1 x 1 block.  The mark pass sets flag[t] for every tile a block covers
+// (info[0] = 1 for a block not wholly inside the raster); the compaction pass, one CTA, scans the flags in tile-index order:
+// the k-th touched tile t gets slot[t] = k, tilesOut[k] = t, its payload location and absent flag as launch_window_gather
+// gives them, and info[1] = K.  The compaction leaves every flag zero again, so the flag array (nTiles rounded up to 16
+// bytes, zero padded) is zero between calls; info[0] is cleared by the caller that reads it set.
 struct PointArgs {
   const int64_t* rows;
   const int64_t* cols;
   int64_t n;
-  int64_t rasterRows, rasterCols;  // points must lie in [0, rasterRows) x [0, rasterCols)
+  int64_t rasterRows, rasterCols;  // blocks must lie in [0, rasterRows) x [0, rasterCols)
   int R, C, tilesAcross, nTiles;
   uint8_t* flag;                   // [nTiles rounded up to 16]
   int32_t* info;                   // [0] a point outside the raster, [1] K
@@ -224,6 +225,8 @@ struct PointArgs {
   uint64_t* offK;                  // [K] payload locations in slot order (zero-length for tiles not G4_OK)
   uint32_t* lenK;
   uint8_t* absentK;                // [K] 1 for G4_DECLINED
+  int64_t blockRows, blockCols;    // 1 x 1 for points
+  int coverTd, coverTa;            // most tile rows / columns one block can cover (1 x 1 for points)
 };
 cudaError_t launch_point_mark(const PointArgs& a, int smCount, cudaStream_t s);
 cudaError_t launch_point_compact(const PointArgs& a, cudaStream_t s);
@@ -231,6 +234,8 @@ cudaError_t launch_point_compact(const PointArgs& a, cudaStream_t s);
 // order (w.nW = K).  out[i] = the converted sample of point i, or the fill sample for an absent tile; absent tiles' status
 // becomes G4_DECLINED.
 cudaError_t launch_point_store(const PointArgs& p, const WindowStore& w, int smCount, cudaStream_t s);
+// The same staging and slots; out + i * blockRows * blockCols = block i, rows contiguous, converted and filled as above.
+cudaError_t launch_block_store(const PointArgs& p, const WindowStore& w, int smCount, cudaStream_t s);
 
 // ---- codec kernels -----------------------------------------------------------------------------
 // Host-side launchers (defined next to their kernels).  nCtas persistent CTAs of kThreads threads.

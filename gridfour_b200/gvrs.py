@@ -408,8 +408,9 @@ class GvrsDeviceImage:
         self.image, self.payload_off, self.lens, self.status = image, payload_off, lens, status  # [n] / [E, n] / [E, n] / [n]
         self.context = context
         self.device = image.device
-        self.lastStatus = None  # per covering tile of the latest read, window-tile order (device tensor); read_values: per lastTiles
-        self.lastTiles = None   # read_values: the tiles the latest point read touched, ascending tile index (device tensor)
+        self.lastStatus = None  # per covering tile of the latest read, window-tile order (device tensor); read_values /
+                                # read_blocks: per lastTiles
+        self.lastTiles = None   # read_values / read_blocks: the tiles the latest read touched, ascending tile index (device tensor)
 
     def _element(self, element):
         if not 0 <= element < len(self.spec.elements):
@@ -478,6 +479,54 @@ class GvrsDeviceImage:
         if st == _lib.G4_ERR_ARG:
             raise ValueError("a point outside the raster")
         check(st, "g4_decode_points")
+        return out
+
+    def read_blocks(self, master, rows, cols, n_rows, n_cols, element=0, as_float=False, out=None):
+        """GvrsElement.readBlock for many blocks of one size at once: block i is the n_rows x n_cols window at (rows[i],
+        cols[i]), and the result is an [N, n_rows, n_cols] tensor with the dtype read_block gives the element.  rows and
+        cols are 1-D integer CUDA tensors (int32 or int64) of length N on the image's device.  Blocks may repeat, overlap and
+        come in any order; each tile they cover is decoded once (g4_decode_blocks).  A block not wholly inside the raster
+        raises ValueError.  `out`, if given, is a contiguous tensor of that dtype and shape.  Afterwards lastTiles holds the
+        covered tile indices (ascending) and lastStatus their statuses."""
+        import torch
+
+        self._element(element)
+        for name, x in (("rows", rows), ("cols", cols)):
+            if not (isinstance(x, torch.Tensor) and x.device == self.device and x.dtype in (torch.int32, torch.int64) and x.dim() == 1):
+                raise ValueError("%s: a 1-D int32 or int64 tensor on %s" % (name, self.device))
+        if rows.shape != cols.shape:
+            raise ValueError("rows and cols differ in length")
+        if not (isinstance(n_rows, (int, np.integer)) and isinstance(n_cols, (int, np.integer)) and n_rows >= 1 and n_cols >= 1):
+            raise ValueError("n_rows and n_cols: positive integers")
+        band, dtype, fill, icf = self._layout(element, as_float)
+        shape = (rows.numel(), int(n_rows), int(n_cols))
+        if out is None:
+            out = torch.empty(shape, dtype=dtype, device=self.device)
+        elif not (isinstance(out, torch.Tensor) and out.device == self.device and out.dtype == dtype and tuple(out.shape) == shape
+                  and out.is_contiguous()):
+            raise ValueError("out: a contiguous %s tensor of shape %s on %s" % (dtype, shape, self.device))
+        r = rows.to(torch.int64).contiguous()
+        c = cols.to(torch.int64).contiguous()
+        spec = self.spec
+        cover = min(spec.tiles_down, (n_rows + spec.tile_rows - 2) // spec.tile_rows + 1) * \
+            min(spec.tiles_across, (n_cols + spec.tile_cols - 2) // spec.tile_cols + 1)
+        k_max = min(r.numel() * cover, spec.tiles_down * spec.tiles_across)
+        tiles = torch.empty(k_max, dtype=torch.int32, device=self.device)
+        status = torch.empty(k_max, dtype=torch.int32, device=self.device)
+        k = C.c_int32(0)
+        d = icf.desc() if icf is not None else None
+        ctx = self.context
+        ctx.after_torch_stream(self.device)  # the index copies above and `out` are on torch's stream
+        st = _lib.lib().g4_decode_blocks(ctx._h, C.byref(master._native_list()), C.byref(band), None if d is None else C.byref(d),
+                                         self.image.data_ptr(), int(self.image.numel()), self.payload_off[element].data_ptr(),
+                                         self.lens[element].data_ptr(), self.status.data_ptr(), fill, spec.n_rows, spec.n_cols,
+                                         r.numel(), r.data_ptr(), c.data_ptr(), int(n_rows), int(n_cols), out.data_ptr(),
+                                         tiles.data_ptr(), status.data_ptr(), C.byref(k))
+        ctx.before_torch_stream(self.device)
+        self.lastTiles, self.lastStatus = tiles[:k.value], status[:k.value]
+        if st == _lib.G4_ERR_ARG:
+            raise ValueError("a block outside the raster")
+        check(st, "g4_decode_blocks")
         return out
 
     def _layout(self, element, as_float):

@@ -273,6 +273,37 @@ int g4_decode_points(g4_context* ctx, const g4_codec_list* codecs, const g4_band
                      int64_t n_points, const int64_t* rows, const int64_t* cols, void* out,
                      int32_t* tiles_out, int32_t* status, int32_t* n_tiles_out);
 
+/* ---- block reads: GvrsElement.readBlock on the device, many blocks of one size at once (gvrs/GvrsElement.java:298-404) ----
+ * Block i is the block_rows x block_cols window at (rows0[i], cols0[i]) of one element of a raster whose file image is
+ * resident on the device, for i < n_blocks.  It goes to out + i * block_rows * block_cols, rows contiguous: `out` is a
+ * contiguous [n_blocks, block_rows, block_cols] array.  Every pointer except n_tiles_out is a device pointer; rows0, cols0,
+ * out, tiles_out or status in host memory or on another device are refused.
+ * Each tile that blocks cover is decoded once, however many blocks overlap it; blocks may repeat, overlap and come in any
+ * order.
+ *   raster, icf, image, image_len, payload_offsets, lens, tile_status, fill_bits
+ *                as in g4_decode_window; a cell is converted exactly as there (int32 / float32 bits copied, G4_ELEM_I16
+ *                narrowed with null -> -32768, G4_ELEM_ICF with `icf` mapped to float32, cells of absent tiles = fill_bits).
+ *   raster_rows, raster_cols
+ *                the raster's extent, at most the tile grid's: every block must lie wholly in [0, raster_rows) x
+ *                [0, raster_cols).
+ *   tiles_out    the K distinct covered tiles, ascending tile index; *n_tiles_out = K (host pointer).
+ *   status       status[k] of tiles_out[k], with the meanings of g4_decode_points' status.
+ *                tiles_down * tiles_across entries of tiles_out and status always suffice.
+ * Returns the first bad status, absent tiles not counted, as g4_decode_points does; with g4_context_set_async the decode is
+ * only enqueued and G4_OK returned, but the call always waits once first for the covered-tile count and a flag for blocks
+ * outside the raster.
+ * G4_ERR_ARG, with nothing decoded and `out` not written, for n_blocks < 0, block_rows < 1 or block_cols < 1,
+ * n_blocks * block_rows * block_cols overflowing int64, a bad `raster` or `icf` (as g4_decode_window), a raster extent
+ * larger than the tile grid, or any block not wholly inside the raster.  n_blocks == 0 returns G4_OK with K = 0 and launches
+ * nothing; rows0, cols0, out, tiles_out and status may then be null.
+ * The K covered tiles are decoded into the int32 staging buffer of g4_decode_points: 4 * K * tile_rows * tile_cols bytes.
+ * Launches: those of g4_decode_tiles_bounded on the K tiles, plus three (mark, compact, store). */
+int g4_decode_blocks(g4_context* ctx, const g4_codec_list* codecs, const g4_band_desc* raster, const g4_icf_desc* icf,
+                     const uint8_t* image, uint64_t image_len, const uint64_t* payload_offsets, const uint32_t* lens,
+                     const int32_t* tile_status, uint32_t fill_bits, int64_t raster_rows, int64_t raster_cols,
+                     int64_t n_blocks, const int64_t* rows0, const int64_t* cols0, int64_t block_rows, int64_t block_cols,
+                     void* out, int32_t* tiles_out, int32_t* status, int32_t* n_tiles_out);
+
 /* ---- window writes: a raster of any dimensions on the device, padded to whole tiles there --------------------------------
  * g4_encode_tiles (or g4_encode_tiles_icf) of the n_rows x n_cols raster at src (row pitch src_pitch samples) padded to the
  * tile grid with the margin sample fill_bits: the same arena bytes, offsets, lengths, codec and predictor bytes, statuses
